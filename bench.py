@@ -10,6 +10,7 @@ BASELINE.json names for 1/2/4/8 GPUs; frames are sharded over the ranks with no 
   roofline the dominant kernel's algorithmic bytes / its CUDA-event duration against MEASURED_PEAKS.json
   cpu_baseline  the CPU oracle (port of the PCL 1.8.1 path; the reference's own PCL build is not installable here)
 --impl reference times that CPU path alone, on all host cores, for the driver's own ratio.
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy, so that two builds can be compared.
 """
 from __future__ import annotations
 
@@ -24,6 +25,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is written next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -47,8 +49,11 @@ def parse_args():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-latency", action="store_true", help="skip the single-frame p50/p99 latency measurement")
     ap.add_argument("--points", type=int, default=0, help="cfg4 / cfg5: points of the cloud (0 = 100 M / 16 Mi)")
-    ap.add_argument("--sustained-seconds", type=float, default=2.0,
-                    help="length of the extra back-to-back leg that shows the number holds at steady-state clocks (0 = skip)")
+    ap.add_argument("--sustained-seconds", type=float, default=0.0,
+                    help="length of an extra back-to-back leg that shows the number holds at steady-state clocks (0 = skip, "
+                         "the default: then --steps is the number of timed steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed (on rank 0) to DIR/<name>.npy (frame workloads cfg1-cfg3)")
     return ap.parse_args()
 
 
@@ -214,6 +219,28 @@ def make_host_frames(spec, name: str, rank: int, pinned: bool):
             row.append((view, (addr + off) if pinned else view.ctypes.data))
         bufs.append(row)
     return arena, bufs
+
+
+DUMP_ROWS = 1 << 18
+
+
+def dump_outputs(cm, out_dir: str):
+    """--dump-outputs: the results the last cm_run_batch left for its caller, as .npy files in float32 / float64.
+    frame_info: one row per frame (survivor_begin, survivor_end, voxel_begin, voxel_end, min_b[3], max_b[3], div_b[3],
+    pcl_overflow). survivor_xyzi / survivor_src and voxel_xyzi / voxel_count / voxel_idx: the same DUMP_ROWS rows of each
+    kind, drawn with a fixed seed from its count (all rows when there are fewer), which keeps the dump near 15 MB."""
+    r = cm.fetch_batch_outputs(want_sorted=False)
+    arrays = {"frame_info": np.array([[f.survivor_begin, f.survivor_end, f.voxel_begin, f.voxel_end, *f.min_b, *f.max_b,
+                                       *f.div_b, f.pcl_overflow] for f in r["frames"]], np.float64)}
+    for kind, fields in (("survivor", ("xyzi", "src")), ("voxel", ("xyzi", "count", "idx"))):
+        n = len(r[kind + "_xyzi"])
+        rows = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_ROWS), replace=False))
+        for f in fields:
+            a = r[kind + "_" + f][rows]
+            arrays[kind + "_" + f] = a if a.dtype == np.float32 else a.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def cpu_port(spec, host_frames, seconds: float, threads_frames: int, sensor_threads: int):
@@ -556,6 +583,8 @@ def emit(line: dict):
 def main():
     args = parse_args()
     guard_stdout()
+    if args.dump_outputs and (args.impl != "b200" or args.workload in CLOUD_WORKLOADS):
+        raise SystemExit("bench.py: --dump-outputs writes the outputs of the GPU path of the frame workloads cfg1-cfg3")
     if args.impl == "reference":
         return run_cloud_reference(args) if args.workload in CLOUD_WORKLOADS else run_reference(args)
     if args.workload in CLOUD_WORKLOADS:
@@ -644,6 +673,8 @@ def main():
     value = pts_step * world * args.steps / (ms_total / 1e3) / 1e6
     st = cm.stats()
     M, V, P, kb = int(st.survivors), int(st.voxels_out), int(st.sort_passes), int(st.key_bytes)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(cm, args.dump_outputs)   # before any later leg overwrites the last timed step's outputs
 
     # ---- sustained leg: the same step back to back for >= --sustained-seconds (the K-step region above lasts milliseconds,
     # too short for the GPU to reach its steady-state power / clocks) ---------------------------------------------------------
