@@ -451,6 +451,7 @@ void fill_voxel_params(cm_handle_t h, Workspace& w, VoxelParams& vp, const float
   for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = h->inv_leaf[k];
   vp.min_points = h->min_points;
   vp.downsample_all = h->downsample_all;
+  vp.pcl_refuses = h->overflow_mode == 1 ? 1u : 0u;
   vp.key_bytes = 8;
   vp.out_step = (uint32_t)w.out_step;
   vp.ctrl = reinterpret_cast<Ctrl*>(w.meta + w.ml.off_ctrl);
@@ -957,6 +958,7 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
     key.append(reinterpret_cast<const char*>(h->inv_leaf), sizeof(h->inv_leaf));
     key.append(reinterpret_cast<const char*>(&h->min_points), sizeof(h->min_points));
     key.append(reinterpret_cast<const char*>(&h->downsample_all), sizeof(h->downsample_all));
+    key.append(reinterpret_cast<const char*>(&h->overflow_mode), sizeof(h->overflow_mode));  // read by k_grid_setup
   }
   bool launched = false;
   if (graphable && sl.graph && sl.graph_key == key) {
@@ -1850,6 +1852,7 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   VoxelParams vp;
   fill_voxel_params(h, w, vp, pts, (uint32_t)n_clouds, (uint32_t)n_points);
   for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = 1.0f / cell;
+  vp.pcl_refuses = 0;  // a cell grid of the neighbour search beyond the key range is always an error
   uint32_t* fss = const_cast<uint32_t*>(vp.frame_surv_start);
   for (int c = 0; c < n_clouds; ++c) {  // bounding box of every cloud (its own cell grid)
     const uint32_t n_here = (uint32_t)(begin[c + 1] - begin[c]);

@@ -124,6 +124,8 @@ struct GridDev {
   int32_t pcl_overflow;
   uint32_t bits;
   uint32_t empty;
+  uint32_t zero_keys;             // 1: the grid is outside the key range (or PCL refuses the frame in overflow mode 1): every
+                                  // point of the frame gets voxel index 0, so no key leaves the frame's (1-cell) grid
   unsigned long long mul1, mul2;  // div0, div0*div1
 };
 

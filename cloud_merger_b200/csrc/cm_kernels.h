@@ -68,6 +68,8 @@ struct VoxelParams {
   float inv_leaf[3];
   uint32_t min_points;
   uint32_t downsample_all;
+  uint32_t pcl_refuses;              // overflow mode 1: a frame PCL refuses is returned as its cropped cloud, so a grid of that
+                                     // frame beyond the key range is not an error
   uint32_t key_bytes;                // 4 or 8
   uint32_t out_step;                 // 16 or 32
   Ctrl* ctrl;

@@ -242,6 +242,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
     g.bits = 0;
     g.mul1 = 0;
     g.mul2 = 0;
+    g.zero_keys = 0;
     g.empty = (a.max_enc[0] == 0u && a.nmin_enc[0] == 0u) ? 1u : 0u;
     if (g.empty) {
       for (int k = 0; k < 3; ++k) { g.min_b[k] = 0; g.max_b[k] = 0; g.div_b[k] = 0; }
@@ -272,8 +273,12 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
       }
       g.pcl_overflow = ovf ? 1 : 0;
       if (range_err) {
-        atomicExch(&p.ctrl->error, (uint32_t)CM_DEV_E_KEY_RANGE);
+        // No key of such a frame can be formed, so every point gets index 0 of a 1-cell grid: keys stay below the frame's
+        // limit whatever idx_bits comes out (0 when no frame has a usable grid), and no kernel derives a frame from garbage.
+        // Overflow mode 1 returns a frame PCL refuses as its cropped cloud: its voxels are not used, so no error then.
+        if (!(p.pcl_refuses && ovf)) atomicExch(&p.ctrl->error, (uint32_t)CM_DEV_E_KEY_RANGE);
         div[0] = div[1] = div[2] = 1;
+        g.zero_keys = 1;
       }
       g.mul1 = div[0];
       g.mul2 = div[0] * div[1];
@@ -446,6 +451,7 @@ __device__ __forceinline__ void key_hist_tiles(const VoxelParams& p, uint32_t (*
     const GridDev* __restrict__ g = p.grid + r.frame;
     const KeyT fbits = SEG ? (KeyT)0 : (KeyT)((unsigned long long)r.frame << idx_bits);
     const KeyT mul1 = (KeyT)g->mul1, mul2 = (KeyT)g->mul2;  // 32-bit arithmetic when the key is 32-bit
+    const KeyT idx_keep = g->zero_keys ? (KeyT)0 : ~(KeyT)0;  // a frame without a usable grid: index 0 (see k_grid_setup)
     const int mb0 = g->min_b[0], mb1 = g->min_b[1], mb2 = g->min_b[2];
     const float4* __restrict__ src = p.pts + r.slot0;
     constexpr int U = KH_UNROLL;  // points per thread in flight
@@ -471,7 +477,7 @@ __device__ __forceinline__ void key_hist_tiles(const VoxelParams& p, uint32_t (*
         const KeyT i0 = (KeyT)(__float2int_rd(__fmul_rn(v.x, inv0)) - mb0);
         const KeyT i1 = (KeyT)(__float2int_rd(__fmul_rn(v.y, inv1)) - mb1);
         const KeyT i2 = (KeyT)(__float2int_rd(__fmul_rn(v.z, inv2)) - mb2);
-        KeyT key = fbits | (KeyT)(i0 + i1 * mul1 + i2 * mul2);
+        KeyT key = fbits | ((KeyT)(i0 + i1 * mul1 + i2 * mul2) & idx_keep);
         if (CHECK && !(finite_f32(v.x) && finite_f32(v.y) && finite_f32(v.z))) key = (KeyT)sentinel;
         if (sizeof(KeyT) == 4) {  // 32-bit keys travel as 8-byte (key, value) records
           recs[r.dense0 + j] = make_uint2((uint32_t)key, r.slot0 + j);

@@ -257,7 +257,10 @@ CM_API int cm_set_voxel(cm_handle_t h, const float* leaf3, int min_points, int d
  * every rank builds the same grid (same min_b / div_b / voxel indices). NULL, NULL switches it off. */
 CM_API int cm_set_voxel_bounds(cm_handle_t h, const float* min3, const float* max3);
 /* PCL 1.8.1 returns the input cloud unchanged when dx*dy*dz > INT32_MAX. mode 0 (default): keep going with the 64-bit
- * key and report it in cm_frame_info_t.pcl_overflow; mode 1: behave like PCL (the frame's output is its cropped cloud). */
+ * key and report it in cm_frame_info_t.pcl_overflow; mode 1: behave like PCL (the frame's output is its cropped cloud).
+ * A frame whose grid is beyond the key range (more than 2^21 cells on an axis, or a cell origin beyond +-2^30) fails with
+ * CM_E_KEY_RANGE, except in mode 1 when PCL refuses it too: cm_wait_frame / cm_merge_frame then return its cropped cloud
+ * (in a device batch its voxels are meaningless and frame_info.pcl_overflow says so). */
 CM_API int cm_set_overflow_mode(cm_handle_t h, int mode);
 
 /* ---- host path: one frame at a time, callable from the ROS callbacks ----

@@ -9,7 +9,8 @@ import pytest
 
 from cloud_merger_b200 import CloudMerger, CloudMergerError, _lib, make_layout, synth
 
-from helpers import assert_bit_equal, assert_centroids_close, cloud_dict, known_answer
+from helpers import (assert_bit_equal, assert_centroids_close, check_survivors, check_voxels, cloud_dict, known_answer,
+                     upload_segments)
 
 pytestmark = pytest.mark.gpu
 
@@ -27,60 +28,6 @@ LAYOUTS = {
 
 def _layout(t, dense=1):
     return make_layout(t[0], t[1], t[2], t[3], t[4], dense)
-
-
-def _upload_segments(cm, frames, layout_of):
-    """frames: list (per frame) of list (per sensor) of (xyzi, is_dense). Returns (segments, oracle cloud dicts per frame)."""
-    items, per_frame = [], []
-    for f, sensors in enumerate(frames):
-        cds = []
-        for s, (xyzi, dense) in enumerate(sensors):
-            lt = layout_of(f, s)
-            data = synth.pack_cloud(xyzi, *lt)
-            buf = cm.upload(data if len(data) else np.zeros(16, np.uint8))
-            items.append((buf.ptr, len(xyzi), _layout(lt, dense), s, f))
-            cds.append(dict(data=data, n_points=len(xyzi), point_step=lt[0], off_x=lt[1], off_y=lt[2], off_z=lt[3],
-                            off_i=lt[4], is_dense=int(dense), m=cm.get_extrinsic(s)))
-        per_frame.append(cds)
-    return cm.make_segments(items), per_frame
-
-
-def _check_survivors(out, frames_info, oracle_frames):
-    for f, (fi, o) in enumerate(zip(frames_info, oracle_frames)):
-        sx = out["survivor_xyzi"][fi.survivor_begin:fi.survivor_end]
-        ss = out["survivor_src"][fi.survivor_begin:fi.survivor_end]
-        assert len(ss) == o["n_survivors"], "frame %d: %d survivors vs oracle %d" % (f, len(ss), o["n_survivors"])
-        assert (ss == o["survivor_src"]).all(), "frame %d: surviving-point indices differ" % f
-        assert_bit_equal(sx, o["survivor_xyzi"], "frame %d survivor coordinates" % f)
-
-
-def _check_voxels(out, frames_info, oracle_frames, check_membership=True):
-    worst = 0.0
-    idx_bits = out["key_idx_bits"]
-    mask = (1 << idx_bits) - 1 if idx_bits < 64 else (1 << 64) - 1
-    for f, (fi, o) in enumerate(zip(frames_info, oracle_frames)):
-        v0, v1 = fi.voxel_begin, fi.voxel_end
-        assert v1 - v0 == o["n_voxels"], "frame %d: %d voxels vs oracle %d" % (f, v1 - v0, o["n_voxels"])
-        if o["n_survivors"]:
-            assert list(fi.min_b) == o["min_b"].tolist() and list(fi.div_b) == o["div_b"].tolist(), "frame %d grid" % f
-            assert fi.pcl_overflow == o["pcl_overflow"]
-        assert (out["voxel_idx"][v0:v1].astype(np.int64) == o["idx"]).all(), "frame %d: voxel ids / order differ" % f
-        assert (out["voxel_count"][v0:v1] == o["count"]).all(), "frame %d: voxel counts differ" % f
-        assert_bit_equal(out["voxel_xyzi"][v0:v1], o["centroid"], "frame %d centroid vs float oracle (asc. index)" % f)
-        worst = max(worst, assert_centroids_close(out["voxel_xyzi"][v0:v1], o["centroid_f64"], "frame %d centroid" % f))
-        if check_membership:
-            s0, s1 = fi.survivor_begin, fi.survivor_end
-            keys = out["sorted_key"][s0:s1]
-            pts = out["sorted_point"][s0:s1].astype(np.int64)
-            assert (np.diff(keys.astype(np.float64)) >= 0).all() and (keys[1:] >= keys[:-1]).all(), "keys not sorted"
-            assert ((keys >> np.uint64(idx_bits)) == f).all() if idx_bits < 64 else True
-            member = np.full(s1 - s0, -2, np.int64)
-            member[pts - s0] = (keys & np.uint64(mask)).astype(np.int64)
-            assert (member == o["point_idx"]).all(), "frame %d: voxel membership differs" % f
-            # stable sort: inside a voxel the points are in ascending index order
-            same = keys[1:] == keys[:-1]
-            assert (pts[1:][same] > pts[:-1][same]).all(), "sort is not stable"
-    return worst
 
 
 def _oracle_frames(oracle, per_frame, passes, leaf, min_points, downsample_all=True):
@@ -131,11 +78,11 @@ def test_transform_crop_layouts(gpu_ok, oracle, name, dense):
         for s in range(len(sizes)):
             cm.set_extrinsic(s, synth.extrinsic(s, len(sizes)))
         cm.set_crop(synth.ROI_BOX)
-        segs, per_frame = _upload_segments(cm, [sensors], lambda f, s: lt)
+        segs, per_frame = upload_segments(cm, [sensors], lambda f, s: lt)
         cm.dev_transform_crop(segs)
         out = cm.fetch_batch_outputs()
         o = _oracle_frames(oracle, per_frame, synth.ROI_BOX, [0.1] * 3, 1)
-        _check_survivors(out, out["frames"], o)
+        check_survivors(out, out["frames"], o)
         assert out["stats"].survivors == o[0]["n_survivors"] > 100
         assert out["stats"].points_in == sum(sizes)
 
@@ -150,11 +97,11 @@ def test_transform_crop_mixed_layouts_and_pass_kinds(gpu_ok, oracle):
         for s in range(len(names)):
             cm.set_extrinsic(s, synth.extrinsic(s, len(names)))
         cm.set_crop(passes)
-        segs, per_frame = _upload_segments(cm, [sensors], lambda f, s: LAYOUTS[names[s]])
+        segs, per_frame = upload_segments(cm, [sensors], lambda f, s: LAYOUTS[names[s]])
         cm.dev_transform_crop(segs)
         out = cm.fetch_batch_outputs()
         o = _oracle_frames(oracle, per_frame, passes, [0.1] * 3, 1)
-        _check_survivors(out, out["frames"], o)
+        check_survivors(out, out["frames"], o)
         assert 0 < out["stats"].survivors < out["stats"].points_in
 
 
@@ -167,14 +114,14 @@ def test_no_crop_keeps_everything_and_voxel_skips_invalid(gpu_ok, oracle):
             cm.set_extrinsic(s, synth.extrinsic(s, 3))
         cm.set_crop([])
         cm.set_voxel(0.5, 1, True)
-        segs, per_frame = _upload_segments(cm, [sensors], lambda f, s: LAYOUTS["packed16"])
+        segs, per_frame = upload_segments(cm, [sensors], lambda f, s: LAYOUTS["packed16"])
         cm.run_batch(segs)
         out = cm.fetch_batch_outputs()
         o = _oracle_frames(oracle, per_frame, [], [0.5] * 3, 1)
         assert out["stats"].survivors == 3 * 5600
-        _check_survivors(out, out["frames"], o)
+        check_survivors(out, out["frames"], o)
         assert np.isnan(out["survivor_xyzi"]).any()
-        _check_voxels(out, out["frames"], o, check_membership=False)
+        check_voxels(out, out["frames"], o, check_membership=False)
         # membership: invalid points carry the sentinel frame and are sorted to the end
         n_bad = int((~np.isfinite(out["survivor_xyzi"][:, :3]).all(axis=1)).sum())
         tail = out["sorted_point"][len(out["sorted_point"]) - n_bad:]
@@ -196,7 +143,7 @@ def test_voxelgrid_only_leaf_sweep(gpu_ok, oracle, leaf, min_points):
     o.update(n_voxels=o["n"], n_survivors=len(x))
     assert out["stats"].pcl_overflow == int(o["pcl_overflow"])
     assert out["key_bytes"] == (4 if out["stats"].key_bits <= 32 else 8)
-    worst = _check_voxels(out, out["frames"], [o])
+    worst = check_voxels(out, out["frames"], [o])
     assert worst <= 1e-5
 
 
@@ -241,13 +188,13 @@ def test_batch_of_frames_matches_per_frame_oracle(gpu_ok, oracle):
             cm.set_extrinsic(s, synth.extrinsic(s, S))
         cm.set_crop(synth.ROI_BOX)
         cm.set_voxel(0.1, 2, True)
-        segs, per_frame = _upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16" if (f + s) % 2 else "pcl32"])
+        segs, per_frame = upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16" if (f + s) % 2 else "pcl32"])
         cm.run_batch(segs)
         out = cm.fetch_batch_outputs()
         o = _oracle_frames(oracle, per_frame, synth.ROI_BOX, [0.1] * 3, 2)
         assert out["stats"].frames == F and out["key_bytes"] == 4
-        _check_survivors(out, out["frames"], o)
-        _check_voxels(out, out["frames"], o)
+        check_survivors(out, out["frames"], o)
+        check_voxels(out, out["frames"], o)
         assert out["frames"][3].survivor_begin == out["frames"][3].survivor_end
         assert cm.launch_count() >= 5
 
@@ -451,7 +398,7 @@ def test_full_size_batch_properties(gpu_ok, oracle):
         cm.set_crop(c["passes"])
         cm.set_voxel(c["leaf"], c["min_points"], True)
         frames = [[(synth.lidar_cloud(2000, s, f, c["rings"], c["azimuth"]), 1) for s in range(S)] for f in range(F)]
-        segs, per_frame = _upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
+        segs, per_frame = upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
         cm.run_batch(segs)
         out = cm.fetch_batch_outputs()
         st = out["stats"]
@@ -534,7 +481,7 @@ def test_sort_64bit_big_tile_at_size(gpu_ok, oracle, leaf):
     o.update(n_voxels=o["n"], n_survivors=n)
     assert out["key_bytes"] == 8 and out["stats"].key_bits > 32 and out["stats"].sort_passes >= 5
     assert out["stats"].pcl_overflow == 1 and o["pcl_overflow"]
-    assert _check_voxels(out, out["frames"], [o]) <= 1e-5
+    assert check_voxels(out, out["frames"], [o]) <= 1e-5
 
 
 def test_cfg1_batch_of_64_frames_at_size(gpu_ok, oracle):
@@ -549,15 +496,15 @@ def test_cfg1_batch_of_64_frames_at_size(gpu_ok, oracle):
         cm.set_crop(c["passes"])
         cm.set_voxel(c["leaf"], c["min_points"], True)
         frames = [[(synth.lidar_cloud(1000, s, f, c["rings"], c["azimuth"]), 1) for s in range(S)] for f in range(F)]
-        segs, per_frame = _upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
+        segs, per_frame = upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
         cm.run_batch(segs)
         out = cm.fetch_batch_outputs()
     assert out["stats"].frames == F and out["stats"].device_error == 0 and out["stats"].survivors > 1363968
     # frame-segmented: the 6 frame bits are not sorted -- 32-bit records and 4 passes where (frame, index) took 64 bits and 5
     assert out["stats"].key_bytes == 4 and out["stats"].sort_passes == 4 and out["stats"].key_bits == out["key_idx_bits"]
     o = _oracle_frames(oracle, per_frame, c["passes"], [c["leaf"]] * 3, c["min_points"])
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
 
 
 def _ragged_batch(cm, oracle, sizes, passes, leaf, min_points, extent, same_cloud=False, seed=7000):
@@ -566,7 +513,7 @@ def _ragged_batch(cm, oracle, sizes, passes, leaf, min_points, extent, same_clou
     cm.set_crop(passes)
     cm.set_voxel(leaf, min_points, True)
     frames = [[(synth.uniform_cloud(seed if same_cloud else seed + f, n, extent=extent)[:n], 1)] for f, n in enumerate(sizes)]
-    segs, per_frame = _upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
+    segs, per_frame = upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
     cm.run_batch(segs)
     out = cm.fetch_batch_outputs()
     return out, _oracle_frames(oracle, per_frame, passes, [leaf] * 3, min_points)
@@ -584,8 +531,8 @@ def test_frame_segmented_sort_ragged_frames(gpu_ok, oracle, min_points):
     st = out["stats"]
     assert st.device_error == 0 and st.frames == len(sizes) and st.key_bytes == 4
     assert st.key_bits == out["key_idx_bits"], "no frame bits were sorted"
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
 
 
 def test_frame_segmented_sort_same_cells_in_adjacent_frames(gpu_ok, oracle):
@@ -599,8 +546,8 @@ def test_frame_segmented_sort_same_cells_in_adjacent_frames(gpu_ok, oracle):
     st = out["stats"]
     assert st.device_error == 0 and st.key_bytes == 4 and st.key_bits == out["key_idx_bits"]
     assert all(fo["n_voxels"] == o[0]["n_voxels"] for fo in o)
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
 
 
 def test_frame_segmented_sort_more_frames_than_threads(gpu_ok, oracle):
@@ -613,8 +560,8 @@ def test_frame_segmented_sort_more_frames_than_threads(gpu_ok, oracle):
         out, o = _ragged_batch(cm, oracle, sizes, z_only, 0.3, 2, (20.0, 20.0, 4.0))
     st = out["stats"]
     assert st.device_error == 0 and st.frames == len(sizes) and st.key_bytes == 4 and st.key_bits == out["key_idx_bits"]
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
 
 
 def test_frame_segmented_sort_big_tile_and_bounded_plan(gpu_ok, oracle):
@@ -627,16 +574,16 @@ def test_frame_segmented_sort_big_tile_and_bounded_plan(gpu_ok, oracle):
         out, o = _ragged_batch(cm, oracle, sizes, z_only, 0.1, 2, (150.0, 150.0, 4.0))
     st = out["stats"]
     assert st.device_error == 0 and st.key_bytes == 4 and st.key_bits == out["key_idx_bits"] and st.survivors > 400000
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
     sizes = [60000, 80000, 0, 70000, 50000]
     box = [(2, -1.0, 1.0, 0), (1, -60.0, 60.0, 0), (0, -60.0, 60.0, 0)]       # 0.02 m: 6001 x 6001 x 101 cells: 32 bits
     with CloudMerger(max_sensors=1, max_batch_points=sum(sizes), max_batch_frames=len(sizes)) as cm:
         out, o = _ragged_batch(cm, oracle, sizes, box, 0.02, 1, (100.0, 100.0, 3.0))
     st = out["stats"]
     assert st.device_error == 0 and st.key_bytes == 4 and st.sort_passes == 4 and st.key_bits == out["key_idx_bits"]
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
 
 
 def test_cfg3_full_size_host_path_and_batch(gpu_ok, oracle):
@@ -656,7 +603,7 @@ def test_cfg3_full_size_host_path_and_batch(gpu_ok, oracle):
         for s in range(S):
             cm.submit_cloud(s, frames[0][s][0], n, make_layout(), stamp=s)
         r = cm.merge_frame(capacity=S * n)
-        segs, per_frame = _upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
+        segs, per_frame = upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16"])
         cm.run_batch(segs)
         out = cm.fetch_batch_outputs()
     o = _oracle_frames(oracle, per_frame, c["passes"], [c["leaf"]] * 3, c["min_points"])
@@ -665,8 +612,8 @@ def test_cfg3_full_size_host_path_and_batch(gpu_ok, oracle):
     assert (r.voxel_idx.astype(np.int64) == o[0]["idx"]).all() and (r.voxel_count == o[0]["count"]).all()
     assert_bit_equal(r.voxel_xyzi, o[0]["centroid"], "host path centroids")
     assert out["stats"].frames == F and out["stats"].points_in == F * S * n and out["key_bytes"] == 4
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
 
 
 @pytest.mark.parametrize("leaf,min_points", [(0.05, 1), (1.0, 2)])
@@ -681,7 +628,7 @@ def test_cfg5_leaf_sweep_at_16mi_points(gpu_ok, oracle, leaf, min_points):
     o.update(n_voxels=o["n"], n_survivors=n)
     assert out["stats"].pcl_overflow == int(o["pcl_overflow"])
     assert out["key_bytes"] == (4 if out["stats"].key_bits <= 32 else 8)
-    assert _check_voxels(out, out["frames"], [o]) <= 1e-5
+    assert check_voxels(out, out["frames"], [o]) <= 1e-5
 
 
 def test_submit_policy_and_unmasked_submissions(gpu_ok, oracle):
@@ -870,13 +817,13 @@ def test_keys_from_the_crop_box_grid(gpu_ok, oracle, leaf, box):
             cm.set_extrinsic(s, synth.extrinsic(s, S))
         cm.set_crop(box)
         cm.set_voxel(leaf, 1, True)
-        segs, per_frame = _upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16" if s != 1 else "pcl32"])
+        segs, per_frame = upload_segments(cm, frames, lambda f, s: LAYOUTS["packed16" if s != 1 else "pcl32"])
         cm.run_batch(segs)
         out = cm.fetch_batch_outputs()
     o = _oracle_frames(oracle, per_frame, box, [leaf] * 3, 1)
     assert out["key_bytes"] == 4 and out["stats"].device_error == 0
     if leaf == 0.035:
         assert out["stats"].key_bits == 32
-    _check_survivors(out, out["frames"], o)
-    assert _check_voxels(out, out["frames"], o) <= 1e-5
+    check_survivors(out, out["frames"], o)
+    assert check_voxels(out, out["frames"], o) <= 1e-5
     assert sum(fo["n_voxels"] for fo in o) > 1000
