@@ -18,10 +18,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <random>
 #include <string>
+#include <type_traits>
 #include <unordered_map>
 #include <vector>
 
@@ -34,6 +36,18 @@ namespace {
 
 constexpr size_t kAlign = 256;
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Owners of the CUDA resources: a set-up that fails part-way leaves nothing behind once its struct is reset or destroyed.
+struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(void* p) const { cudaFreeHost(p); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct GraphExecDestroy { void operator()(cudaGraphExec_t g) const { cudaGraphExecDestroy(g); } };
+template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <typename T> using HostPtr = std::unique_ptr<T, CudaFreeHost>;  // default and mapped page-locked memory
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using GraphExec = std::unique_ptr<std::remove_pointer_t<cudaGraphExec_t>, GraphExecDestroy>;
 
 struct MetaLayout {
   size_t off_ctrl, off_acc, off_hist, zero_bytes, off_info, off_fstart, off_segstart, off_grid, total;
@@ -58,43 +72,43 @@ struct Workspace {
   uint32_t plan_idx_bits = 0, plan_total_bits = 0;  // key plan of the last unbounded run (fetched from the device)
   int out_step = 16;
   MetaLayout ml{};
-  uint8_t* meta = nullptr;
-  uint8_t* report = nullptr;  // pinned host mirror of meta
-  SegDev* segs = nullptr;
+  DevPtr<uint8_t> meta;
+  HostPtr<uint8_t> report;  // pinned host mirror of meta
+  DevPtr<SegDev> segs;
   std::vector<SegDev> segs_host;  // what is currently uploaded
-  uint32_t* tile_seg = nullptr;
+  DevPtr<uint32_t> tile_seg;
   std::vector<uint32_t> tile_seg_host;
-  float4* surv_xyzi = nullptr;
-  uint32_t* surv_src = nullptr;
-  uint32_t* surv_key = nullptr;          // box-grid voxel keys written by K1 (fused-key runs)
-  uint32_t* first_k1 = nullptr;          // [sort tiles] K1 tile holding the first key of every radix tile
-  SegTile* seg_tile = nullptr;           // frame-segmented sort (batches of several frames): [sort tiles + frames]
-  uint32_t* seg_hist = nullptr;          //   [frames][CM_SEG_PASSES][256]
-  uint32_t* seg_frame_tile0 = nullptr;   //   [frames + 1]
-  uint2* seg_cent_range = nullptr;       //   [centroid tiles]
+  DevPtr<float4> surv_xyzi;
+  DevPtr<uint32_t> surv_src;
+  DevPtr<uint32_t> surv_key;             // box-grid voxel keys written by K1 (fused-key runs)
+  DevPtr<uint32_t> first_k1;             // [sort tiles] K1 tile holding the first key of every radix tile
+  DevPtr<SegTile> seg_tile;              // frame-segmented sort (batches of several frames): [sort tiles + frames]
+  DevPtr<uint32_t> seg_hist;             //   [frames][CM_SEG_PASSES][256]
+  DevPtr<uint32_t> seg_frame_tile0;      //   [frames + 1]
+  DevPtr<uint2> seg_cent_range;          //   [centroid tiles]
   bool timed_pass0 = false;              // last run: an event was recorded after radix pass 0 (profiling, host-planned key width)
   bool segmented = false;                // last run: the frame-segmented kernels were enqueued (SortInfo says whether they ran)
   bool fused_keys = false;               // last run: K1 produced the keys
   BoxGrid box{};
-  void *keys_a = nullptr, *keys_b = nullptr;
-  uint32_t *vals_a = nullptr, *vals_b = nullptr;
-  TileRec* tile_rec = nullptr;          // [lb_k1_n] K1 tile records
-  unsigned long long* cent_status = nullptr;  // [lb_cent_n] look-back words of the voxel compaction
-  unsigned long long* lb_sort = nullptr;
-  uint32_t* epoch_dev = nullptr;        // run epoch of the look-back words (device-resident, see VoxelParams)
+  DevPtr<unsigned long long> keys_a, keys_b;
+  DevPtr<uint32_t> vals_a, vals_b;
+  DevPtr<TileRec> tile_rec;             // [lb_k1_n] K1 tile records
+  DevPtr<unsigned long long> cent_status;  // [lb_cent_n] look-back words of the voxel compaction
+  DevPtr<unsigned long long> lb_sort;
+  DevPtr<uint32_t> epoch_dev;           // run epoch of the look-back words (device-resident, see VoxelParams)
   size_t lb_k1_n = 0, lb_sort_n = 0, lb_cent_n = 0;
-  float4* dense_xyzi = nullptr;         // dense merged cloud, allocated and filled on request only
-  uint32_t* dense_src = nullptr;
-  uint32_t* dense_slot = nullptr;
+  DevPtr<float4> dense_xyzi;            // dense merged cloud, allocated and filled on request only
+  DevPtr<uint32_t> dense_src;
+  DevPtr<uint32_t> dense_slot;
   bool dense_valid = false;
   uint32_t n_k1_tiles = 0;
-  void* out_xyzi = nullptr;
-  uint32_t* out_count = nullptr;
-  unsigned long long* out_idx = nullptr;
-  unsigned long long* trace_k1 = nullptr;    // debug traces (CM_TRACE=1): 8 stamps per tile
-  unsigned long long* trace_sort = nullptr;
+  DevPtr<uint8_t> out_xyzi;
+  DevPtr<uint32_t> out_count;
+  DevPtr<unsigned long long> out_idx;
+  DevPtr<unsigned long long> trace_k1;  // debug traces (CM_TRACE=1): 8 stamps per tile
+  DevPtr<unsigned long long> trace_sort;
   size_t trace_k1_n = 0, trace_sort_n = 0;
-  cudaEvent_t ev[EV_COUNT]{};
+  Event ev[EV_COUNT];
   // description of the last run
   bool has_run = false, report_valid = false, profiled = false;
   uint32_t n_frames = 0, n_segs = 0;
@@ -114,26 +128,26 @@ struct SensorState {
   int64_t n_points = 0;
   cm_layout_t layout{};
   uint64_t stamp = 0;
-  cudaEvent_t copied = nullptr;
+  Event copied;
 };
 
 struct Slot {
   Workspace ws;
-  uint8_t* raw_dev = nullptr;     // one region per sensor (single submissions, carried-over clouds)
-  uint8_t* raw_pinned = nullptr;
+  DevPtr<uint8_t> raw_dev;        // one region per sensor (single submissions, carried-over clouds)
+  HostPtr<uint8_t> raw_pinned;
   // cm_submit_clouds_pinned: host-adjacent clouds travel as one copy into this bump-allocated arena, so a coalesced run
   // never shares bytes with a sensor's own region or with another run; reset when the slot's frame has been merged
-  uint8_t* arena_dev = nullptr;
+  DevPtr<uint8_t> arena_dev;
   size_t arena_bytes = 0, arena_used = 0;
   // page-locked, device-mapped mirrors of the frame's voxel outputs: the last kernel of the frame (k_export_voxels) writes
   // them over PCIe, sized on the device, so cm_wait_frame needs ONE synchronisation and no copy of its own
-  uint8_t* exp_xyzi = nullptr;
-  uint32_t* exp_count = nullptr;
-  unsigned long long* exp_idx = nullptr;
+  HostPtr<uint8_t> exp_xyzi;
+  HostPtr<uint32_t> exp_count;
+  HostPtr<unsigned long long> exp_idx;
   uint32_t exp_cap = 0;
   std::vector<SensorState> sensor;
-  cudaStream_t stream = nullptr;
-  cudaEvent_t done = nullptr;
+  Stream stream;
+  Event done;
   int64_t ticket = -1;
   bool busy = false;
   uint64_t used_mask = 0, stamp = 0;
@@ -141,7 +155,7 @@ struct Slot {
   // path is ~12 stream operations on half a million points, and enqueueing them one by one costs more host time than
   // the GPU needs to run them. graph_seen: configuration of the previous frame (run the plain way, which also uploads
   // the segment table); graph_key: configuration the instantiated graph belongs to.
-  cudaGraphExec_t graph = nullptr;
+  GraphExec graph;
   std::string graph_key, graph_seen;
 };
 
@@ -174,13 +188,13 @@ struct cm_handle_s {
   ZoneSet zones{};
   struct ZoneWs {
     size_t cap_points = 0, cap_out = 0;
-    unsigned short* mask = nullptr;
-    uint32_t *tile_count = nullptr, *tile_offset = nullptr, *zone_begin = nullptr, *overflow = nullptr;
-    uint32_t* zone_total = nullptr;  // [CM_MAX_ZONES] + the scan ticket behind it
-    float4* out_xyzi = nullptr;
-    uint32_t* out_src = nullptr;
-    float4* in_stage = nullptr;  // host-buffer form: the uploaded cloud
-    uint32_t* report = nullptr;  // pinned: zone_begin[CM_MAX_ZONES + 1] + overflow
+    DevPtr<unsigned short> mask;
+    DevPtr<uint32_t> tile_count, tile_offset, zone_begin, overflow;
+    DevPtr<uint32_t> zone_total;  // [CM_MAX_ZONES] + the scan ticket behind it
+    DevPtr<float4> out_xyzi;
+    DevPtr<uint32_t> out_src;
+    DevPtr<float4> in_stage;      // host-buffer form: the uploaded cloud
+    HostPtr<uint32_t> report;     // pinned: zone_begin[CM_MAX_ZONES + 1] + overflow
     cudaStream_t stream = nullptr;
     bool ran = false;
     int64_t launches = 0;
@@ -188,34 +202,33 @@ struct cm_handle_s {
     int n_zones_run = 0;         // zones of the last split (1 for a radius outlier removal)
   } zw;
   // radius outlier removal: first sorted position of every cell key (allocated on first use, grows)
-  uint32_t* ror_table = nullptr;
+  DevPtr<uint32_t> ror_table;
   size_t ror_table_cap = 0;
   // RANSAC ground plane (allocated on first use): one batch of draws and its scores, device + pinned mirrors
   struct PlaneWs {
     size_t cap_draws = 0;
-    int32_t* samples_dev = nullptr;  // [cap_draws][3]
-    int32_t* counts_dev = nullptr;   // [cap_draws] counts, then [cap_draws] good flags
-    float4* models_dev = nullptr;    // [cap_draws]
-    float* acc_dev = nullptr;        // [10] running sums + count
-    int32_t* samples_pin = nullptr;
-    int32_t* counts_pin = nullptr;
-    float4* models_pin = nullptr;
-    float* acc_pin = nullptr;
+    DevPtr<int32_t> samples_dev;  // [cap_draws][3]
+    DevPtr<int32_t> counts_dev;   // [cap_draws] counts, then [cap_draws] good flags
+    DevPtr<float4> models_dev;    // [cap_draws]
+    DevPtr<float> acc_dev;        // [10] running sums + count
+    HostPtr<int32_t> samples_pin;
+    HostPtr<int32_t> counts_pin;
+    HostPtr<float4> models_pin;
+    HostPtr<float> acc_pin;
   } pw;
   // cm_*proceed_zones: stage results parked between the three multi-cloud stages, and the two result clouds
   struct ProceedWs {
     size_t cap = 0;
-    float4 *low = nullptr, *high = nullptr, *rest = nullptr, *planes = nullptr;  // [cap] each
-    float4 *no_ground = nullptr, *ground = nullptr;                              // [2 cap] (windows share their end points)
-    float4* in_stage = nullptr;                                                  // host-buffer form: the uploaded ROI cloud
+    DevPtr<float4> low, high, rest, planes;  // [cap] each
+    DevPtr<float4> no_ground, ground;        // [2 cap] (windows share their end points)
+    DevPtr<float4> in_stage;                 // host-buffer form: the uploaded ROI cloud
   } prz;
-  // host path
+  // host path: slots and streams are set up together on first use (empty until then)
   std::vector<Slot> slots;
-  std::vector<cudaStream_t> sensor_stream;
+  std::vector<Stream> sensor_stream;
   size_t slot_stride = 0;
   int fill = 0;
   int64_t ticket_counter = 0;
-  bool host_ready = false;
   bool use_graph = true;  // CM_NO_GRAPH=1 switches the frame graphs off
   int submit_policy = CM_SUBMIT_LATEST_WINS;
 };
@@ -278,7 +291,8 @@ bool cpus_of_node(int node, cpu_set_t* set) {
   fclose(f);
   return n > 0;
 }
-cudaError_t pinned_alloc(void** p, size_t bytes, unsigned flags) {
+template <typename T>
+cudaError_t pinned_alloc(HostPtr<T>& p, size_t bytes, unsigned flags) {
   static const bool no_numa = getenv("CM_NO_NUMA") != nullptr;
   cpu_set_t old_set, local;
   bool moved = false;
@@ -290,74 +304,77 @@ cudaError_t pinned_alloc(void** p, size_t bytes, unsigned flags) {
       if (CPU_COUNT(&both) > 0 && !CPU_EQUAL(&both, &old_set)) moved = sched_setaffinity(0, sizeof(both), &both) == 0;
     }
   }
-  const cudaError_t e = cudaHostAlloc(p, bytes ? bytes : 1, flags);
+  void* raw = nullptr;
+  const cudaError_t e = cudaHostAlloc(&raw, bytes ? bytes : 1, flags);
   if (moved) sched_setaffinity(0, sizeof(old_set), &old_set);
+  p.reset(e == cudaSuccess ? static_cast<T*>(raw) : nullptr);
   return e;
 }
 
+// `count` elements, at least `min_bytes`
 template <typename T>
-cudaError_t dev_alloc(T** p, size_t count) {
-  return cudaMalloc(reinterpret_cast<void**>(p), std::max<size_t>(count * sizeof(T), kAlign));
+cudaError_t dev_alloc(DevPtr<T>& p, size_t count, size_t min_bytes = kAlign) {
+  void* raw = nullptr;
+  const cudaError_t e = cudaMalloc(&raw, std::max<size_t>(count * sizeof(T), min_bytes));
+  p.reset(e == cudaSuccess ? static_cast<T*>(raw) : nullptr);
+  return e;
 }
 
-void ws_free(Workspace& w) {
-  if (!w.ready) return;
-  cudaFree(w.meta); cudaFreeHost(w.report); cudaFree(w.segs); cudaFree(w.tile_seg); cudaFree(w.surv_xyzi); cudaFree(w.surv_src);
-  cudaFree(w.surv_key); cudaFree(w.first_k1); cudaFree(w.seg_tile); cudaFree(w.seg_hist); cudaFree(w.seg_frame_tile0); cudaFree(w.seg_cent_range);
-  cudaFree(w.keys_a); cudaFree(w.keys_b); cudaFree(w.vals_a); cudaFree(w.vals_b);
-  cudaFree(w.tile_rec); cudaFree(w.lb_sort); cudaFree(w.cent_status); cudaFree(w.epoch_dev);
-  cudaFree(w.dense_xyzi); cudaFree(w.dense_src); cudaFree(w.dense_slot);
-  cudaFree(w.out_xyzi); cudaFree(w.out_count); cudaFree(w.out_idx);
-  cudaFree(w.trace_k1); cudaFree(w.trace_sort);
-  for (auto& e : w.ev) if (e) cudaEventDestroy(e);
-  w = Workspace();
+// An event or stream made by cudaEventCreateWithFlags / cudaStreamCreateWithFlags (left empty if the call fails).
+template <typename Owner>
+cudaError_t create(Owner& p, cudaError_t (*make)(typename Owner::pointer*, unsigned), unsigned flags) {
+  typename Owner::pointer raw = nullptr;
+  const cudaError_t e = make(&raw, flags);
+  p.reset(e == cudaSuccess ? raw : nullptr);
+  return e;
 }
 
 int ws_alloc(cm_handle_t h, Workspace& w, uint32_t points, uint32_t frames, uint32_t segs, int out_step) {
+  w = Workspace();  // frees what an earlier, failed call left behind
   w.cap_points = points; w.cap_frames = frames; w.cap_segs = segs; w.out_step = out_step;
   w.ml.build(frames, segs);
   const size_t np = std::max<uint32_t>(points, 1);
-  CM_CUDA(h, dev_alloc(&w.meta, w.ml.total));
-  CM_CUDA(h, cudaMemset(w.meta, 0, w.ml.total));
-  CM_CUDA(h, pinned_alloc(reinterpret_cast<void**>(&w.report), w.ml.total, cudaHostAllocDefault));
-  memset(w.report, 0, w.ml.total);
-  CM_CUDA(h, dev_alloc(&w.segs, segs));
-  CM_CUDA(h, dev_alloc(&w.surv_xyzi, np));
-  CM_CUDA(h, dev_alloc(&w.surv_src, np));
-  CM_CUDA(h, dev_alloc(&w.surv_key, np));
-  CM_CUDA(h, dev_alloc(&w.first_k1, sort_lookback_rows((uint32_t)np)));
-  CM_CUDA(h, cudaMalloc(&w.keys_a, np * 8));
-  CM_CUDA(h, cudaMalloc(&w.keys_b, np * 8));
-  CM_CUDA(h, dev_alloc(&w.vals_a, np));
-  CM_CUDA(h, dev_alloc(&w.vals_b, np));
+  CM_CUDA(h, dev_alloc(w.meta, w.ml.total));
+  CM_CUDA(h, cudaMemset(w.meta.get(), 0, w.ml.total));
+  CM_CUDA(h, pinned_alloc(w.report, w.ml.total, cudaHostAllocDefault));
+  memset(w.report.get(), 0, w.ml.total);
+  CM_CUDA(h, dev_alloc(w.segs, segs));
+  CM_CUDA(h, dev_alloc(w.surv_xyzi, np));
+  CM_CUDA(h, dev_alloc(w.surv_src, np));
+  CM_CUDA(h, dev_alloc(w.surv_key, np));
+  CM_CUDA(h, dev_alloc(w.first_k1, sort_lookback_rows((uint32_t)np)));
+  CM_CUDA(h, dev_alloc(w.keys_a, np, 0));
+  CM_CUDA(h, dev_alloc(w.keys_b, np, 0));
+  CM_CUDA(h, dev_alloc(w.vals_a, np));
+  CM_CUDA(h, dev_alloc(w.vals_b, np));
   // every segment owns at least one K1 tile
   w.lb_k1_n = np / k1_min_tile_points() + segs + 2;
-  CM_CUDA(h, dev_alloc(&w.tile_seg, w.lb_k1_n));
+  CM_CUDA(h, dev_alloc(w.tile_seg, w.lb_k1_n));
   w.lb_sort_n = (sort_lookback_rows((uint32_t)np) + (frames > 1 ? frames : 0u)) * CM_RADIX;  // segmented: a partial tile per frame
   if (frames > 1) {
-    CM_CUDA(h, dev_alloc(&w.seg_tile, sort_lookback_rows((uint32_t)np) + frames));
-    CM_CUDA(h, dev_alloc(&w.seg_hist, (size_t)frames * CM_SEG_PASSES * CM_RADIX));
-    CM_CUDA(h, dev_alloc(&w.seg_frame_tile0, (size_t)frames + 1));
-    CM_CUDA(h, dev_alloc(&w.seg_cent_range, np / centroid_tile_items() + 2));
+    CM_CUDA(h, dev_alloc(w.seg_tile, sort_lookback_rows((uint32_t)np) + frames));
+    CM_CUDA(h, dev_alloc(w.seg_hist, (size_t)frames * CM_SEG_PASSES * CM_RADIX));
+    CM_CUDA(h, dev_alloc(w.seg_frame_tile0, (size_t)frames + 1));
+    CM_CUDA(h, dev_alloc(w.seg_cent_range, np / centroid_tile_items() + 2));
   }
   w.lb_cent_n = np / centroid_tile_items() + 2;
-  CM_CUDA(h, dev_alloc(&w.tile_rec, w.lb_k1_n));
-  CM_CUDA(h, dev_alloc(&w.lb_sort, w.lb_sort_n));
-  CM_CUDA(h, dev_alloc(&w.cent_status, w.lb_cent_n));
-  CM_CUDA(h, cudaMemset(w.cent_status, 0, w.lb_cent_n * 8));
-  CM_CUDA(h, cudaMemset(w.lb_sort, 0, w.lb_sort_n * 8));
-  CM_CUDA(h, dev_alloc(&w.epoch_dev, (size_t)1));
-  CM_CUDA(h, cudaMemset(w.epoch_dev, 0, sizeof(uint32_t)));
-  CM_CUDA(h, cudaMalloc(&w.out_xyzi, np * (size_t)out_step));
-  CM_CUDA(h, dev_alloc(&w.out_count, np));
-  CM_CUDA(h, dev_alloc(&w.out_idx, np));
-  for (auto& e : w.ev) CM_CUDA(h, cudaEventCreate(&e));
+  CM_CUDA(h, dev_alloc(w.tile_rec, w.lb_k1_n));
+  CM_CUDA(h, dev_alloc(w.lb_sort, w.lb_sort_n));
+  CM_CUDA(h, dev_alloc(w.cent_status, w.lb_cent_n));
+  CM_CUDA(h, cudaMemset(w.cent_status.get(), 0, w.lb_cent_n * 8));
+  CM_CUDA(h, cudaMemset(w.lb_sort.get(), 0, w.lb_sort_n * 8));
+  CM_CUDA(h, dev_alloc(w.epoch_dev, (size_t)1));
+  CM_CUDA(h, cudaMemset(w.epoch_dev.get(), 0, sizeof(uint32_t)));
+  CM_CUDA(h, dev_alloc(w.out_xyzi, np * (size_t)out_step, 0));
+  CM_CUDA(h, dev_alloc(w.out_count, np));
+  CM_CUDA(h, dev_alloc(w.out_idx, np));
+  for (auto& e : w.ev) CM_CUDA(h, create(e, cudaEventCreateWithFlags, cudaEventDefault));
   if (getenv("CM_TRACE")) {
     w.trace_k1_n = w.lb_k1_n * 8; w.trace_sort_n = (w.lb_sort_n / CM_RADIX) * 8;
-    CM_CUDA(h, dev_alloc(&w.trace_k1, w.trace_k1_n));
-    CM_CUDA(h, dev_alloc(&w.trace_sort, w.trace_sort_n));
-    CM_CUDA(h, cudaMemset(w.trace_k1, 0, w.trace_k1_n * 8));
-    CM_CUDA(h, cudaMemset(w.trace_sort, 0, w.trace_sort_n * 8));
+    CM_CUDA(h, dev_alloc(w.trace_k1, w.trace_k1_n));
+    CM_CUDA(h, dev_alloc(w.trace_sort, w.trace_sort_n));
+    CM_CUDA(h, cudaMemset(w.trace_k1.get(), 0, w.trace_k1_n * 8));
+    CM_CUDA(h, cudaMemset(w.trace_sort.get(), 0, w.trace_sort_n * 8));
   }
   // the clears above ran on the default stream: callers may go on with a non-blocking stream of their own
   CM_CUDA(h, cudaDeviceSynchronize());
@@ -445,7 +462,7 @@ bool crop_box_grid(cm_handle_t h, uint32_t n_frames, BoxGrid* g) {
 void fill_voxel_params(cm_handle_t h, Workspace& w, VoxelParams& vp, const float4* pts, uint32_t n_frames,
                        uint32_t max_points) {
   vp.pts = pts;
-  vp.frame_surv_start = reinterpret_cast<uint32_t*>(w.meta + w.ml.off_fstart);
+  vp.frame_surv_start = reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_fstart);
   vp.n_frames = n_frames;
   vp.max_points = max_points;
   for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = h->inv_leaf[k];
@@ -454,26 +471,26 @@ void fill_voxel_params(cm_handle_t h, Workspace& w, VoxelParams& vp, const float
   vp.pcl_refuses = h->overflow_mode == 1 ? 1u : 0u;
   vp.key_bytes = 8;
   vp.out_step = (uint32_t)w.out_step;
-  vp.ctrl = reinterpret_cast<Ctrl*>(w.meta + w.ml.off_ctrl);
-  vp.acc = reinterpret_cast<FrameAcc*>(w.meta + w.ml.off_acc);
-  vp.grid = reinterpret_cast<GridDev*>(w.meta + w.ml.off_grid);
-  vp.info = reinterpret_cast<SortInfo*>(w.meta + w.ml.off_info);
-  vp.hist = reinterpret_cast<uint32_t*>(w.meta + w.ml.off_hist);
-  vp.keys_a = w.keys_a; vp.keys_b = w.keys_b; vp.vals_a = w.vals_a; vp.vals_b = w.vals_b;
-  vp.lb_sort = w.lb_sort; vp.cent_status = w.cent_status;
+  vp.ctrl = reinterpret_cast<Ctrl*>(w.meta.get() + w.ml.off_ctrl);
+  vp.acc = reinterpret_cast<FrameAcc*>(w.meta.get() + w.ml.off_acc);
+  vp.grid = reinterpret_cast<GridDev*>(w.meta.get() + w.ml.off_grid);
+  vp.info = reinterpret_cast<SortInfo*>(w.meta.get() + w.ml.off_info);
+  vp.hist = reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_hist);
+  vp.keys_a = w.keys_a.get(); vp.keys_b = w.keys_b.get(); vp.vals_a = w.vals_a.get(); vp.vals_b = w.vals_b.get();
+  vp.lb_sort = w.lb_sort.get(); vp.cent_status = w.cent_status.get();
   vp.cent_status_words = (uint32_t)std::min<size_t>(w.lb_cent_n, 0xFFFFFFFFu);
-  vp.tile_rec = w.ran_k1 ? w.tile_rec : nullptr;
+  vp.tile_rec = w.ran_k1 ? w.tile_rec.get() : nullptr;
   vp.n_k1_tiles = w.n_k1_tiles;
-  vp.epoch_dev = w.epoch_dev;
+  vp.epoch_dev = w.epoch_dev.get();
   vp.lb_sort_words = (uint32_t)std::min<size_t>(w.lb_sort_n, 0xFFFFFFFFu);
   vp.max_passes = CM_MAX_SORT_PASSES;
-  vp.fused_keys = 0; vp.surv_key = w.surv_key; vp.box = BoxGrid{}; vp.first_k1 = w.first_k1;
+  vp.fused_keys = 0; vp.surv_key = w.surv_key.get(); vp.box = BoxGrid{}; vp.first_k1 = w.first_k1.get();
   vp.sort_tile = sort_tile_items(4, max_points);
   vp.dual_width = 0;
-  vp.segmented = 0; vp.seg_tile = w.seg_tile; vp.seg_hist = w.seg_hist; vp.seg_frame_tile0 = w.seg_frame_tile0;
-  vp.seg_cent_range = w.seg_cent_range;
-  vp.out_xyzi = w.out_xyzi; vp.out_count = w.out_count; vp.out_idx = w.out_idx;
-  vp.trace = w.trace_sort;
+  vp.segmented = 0; vp.seg_tile = w.seg_tile.get(); vp.seg_hist = w.seg_hist.get(); vp.seg_frame_tile0 = w.seg_frame_tile0.get();
+  vp.seg_cent_range = w.seg_cent_range.get();
+  vp.out_xyzi = w.out_xyzi.get(); vp.out_count = w.out_count.get(); vp.out_idx = w.out_idx.get();
+  vp.trace = w.trace_sort.get();
   const char* tp = getenv("CM_TRACE_PASS");
   vp.trace_pass = tp ? (uint32_t)atoi(tp) : 1u;
 }
@@ -524,14 +541,14 @@ int run_voxel(cm_handle_t h, Workspace& w, VoxelParams& vp, cudaStream_t st, boo
   }
   w.segmented = vp.segmented != 0;
   if (vp.segmented)
-    CM_CUDA(h, cudaMemsetAsync(w.seg_hist, 0, (size_t)vp.n_frames * CM_SEG_PASSES * CM_RADIX * sizeof(uint32_t), st));
+    CM_CUDA(h, cudaMemsetAsync(w.seg_hist.get(), 0, (size_t)vp.n_frames * CM_SEG_PASSES * CM_RADIX * sizeof(uint32_t), st));
   if (scan_k1_tiles)
-    CM_CUDA(h, launch_grid_setup(vp, st, w.tile_rec, w.n_k1_tiles, w.segs, w.n_segs,
-                                 reinterpret_cast<uint32_t*>(w.meta + w.ml.off_segstart)));
+    CM_CUDA(h, launch_grid_setup(vp, st, w.tile_rec.get(), w.n_k1_tiles, w.segs.get(), w.n_segs,
+                                 reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_segstart)));
   else
     CM_CUDA(h, launch_grid_setup(vp, st));
   ++w.launches;
-  if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_GRID], st));
+  if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_GRID].get(), st));
   if (dual) {
     w.key_bytes = 0;  // known with the report (fetch_report)
     w.max_passes = CM_MAX_SORT_PASSES;
@@ -544,24 +561,24 @@ int run_voxel(cm_handle_t h, Workspace& w, VoxelParams& vp, cudaStream_t st, boo
       CM_CUDA(h, launch_seg_base(v4, st));
       ++w.launches;
     }
-    if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_KEY], st));
+    if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_KEY].get(), st));
     for (uint32_t ps = 0; ps < 4; ++ps) CM_CUDA(h, launch_sort_pass(v4, (int)ps, st));
     for (uint32_t ps = 0; ps < CM_MAX_SORT_PASSES; ++ps) CM_CUDA(h, launch_sort_pass(v8, (int)ps, st));
     w.launches += 4 + CM_MAX_SORT_PASSES;
-    if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT], st));
+    if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT].get(), st));
     CM_CUDA(h, launch_centroid(v4, st));
     CM_CUDA(h, launch_centroid(v8, st));
     w.launches += 2 * CM_CENTROID_LAUNCHES;
-    if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT], st));
+    if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
     w.ran_voxel = true;
     return CM_OK;
   }
   if (!bounded) {
     // the key width is only known on the device: fetch the plan (one small round trip), then size the sort to it
     SortInfo si;
-    CM_CUDA(h, cudaMemcpyAsync(w.report + w.ml.off_info, w.meta + w.ml.off_info, sizeof(SortInfo), cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaMemcpyAsync(w.report.get() + w.ml.off_info, w.meta.get() + w.ml.off_info, sizeof(SortInfo), cudaMemcpyDeviceToHost, st));
     CM_CUDA(h, cudaStreamSynchronize(st));
-    memcpy(&si, w.report + w.ml.off_info, sizeof(si));
+    memcpy(&si, w.report.get() + w.ml.off_info, sizeof(si));
     vp.key_bytes = si.total_bits <= 32 ? 4 : 8;
     vp.max_passes = si.num_passes;
     w.plan_idx_bits = si.idx_bits; w.plan_total_bits = si.total_bits;
@@ -576,24 +593,24 @@ int run_voxel(cm_handle_t h, Workspace& w, VoxelParams& vp, cudaStream_t st, boo
     CM_CUDA(h, launch_seg_base(vp, st));
     ++w.launches;
   }
-  if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_KEY], st));
+  if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_KEY].get(), st));
   w.timed_pass0 = false;
   for (uint32_t ps = 0; ps < vp.max_passes; ++ps) {
     CM_CUDA(h, launch_sort_pass(vp, (int)ps, st));
     ++w.launches;
     if (ps == 0 && h->profiling) {  // pass 0 of a fused-key run does the key kernel's histogram work too: timed on its own
-      CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT0], st));
+      CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT0].get(), st));
       w.timed_pass0 = true;
     }
   }
-  if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT], st));
+  if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT].get(), st));
   if (!with_centroid) {  // the caller only wants the points sorted by cell (radius outlier removal)
     w.ran_voxel = false;
     return CM_OK;
   }
   CM_CUDA(h, launch_centroid(vp, st));
   w.launches += CM_CENTROID_LAUNCHES;
-  if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT], st));
+  if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
   w.ran_voxel = true;
   return CM_OK;
 }
@@ -701,11 +718,11 @@ int run_pipeline(cm_handle_t h, Workspace& w, const cm_segment_t* segs, int n_se
   int rc = build_segments(h, w, segs, n_seg, sd, ts, &plan);
   if (rc != CM_OK) return rc;
   if (sd.size() != w.segs_host.size() || memcmp(sd.data(), w.segs_host.data(), sd.size() * sizeof(SegDev)) != 0) {
-    CM_CUDA(h, cudaMemcpyAsync(w.segs, sd.data(), sd.size() * sizeof(SegDev), cudaMemcpyHostToDevice, st));
+    CM_CUDA(h, cudaMemcpyAsync(w.segs.get(), sd.data(), sd.size() * sizeof(SegDev), cudaMemcpyHostToDevice, st));
     w.segs_host = sd;
   }
   if (!ts.empty() && ts != w.tile_seg_host) {
-    CM_CUDA(h, cudaMemcpyAsync(w.tile_seg, ts.data(), ts.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    CM_CUDA(h, cudaMemcpyAsync(w.tile_seg.get(), ts.data(), ts.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     w.tile_seg_host = ts;
   }
   const uint32_t n_frames = plan.n_frames;
@@ -713,44 +730,44 @@ int run_pipeline(cm_handle_t h, Workspace& w, const cm_segment_t* segs, int n_se
   w.has_run = true; w.report_valid = false; w.profiled = h->profiling;
   w.n_frames = n_frames; w.n_segs = (uint32_t)n_seg; w.points_in = total; w.launches = 0;
   w.ran_k1 = true; w.ran_voxel = false; w.stream = st;
-  w.voxel_pts = w.surv_xyzi;
+  w.voxel_pts = w.surv_xyzi.get();
   h->last = &w;
 
-  if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_START], st));
-  CM_CUDA(h, cudaMemsetAsync(w.meta, 0, w.ml.zero_bytes, st));
+  if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
+  CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
   K1Params kp;
-  kp.segs = w.segs; kp.n_seg = (uint32_t)n_seg; kp.n_tiles = plan.n_tiles; kp.n_frames = n_frames;
-  kp.tiles_per_seg = plan.tiles_per_seg; kp.tile_seg = w.tile_seg;
+  kp.segs = w.segs.get(); kp.n_seg = (uint32_t)n_seg; kp.n_tiles = plan.n_tiles; kp.n_frames = n_frames;
+  kp.tiles_per_seg = plan.tiles_per_seg; kp.tile_seg = w.tile_seg.get();
   kp.crop = h->crop;
-  kp.surv_xyzi = w.surv_xyzi; kp.surv_src = w.surv_src;
-  kp.ctrl = reinterpret_cast<Ctrl*>(w.meta + w.ml.off_ctrl);
-  kp.acc = reinterpret_cast<FrameAcc*>(w.meta + w.ml.off_acc);
-  kp.tile_rec = w.tile_rec;
-  kp.trace = w.trace_k1;
+  kp.surv_xyzi = w.surv_xyzi.get(); kp.surv_src = w.surv_src.get();
+  kp.ctrl = reinterpret_cast<Ctrl*>(w.meta.get() + w.ml.off_ctrl);
+  kp.acc = reinterpret_cast<FrameAcc*>(w.meta.get() + w.ml.off_acc);
+  kp.tile_rec = w.tile_rec.get();
+  kp.trace = w.trace_k1.get();
   // K1 keys the survivors itself when the crop is a box that bounds the grid (no k_voxel_key_hist): CM_NO_FUSED_KEYS=1 keeps
   // the separate key kernel (A/B and test hook)
   static const bool no_fused = getenv("CM_NO_FUSED_KEYS") != nullptr;
   BoxGrid box{};
   const bool fused = with_voxel && !no_fused && crop_box_grid(h, n_frames, &box);
   w.fused_keys = fused; w.box = box;
-  kp.surv_key = fused ? w.surv_key : nullptr;
-  kp.hist = reinterpret_cast<uint32_t*>(w.meta + w.ml.off_hist);
+  kp.surv_key = fused ? w.surv_key.get() : nullptr;
+  kp.hist = reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_hist);
   kp.box = box;
   w.n_k1_tiles = plan.n_tiles;
   w.dense_valid = false;
   CM_CUDA(h, launch_transform_crop(kp, plan.tile_points, plan.mode, plan.staged_smem, st));
   ++w.launches;
   if (!with_voxel) {
-    CM_CUDA(h, launch_tile_scan(w.tile_rec, plan.n_tiles, w.segs, (uint32_t)n_seg, n_frames,
-                                reinterpret_cast<uint32_t*>(w.meta + w.ml.off_fstart),
-                                reinterpret_cast<uint32_t*>(w.meta + w.ml.off_segstart), st));
+    CM_CUDA(h, launch_tile_scan(w.tile_rec.get(), plan.n_tiles, w.segs.get(), (uint32_t)n_seg, n_frames,
+                                reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_fstart),
+                                reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_segstart), st));
     ++w.launches;
-    CM_CUDA(h, cudaEventRecord(w.ev[EV_K1], st));
+    CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
     return CM_OK;
   }
-  if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_K1], st));
+  if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
   VoxelParams vp;
-  fill_voxel_params(h, w, vp, w.surv_xyzi, n_frames, (uint32_t)total);
+  fill_voxel_params(h, w, vp, w.surv_xyzi.get(), n_frames, (uint32_t)total);
   vp.fused_keys = fused ? 1u : 0u;
   vp.box = box;
   return run_voxel(h, w, vp, st, true);  // the tile scan rides in the grid-setup launch
@@ -760,13 +777,15 @@ int run_pipeline(cm_handle_t h, Workspace& w, const cm_segment_t* segs, int n_se
 int materialize_dense(cm_handle_t h, Workspace& w) {
   if (!w.ran_k1 || w.dense_valid) return CM_OK;
   const size_t np = std::max<uint32_t>(w.cap_points, 1);
-  if (!w.dense_xyzi) {
-    CM_CUDA(h, dev_alloc(&w.dense_xyzi, np));
-    CM_CUDA(h, dev_alloc(&w.dense_src, np));
-    CM_CUDA(h, dev_alloc(&w.dense_slot, np));
+  if (!w.dense_xyzi) {  // all three or none
+    DevPtr<float4> xyzi; DevPtr<uint32_t> src, slot;
+    CM_CUDA(h, dev_alloc(xyzi, np));
+    CM_CUDA(h, dev_alloc(src, np));
+    CM_CUDA(h, dev_alloc(slot, np));
+    w.dense_xyzi = std::move(xyzi); w.dense_src = std::move(src); w.dense_slot = std::move(slot);
   }
-  CM_CUDA(h, launch_compact_survivors(w.tile_rec, w.n_k1_tiles, w.surv_xyzi, w.surv_src, w.dense_xyzi, w.dense_src,
-                                      w.dense_slot, w.stream));
+  CM_CUDA(h, launch_compact_survivors(w.tile_rec.get(), w.n_k1_tiles, w.surv_xyzi.get(), w.surv_src.get(), w.dense_xyzi.get(),
+                                      w.dense_src.get(), w.dense_slot.get(), w.stream));
   w.dense_valid = true;
   return CM_OK;
 }
@@ -778,14 +797,14 @@ int fetch_report(cm_handle_t h, Workspace& w, cudaEvent_t already_copied = nullp
   if (already_copied) {
     CM_CUDA(h, cudaEventSynchronize(already_copied));  // the run enqueued the report copy itself
   } else {
-    CM_CUDA(h, cudaMemcpyAsync(w.report, w.meta, w.ml.total, cudaMemcpyDeviceToHost, w.stream));
+    CM_CUDA(h, cudaMemcpyAsync(w.report.get(), w.meta.get(), w.ml.total, cudaMemcpyDeviceToHost, w.stream));
     CM_CUDA(h, cudaStreamSynchronize(w.stream));
   }
-  const Ctrl* ctrl = reinterpret_cast<const Ctrl*>(w.report + w.ml.off_ctrl);
-  const FrameAcc* acc = reinterpret_cast<const FrameAcc*>(w.report + w.ml.off_acc);
-  const SortInfo* si = reinterpret_cast<const SortInfo*>(w.report + w.ml.off_info);
-  const uint32_t* fstart = reinterpret_cast<const uint32_t*>(w.report + w.ml.off_fstart);
-  const GridDev* grid = reinterpret_cast<const GridDev*>(w.report + w.ml.off_grid);
+  const Ctrl* ctrl = reinterpret_cast<const Ctrl*>(w.report.get() + w.ml.off_ctrl);
+  const FrameAcc* acc = reinterpret_cast<const FrameAcc*>(w.report.get() + w.ml.off_acc);
+  const SortInfo* si = reinterpret_cast<const SortInfo*>(w.report.get() + w.ml.off_info);
+  const uint32_t* fstart = reinterpret_cast<const uint32_t*>(w.report.get() + w.ml.off_fstart);
+  const GridDev* grid = reinterpret_cast<const GridDev*>(w.report.get() + w.ml.off_grid);
   cm_stats_t& s = h->stats;
   memset(&s, 0, sizeof(s));
   s.points_in = w.points_in;
@@ -816,19 +835,19 @@ int fetch_report(cm_handle_t h, Workspace& w, cudaEvent_t already_copied = nullp
   }
   const int last_ev = w.ran_voxel ? EV_CENT : EV_K1;
   float ms = 0.f;
-  if (cudaEventElapsedTime(&ms, w.ev[EV_START], w.ev[last_ev]) == cudaSuccess) s.gpu_ms = ms;
+  if (cudaEventElapsedTime(&ms, w.ev[EV_START].get(), w.ev[last_ev].get()) == cudaSuccess) s.gpu_ms = ms;
   else cudaGetLastError();  // a failed query must not surface later as the result of an unrelated launch
   for (auto& v : h->stage_ms) v = -1.f;
   h->stage_ms[EV_START] = s.gpu_ms;
   if (w.profiled) {
     float t;
-    if (cudaEventElapsedTime(&t, w.ev[EV_START], w.ev[EV_K1]) == cudaSuccess) h->stage_ms[EV_K1] = t;
+    if (cudaEventElapsedTime(&t, w.ev[EV_START].get(), w.ev[EV_K1].get()) == cudaSuccess) h->stage_ms[EV_K1] = t;
     if (w.ran_voxel) {
-      if (cudaEventElapsedTime(&t, w.ev[EV_K1], w.ev[EV_GRID]) == cudaSuccess) h->stage_ms[EV_GRID] = t;
-      if (cudaEventElapsedTime(&t, w.ev[EV_GRID], w.ev[EV_KEY]) == cudaSuccess) h->stage_ms[EV_KEY] = t;
-      if (cudaEventElapsedTime(&t, w.ev[EV_KEY], w.ev[EV_SORT]) == cudaSuccess) h->stage_ms[EV_SORT] = t;
-      if (w.timed_pass0 && cudaEventElapsedTime(&t, w.ev[EV_KEY], w.ev[EV_SORT0]) == cudaSuccess) h->stage_ms[EV_SORT0] = t;
-      if (cudaEventElapsedTime(&t, w.ev[EV_SORT], w.ev[EV_CENT]) == cudaSuccess) h->stage_ms[EV_CENT] = t;
+      if (cudaEventElapsedTime(&t, w.ev[EV_K1].get(), w.ev[EV_GRID].get()) == cudaSuccess) h->stage_ms[EV_GRID] = t;
+      if (cudaEventElapsedTime(&t, w.ev[EV_GRID].get(), w.ev[EV_KEY].get()) == cudaSuccess) h->stage_ms[EV_KEY] = t;
+      if (cudaEventElapsedTime(&t, w.ev[EV_KEY].get(), w.ev[EV_SORT].get()) == cudaSuccess) h->stage_ms[EV_SORT] = t;
+      if (w.timed_pass0 && cudaEventElapsedTime(&t, w.ev[EV_KEY].get(), w.ev[EV_SORT0].get()) == cudaSuccess) h->stage_ms[EV_SORT0] = t;
+      if (cudaEventElapsedTime(&t, w.ev[EV_SORT].get(), w.ev[EV_CENT].get()) == cudaSuccess) h->stage_ms[EV_CENT] = t;
     }
   }
   w.report_valid = true;
@@ -844,33 +863,36 @@ int ensure_batch_ws(cm_handle_t h) {
                   c.out_point_step);
 }
 
+// Sets up the slots and the sensor streams in locals and commits them only when all of it succeeded: a failure leaves the
+// handle as it was, and the slots never move once a run (h->last, a captured graph) can point into them.
 int ensure_host_path(cm_handle_t h) {
-  if (h->host_ready) return CM_OK;
+  if (!h->slots.empty()) return CM_OK;
   const cm_config_t& c = h->cfg;
   h->slot_stride = align_up((size_t)c.max_points_per_sensor * (size_t)c.max_point_step + 16, kAlign);
-  h->sensor_stream.resize(c.max_sensors);
-  for (auto& s : h->sensor_stream) CM_CUDA(h, cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-  h->slots.resize(c.frames_in_flight);
+  std::vector<Stream> streams(c.max_sensors);
+  for (auto& s : streams) CM_CUDA(h, create(s, cudaStreamCreateWithFlags, cudaStreamNonBlocking));
+  std::vector<Slot> slots(c.frames_in_flight);
   const uint64_t pts = (uint64_t)c.max_sensors * (uint64_t)c.max_points_per_sensor;
   if (pts > 0xFFFFFFF0ull) return fail(h, CM_E_CAPACITY, "max_sensors * max_points_per_sensor too large");
-  for (auto& sl : h->slots) {
+  for (auto& sl : slots) {
     int rc = ws_alloc(h, sl.ws, (uint32_t)pts, 1, (uint32_t)c.max_sensors, c.out_point_step);
     if (rc != CM_OK) return rc;
-    CM_CUDA(h, cudaMalloc(reinterpret_cast<void**>(&sl.raw_dev), h->slot_stride * c.max_sensors));
-    CM_CUDA(h, pinned_alloc(reinterpret_cast<void**>(&sl.raw_pinned), h->slot_stride * c.max_sensors, cudaHostAllocDefault));
+    CM_CUDA(h, dev_alloc(sl.raw_dev, h->slot_stride * c.max_sensors, 0));
+    CM_CUDA(h, pinned_alloc(sl.raw_pinned, h->slot_stride * c.max_sensors, cudaHostAllocDefault));
     sl.arena_bytes = 2 * h->slot_stride * c.max_sensors;
-    CM_CUDA(h, cudaMalloc(reinterpret_cast<void**>(&sl.arena_dev), sl.arena_bytes));
+    CM_CUDA(h, dev_alloc(sl.arena_dev, sl.arena_bytes, 0));
     sl.exp_cap = (uint32_t)pts;
     const size_t ecap = std::max<size_t>(sl.exp_cap, 1);
-    CM_CUDA(h, pinned_alloc(reinterpret_cast<void**>(&sl.exp_xyzi), ecap * (size_t)c.out_point_step, cudaHostAllocMapped));
-    CM_CUDA(h, pinned_alloc(reinterpret_cast<void**>(&sl.exp_count), ecap * sizeof(uint32_t), cudaHostAllocMapped));
-    CM_CUDA(h, pinned_alloc(reinterpret_cast<void**>(&sl.exp_idx), ecap * sizeof(unsigned long long), cudaHostAllocMapped));
+    CM_CUDA(h, pinned_alloc(sl.exp_xyzi, ecap * (size_t)c.out_point_step, cudaHostAllocMapped));
+    CM_CUDA(h, pinned_alloc(sl.exp_count, ecap * sizeof(uint32_t), cudaHostAllocMapped));
+    CM_CUDA(h, pinned_alloc(sl.exp_idx, ecap * sizeof(unsigned long long), cudaHostAllocMapped));
     sl.sensor.resize(c.max_sensors);
-    for (auto& ss : sl.sensor) CM_CUDA(h, cudaEventCreateWithFlags(&ss.copied, cudaEventDisableTiming));
-    CM_CUDA(h, cudaStreamCreateWithFlags(&sl.stream, cudaStreamNonBlocking));
-    CM_CUDA(h, cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
+    for (auto& ss : sl.sensor) CM_CUDA(h, create(ss.copied, cudaEventCreateWithFlags, cudaEventDisableTiming));
+    CM_CUDA(h, create(sl.stream, cudaStreamCreateWithFlags, cudaStreamNonBlocking));
+    CM_CUDA(h, create(sl.done, cudaEventCreateWithFlags, cudaEventDisableTiming));
   }
-  h->host_ready = true;
+  h->sensor_stream = std::move(streams);
+  h->slots = std::move(slots);
   return CM_OK;
 }
 
@@ -893,19 +915,19 @@ int submit_impl(cm_handle_t h, int sensor, const void* data, int64_t n_points, c
   // arrives while the sensor's previous one is still waiting to be fused is dropped
   if (h->submit_policy == CM_SUBMIT_FIRST_WINS && ss.submitted) return CM_OK;
   const size_t bytes = (size_t)n_points * (size_t)layout->point_step;
-  uint8_t* dst = sl.raw_dev + (size_t)sensor * h->slot_stride;
-  cudaStream_t st = h->sensor_stream[sensor];
+  uint8_t* dst = sl.raw_dev.get() + (size_t)sensor * h->slot_stride;
+  cudaStream_t st = h->sensor_stream[sensor].get();
   if (bytes) {
     if (pinned_src) {
       CM_CUDA(h, cudaMemcpyAsync(dst, data, bytes, cudaMemcpyHostToDevice, st));
     } else {
-      uint8_t* stg = sl.raw_pinned + (size_t)sensor * h->slot_stride;
-      CM_CUDA(h, cudaEventSynchronize(ss.copied));  // the previous copy out of this staging buffer is done
+      uint8_t* stg = sl.raw_pinned.get() + (size_t)sensor * h->slot_stride;
+      CM_CUDA(h, cudaEventSynchronize(ss.copied.get()));  // the previous copy out of this staging buffer is done
       memcpy(stg, data, bytes);
       CM_CUDA(h, cudaMemcpyAsync(dst, stg, bytes, cudaMemcpyHostToDevice, st));
     }
   }
-  CM_CUDA(h, cudaEventRecord(ss.copied, st));
+  CM_CUDA(h, cudaEventRecord(ss.copied.get(), st));
   ss.submitted = true; ss.n_points = n_points; ss.layout = *layout; ss.stamp = stamp; ss.dev = dst;
   return CM_OK;
 }
@@ -916,15 +938,15 @@ int submit_impl(cm_handle_t h, int sensor, const void* data, int64_t n_points, c
 cudaError_t enqueue_frame_export(cm_handle_t h, Slot& sl) {
   Workspace& w = sl.ws;
   VoxelParams vp;
-  fill_voxel_params(h, w, vp, w.surv_xyzi, 1, 0);
+  fill_voxel_params(h, w, vp, w.surv_xyzi.get(), 1, 0);
   void *dx = nullptr, *dc = nullptr, *di = nullptr;
-  cudaError_t e = cudaHostGetDevicePointer(&dx, sl.exp_xyzi, 0);
-  if (e == cudaSuccess) e = cudaHostGetDevicePointer(&dc, sl.exp_count, 0);
-  if (e == cudaSuccess) e = cudaHostGetDevicePointer(&di, sl.exp_idx, 0);
-  if (e == cudaSuccess) e = launch_export_voxels(vp, dx, static_cast<uint32_t*>(dc), static_cast<unsigned long long*>(di), sl.exp_cap, sl.stream);
+  cudaError_t e = cudaHostGetDevicePointer(&dx, sl.exp_xyzi.get(), 0);
+  if (e == cudaSuccess) e = cudaHostGetDevicePointer(&dc, sl.exp_count.get(), 0);
+  if (e == cudaSuccess) e = cudaHostGetDevicePointer(&di, sl.exp_idx.get(), 0);
+  if (e == cudaSuccess) e = launch_export_voxels(vp, dx, static_cast<uint32_t*>(dc), static_cast<unsigned long long*>(di), sl.exp_cap, sl.stream.get());
   if (e != cudaSuccess) return e;
   ++w.launches;
-  return cudaMemcpyAsync(w.report, w.meta, w.ml.total, cudaMemcpyDeviceToHost, sl.stream);
+  return cudaMemcpyAsync(w.report.get(), w.meta.get(), w.ml.total, cudaMemcpyDeviceToHost, sl.stream.get());
 }
 
 int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
@@ -932,6 +954,7 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
   if (rc != CM_OK) return rc;
   Slot& sl = h->slots[h->fill];
   if (sl.busy) return fail(h, CM_E_CAPACITY, "frame slot still in flight");
+  cudaStream_t st = sl.stream.get();
   std::vector<cm_segment_t> segs;
   uint64_t used = 0, stamp = 0;
   for (int s = 0; s < h->cfg.max_sensors; ++s) {
@@ -944,7 +967,7 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
     segs.push_back(g);
     used |= 1ull << s;
     stamp = std::max(stamp, ss.stamp);  // operator+= keeps the newest stamp
-    CM_CUDA(h, cudaStreamWaitEvent(sl.stream, ss.copied, 0));
+    CM_CUDA(h, cudaStreamWaitEvent(st, ss.copied.get(), 0));
   }
   if (segs.empty()) return fail(h, CM_E_NOT_READY, "no submitted cloud for any sensor in the mask");
   // ---- replay / capture / plain enqueue ---------------------------------------------------------------------------------
@@ -963,34 +986,35 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
   bool launched = false;
   if (graphable && sl.graph && sl.graph_key == key) {
     Workspace& w = sl.ws;  // same configuration as the captured frame: every host-side field of the run is unchanged
-    w.has_run = true; w.report_valid = false; w.dense_valid = false; w.stream = sl.stream;
+    w.has_run = true; w.report_valid = false; w.dense_valid = false; w.stream = st;
     h->last = &w;
-    CM_CUDA(h, cudaEventRecord(w.ev[EV_START], sl.stream));
-    CM_CUDA(h, cudaGraphLaunch(sl.graph, sl.stream));
-    CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT], sl.stream));
+    CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
+    CM_CUDA(h, cudaGraphLaunch(sl.graph.get(), st));
+    CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
     launched = true;
   } else if (graphable && sl.graph_seen == key) {
     // second frame with this configuration (its segment table is already on the device): capture, instantiate, launch
-    if (sl.graph) { cudaGraphExecDestroy(sl.graph); sl.graph = nullptr; sl.graph_key.clear(); }
+    sl.graph.reset(); sl.graph_key.clear();
     cudaGraph_t g = nullptr;
-    if (cudaStreamBeginCapture(sl.stream, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
+    if (cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
       sl.ws.capturing = true;
-      rc = run_pipeline(h, sl.ws, segs.data(), (int)segs.size(), sl.stream, true);
+      rc = run_pipeline(h, sl.ws, segs.data(), (int)segs.size(), st, true);
       sl.ws.capturing = false;
       cudaError_t ce = cudaSuccess;
       if (rc == CM_OK) ce = enqueue_frame_export(h, sl);
-      const cudaError_t ee = cudaStreamEndCapture(sl.stream, &g);
+      const cudaError_t ee = cudaStreamEndCapture(st, &g);
+      cudaGraphExec_t exec = nullptr;
       if (rc == CM_OK && ce == cudaSuccess && ee == cudaSuccess && g &&
-          cudaGraphInstantiate(&sl.graph, g, 0) == cudaSuccess) {
+          cudaGraphInstantiate(&exec, g, 0) == cudaSuccess) {
+        sl.graph.reset(exec);
         sl.graph_key = key;
         cudaGraphDestroy(g);
-        CM_CUDA(h, cudaEventRecord(sl.ws.ev[EV_START], sl.stream));
-        CM_CUDA(h, cudaGraphLaunch(sl.graph, sl.stream));
-        CM_CUDA(h, cudaEventRecord(sl.ws.ev[EV_CENT], sl.stream));
+        CM_CUDA(h, cudaEventRecord(sl.ws.ev[EV_START].get(), st));
+        CM_CUDA(h, cudaGraphLaunch(sl.graph.get(), st));
+        CM_CUDA(h, cudaEventRecord(sl.ws.ev[EV_CENT].get(), st));
         launched = true;
       } else {
         if (g) cudaGraphDestroy(g);
-        sl.graph = nullptr;
         h->use_graph = false;  // not capturable here: stay on the plain path
         cudaGetLastError();
       }
@@ -1000,13 +1024,13 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
     }
   }
   if (!launched) {
-    if (sl.graph && sl.graph_key != key) { cudaGraphExecDestroy(sl.graph); sl.graph = nullptr; sl.graph_key.clear(); }
-    rc = run_pipeline(h, sl.ws, segs.data(), (int)segs.size(), sl.stream, true);
+    if (sl.graph && sl.graph_key != key) { sl.graph.reset(); sl.graph_key.clear(); }
+    rc = run_pipeline(h, sl.ws, segs.data(), (int)segs.size(), st, true);
     if (rc != CM_OK) return rc;
     CM_CUDA(h, enqueue_frame_export(h, sl));
     sl.graph_seen = key;
   }
-  CM_CUDA(h, cudaEventRecord(sl.done, sl.stream));
+  CM_CUDA(h, cudaEventRecord(sl.done.get(), st));
   // Every submission of this slot ends here: merged clouds are consumed; a cloud submitted for a sensor outside the mask is
   // discarded (it would otherwise resurface, stale, when the slot comes round again frames_in_flight frames later).
   for (int s = 0; s < h->cfg.max_sensors; ++s) sl.sensor[s].submitted = false;
@@ -1024,7 +1048,7 @@ int wait_impl(cm_handle_t h, int64_t ticket, cm_frame_out_t* out, uint64_t* used
   if (!sl) return fail(h, CM_E_INVALID, "unknown ticket %lld", (long long)ticket);
   Workspace& w = sl->ws;
   h->last = &w;
-  int rc = fetch_report(h, w, sl->done);
+  int rc = fetch_report(h, w, sl->done.get());
   sl->busy = false;
   if (rc != CM_OK) return rc;
   if (used_mask) *used_mask = sl->used_mask;
@@ -1040,7 +1064,7 @@ int wait_impl(cm_handle_t h, int64_t ticket, cm_frame_out_t* out, uint64_t* used
     return fail(h, CM_E_CAPACITY, "voxel_capacity %lld < %lld voxels", (long long)out->voxel_capacity, (long long)out->n_voxels);
   if ((out->survivor_xyzi || out->survivor_src) && out->n_survivors > out->survivor_capacity)
     return fail(h, CM_E_CAPACITY, "survivor_capacity %lld < %lld survivors", (long long)out->survivor_capacity, (long long)out->n_survivors);
-  cudaStream_t st = sl->stream;
+  cudaStream_t st = sl->stream.get();
   const size_t nv = (size_t)out->n_voxels, ns = (size_t)out->n_survivors;
   if ((out->survivor_xyzi || out->survivor_src || pcl_refuses) && ns) {
     rc = materialize_dense(h, w);
@@ -1049,11 +1073,11 @@ int wait_impl(cm_handle_t h, int64_t ticket, cm_frame_out_t* out, uint64_t* used
   if (pcl_refuses) {
     if (out->voxel_xyzi && nv) {
       if (w.out_step == 16) {
-        CM_CUDA(h, cudaMemcpyAsync(out->voxel_xyzi, w.dense_xyzi, nv * 16, cudaMemcpyDeviceToHost, st));
+        CM_CUDA(h, cudaMemcpyAsync(out->voxel_xyzi, w.dense_xyzi.get(), nv * 16, cudaMemcpyDeviceToHost, st));
       } else {
         // expand packed survivors into pcl::PointXYZI records on the host side of the copy
         std::vector<float> tmp(nv * 4);
-        CM_CUDA(h, cudaMemcpyAsync(tmp.data(), w.dense_xyzi, nv * 16, cudaMemcpyDeviceToHost, st));
+        CM_CUDA(h, cudaMemcpyAsync(tmp.data(), w.dense_xyzi.get(), nv * 16, cudaMemcpyDeviceToHost, st));
         CM_CUDA(h, cudaStreamSynchronize(st));
         float* o = static_cast<float*>(out->voxel_xyzi);
         for (size_t i = 0; i < nv; ++i) {
@@ -1066,17 +1090,17 @@ int wait_impl(cm_handle_t h, int64_t ticket, cm_frame_out_t* out, uint64_t* used
     if (out->voxel_idx) for (size_t i = 0; i < nv; ++i) out->voxel_idx[i] = 0;
   } else if (nv <= (size_t)sl->exp_cap) {
     // the frame's own stream already wrote the voxels to the slot's page-locked mirrors (k_export_voxels): plain memcpy
-    if (out->voxel_xyzi && nv) memcpy(out->voxel_xyzi, sl->exp_xyzi, nv * (size_t)w.out_step);
-    if (out->voxel_count && nv) memcpy(out->voxel_count, sl->exp_count, nv * 4);
-    if (out->voxel_idx && nv) memcpy(out->voxel_idx, sl->exp_idx, nv * 8);
+    if (out->voxel_xyzi && nv) memcpy(out->voxel_xyzi, sl->exp_xyzi.get(), nv * (size_t)w.out_step);
+    if (out->voxel_count && nv) memcpy(out->voxel_count, sl->exp_count.get(), nv * 4);
+    if (out->voxel_idx && nv) memcpy(out->voxel_idx, sl->exp_idx.get(), nv * 8);
     if (!((out->survivor_xyzi || out->survivor_src) && ns)) return CM_OK;
   } else {
-    if (out->voxel_xyzi && nv) CM_CUDA(h, cudaMemcpyAsync(out->voxel_xyzi, w.out_xyzi, nv * (size_t)w.out_step, cudaMemcpyDeviceToHost, st));
-    if (out->voxel_count && nv) CM_CUDA(h, cudaMemcpyAsync(out->voxel_count, w.out_count, nv * 4, cudaMemcpyDeviceToHost, st));
-    if (out->voxel_idx && nv) CM_CUDA(h, cudaMemcpyAsync(out->voxel_idx, w.out_idx, nv * 8, cudaMemcpyDeviceToHost, st));
+    if (out->voxel_xyzi && nv) CM_CUDA(h, cudaMemcpyAsync(out->voxel_xyzi, w.out_xyzi.get(), nv * (size_t)w.out_step, cudaMemcpyDeviceToHost, st));
+    if (out->voxel_count && nv) CM_CUDA(h, cudaMemcpyAsync(out->voxel_count, w.out_count.get(), nv * 4, cudaMemcpyDeviceToHost, st));
+    if (out->voxel_idx && nv) CM_CUDA(h, cudaMemcpyAsync(out->voxel_idx, w.out_idx.get(), nv * 8, cudaMemcpyDeviceToHost, st));
   }
-  if (out->survivor_xyzi && ns) CM_CUDA(h, cudaMemcpyAsync(out->survivor_xyzi, w.dense_xyzi, ns * 16, cudaMemcpyDeviceToHost, st));
-  if (out->survivor_src && ns) CM_CUDA(h, cudaMemcpyAsync(out->survivor_src, w.dense_src, ns * 4, cudaMemcpyDeviceToHost, st));
+  if (out->survivor_xyzi && ns) CM_CUDA(h, cudaMemcpyAsync(out->survivor_xyzi, w.dense_xyzi.get(), ns * 16, cudaMemcpyDeviceToHost, st));
+  if (out->survivor_src && ns) CM_CUDA(h, cudaMemcpyAsync(out->survivor_src, w.dense_src.get(), ns * 4, cudaMemcpyDeviceToHost, st));
   CM_CUDA(h, cudaStreamSynchronize(st));
   return CM_OK;
 }
@@ -1202,35 +1226,6 @@ int cm_destroy(cm_handle_t h) {
   if (!h) return CM_E_INVALID;
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
-  ws_free(h->batch);
-  for (auto& sl : h->slots) {
-    ws_free(sl.ws);
-    cudaFree(sl.raw_dev); cudaFreeHost(sl.raw_pinned); cudaFree(sl.arena_dev);
-    if (sl.exp_xyzi) cudaFreeHost(sl.exp_xyzi);
-    if (sl.exp_count) cudaFreeHost(sl.exp_count);
-    if (sl.exp_idx) cudaFreeHost(sl.exp_idx);
-    for (auto& ss : sl.sensor) if (ss.copied) cudaEventDestroy(ss.copied);
-    if (sl.graph) cudaGraphExecDestroy(sl.graph);
-    if (sl.stream) cudaStreamDestroy(sl.stream);
-    if (sl.done) cudaEventDestroy(sl.done);
-  }
-  for (auto& s : h->sensor_stream) if (s) cudaStreamDestroy(s);
-  {
-    auto& z = h->zw;
-    cudaFree(z.mask); cudaFree(z.tile_count); cudaFree(z.tile_offset); cudaFree(z.zone_begin); cudaFree(z.overflow);
-    cudaFree(z.zone_total);
-    cudaFree(z.out_xyzi); cudaFree(z.out_src); cudaFree(z.in_stage);
-    if (z.report) cudaFreeHost(z.report);
-    cudaFree(h->ror_table);
-    cudaFree(h->prz.low); cudaFree(h->prz.high); cudaFree(h->prz.rest); cudaFree(h->prz.planes);
-    cudaFree(h->prz.no_ground); cudaFree(h->prz.ground); cudaFree(h->prz.in_stage);
-    auto& q = h->pw;
-    cudaFree(q.samples_dev); cudaFree(q.counts_dev); cudaFree(q.models_dev); cudaFree(q.acc_dev);
-    if (q.samples_pin) cudaFreeHost(q.samples_pin);
-    if (q.counts_pin) cudaFreeHost(q.counts_pin);
-    if (q.models_pin) cudaFreeHost(q.models_pin);
-    if (q.acc_pin) cudaFreeHost(q.acc_pin);
-  }
   delete h;
   return CM_OK;
 }
@@ -1373,21 +1368,21 @@ int cm_submit_clouds_pinned(cm_handle_t h, int count, const int* sensors, const 
     }
     const size_t need = align_up(run_bytes, kAlign);
     if (b - a >= 2 && sl.arena_used + need > sl.arena_bytes) b = a + 1;  // arena full: this cloud alone, into its own region
-    cudaStream_t st = h->sensor_stream[sensors[i]];
+    cudaStream_t st = h->sensor_stream[sensors[i]].get();
     uint8_t* dst;
     if (b - a >= 2) {
-      dst = sl.arena_dev + sl.arena_used;
+      dst = sl.arena_dev.get() + sl.arena_used;
       sl.arena_used += need;
     } else {
       run_bytes = (size_t)n_points[i] * (size_t)layouts[i].point_step;
-      dst = sl.raw_dev + (size_t)sensors[i] * h->slot_stride;
+      dst = sl.raw_dev.get() + (size_t)sensors[i] * h->slot_stride;
     }
     if (run_bytes) CM_CUDA(h, cudaMemcpyAsync(dst, data[i], run_bytes, cudaMemcpyHostToDevice, st));
     size_t off = 0;
     for (size_t k = a; k < b; ++k) {
       const int c = pick[k];
       SensorState& ss = sl.sensor[sensors[c]];
-      CM_CUDA(h, cudaEventRecord(ss.copied, st));
+      CM_CUDA(h, cudaEventRecord(ss.copied.get(), st));
       ss.submitted = true; ss.n_points = n_points[c]; ss.layout = layouts[c]; ss.stamp = stamps ? stamps[c] : 0;
       ss.dev = dst + off;
       off += (size_t)n_points[c] * (size_t)layouts[c].point_step;
@@ -1430,9 +1425,9 @@ int cm_wait_frame_view(cm_handle_t h, int64_t ticket, cm_frame_view_t* view) {
   if (h->overflow_mode == 1 && fi.pcl_overflow)
     return fail(h, CM_E_INVALID, "PCL would refuse this frame (leaf too small): its result is the merged cloud, use cm_wait_frame");
   if ((uint64_t)view->n_voxels > sl->exp_cap) return fail(h, CM_E_CAPACITY, "more voxels than the result mirror holds");
-  view->voxel_xyzi = sl->exp_xyzi;
-  view->voxel_count = sl->exp_count;
-  view->voxel_idx = reinterpret_cast<const uint64_t*>(sl->exp_idx);
+  view->voxel_xyzi = sl->exp_xyzi.get();
+  view->voxel_count = sl->exp_count.get();
+  view->voxel_idx = reinterpret_cast<const uint64_t*>(sl->exp_idx.get());
   return CM_OK;
 }
 
@@ -1448,7 +1443,10 @@ int cm_merge_frame(cm_handle_t h, uint64_t sensor_mask, cm_frame_out_t* out, uin
 
 int cm_host_alloc(void** p, size_t bytes) {
   if (!p) return CM_E_INVALID;
-  return pinned_alloc(p, bytes, cudaHostAllocDefault) == cudaSuccess ? CM_OK : CM_E_CUDA;
+  HostPtr<void> mem;
+  const cudaError_t e = pinned_alloc(mem, bytes, cudaHostAllocDefault);
+  *p = mem.release();  // the caller's from here on (cm_host_free)
+  return e == cudaSuccess ? CM_OK : CM_E_CUDA;
 }
 int cm_host_free(void* p) { return cudaFreeHost(p) == cudaSuccess ? CM_OK : CM_E_CUDA; }
 
@@ -1484,8 +1482,8 @@ int voxelgrid_run(cm_handle_t h, const float4* pts, int64_t n_points, cudaStream
   w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
   w.voxel_pts = pts; w.fused_keys = false;
   h->last = &w;
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_START], st));
-  CM_CUDA(h, cudaMemsetAsync(w.meta, 0, w.ml.zero_bytes, st));
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
+  CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
   VoxelParams vp;
   fill_voxel_params(h, w, vp, w.voxel_pts, 1, (uint32_t)n_points);
   CM_CUDA(h, launch_minmax(w.voxel_pts, (uint32_t)n_points, vp.ctrl, vp.acc, const_cast<uint32_t*>(vp.frame_surv_start), st));
@@ -1497,7 +1495,7 @@ int voxelgrid_run(cm_handle_t h, const float4* pts, int64_t n_points, cudaStream
     CM_CUDA(h, launch_seed_bounds(vp.acc, h->bounds_min, h->bounds_max, st));
     ++w.launches;
   }
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_K1], st));
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
   return run_voxel(h, w, vp, st, false, true, known_idx_bits);
 }
 }  // namespace
@@ -1549,33 +1547,25 @@ int cm_set_zones(cm_handle_t h, int n_zones, const cm_zone_t* zones) {
 }
 
 namespace {
-void zone_ws_free(cm_handle_s::ZoneWs& z) {
-  cudaFree(z.mask); cudaFree(z.tile_count); cudaFree(z.tile_offset); cudaFree(z.zone_begin); cudaFree(z.overflow);
-  cudaFree(z.zone_total);
-  cudaFree(z.out_xyzi); cudaFree(z.out_src); cudaFree(z.in_stage);
-  if (z.report) cudaFreeHost(z.report);
-  z = cm_handle_s::ZoneWs();
-}
-
 // capacity: the input may hold up to `points`; the zones together up to twice that (boundary duplicates are rare, but
 // zones are free to overlap)
 int zone_ws_ensure(cm_handle_t h, size_t points) {
   cm_handle_s::ZoneWs& z = h->zw;
   const size_t want = std::max<size_t>({points, (size_t)h->cfg.max_batch_points, (size_t)1});
   if (z.cap_points >= want) return CM_OK;
-  zone_ws_free(z);
+  z = cm_handle_s::ZoneWs();  // the old buffers go before the larger ones are allocated
   const size_t tiles = want / zone_tile_points() + 2;
-  CM_CUDA(h, dev_alloc(&z.mask, want));
-  CM_CUDA(h, dev_alloc(&z.tile_count, tiles * CM_MAX_ZONES));
-  CM_CUDA(h, dev_alloc(&z.tile_offset, tiles * CM_MAX_ZONES));
-  CM_CUDA(h, dev_alloc(&z.zone_begin, (size_t)CM_MAX_ZONES + 2));
-  CM_CUDA(h, dev_alloc(&z.overflow, (size_t)1));
-  CM_CUDA(h, dev_alloc(&z.zone_total, (size_t)CM_MAX_ZONES + 2));
-  CM_CUDA(h, cudaMemset(z.zone_total, 0, sizeof(uint32_t) * (CM_MAX_ZONES + 2)));
+  CM_CUDA(h, dev_alloc(z.mask, want));
+  CM_CUDA(h, dev_alloc(z.tile_count, tiles * CM_MAX_ZONES));
+  CM_CUDA(h, dev_alloc(z.tile_offset, tiles * CM_MAX_ZONES));
+  CM_CUDA(h, dev_alloc(z.zone_begin, (size_t)CM_MAX_ZONES + 2));
+  CM_CUDA(h, dev_alloc(z.overflow, (size_t)1));
+  CM_CUDA(h, dev_alloc(z.zone_total, (size_t)CM_MAX_ZONES + 2));
+  CM_CUDA(h, cudaMemset(z.zone_total.get(), 0, sizeof(uint32_t) * (CM_MAX_ZONES + 2)));
   z.cap_out = 2 * want;
-  CM_CUDA(h, dev_alloc(&z.out_xyzi, z.cap_out));
-  CM_CUDA(h, dev_alloc(&z.out_src, z.cap_out));
-  CM_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&z.report), sizeof(uint32_t) * (CM_MAX_ZONES + 2)));
+  CM_CUDA(h, dev_alloc(z.out_xyzi, z.cap_out));
+  CM_CUDA(h, dev_alloc(z.out_src, z.cap_out));
+  CM_CUDA(h, pinned_alloc(z.report, sizeof(uint32_t) * (CM_MAX_ZONES + 2), cudaHostAllocDefault));
   CM_CUDA(h, cudaDeviceSynchronize());  // the clear above ran on the default stream (see ws_alloc)
   z.cap_points = want;
   return CM_OK;
@@ -1587,7 +1577,7 @@ bool in_zone_outputs(cm_handle_t h, const void* p, int64_t n_points) {
   const cm_handle_s::ZoneWs& z = h->zw;
   if (!p || !z.out_xyzi || n_points <= 0) return false;
   const uintptr_t a = reinterpret_cast<uintptr_t>(p), b = a + (uintptr_t)n_points * 16u;
-  const uintptr_t lo = reinterpret_cast<uintptr_t>(z.out_xyzi), hi = lo + (uintptr_t)z.cap_out * 16u;
+  const uintptr_t lo = reinterpret_cast<uintptr_t>(z.out_xyzi.get()), hi = lo + (uintptr_t)z.cap_out * 16u;
   return a < hi && b > lo;
 }
 
@@ -1604,10 +1594,10 @@ ZoneParams zone_params(cm_handle_t h, const float4* pts, int64_t n_points, bool 
     zp.zones.n_zones = given_zones;
   }
   z.n_zones_run = zp.zones.n_zones;
-  zp.mask = z.mask; zp.tile_count = z.tile_count; zp.tile_offset = z.tile_offset; zp.zone_begin = z.zone_begin;
-  zp.zone_total = z.zone_total; zp.scan_ticket = z.zone_total + CM_MAX_ZONES;
-  zp.overflow = z.overflow; zp.out_capacity = (uint32_t)std::min<size_t>(z.cap_out, 0xFFFFFFF0u);
-  zp.out_xyzi = z.out_xyzi; zp.out_src = z.out_src;
+  zp.mask = z.mask.get(); zp.tile_count = z.tile_count.get(); zp.tile_offset = z.tile_offset.get(); zp.zone_begin = z.zone_begin.get();
+  zp.zone_total = z.zone_total.get(); zp.scan_ticket = z.zone_total.get() + CM_MAX_ZONES;
+  zp.overflow = z.overflow.get(); zp.out_capacity = (uint32_t)std::min<size_t>(z.cap_out, 0xFFFFFFF0u);
+  zp.out_xyzi = z.out_xyzi.get(); zp.out_src = z.out_src.get();
   for (int i = 0; i < CM_MAX_ZONES; ++i) zp.zone_ptr[i] = nullptr;
   zp.zone_remote_base = nullptr;
   zp.giant_plan = nullptr; zp.giant_invalid_part = 0;
@@ -1626,10 +1616,10 @@ int zone_run(cm_handle_t h, const float4* pts, int64_t n_points, cudaStream_t st
   if (rc != CM_OK) return rc;
   ZoneParams zp = zone_params(h, pts, n_points, mask_given, given_zones);
   if (giant) { zp.mask_given = 0; zp.giant_plan = giant; zp.giant_invalid_part = giant_invalid_part; }
-  CM_CUDA(h, cudaMemsetAsync(z.overflow, 0, sizeof(uint32_t), st));
+  CM_CUDA(h, cudaMemsetAsync(z.overflow.get(), 0, sizeof(uint32_t), st));
   CM_CUDA(h, launch_zone_split(zp, st));
-  CM_CUDA(h, cudaMemcpyAsync(z.report, z.zone_begin, sizeof(uint32_t) * (CM_MAX_ZONES + 1), cudaMemcpyDeviceToHost, st));
-  CM_CUDA(h, cudaMemcpyAsync(z.report + CM_MAX_ZONES + 1, z.overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  CM_CUDA(h, cudaMemcpyAsync(z.report.get(), z.zone_begin.get(), sizeof(uint32_t) * (CM_MAX_ZONES + 1), cudaMemcpyDeviceToHost, st));
+  CM_CUDA(h, cudaMemcpyAsync(z.report.get() + CM_MAX_ZONES + 1, z.overflow.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
   z.stream = st; z.ran = true; z.launches = zp.n_tiles ? CM_ZONE_LAUNCHES : 1; z.last = zp;
   return CM_OK;
 }
@@ -1652,7 +1642,7 @@ int cm_dev_zone_split(cm_handle_t h, const float* xyzi_dev, int64_t n_points, vo
   rc = materialize_dense(h, w);
   if (rc != CM_OK) return rc;
   CM_CUDA(h, cudaStreamSynchronize(w.stream));
-  return zone_run(h, w.dense_xyzi, h->stats.survivors, st);
+  return zone_run(h, w.dense_xyzi.get(), h->stats.survivors, st);
 }
 
 namespace {
@@ -1669,29 +1659,29 @@ int zone_out_locked(cm_handle_t h, cm_zone_out_t* out) {
   if (!z.ran) return fail(h, CM_E_INVALID, "no zone split has run on this handle");
   CM_CUDA(h, cudaSetDevice(h->device));
   CM_CUDA(h, cudaStreamSynchronize(z.stream));
-  if (z.report[CM_MAX_ZONES + 1] && (size_t)z.report[CM_MAX_ZONES + 1] <= 0xFFFFFFF0u) {
+  uint32_t* report = z.report.get();
+  if (report[CM_MAX_ZONES + 1] && (size_t)report[CM_MAX_ZONES + 1] <= 0xFFFFFFF0u) {
     // Overlapping zones hold more points together than the output arrays were sized for (twice the input): grow them to
     // the size the scan found and repeat the scatter. The input cloud must still be where it was.
-    const size_t need = z.report[CM_MAX_ZONES + 1];
-    cudaFree(z.out_xyzi); cudaFree(z.out_src);
-    z.out_xyzi = nullptr; z.out_src = nullptr; z.cap_out = 0;
-    CM_CUDA(h, dev_alloc(&z.out_xyzi, need));
-    CM_CUDA(h, dev_alloc(&z.out_src, need));
+    const size_t need = report[CM_MAX_ZONES + 1];
+    z.out_xyzi.reset(); z.out_src.reset(); z.cap_out = 0;  // the old outputs go before the larger ones are allocated
+    CM_CUDA(h, dev_alloc(z.out_xyzi, need));
+    CM_CUDA(h, dev_alloc(z.out_src, need));
     z.cap_out = need;
-    z.last.out_xyzi = z.out_xyzi; z.last.out_src = z.out_src; z.last.out_capacity = (uint32_t)need;
-    CM_CUDA(h, cudaMemsetAsync(z.overflow, 0, sizeof(uint32_t), z.stream));
+    z.last.out_xyzi = z.out_xyzi.get(); z.last.out_src = z.out_src.get(); z.last.out_capacity = (uint32_t)need;
+    CM_CUDA(h, cudaMemsetAsync(z.overflow.get(), 0, sizeof(uint32_t), z.stream));
     CM_CUDA(h, launch_zone_scatter(z.last, z.stream));
     CM_CUDA(h, cudaStreamSynchronize(z.stream));
-    z.report[CM_MAX_ZONES + 1] = 0;
+    report[CM_MAX_ZONES + 1] = 0;
     ++z.launches;
   }
   memset(out, 0, sizeof(*out));
   out->n_zones = z.n_zones_run;
-  for (int k = 0; k <= z.n_zones_run; ++k) out->begin[k] = z.report[k];
-  out->xyzi = reinterpret_cast<const float*>(z.out_xyzi);
-  out->src = z.out_src;
-  if (z.report[CM_MAX_ZONES + 1])
-    return fail(h, CM_E_CAPACITY, "the zones hold %u points together, capacity is %zu", z.report[CM_MAX_ZONES + 1], z.cap_out);
+  for (int k = 0; k <= z.n_zones_run; ++k) out->begin[k] = report[k];
+  out->xyzi = reinterpret_cast<const float*>(z.out_xyzi.get());
+  out->src = z.out_src.get();
+  if (report[CM_MAX_ZONES + 1])
+    return fail(h, CM_E_CAPACITY, "the zones hold %u points together, capacity is %zu", report[CM_MAX_ZONES + 1], z.cap_out);
   return CM_OK;
 }
 }  // namespace
@@ -1706,9 +1696,10 @@ int cm_zone_split(cm_handle_t h, const float* xyzi_host, int64_t n_points, float
     int rc = zone_ws_ensure(h, (size_t)n_points);
     if (rc != CM_OK) return rc;
     cm_handle_s::ZoneWs& z = h->zw;
-    if (!z.in_stage) CM_CUDA(h, dev_alloc(&z.in_stage, z.cap_points));
-    CM_CUDA(h, cudaMemcpyAsync(z.in_stage, xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-    rc = zone_run(h, z.in_stage, n_points, nullptr);
+    if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
+    CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
+    rc = zone_run(h, z.in_stage.get(), n_points, nullptr);
+
     if (rc != CM_OK) return rc;
   }
   int rc = cm_get_zone_out(h, &zo);
@@ -1752,11 +1743,11 @@ int cm_dev_bounds(cm_handle_t h, const float* xyzi_dev, int64_t n_points, float*
   if (rc != CM_OK) return rc;
   Workspace& w = h->batch;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CM_CUDA(h, cudaMemsetAsync(w.meta, 0, w.ml.zero_bytes, st));
-  Ctrl* ctrl = reinterpret_cast<Ctrl*>(w.meta + w.ml.off_ctrl);
-  FrameAcc* acc = reinterpret_cast<FrameAcc*>(w.meta + w.ml.off_acc);
+  CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
+  Ctrl* ctrl = reinterpret_cast<Ctrl*>(w.meta.get() + w.ml.off_ctrl);
+  FrameAcc* acc = reinterpret_cast<FrameAcc*>(w.meta.get() + w.ml.off_acc);
   CM_CUDA(h, launch_minmax(reinterpret_cast<const float4*>(xyzi_dev), (uint32_t)n_points, ctrl, acc,
-                           reinterpret_cast<uint32_t*>(w.meta + w.ml.off_fstart), st));
+                           reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_fstart), st));
   FrameAcc a;
   CM_CUDA(h, cudaMemcpyAsync(&a, acc, sizeof(a), cudaMemcpyDeviceToHost, st));
   CM_CUDA(h, cudaStreamSynchronize(st));
@@ -1807,7 +1798,7 @@ int cm_dev_route_by_key(cm_handle_t h, const float* xyzi_dev, int64_t n_points, 
   sp.n_parts = n_parts; sp.invalid_part = (uint32_t)invalid_part;
   for (int k = 0; k + 1 < n_parts; ++k) sp.splitter[k] = splitters[k];
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CM_CUDA(h, launch_route_mask(reinterpret_cast<const float4*>(xyzi_dev), (uint32_t)n_points, g, sp, h->zw.mask, st));
+  CM_CUDA(h, launch_route_mask(reinterpret_cast<const float4*>(xyzi_dev), (uint32_t)n_points, g, sp, h->zw.mask.get(), st));
   return zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st, true, n_parts);
 }
 
@@ -1847,8 +1838,8 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
   w.voxel_pts = pts; w.fused_keys = false;
   h->last = &w;
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_START], st));
-  CM_CUDA(h, cudaMemsetAsync(w.meta, 0, w.ml.zero_bytes, st));
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
+  CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
   VoxelParams vp;
   fill_voxel_params(h, w, vp, pts, (uint32_t)n_clouds, (uint32_t)n_points);
   for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = 1.0f / cell;
@@ -1865,7 +1856,7 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
     for (int c = 0; c <= n_clouds; ++c) starts[c] = (uint32_t)begin[c];
     CM_CUDA(h, cudaMemcpyAsync(fss, starts, sizeof(uint32_t) * (size_t)(n_clouds + 1), cudaMemcpyHostToDevice, st));
   }
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_K1], st));
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
   rc = run_voxel(h, w, vp, st, false, false);  // keys + sort only
   if (rc != CM_OK) return rc;
   vp.key_bytes = w.key_bytes;
@@ -1873,7 +1864,7 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   rp.r2 = (float)(radius * radius);
   rp.min_pts = (uint32_t)min_neighbors;
   rp.negative = negative ? 1u : 0u;
-  rp.mask = h->zw.mask;
+  rp.mask = h->zw.mask.get();
   rp.cell_start = nullptr; rp.table_keys = 0;
   // a small key space (the usual case: a cropped cloud) gets a direct-address table of the cells' first sorted positions
   // instead of nine binary searches per point
@@ -1882,19 +1873,18 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
       !getenv("CM_ROR_NO_TABLE")) {
     const size_t keys = (size_t)n_clouds << w.plan_idx_bits;
     if (h->ror_table_cap < keys + 1) {
-      cudaFree(h->ror_table);
-      h->ror_table = nullptr; h->ror_table_cap = 0;
-      CM_CUDA(h, dev_alloc(&h->ror_table, keys + 1));
+      h->ror_table.reset(); h->ror_table_cap = 0;  // the old table goes before the larger one is allocated
+      CM_CUDA(h, dev_alloc(h->ror_table, keys + 1));
       h->ror_table_cap = keys + 1;
     }
-    rp.cell_start = h->ror_table; rp.table_keys = (uint32_t)keys;
+    rp.cell_start = h->ror_table.get(); rp.table_keys = (uint32_t)keys;
     CM_CUDA(h, launch_radius_table(vp, rp, st));
     ++w.launches;
   }
-  if (n_points) CM_CUDA(h, cudaMemsetAsync(h->zw.mask, 0, (size_t)n_points * sizeof(unsigned short), st));
+  if (n_points) CM_CUDA(h, cudaMemsetAsync(h->zw.mask.get(), 0, (size_t)n_points * sizeof(unsigned short), st));
   CM_CUDA(h, launch_radius_count(vp, rp, st));
   ++w.launches;
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT], st));
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
   return zone_run(h, pts, n_points, st, true, n_clouds);
 }
 }  // namespace
@@ -1936,9 +1926,9 @@ int cm_radius_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t
     int rc = zone_ws_ensure(h, (size_t)n_points);
     if (rc != CM_OK) return rc;
     cm_handle_s::ZoneWs& z = h->zw;
-    if (!z.in_stage) CM_CUDA(h, dev_alloc(&z.in_stage, z.cap_points));
-    if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage, xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-    rc = radius_outlier_run(h, z.in_stage, begin, n_clouds, radius, min_neighbors, negative, nullptr);
+    if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
+    if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
+    rc = radius_outlier_run(h, z.in_stage.get(), begin, n_clouds, radius, min_neighbors, negative, nullptr);
     if (rc != CM_OK) return rc;
   }
   int rc = cm_get_zone_out(h, &zo);
@@ -1949,7 +1939,7 @@ int cm_radius_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t
     // device-side errors of the key / sort stage (e.g. the radius is too small for the extent of the cloud)
     uint32_t dev_err = 0;
     Workspace& w = h->batch;
-    CM_CUDA(h, cudaMemcpy(&dev_err, &reinterpret_cast<Ctrl*>(w.meta + w.ml.off_ctrl)->error, sizeof(dev_err), cudaMemcpyDeviceToHost));
+    CM_CUDA(h, cudaMemcpy(&dev_err, &reinterpret_cast<Ctrl*>(w.meta.get() + w.ml.off_ctrl)->error, sizeof(dev_err), cudaMemcpyDeviceToHost));
     if (dev_err == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of the cloud (cell grid exceeds the key range)");
     if (dev_err) return fail(h, CM_E_INTERNAL, "device error %u", dev_err);
     const int64_t total = zo.begin[n_clouds];
@@ -1979,15 +1969,16 @@ constexpr size_t PLANE_BATCH = 1024;  // draws per cloud and batch
 int plane_ws_ensure(cm_handle_t h) {
   cm_handle_s::PlaneWs& q = h->pw;
   if (q.cap_draws) return CM_OK;
+  q = cm_handle_s::PlaneWs();  // frees what an earlier, failed call left behind
   const size_t draws = PLANE_BATCH * CM_MAX_PLANE_CLOUDS;
-  CM_CUDA(h, dev_alloc(&q.samples_dev, draws * 3));
-  CM_CUDA(h, dev_alloc(&q.counts_dev, draws * 2));
-  CM_CUDA(h, dev_alloc(&q.models_dev, draws));
-  CM_CUDA(h, dev_alloc(&q.acc_dev, (size_t)16 * CM_MAX_PLANE_CLOUDS));
-  CM_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&q.samples_pin), draws * 3 * sizeof(int32_t)));
-  CM_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&q.counts_pin), draws * 2 * sizeof(int32_t)));
-  CM_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&q.models_pin), draws * sizeof(float4)));
-  CM_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&q.acc_pin), 16 * CM_MAX_PLANE_CLOUDS * sizeof(float)));
+  CM_CUDA(h, dev_alloc(q.samples_dev, draws * 3));
+  CM_CUDA(h, dev_alloc(q.counts_dev, draws * 2));
+  CM_CUDA(h, dev_alloc(q.models_dev, draws));
+  CM_CUDA(h, dev_alloc(q.acc_dev, (size_t)16 * CM_MAX_PLANE_CLOUDS));
+  CM_CUDA(h, pinned_alloc(q.samples_pin, draws * 3 * sizeof(int32_t), cudaHostAllocDefault));
+  CM_CUDA(h, pinned_alloc(q.counts_pin, draws * 2 * sizeof(int32_t), cudaHostAllocDefault));
+  CM_CUDA(h, pinned_alloc(q.models_pin, draws * sizeof(float4), cudaHostAllocDefault));
+  CM_CUDA(h, pinned_alloc(q.acc_pin, 16 * CM_MAX_PLANE_CLOUDS * sizeof(float), cudaHostAllocDefault));
   q.cap_draws = draws;
   return CM_OK;
 }
@@ -2143,7 +2134,7 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
   PlaneParams pp{};
   pp.pts = pts; pp.n_clouds = (uint32_t)n_clouds; pp.draw_stride = (uint32_t)PLANE_BATCH;
   pp.threshold = thr; pp.sum_order = (uint32_t)cfg.sum_order;
-  pp.samples = q.samples_dev; pp.models = q.models_dev; pp.counts = q.counts_dev; pp.good = q.counts_dev + q.cap_draws;
+  pp.samples = q.samples_dev.get(); pp.models = q.models_dev.get(); pp.counts = q.counts_dev.get(); pp.good = q.counts_dev.get() + q.cap_draws;
   std::vector<PlaneSearch> search((size_t)n_clouds);
   // CM_PLANE_TRACE=1: where the wall time of a call goes (host draws / scoring round trips / select + refit), to stderr
   static const bool trace = getenv("CM_PLANE_TRACE") != nullptr;
@@ -2176,7 +2167,7 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
       if (!s.running()) continue;
       any = true;
       pp.n_draws[c] = (uint32_t)batch;
-      int32_t* smp = q.samples_pin + 3 * (size_t)c * PLANE_BATCH;
+      int32_t* smp = q.samples_pin.get() + 3 * (size_t)c * PLANE_BATCH;
       for (size_t d = 0; d < batch; ++d) {
         for (int64_t i = 0; i < 3; ++i) {
           const uint64_t r = (uint64_t)((uint32_t)s.engine() >> 1);  // boost::uniform_int<>(0, INT_MAX) on mt19937
@@ -2188,20 +2179,20 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
     if (!any) break;
     const auto t1 = now();
     const size_t used = (size_t)(n_clouds - 1) * PLANE_BATCH + batch;  // the per-draw arrays up to the last cloud's batch
-    CM_CUDA(h, cudaMemcpyAsync(q.samples_dev, q.samples_pin, used * 3 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    CM_CUDA(h, cudaMemsetAsync(q.counts_dev, 0, used * sizeof(int32_t), st));
+    CM_CUDA(h, cudaMemcpyAsync(q.samples_dev.get(), q.samples_pin.get(), used * 3 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CM_CUDA(h, cudaMemsetAsync(q.counts_dev.get(), 0, used * sizeof(int32_t), st));
     CM_CUDA(h, launch_plane_score(pp, st));
     ++launches;
-    CM_CUDA(h, cudaMemcpyAsync(q.counts_pin, q.counts_dev, used * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CM_CUDA(h, cudaMemcpyAsync(q.counts_pin + q.cap_draws, q.counts_dev + q.cap_draws, used * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CM_CUDA(h, cudaMemcpyAsync(q.models_pin, q.models_dev, used * sizeof(float4), cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaMemcpyAsync(q.counts_pin.get(), q.counts_dev.get(), used * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaMemcpyAsync(q.counts_pin.get() + q.cap_draws, q.counts_dev.get() + q.cap_draws, used * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaMemcpyAsync(q.models_pin.get(), q.models_dev.get(), used * sizeof(float4), cudaMemcpyDeviceToHost, st));
     CM_CUDA(h, cudaStreamSynchronize(st));
     const auto t2 = now();
     for (int c = 0; c < n_clouds; ++c) {
       PlaneSearch& s = search[(size_t)c];
       const size_t n_draws = pp.n_draws[c], off = (size_t)c * PLANE_BATCH;
-      const int32_t* counts = q.counts_pin + off;
-      const int32_t* good = q.counts_pin + q.cap_draws + off;
+      const int32_t* counts = q.counts_pin.get() + off;
+      const int32_t* good = q.counts_pin.get() + q.cap_draws + off;
       for (size_t d = 0; d < n_draws && s.running(); ++d) {
         ++s.draws;
         if (!good[d]) {  // getSamples draws again; after max_sample_checks_ (1000) failures in a row it gives up
@@ -2213,8 +2204,8 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
           s.best = counts[d];
           s.found = true;
           out[c].best_count = counts[d];
-          for (int i = 0; i < 3; ++i) out[c].sample[i] = q.samples_pin[3 * (off + d) + i];
-          const float4 m = q.models_pin[off + d];
+          for (int i = 0; i < 3; ++i) out[c].sample[i] = q.samples_pin.get()[3 * (off + d) + i];
+          const float4 m = q.models_pin.get()[off + d];
           out[c].coeff_ransac[0] = m.x; out[c].coeff_ransac[1] = m.y; out[c].coeff_ransac[2] = m.z; out[c].coeff_ransac[3] = m.w;
           const double w = (double)s.best * s.one_over_indices;
           double p_no_outliers = 1.0 - std::pow(w, 3.0);
@@ -2234,7 +2225,7 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
 
   // what follows the search: zone 2k = inliers of cloud k, zone 2k + 1 = its other points
   PlaneSelect ps{};
-  ps.pts = pts; ps.n_clouds = (uint32_t)n_clouds; ps.threshold = thr; ps.mask = h->zw.mask;
+  ps.pts = pts; ps.n_clouds = (uint32_t)n_clouds; ps.threshold = thr; ps.mask = h->zw.mask.get();
   for (int c = 0; c <= n_clouds; ++c) ps.begin[c] = (uint32_t)begin[c];
   bool any_found = false;
   for (int c = 0; c < n_clouds; ++c) {
@@ -2249,22 +2240,22 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
   }
   if (any_found && cfg.optimize) {
     // optimizeModelCoefficients on the inliers of the RANSAC model: the running sums on the device, the 3 x 3 part here
-    CM_CUDA(h, launch_plane_moments(ps, (uint32_t)cfg.sum_order, q.acc_dev, st));
+    CM_CUDA(h, launch_plane_moments(ps, (uint32_t)cfg.sum_order, q.acc_dev.get(), st));
     ++launches;
-    CM_CUDA(h, cudaMemcpyAsync(q.acc_pin, q.acc_dev, (size_t)16 * n_clouds * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaMemcpyAsync(q.acc_pin.get(), q.acc_dev.get(), (size_t)16 * n_clouds * sizeof(float), cudaMemcpyDeviceToHost, st));
     CM_CUDA(h, cudaStreamSynchronize(st));
     for (int c = 0; c < n_clouds; ++c) {
       uint32_t n_in;
-      memcpy(&n_in, q.acc_pin + 16 * c + 9, sizeof(n_in));
+      memcpy(&n_in, q.acc_pin.get() + 16 * c + 9, sizeof(n_in));
 #ifdef CM_PLANE_CYCLES
       if (trace) {
         uint32_t cyc[2];
-        memcpy(cyc, q.acc_pin + 16 * c + 10, sizeof(cyc));
+        memcpy(cyc, q.acc_pin.get() + 16 * c + 10, sizeof(cyc));
         fprintf(stderr, "[cm plane] cloud %d: moments kernel %u cycles, adding warp busy %u cycles, %u inliers\n", c, cyc[0], cyc[1], n_in);
       }
 #endif
       if (!search[(size_t)c].found || n_in < 4) continue;  // below 4 inliers PCL keeps the RANSAC model
-      plane_refit(q.acc_pin + 16 * c, n_in, cfg.sum_order, out[c].coeff);
+      plane_refit(q.acc_pin.get() + 16 * c, n_in, cfg.sum_order, out[c].coeff);
       ps.coeff[c] = make_float4(out[c].coeff[0], out[c].coeff[1], out[c].coeff[2], out[c].coeff[3]);
     }
   }
@@ -2320,9 +2311,9 @@ int cm_plane_ransac_multi(cm_handle_t h, const float* xyzi_host, const int64_t* 
   int rc = zone_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
   cm_handle_s::ZoneWs& z = h->zw;
-  if (!z.in_stage) CM_CUDA(h, dev_alloc(&z.in_stage, z.cap_points));
-  if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage, xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-  rc = plane_ransac_run(h, z.in_stage, begin, n_clouds, *cfg, out, nullptr);
+  if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
+  if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
+  rc = plane_ransac_run(h, z.in_stage.get(), begin, n_clouds, *cfg, out, nullptr);
   if (rc != CM_OK) return rc;
   cm_zone_out_t zo;
   rc = zone_out_locked(h, &zo);
@@ -2348,14 +2339,13 @@ int proceed_ws_ensure(cm_handle_t h, size_t points) {
   cm_handle_s::ProceedWs& w = h->prz;
   const size_t want = std::max<size_t>({points, (size_t)h->cfg.max_batch_points, (size_t)1});
   if (w.cap >= want) return CM_OK;
-  cudaFree(w.low); cudaFree(w.high); cudaFree(w.rest); cudaFree(w.planes); cudaFree(w.no_ground); cudaFree(w.ground); cudaFree(w.in_stage);
-  w = cm_handle_s::ProceedWs();
-  CM_CUDA(h, dev_alloc(&w.low, want));
-  CM_CUDA(h, dev_alloc(&w.high, 2 * want));
-  CM_CUDA(h, dev_alloc(&w.rest, want));
-  CM_CUDA(h, dev_alloc(&w.planes, want));
-  CM_CUDA(h, dev_alloc(&w.no_ground, 2 * want));
-  CM_CUDA(h, dev_alloc(&w.ground, 2 * want));
+  w = cm_handle_s::ProceedWs();  // the old buffers go before the larger ones are allocated
+  CM_CUDA(h, dev_alloc(w.low, want));
+  CM_CUDA(h, dev_alloc(w.high, 2 * want));
+  CM_CUDA(h, dev_alloc(w.rest, want));
+  CM_CUDA(h, dev_alloc(w.planes, want));
+  CM_CUDA(h, dev_alloc(w.no_ground, 2 * want));
+  CM_CUDA(h, dev_alloc(w.ground, 2 * want));
   w.cap = want;
   return CM_OK;
 }
@@ -2378,8 +2368,8 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
   if (rc != CM_OK) return rc;
   cm_handle_s::ProceedWs& w = h->prz;
   memset(out, 0, sizeof(*out));
-  out->no_ground_xyzi = reinterpret_cast<const float*>(w.no_ground);
-  out->ground_xyzi = reinterpret_cast<const float*>(w.ground);
+  out->no_ground_xyzi = reinterpret_cast<const float*>(w.no_ground.get());
+  out->ground_xyzi = reinterpret_cast<const float*>(w.ground.get());
   out->n_planes = G;
   // ---- one zone-slicing pass: zones [0, G) the ground windows, [G, 2G) the upper windows, [2G, 2G + P) the plain parts
   const ZoneSet saved = h->zones;
@@ -2426,8 +2416,8 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
   if (rc != CM_OK) return rc;
   const int64_t n_low = zo.begin[G], n_high = zo.begin[2 * G + P] - n_low;
   if ((size_t)n_low > w.cap || (size_t)n_high > 2 * w.cap) return fail(h, CM_E_CAPACITY, "zone windows larger than the workspace");
-  if (n_low) CM_CUDA(h, cudaMemcpyAsync(w.low, zo.xyzi, (size_t)n_low * 16, cudaMemcpyDeviceToDevice, st));
-  if (n_high) CM_CUDA(h, cudaMemcpyAsync(w.high, zo.xyzi + n_low * 4, (size_t)n_high * 16, cudaMemcpyDeviceToDevice, st));
+  if (n_low) CM_CUDA(h, cudaMemcpyAsync(w.low.get(), zo.xyzi, (size_t)n_low * 16, cudaMemcpyDeviceToDevice, st));
+  if (n_high) CM_CUDA(h, cudaMemcpyAsync(w.high.get(), zo.xyzi + n_low * 4, (size_t)n_high * 16, cudaMemcpyDeviceToDevice, st));
   int64_t zb[CM_MAX_ZONES + 1];
   for (int z = 0; z <= 2 * G + P; ++z) zb[z] = zo.begin[z];
 
@@ -2435,19 +2425,19 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
   int64_t pb[2 * CM_MAX_PLANE_CLOUDS + 1] = {0}, kb[CM_MAX_PLANE_CLOUDS + 1] = {0}, rb[CM_MAX_PLANE_CLOUDS + 1] = {0};
   const float4* kept = nullptr;
   if (G > 0) {
-    rc = plane_ransac_run(h, w.low, zb, G, cfg.plane, out->plane, st);  // ends with the sizes on the host
+    rc = plane_ransac_run(h, w.low.get(), zb, G, cfg.plane, out->plane, st);  // ends with the sizes on the host
     out->host_syncs += 2 + (cfg.plane.optimize ? 1 : 0);
     if (rc != CM_OK) return rc;
     rc = zone_out_locked(h, &zo);
     if (rc != CM_OK) return rc;
     for (int z = 0; z <= 2 * G; ++z) pb[z] = zo.begin[z];
-    if (pb[2 * G]) CM_CUDA(h, cudaMemcpyAsync(w.planes, zo.xyzi, (size_t)pb[2 * G] * 16, cudaMemcpyDeviceToDevice, st));
+    if (pb[2 * G]) CM_CUDA(h, cudaMemcpyAsync(w.planes.get(), zo.xyzi, (size_t)pb[2 * G] * 16, cudaMemcpyDeviceToDevice, st));
     for (int c = 0; c < G; ++c) {  // the non-ground points of every window side by side
       const int64_t cnt = pb[2 * c + 2] - pb[2 * c + 1];
-      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.rest + rb[c], w.planes + pb[2 * c + 1], (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
+      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.rest.get() + rb[c], w.planes.get() + pb[2 * c + 1], (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
       rb[c + 1] = rb[c] + cnt;
     }
-    rc = radius_outlier_run(h, w.rest, rb, G, cfg.radius, cfg.min_neighbors, 0, st);
+    rc = radius_outlier_run(h, w.rest.get(), rb, G, cfg.radius, cfg.min_neighbors, 0, st);
     if (rc != CM_OK) return rc;
     rc = zone_out_locked(h, &zo);
     out->host_syncs += 2;
@@ -2455,7 +2445,7 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
     for (int c = 0; c <= G; ++c) kb[c] = zo.begin[c];
     kept = reinterpret_cast<const float4*>(zo.xyzi);
     uint32_t dev_err = 0;  // key-range / watchdog errors of the cell sort
-    CM_CUDA(h, cudaMemcpyAsync(&dev_err, &reinterpret_cast<Ctrl*>(h->batch.meta + h->batch.ml.off_ctrl)->error, sizeof(dev_err), cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaMemcpyAsync(&dev_err, &reinterpret_cast<Ctrl*>(h->batch.meta.get() + h->batch.ml.off_ctrl)->error, sizeof(dev_err), cudaMemcpyDeviceToHost, st));
     CM_CUDA(h, cudaStreamSynchronize(st));
     if (dev_err == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a zone (cell grid exceeds the key range)");
     if (dev_err) return fail(h, CM_E_INTERNAL, "device error %u", dev_err);
@@ -2466,18 +2456,18 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
     if (ground_of[k] >= 0) {
       const int c = ground_of[k];
       int64_t cnt = kb[c + 1] - kb[c];                    // outlierRemoval(no_ground_cloud_ptr) ...
-      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.no_ground + n_ng, kept + kb[c], (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
+      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.no_ground.get() + n_ng, kept + kb[c], (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
       n_ng += cnt;
       cnt = zb[G + c + 1] - zb[G + c];                    // ... += *no_ground_part_ptr (the upper window)
-      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.no_ground + n_ng, w.high + (zb[G + c] - n_low), (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
+      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.no_ground.get() + n_ng, w.high.get() + (zb[G + c] - n_low), (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
       n_ng += cnt;
       cnt = pb[2 * c + 1] - pb[2 * c];                    // ground: the inliers
-      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.ground + n_g, w.planes + pb[2 * c], (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
+      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.ground.get() + n_g, w.planes.get() + pb[2 * c], (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
       n_g += cnt;
     } else {
       const int z = 2 * G + plain_of[k];
       const int64_t cnt = zb[z + 1] - zb[z];
-      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.no_ground + n_ng, w.high + (zb[z] - n_low), (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
+      if (cnt) CM_CUDA(h, cudaMemcpyAsync(w.no_ground.get() + n_ng, w.high.get() + (zb[z] - n_low), (size_t)cnt * 16, cudaMemcpyDeviceToDevice, st));
       n_ng += cnt;
     }
   }
@@ -2505,10 +2495,10 @@ int cm_proceed_zones(cm_handle_t h, const float* roi_xyzi_host, int64_t n_points
   int rc = proceed_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
   cm_handle_s::ProceedWs& w = h->prz;
-  if (!w.in_stage) CM_CUDA(h, dev_alloc(&w.in_stage, w.cap));
-  if (n_points) CM_CUDA(h, cudaMemcpyAsync(w.in_stage, roi_xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
+  if (!w.in_stage) CM_CUDA(h, dev_alloc(w.in_stage, w.cap));
+  if (n_points) CM_CUDA(h, cudaMemcpyAsync(w.in_stage.get(), roi_xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
   cm_proceed_out_t po;
-  rc = proceed_run(h, w.in_stage, n_points, *cfg, &po, nullptr);
+  rc = proceed_run(h, w.in_stage.get(), n_points, *cfg, &po, nullptr);
   if (rc != CM_OK) return rc;
   *n_no_ground = po.n_no_ground;
   *n_ground = po.n_ground;
@@ -2574,19 +2564,19 @@ struct cm_giant_s {
   ncclComm_t comm = nullptr;
   NcclApi* api = nullptr;
   uint32_t bins = 1u << 14;
-  GiantPlan* plan = nullptr;            // device
-  unsigned long long* hist = nullptr;   // device [bins]
-  uint32_t* counts = nullptr;           // device [world][CM_MAX_ZONES + 2]: every rank's zone_begin
-  float4* recv = nullptr;               // device [recv_cap]: what the all-to-all delivers
+  DevPtr<GiantPlan> plan;               // device
+  DevPtr<unsigned long long> hist;      // device [bins]
+  DevPtr<uint32_t> counts;              // device [world][CM_MAX_ZONES + 2]: every rank's zone_begin
+  DevPtr<float4> recv;                  // device [recv_cap]: what the all-to-all delivers
   size_t recv_cap = 0;
-  GiantPlan* plan_pin = nullptr;        // pinned mirrors
-  uint32_t* counts_pin = nullptr;       // [world][stride] + 1: the overflow word of the peer exchange
+  HostPtr<GiantPlan> plan_pin;          // pinned mirrors
+  HostPtr<uint32_t> counts_pin;         // [world][stride] + 1: the overflow word of the peer exchange
   // the exchange fused into the grouping kernel: every rank's receive buffer mapped here through CUDA IPC
   bool p2p = false;
   float4* peer_recv[CM_MAX_ZONES] = {};
-  uint32_t* p2p_words = nullptr;        // device: [0..world) remote_base, [world] barrier word, [world + 1] my receive capacity
-  cudaEvent_t plan_ready = nullptr;     // the host waits for the counts, not for the exchange
-  cudaEvent_t prof[5] = {};             // stage boundaries (cm_set_profiling)
+  DevPtr<uint32_t> p2p_words;           // device: [0..world) remote_base, [world] barrier word, [world + 1] my receive capacity
+  Event plan_ready;                     // the host waits for the counts, not for the exchange
+  Event prof[5];                        // stage boundaries (cm_set_profiling)
   std::string err;
 };
 
@@ -2622,23 +2612,22 @@ void giant_setup_p2p(cm_giant_t g) {
   const int W = g->world;
   cudaIpcMemHandle_t mine;
   memset(&mine, 0, sizeof(mine));
-  if (want && cudaIpcGetMemHandle(&mine, g->recv) != cudaSuccess) { want = 0; cudaGetLastError(); }
-  cudaIpcMemHandle_t* all_dev = nullptr;
-  int* ok_dev = nullptr;
+  if (want && cudaIpcGetMemHandle(&mine, g->recv.get()) != cudaSuccess) { want = 0; cudaGetLastError(); }
+  DevPtr<cudaIpcMemHandle_t> all_dev;
+  DevPtr<int> ok_dev;
   std::vector<cudaIpcMemHandle_t> all((size_t)W);
   int ok = want;
-  if (cudaMalloc(reinterpret_cast<void**>(&all_dev), sizeof(mine) * (size_t)(W + 1)) != cudaSuccess ||
-      cudaMalloc(reinterpret_cast<void**>(&ok_dev), sizeof(int)) != cudaSuccess) { cudaGetLastError(); ok = 0; }
+  if (dev_alloc(all_dev, (size_t)W + 1, 0) != cudaSuccess || dev_alloc(ok_dev, 1, 0) != cudaSuccess) { cudaGetLastError(); ok = 0; }
   // every rank takes part in both collectives whatever its own state, or the others would hang
   if (all_dev && ok_dev) {
-    cudaMemcpy(all_dev + W, &mine, sizeof(mine), cudaMemcpyHostToDevice);
-    if (g->api->AllGather(all_dev + W, all_dev, sizeof(mine), ncclUint8, g->comm, nullptr) != ncclSuccess) ok = 0;
-    if (cudaMemcpy(all.data(), all_dev, sizeof(mine) * (size_t)W, cudaMemcpyDeviceToHost) != cudaSuccess) { ok = 0; cudaGetLastError(); }
+    cudaMemcpy(all_dev.get() + W, &mine, sizeof(mine), cudaMemcpyHostToDevice);
+    if (g->api->AllGather(all_dev.get() + W, all_dev.get(), sizeof(mine), ncclUint8, g->comm, nullptr) != ncclSuccess) ok = 0;
+    if (cudaMemcpy(all.data(), all_dev.get(), sizeof(mine) * (size_t)W, cudaMemcpyDeviceToHost) != cudaSuccess) { ok = 0; cudaGetLastError(); }
   }
   int opened = 0;
   if (ok) {
     for (int r = 0; r < W && ok; ++r) {
-      if (r == g->rank) { g->peer_recv[r] = g->recv; continue; }
+      if (r == g->rank) { g->peer_recv[r] = g->recv.get(); continue; }
       void* p = nullptr;
       if (cudaIpcOpenMemHandle(&p, all[(size_t)r], cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { ok = 0; cudaGetLastError(); break; }
       g->peer_recv[r] = static_cast<float4*>(p);
@@ -2646,19 +2635,18 @@ void giant_setup_p2p(cm_giant_t g) {
     }
   }
   if (all_dev && ok_dev) {
-    cudaMemcpy(ok_dev, &ok, sizeof(int), cudaMemcpyHostToDevice);
+    cudaMemcpy(ok_dev.get(), &ok, sizeof(int), cudaMemcpyHostToDevice);
     int agreed = 0;
-    if (g->api->AllReduce(ok_dev, ok_dev, 1, ncclInt32, ncclMin, g->comm, nullptr) == ncclSuccess &&
-        cudaMemcpy(&agreed, ok_dev, sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess) ok = ok && agreed;
+    if (g->api->AllReduce(ok_dev.get(), ok_dev.get(), 1, ncclInt32, ncclMin, g->comm, nullptr) == ncclSuccess &&
+        cudaMemcpy(&agreed, ok_dev.get(), sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess) ok = ok && agreed;
     else ok = 0;
   }
-  cudaFree(all_dev); cudaFree(ok_dev);
-  if (ok && (cudaMalloc(reinterpret_cast<void**>(&g->p2p_words), sizeof(uint32_t) * (size_t)(W + 2)) != cudaSuccess ||
-             cudaEventCreateWithFlags(&g->plan_ready, cudaEventDisableTiming) != cudaSuccess)) { ok = 0; cudaGetLastError(); }
+  if (ok && (dev_alloc(g->p2p_words, (size_t)W + 2, 0) != cudaSuccess ||
+             create(g->plan_ready, cudaEventCreateWithFlags, cudaEventDisableTiming) != cudaSuccess)) { ok = 0; cudaGetLastError(); }
   if (ok) {
     std::vector<uint32_t> init((size_t)W + 2, 0u);
     init[(size_t)W + 1] = (uint32_t)std::min<size_t>(g->recv_cap, 0xFFFFFFF0u);
-    cudaMemcpy(g->p2p_words, init.data(), sizeof(uint32_t) * init.size(), cudaMemcpyHostToDevice);
+    cudaMemcpy(g->p2p_words.get(), init.data(), sizeof(uint32_t) * init.size(), cudaMemcpyHostToDevice);
   }
   if (!ok) {
     for (int r = 0; r < W; ++r) {
@@ -2669,6 +2657,33 @@ void giant_setup_p2p(cm_giant_t g) {
   }
   (void)opened;
   g->p2p = ok != 0;
+}
+
+// The part of cm_giant_create that can fail: the communicator, the batch workspace and the giant-cloud buffers.
+int giant_setup(cm_giant_t g, const void* nccl_id) {
+  cm_handle_t h = g->h;
+  if (g->world > 1 && nccl_id) {
+    g->api = nccl_api();
+    if (!g->api) { h->last_error = "NCCL unavailable"; return CM_E_CUDA; }
+    ncclUniqueId id;
+    memcpy(&id, nccl_id, sizeof(id));
+    const ncclResult_t r = g->api->CommInitRank(&g->comm, g->world, id, g->rank);
+    if (r != ncclSuccess) { h->last_error = std::string("ncclCommInitRank: ") + g->api->GetErrorString(r); return CM_E_CUDA; }
+  }
+  int rc = ensure_batch_ws(h);
+  if (rc != CM_OK) return rc;
+  g->recv_cap = h->batch.cap_points;
+  if (dev_alloc(g->plan, 1, 0) != cudaSuccess || dev_alloc(g->hist, g->bins, 0) != cudaSuccess ||
+      dev_alloc(g->counts, (size_t)kCountStride * g->world, 0) != cudaSuccess ||
+      (g->world > 1 && g->comm && dev_alloc(g->recv, g->recv_cap) != cudaSuccess) ||
+      pinned_alloc(g->plan_pin, sizeof(GiantPlan), cudaHostAllocDefault) != cudaSuccess ||
+      pinned_alloc(g->counts_pin, sizeof(uint32_t) * (kCountStride * g->world + 1), cudaHostAllocDefault) != cudaSuccess) {
+    h->last_error = "cm_giant_create: allocation failed";
+    cudaGetLastError();
+    return CM_E_CUDA;
+  }
+  if (g->comm && g->recv) giant_setup_p2p(g);
+  return CM_OK;
 }
 }  // namespace
 
@@ -2692,31 +2707,12 @@ int cm_giant_create(cm_handle_t h, int rank, int world, const void* nccl_id, cm_
   cm_giant_t g = new (std::nothrow) cm_giant_s();
   if (!g) return CM_E_INTERNAL;
   g->h = h; g->rank = rank; g->world = world;
-  auto bail = [&](int code) { cudaFree(g->plan); cudaFree(g->hist); cudaFree(g->counts); cudaFree(g->recv);
-                              if (g->plan_pin) cudaFreeHost(g->plan_pin); if (g->counts_pin) cudaFreeHost(g->counts_pin);
-                              delete g; return code; };
-  if (world > 1 && nccl_id) {
-    g->api = nccl_api();
-    if (!g->api) { h->last_error = "NCCL unavailable"; return bail(CM_E_CUDA); }
-    ncclUniqueId id;
-    memcpy(&id, nccl_id, sizeof(id));
-    const ncclResult_t r = g->api->CommInitRank(&g->comm, world, id, rank);
-    if (r != ncclSuccess) { h->last_error = std::string("ncclCommInitRank: ") + g->api->GetErrorString(r); return bail(CM_E_CUDA); }
+  const int rc = giant_setup(g, nccl_id);
+  if (rc != CM_OK) {  // the buffers go with g, the communicator (if one was made) does not
+    if (g->comm) g->api->CommDestroy(g->comm);
+    delete g;
+    return rc;
   }
-  int rc = ensure_batch_ws(h);
-  if (rc != CM_OK) return bail(rc);
-  g->recv_cap = h->batch.cap_points;
-  if (cudaMalloc(reinterpret_cast<void**>(&g->plan), sizeof(GiantPlan)) != cudaSuccess ||
-      cudaMalloc(reinterpret_cast<void**>(&g->hist), sizeof(unsigned long long) * g->bins) != cudaSuccess ||
-      cudaMalloc(reinterpret_cast<void**>(&g->counts), sizeof(uint32_t) * kCountStride * world) != cudaSuccess ||
-      (world > 1 && g->comm && dev_alloc(&g->recv, g->recv_cap) != cudaSuccess) ||
-      cudaMallocHost(reinterpret_cast<void**>(&g->plan_pin), sizeof(GiantPlan)) != cudaSuccess ||
-      cudaMallocHost(reinterpret_cast<void**>(&g->counts_pin), sizeof(uint32_t) * (kCountStride * world + 1)) != cudaSuccess) {
-    h->last_error = "cm_giant_create: allocation failed";
-    cudaGetLastError();
-    return bail(CM_E_CUDA);
-  }
-  if (g->comm && g->recv) giant_setup_p2p(g);
   *out = g;
   return CM_OK;
 }
@@ -2727,13 +2723,7 @@ int cm_giant_destroy(cm_giant_t g) {
   cudaDeviceSynchronize();  // past this rank's last barrier: no peer is still storing into g->recv
   for (int r = 0; r < g->world; ++r)
     if (g->p2p && r != g->rank && g->peer_recv[r]) cudaIpcCloseMemHandle(g->peer_recv[r]);
-  cudaFree(g->p2p_words);
-  if (g->plan_ready) cudaEventDestroy(g->plan_ready);
-  for (auto& e : g->prof) if (e) cudaEventDestroy(e);
   if (g->comm && g->api) g->api->CommDestroy(g->comm);
-  cudaFree(g->plan); cudaFree(g->hist); cudaFree(g->counts); cudaFree(g->recv);
-  if (g->plan_pin) cudaFreeHost(g->plan_pin);
-  if (g->counts_pin) cudaFreeHost(g->counts_pin);
   delete g;
   return CM_OK;
 }
@@ -2752,29 +2742,29 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
   rc = zone_ws_ensure(h, (size_t)n_local);
   if (rc != CM_OK) return rc;
   Workspace& w = h->batch;
-  Ctrl* ctrl = reinterpret_cast<Ctrl*>(w.meta + w.ml.off_ctrl);
-  FrameAcc* acc = reinterpret_cast<FrameAcc*>(w.meta + w.ml.off_acc);
-  uint32_t* fss = reinterpret_cast<uint32_t*>(w.meta + w.ml.off_fstart);
+  Ctrl* ctrl = reinterpret_cast<Ctrl*>(w.meta.get() + w.ml.off_ctrl);
+  FrameAcc* acc = reinterpret_cast<FrameAcc*>(w.meta.get() + w.ml.off_acc);
+  uint32_t* fss = reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_fstart);
   cm_giant_info_t gi;
   memset(&gi, 0, sizeof(gi));
   gi.points_local = n_local;
   ZoneParams zp;
   const bool prof = h->profiling;
   if (prof)
-    for (auto& e : g->prof) if (!e) CM_G_CUDA(g, cudaEventCreate(&e));
-  auto mark = [&](int i) { return prof ? cudaEventRecord(g->prof[i], st) : cudaSuccess; };
+    for (auto& e : g->prof) if (!e) CM_G_CUDA(g, create(e, cudaEventCreateWithFlags, cudaEventDefault));
+  auto mark = [&](int i) { return prof ? cudaEventRecord(g->prof[i].get(), st) : cudaSuccess; };
   CM_G_CUDA(g, mark(0));
   // ---- global bounding box -> grid, on the device
-  CM_G_CUDA(g, cudaMemsetAsync(w.meta, 0, w.ml.zero_bytes, st));
+  CM_G_CUDA(g, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
   CM_G_CUDA(g, launch_minmax(pts, (uint32_t)n_local, ctrl, acc, fss, st));
   if (g->comm) CM_G_NCCL(g, g->api->AllReduce(acc, acc, 6, ncclUint32, ncclMax, g->comm, st));  // max_enc[3], nmin_enc[3]
-  CM_G_CUDA(g, launch_giant_plan(g->plan, acc, h->inv_leaf, g->bins, st));
+  CM_G_CUDA(g, launch_giant_plan(g->plan.get(), acc, h->inv_leaf, g->bins, st));
   // ---- balancing splitters from the all-reduced histogram of the voxel index, on the device
   if (W > 1) {
-    CM_G_CUDA(g, cudaMemsetAsync(g->hist, 0, sizeof(unsigned long long) * g->bins, st));
-    CM_G_CUDA(g, launch_giant_hist(pts, (uint32_t)n_local, g->plan, g->bins, g->hist, st));
-    if (g->comm) CM_G_NCCL(g, g->api->AllReduce(g->hist, g->hist, g->bins, ncclUint64, ncclSum, g->comm, st));
-    CM_G_CUDA(g, launch_giant_splitters(g->plan, g->hist, g->bins, (uint32_t)W, st));
+    CM_G_CUDA(g, cudaMemsetAsync(g->hist.get(), 0, sizeof(unsigned long long) * g->bins, st));
+    CM_G_CUDA(g, launch_giant_hist(pts, (uint32_t)n_local, g->plan.get(), g->bins, g->hist.get(), st));
+    if (g->comm) CM_G_NCCL(g, g->api->AllReduce(g->hist.get(), g->hist.get(), g->bins, ncclUint64, ncclSum, g->comm, st));
+    CM_G_CUDA(g, launch_giant_splitters(g->plan.get(), g->hist.get(), g->bins, (uint32_t)W, st));
     CM_G_CUDA(g, mark(1));
     // ---- group the block by destination (source order kept inside a destination): the send buffer of the all-to-all
     // (the destination masks are derived inside the count sweep from the device-resident plan)
@@ -2782,35 +2772,35 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
       // count + scan only; the scatter below IS the all-to-all (stores into the owners' receive buffers over NVLink)
       if (in_zone_outputs(h, pts, n_local)) return gfail(g, CM_E_INVALID, "the input cloud lies in this handle's own zone outputs");
       zp = zone_params(h, pts, n_local, true, W);
-      zp.mask_given = 0; zp.giant_plan = g->plan; zp.giant_invalid_part = (uint32_t)me;
+      zp.mask_given = 0; zp.giant_plan = g->plan.get(); zp.giant_invalid_part = (uint32_t)me;
       zp.out_capacity = 0xFFFFFFF0u;  // nothing lands in the local outputs; the receivers' capacities are checked on the device
-      CM_G_CUDA(g, cudaMemsetAsync(h->zw.overflow, 0, sizeof(uint32_t), st));
+      CM_G_CUDA(g, cudaMemsetAsync(h->zw.overflow.get(), 0, sizeof(uint32_t), st));
       CM_G_CUDA(g, launch_zone_count_scan(zp, st));
-      CM_G_CUDA(g, cudaMemcpyAsync(h->zw.zone_begin + CM_MAX_ZONES + 1, g->p2p_words + W + 1, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+      CM_G_CUDA(g, cudaMemcpyAsync(h->zw.zone_begin.get() + CM_MAX_ZONES + 1, g->p2p_words.get() + W + 1, sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
       h->zw.ran = false;  // no grouped array on this handle after this call
     } else {
-      rc = zone_run(h, pts, n_local, st, true, W, g->plan, (uint32_t)me);
+      rc = zone_run(h, pts, n_local, st, true, W, g->plan.get(), (uint32_t)me);
       if (rc != CM_OK) return rc;
     }
     // every rank's per-destination offsets (NCCL takes the counts of a send / recv as host arguments)
-    if (g->comm) CM_G_NCCL(g, g->api->AllGather(h->zw.zone_begin, g->counts, kCountStride, ncclUint32, g->comm, st));
-    else CM_G_CUDA(g, cudaMemcpyAsync(g->counts + (size_t)me * kCountStride, h->zw.zone_begin, sizeof(uint32_t) * kCountStride, cudaMemcpyDeviceToDevice, st));
-    CM_G_CUDA(g, cudaMemcpyAsync(g->counts_pin, g->counts, sizeof(uint32_t) * kCountStride * W, cudaMemcpyDeviceToHost, st));
+    if (g->comm) CM_G_NCCL(g, g->api->AllGather(h->zw.zone_begin.get(), g->counts.get(), kCountStride, ncclUint32, g->comm, st));
+    else CM_G_CUDA(g, cudaMemcpyAsync(g->counts.get() + (size_t)me * kCountStride, h->zw.zone_begin.get(), sizeof(uint32_t) * kCountStride, cudaMemcpyDeviceToDevice, st));
+    CM_G_CUDA(g, cudaMemcpyAsync(g->counts_pin.get(), g->counts.get(), sizeof(uint32_t) * kCountStride * W, cudaMemcpyDeviceToHost, st));
     if (g->p2p) {
-      CM_G_CUDA(g, launch_giant_offsets(g->counts, kCountStride, (uint32_t)W, (uint32_t)me, g->p2p_words, h->zw.overflow, st));
-      CM_G_CUDA(g, cudaMemcpyAsync(g->counts_pin + (size_t)kCountStride * W, h->zw.overflow, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+      CM_G_CUDA(g, launch_giant_offsets(g->counts.get(), kCountStride, (uint32_t)W, (uint32_t)me, g->p2p_words.get(), h->zw.overflow.get(), st));
+      CM_G_CUDA(g, cudaMemcpyAsync(g->counts_pin.get() + (size_t)kCountStride * W, h->zw.overflow.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     }
   }
-  CM_G_CUDA(g, cudaMemcpyAsync(g->plan_pin, g->plan, sizeof(GiantPlan), cudaMemcpyDeviceToHost, st));
+  CM_G_CUDA(g, cudaMemcpyAsync(g->plan_pin.get(), g->plan.get(), sizeof(GiantPlan), cudaMemcpyDeviceToHost, st));
   if (W > 1) CM_G_CUDA(g, mark(2));
   if (W > 1 && g->p2p) {
-    CM_G_CUDA(g, cudaEventRecord(g->plan_ready, st));
+    CM_G_CUDA(g, cudaEventRecord(g->plan_ready.get(), st));
     for (int r = 0; r < W; ++r) zp.zone_ptr[r] = g->peer_recv[r];
-    zp.zone_remote_base = g->p2p_words;
+    zp.zone_remote_base = g->p2p_words.get();
     CM_G_CUDA(g, launch_zone_scatter_remote(zp, st));
     // every store of every rank has landed once this one-word all-reduce completes (stream order on each rank)
-    CM_G_NCCL(g, g->api->AllReduce(g->p2p_words + W, g->p2p_words + W, 1, ncclUint32, ncclMax, g->comm, st));
-    CM_G_CUDA(g, cudaEventSynchronize(g->plan_ready));  // the counts are here; the exchange is still in flight
+    CM_G_NCCL(g, g->api->AllReduce(g->p2p_words.get() + W, g->p2p_words.get() + W, 1, ncclUint32, ncclMax, g->comm, st));
+    CM_G_CUDA(g, cudaEventSynchronize(g->plan_ready.get()));  // the counts are here; the exchange is still in flight
   } else {
     CM_G_CUDA(g, cudaStreamSynchronize(st));
   }
@@ -2828,7 +2818,7 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
   const float4* vox_in = pts;
   int64_t n_vox = n_local;
   if (W > 1) {
-    const uint32_t* mine = g->counts_pin + (size_t)me * kCountStride;
+    const uint32_t* mine = g->counts_pin.get() + (size_t)me * kCountStride;
     for (int r = 0; r <= W; ++r) gi.send_begin[r] = mine[r];
     gi.points_sent_away = n_local - (int64_t)(mine[me + 1] - mine[me]);
     if (!g->comm) {  // dry mode: the grouping is the result (cm_get_zone_out)
@@ -2838,34 +2828,34 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
     int64_t roff[CM_MAX_ZONES + 1];
     roff[0] = 0;
     for (int s = 0; s < W; ++s) {
-      const uint32_t* row = g->counts_pin + (size_t)s * kCountStride;
+      const uint32_t* row = g->counts_pin.get() + (size_t)s * kCountStride;
       roff[s + 1] = roff[s] + (int64_t)(row[me + 1] - row[me]);
     }
     gi.points_received = roff[W];
     if (g->p2p) {
       // the device already decided (every rank the same): with an overflow nobody stored anything
-      const uint32_t over = g->counts_pin[(size_t)kCountStride * W];
+      const uint32_t over = g->counts_pin.get()[(size_t)kCountStride * W];
       if (over) return gfail(g, CM_E_CAPACITY, "a rank would receive %u points, more than max_batch_points of its handle", over);
       gi.exchange = CM_GIANT_EXCHANGE_PEER;
-      vox_in = g->recv;
+      vox_in = g->recv.get();
       n_vox = roff[W];
     } else {
       if ((size_t)roff[W] > g->recv_cap)
         return gfail(g, CM_E_CAPACITY, "this rank receives %lld points, max_batch_points of the handle is %zu", (long long)roff[W], g->recv_cap);
       gi.exchange = CM_GIANT_EXCHANGE_NCCL;
       // ---- ONE all-to-all, straight out of the grouped array
-      const float4* send = h->zw.out_xyzi;
+      const float4* send = h->zw.out_xyzi.get();
       CM_G_NCCL(g, g->api->GroupStart());
       for (int r = 0; r < W; ++r) {
         const size_t sc = (size_t)(mine[r + 1] - mine[r]), rcnt = (size_t)(roff[r + 1] - roff[r]);
         if (r == me) continue;
         if (sc) CM_G_NCCL(g, g->api->Send(send + mine[r], sc * 4, ncclFloat, r, g->comm, st));
-        if (rcnt) CM_G_NCCL(g, g->api->Recv(g->recv + roff[r], rcnt * 4, ncclFloat, r, g->comm, st));
+        if (rcnt) CM_G_NCCL(g, g->api->Recv(g->recv.get() + roff[r], rcnt * 4, ncclFloat, r, g->comm, st));
       }
       CM_G_NCCL(g, g->api->GroupEnd());
       const size_t self = (size_t)(mine[me + 1] - mine[me]);
-      if (self) CM_G_CUDA(g, cudaMemcpyAsync(g->recv + roff[me], send + mine[me], self * 16, cudaMemcpyDeviceToDevice, st));
-      vox_in = g->recv;
+      if (self) CM_G_CUDA(g, cudaMemcpyAsync(g->recv.get() + roff[me], send + mine[me], self * 16, cudaMemcpyDeviceToDevice, st));
+      vox_in = g->recv.get();
       n_vox = roff[W];
     }
   } else {
@@ -2873,14 +2863,14 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
   }
   if (info) *info = gi;
   // ---- the ordinary single-GPU VoxelGrid on what arrived, global box folded in, key plan known from the global grid
-  const uint32_t* enc_dev = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(g->plan) + offsetof(GiantPlan, enc));
+  const uint32_t* enc_dev = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(g->plan.get()) + offsetof(GiantPlan, enc));
   CM_G_CUDA(g, mark(3));
   rc = voxelgrid_run(h, vox_in, n_vox, st, enc_dev, (int)P.key_bits);
   if (rc == CM_OK && prof && W > 1) {
     CM_G_CUDA(g, mark(4));
-    CM_G_CUDA(g, cudaEventSynchronize(g->prof[4]));
+    CM_G_CUDA(g, cudaEventSynchronize(g->prof[4].get()));
     for (int i = 0; i < 4; ++i)
-      if (cudaEventElapsedTime(&gi.stage_ms[i], g->prof[i], g->prof[i + 1]) != cudaSuccess) { gi.stage_ms[i] = 0.f; cudaGetLastError(); }
+      if (cudaEventElapsedTime(&gi.stage_ms[i], g->prof[i].get(), g->prof[i + 1].get()) != cudaSuccess) { gi.stage_ms[i] = 0.f; cudaGetLastError(); }
     if (info) *info = gi;
   }
   return rc;
@@ -2912,48 +2902,48 @@ int cm_get_device_out(cm_handle_t h, cm_device_out_t* out) {
     int rc2 = materialize_dense(h, w);
     if (rc2 != CM_OK) return rc2;
     CM_CUDA(h, cudaStreamSynchronize(w.stream));
-    out->survivor_xyzi = reinterpret_cast<const float*>(w.dense_xyzi);
-    out->survivor_src = w.dense_src;
-    out->survivor_slot = w.dense_slot;
-    out->slot_xyzi = reinterpret_cast<const float*>(w.surv_xyzi);
+    out->survivor_xyzi = reinterpret_cast<const float*>(w.dense_xyzi.get());
+    out->survivor_src = w.dense_src.get();
+    out->survivor_slot = w.dense_slot.get();
+    out->slot_xyzi = reinterpret_cast<const float*>(w.surv_xyzi.get());
   } else {
     out->survivor_xyzi = reinterpret_cast<const float*>(w.voxel_pts);
     out->slot_xyzi = out->survivor_xyzi;
   }
   if (w.ran_voxel) {
     const bool odd = (h->stats.sort_passes & 1) != 0;
-    const SortInfo* si_rep = reinterpret_cast<const SortInfo*>(w.report + w.ml.off_info);
+    const SortInfo* si_rep = reinterpret_cast<const SortInfo*>(w.report.get() + w.ml.off_info);
     out->key_bytes = (int32_t)w.key_bytes;
     if (w.key_bytes == 4 && si_rep->segmented) {
       // a frame-segmented run sorted bare voxel indices: hand out (frame << idx_bits | idx), as every other run does,
       // in the ping-pong buffer the last pass did not write
       VoxelParams vp;
       fill_voxel_params(h, w, vp, w.voxel_pts, w.n_frames, (uint32_t)w.points_in);
-      unsigned long long* k64 = reinterpret_cast<unsigned long long*>(odd ? w.keys_a : w.keys_b);
-      CM_CUDA(h, launch_seg_keys64(odd ? w.keys_b : w.keys_a, k64, w.vals_b, vp, w.stream));
+      unsigned long long* k64 = reinterpret_cast<unsigned long long*>(odd ? w.keys_a.get() : w.keys_b.get());
+      CM_CUDA(h, launch_seg_keys64(odd ? w.keys_b.get() : w.keys_a.get(), k64, w.vals_b.get(), vp, w.stream));
       CM_CUDA(h, cudaStreamSynchronize(w.stream));
       out->sorted_key = k64;
-      out->sorted_point = w.vals_b;
+      out->sorted_point = w.vals_b.get();
       out->key_bytes = 8;
     } else if (w.key_bytes == 4) {
       // 32-bit keys are sorted as 8-byte (key, value) records: split them into the two arrays this struct promises
-      const uint32_t* n_ptr = reinterpret_cast<const uint32_t*>(w.meta + w.ml.off_fstart) + w.n_frames;
+      const uint32_t* n_ptr = reinterpret_cast<const uint32_t*>(w.meta.get() + w.ml.off_fstart) + w.n_frames;
       VoxelParams vp;  // fused-key runs sorted box-grid keys: hand out PCL's index, like every other run
       fill_voxel_params(h, w, vp, w.voxel_pts, w.n_frames, (uint32_t)w.points_in);
       vp.fused_keys = w.fused_keys ? 1u : 0u;
       vp.box = w.box;
-      CM_CUDA(h, launch_split_records(odd ? w.keys_b : w.keys_a, w.vals_a, w.vals_b, n_ptr, (uint32_t)w.points_in, w.stream,
+      CM_CUDA(h, launch_split_records(odd ? w.keys_b.get() : w.keys_a.get(), w.vals_a.get(), w.vals_b.get(), n_ptr, (uint32_t)w.points_in, w.stream,
                                       w.fused_keys ? &vp : nullptr));
       CM_CUDA(h, cudaStreamSynchronize(w.stream));
-      out->sorted_key = w.vals_a;
-      out->sorted_point = w.vals_b;
+      out->sorted_key = w.vals_a.get();
+      out->sorted_point = w.vals_b.get();
     } else {
-      out->sorted_key = odd ? w.keys_b : w.keys_a;
-      out->sorted_point = odd ? w.vals_b : w.vals_a;
+      out->sorted_key = odd ? w.keys_b.get() : w.keys_a.get();
+      out->sorted_point = odd ? w.vals_b.get() : w.vals_a.get();
     }
-    out->voxel_xyzi = w.out_xyzi;
-    out->voxel_count = w.out_count;
-    out->voxel_idx = reinterpret_cast<const uint64_t*>(w.out_idx);
+    out->voxel_xyzi = w.out_xyzi.get();
+    out->voxel_count = w.out_count.get();
+    out->voxel_idx = reinterpret_cast<const uint64_t*>(w.out_idx.get());
     out->key_idx_bits = (int32_t)si_rep->idx_bits;
   }
   return rc;
@@ -2998,7 +2988,7 @@ int cm_debug_trace(cm_handle_t h, int which, uint64_t* out, int64_t capacity, in
   std::lock_guard<std::mutex> lk(h->mu);
   if (!h->last) return fail(h, CM_E_INVALID, "nothing has run on this handle");
   Workspace& w = *h->last;
-  const unsigned long long* src = which == 0 ? w.trace_k1 : w.trace_sort;
+  const unsigned long long* src = which == 0 ? w.trace_k1.get() : w.trace_sort.get();
   const size_t cnt = which == 0 ? w.trace_k1_n : w.trace_sort_n;
   *n = (int64_t)cnt;
   if (!src) { *n = 0; return CM_OK; }
