@@ -2812,7 +2812,8 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
     gi.min_b[k] = P.min_b[k]; gi.div_b[k] = P.div_b[k];
   }
   gi.key_bits = (int32_t)P.key_bits;
-  gi.points_total_finite = (int64_t)P.total;
+  // the histogram (and with it P.total) is only built for W > 1; one rank holds the whole cloud
+  gi.points_total_finite = W > 1 ? (int64_t)P.total : n_local - (int64_t)P.n_invalid;
   for (int r = 0; r + 1 < W; ++r) gi.splitter[r] = P.splitter[r];
   if (P.error) return gfail(g, CM_E_KEY_RANGE, "the global voxel grid exceeds the key range (leaf too small for the extent)");
   const float4* vox_in = pts;
@@ -2865,7 +2866,9 @@ int cm_giant_voxelgrid(cm_giant_t g, const float* local_xyzi_dev, int64_t n_loca
   // ---- the ordinary single-GPU VoxelGrid on what arrived, global box folded in, key plan known from the global grid
   const uint32_t* enc_dev = reinterpret_cast<const uint32_t*>(reinterpret_cast<const char*>(g->plan.get()) + offsetof(GiantPlan, enc));
   CM_G_CUDA(g, mark(3));
-  rc = voxelgrid_run(h, vox_in, n_vox, st, enc_dev, (int)P.key_bits);
+  // Non-finite points reach the local VoxelGrid only from this rank's own block (they are never sent away). k_grid_setup keys
+  // them into a sentinel frame, which takes one more key bit: size the key and the pass count for it when there are any.
+  rc = voxelgrid_run(h, vox_in, n_vox, st, enc_dev, (int)P.key_bits + (P.n_invalid ? 1 : 0));
   if (rc == CM_OK && prof && W > 1) {
     CM_G_CUDA(g, mark(4));
     CM_G_CUDA(g, cudaEventSynchronize(g->prof[4].get()));

@@ -245,6 +245,7 @@ struct GiantPlan {
   int32_t min_b[3], div_b[3];
   uint32_t key_bits;                            // bits of the largest voxel index
   uint32_t error;                               // CM_DEV_E_KEY_RANGE: grid outside the key range
+  uint32_t n_invalid;                           // THIS rank's non-finite points (not all-reduced): they stay on this rank
 };
 cudaError_t launch_giant_plan(GiantPlan* plan, const FrameAcc* acc_reduced, const float* inv_leaf3, uint32_t bins, cudaStream_t stream);
 cudaError_t launch_giant_hist(const float4* pts, uint32_t n, const GiantPlan* plan, uint32_t bins, unsigned long long* hist,

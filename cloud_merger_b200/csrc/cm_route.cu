@@ -97,6 +97,7 @@ __global__ void k_giant_plan(GiantPlan* plan, const FrameAcc* __restrict__ acc, 
   if (p.width == 0) p.width = 1;
   p.key_bits = p.cells <= 1ull ? 0u : (uint32_t)(64 - __clzll((long long)(p.cells - 1ull)));
   p.total = 0;
+  p.n_invalid = acc->n_invalid;  // the all-reduce covers max_enc / nmin_enc only: this is the local count
   for (int r = 0; r < CM_MAX_ZONES; ++r) p.splitter[r] = ~0ull;
   *plan = p;
 }

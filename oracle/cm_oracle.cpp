@@ -255,7 +255,12 @@ int64_t voxelgrid_cloud(const Cloud& in, const float* leaf, uint32_t min_points,
   const int64_t dx = static_cast<int64_t>((max_p[0] - min_p[0]) * inv[0]) + 1;
   const int64_t dy = static_cast<int64_t>((max_p[1] - min_p[1]) * inv[1]) + 1;
   const int64_t dz = static_cast<int64_t>((max_p[2] - min_p[2]) * inv[2]) + 1;
-  const bool pcl_overflow = (dx * dy * dz) > static_cast<int64_t>(std::numeric_limits<int32_t>::max());
+  // PCL writes (dx * dy * dz) > INT32_MAX in int64_t, which overflows (undefined) from 2^63 on -- 2^21 cells on every axis.
+  // The product is compared step by step so that every partial product stays below 2^62: the guard trips as it does
+  // mathematically (np_oracle compares the exact product).
+  const int64_t imax = static_cast<int64_t>(std::numeric_limits<int32_t>::max());
+  const bool pcl_overflow = dx > imax || dy > imax || dz > imax || dx < 0 || dy < 0 || dz < 0 || dx * dy > imax ||
+                            dx * dy * dz > imax;
   if (pcl_overflow) {
     if (o.flags) *o.flags |= CMO_FLAG_PCL_OVERFLOW;
     if (!force64) { /* PCL: PCL_WARN(...); output = *input_; return; */

@@ -28,6 +28,7 @@ def main():
     ap.add_argument("--leaf", type=float, default=0.02)
     ap.add_argument("--min-points", type=int, default=1)
     ap.add_argument("--iters", type=int, default=3)
+    ap.add_argument("--nan-every", type=int, default=0, help="K > 0: every K-th point gets a NaN y (non-finite rows, which stay on their rank)")
     ap.add_argument("--check", action="store_true")
     ap.add_argument("--stages", action="store_true", help="one more (profiled, blocking) call after the timed ones: device time per stage")
     a = ap.parse_args()
@@ -40,6 +41,8 @@ def main():
     lo, hi = rank * n // world, (rank + 1) * n // world
     # every rank generates the same cloud chunk-wise and keeps its block (deterministic, no host exchange)
     whole = synth.map_cloud(4, n)
+    if a.nan_every > 0:
+        whole[::a.nan_every, 1] = np.nan
     local = torch.from_numpy(np.ascontiguousarray(whole[lo:hi])).cuda()
     if not a.check:
         whole = None
@@ -102,8 +105,9 @@ def main():
             gathered.sort(key=lambda t: t[0])
             idx = np.concatenate([g[1] for g in gathered]); cnt = np.concatenate([g[2] for g in gathered])
             cen = np.concatenate([g[3] for g in gathered])
-            o = oracle.voxelgrid(whole, [a.leaf] * 3, a.min_points, True, force64=True)
+            o = oracle.voxelgrid(whole, [a.leaf] * 3, a.min_points, True, force64=True, is_dense=a.nan_every <= 0)
             ok = len(idx) == o["n"] and (idx == o["idx"]).all() and (cnt == o["count"]).all()
+            ok = ok and (cen.view(np.uint32) == o["centroid"].view(np.uint32)).all()   # bit-equal to the float oracle
             rel = np.abs(cen - o["centroid_f64"]) / np.maximum(np.abs(o["centroid_f64"]), 1e-2)
             ok = ok and rel.max() <= 1e-5
             check = "ok" if ok else "MISMATCH"

@@ -240,3 +240,135 @@ ORIGIN_BEYOND = 1073741824.0
 
 def bits_for(cells: int) -> int:
     return 0 if cells <= 1 else int(cells - 1).bit_length()
+
+
+# ---- giant-cloud mode: key widths, histogram-bin boundaries, degenerate clouds --------------------------------------------
+# data grids (leaf 1.0) whose voxel index space is exactly 2^bits cells: 8, 16, 24, 40, 48 and 56 are the widths where one
+# more key bit needs one more radix pass, 32 the last one of a 4-byte key
+KEY_WIDTH_DIVS = {8: (16, 16, 1), 16: (256, 256, 1), 24: (256, 256, 256), 31: DIV_2P31, 32: DIV_2P32, 33: DIV_2P32_PLUS,
+                  40: (1 << 20, 1 << 10, 1 << 10), 48: (1 << 16, 1 << 16, 1 << 16), 56: (1 << 21, 1 << 21, 1 << 14),
+                  63: (1 << 21, 1 << 21, 1 << 21)}
+# data grids whose 16384-bin key histogram has a bin width of 1, a power of two (64), an odd non-power of two (63) and one
+# of at least 2^40 (2^40 + 2^28)
+BIN_WIDTH_DIVS = {"w1": (32, 32, 16), "w64": (128, 128, 64), "w63": (101, 101, 101), "w2p40": (1 << 21, 1 << 21, 4097)}
+HIST_BINS = 1 << 14
+
+
+def key_cell_cloud(div, keys, leaf: float = 1.0) -> np.ndarray:
+    """One point at the centre (i + 0.5) * leaf of every given voxel index of the grid div (origin 0; exact in float32 for
+    cells below 2^22 on an axis)."""
+    k = np.asarray(keys, np.int64)
+    d0, d1 = int(div[0]), int(div[1])
+    ijk = np.stack([k % d0, (k // d0) % d1, k // (d0 * d1)], axis=1)
+    out = np.zeros((len(k), 4), F32)
+    out[:, :3] = ((ijk.astype(np.float64) + 0.5) * leaf).astype(F32)
+    out[:, 3] = (k % 251).astype(F32)
+    return out
+
+
+def grid_corner_keys(div) -> list:
+    d0, d1, d2 = (int(v) for v in div)
+    return [i + j * d0 + k * d0 * d1 for k in (0, d2 - 1) for j in (0, d1 - 1) for i in (0, d0 - 1)]
+
+
+def key_width_cloud(seed: int, div, n_filler: int = 20000) -> np.ndarray:
+    """grid_cloud at leaf 1.0 with every filler point inside the box, so that the data grid is div even where an axis has
+    fewer cells than the clump near the origin spans."""
+    x = grid_cloud(seed, div, n_filler=n_filler)
+    hi = (np.asarray(div, np.float64) - 0.5).astype(F32)
+    x[:, :3] = np.minimum(x[:, :3], hi)
+    return x
+
+
+def bin_boundary_keys(div, bins: int = HIST_BINS, ks=None) -> list:
+    """Voxel indices k*width - 1, k*width and k*width + 1 around three bin boundaries (a quarter, half and three quarters of
+    the bins) of the grid's key histogram."""
+    cells = int(div[0]) * int(div[1]) * int(div[2])
+    width = max(1, -(-cells // bins))
+    ks = ks or (bins // 4, bins // 2, 3 * bins // 4)
+    return [k * width + e for k in ks for e in (-1, 0, 1)]
+
+
+def bin_boundary_cloud(div, bins: int = HIST_BINS) -> np.ndarray:
+    """The eight grid corners (they fix the box, so min_b = 0 and div_b = div) and one point at each bin-boundary key. With
+    17 points in all, every running sum from 1 to 15 is a balancing target of 16 ranks: moving any single key into the
+    neighbouring bin moves a splitter."""
+    return key_cell_cloud(div, grid_corner_keys(div) + bin_boundary_keys(div, bins))
+
+
+def with_nonfinite(x, every: int = 500, seed: int = 0) -> np.ndarray:
+    """x with non-finite rows inserted: a copy of a row with NaN on one axis after every `every` rows (at least one), plus
+    three rows with +-inf. The finite rows, and so the grid and the voxels, stay those of x."""
+    rng = np.random.default_rng(seed)
+    x = np.asarray(x, F32)
+    n_nan = max(1, len(x) // every)
+    src = rng.integers(0, max(len(x), 1), size=n_nan + 3) if len(x) else np.zeros(n_nan + 3, np.int64)
+    bad = x[src].copy() if len(x) else np.zeros((n_nan + 3, 4), F32)
+    axis = np.arange(n_nan + 3) % 3
+    bad[np.arange(n_nan), axis[:n_nan]] = np.nan
+    bad[n_nan:, :3][np.arange(3), axis[n_nan:]] = np.array([np.inf, -np.inf, np.inf], F32)
+    pos = np.concatenate([np.minimum(np.arange(1, n_nan + 1) * every, len(x)), rng.integers(0, len(x) + 1, size=3)])
+    return np.insert(x, pos, bad, axis=0)
+
+
+def degenerate_cloud(kind: str, seed: int = 0) -> np.ndarray:
+    """empty; all non-finite; one point; every point in one voxel; 3 finite points (fewer than most rank counts) among
+    non-finite rows; one hot voxel holding 90 % of the points (several balancing targets in one histogram bin)."""
+    rng = np.random.default_rng(seed)
+    if kind == "empty":
+        return np.zeros((0, 4), F32)
+    if kind == "all-nonfinite":
+        x = _filler(rng, 2000, -5.0, 5.0)
+        x[:, 0] = np.nan
+        x[::7, 1] = np.inf
+        x[::11, 2] = -np.inf
+        return x
+    if kind == "one-point":
+        return np.array([[1.25, -3.5, 0.75, 7.0]], F32)
+    if kind == "one-voxel":   # cell 4 of a 0.5 leaf on every axis
+        return _filler(rng, 5000, 2.0625, 2.4375)
+    if kind == "three-finite":
+        x = np.full((300, 4), np.nan, F32)
+        x[[17, 150, 299]] = [[0.5, 0.5, 0.5, 1.0], [-3.5, 7.25, 2.5, 2.0], [9.5, -1.5, -4.5, 3.0]]
+        return x
+    if kind == "hot-voxel":
+        hot = _filler(rng, 27000, 10.125, 10.875)
+        rest = _filler(rng, 3000, -20.0, 20.0)
+        x = np.concatenate([hot, rest])
+        return x[rng.permutation(len(x))]
+    raise ValueError(kind)
+
+
+DEGENERATE_KINDS = ("empty", "all-nonfinite", "one-point", "one-voxel", "three-finite", "hot-voxel")
+
+
+def giant_case(name: str):
+    """(cloud, leaf) of a named giant-cloud edge case (see GIANT_CASES); a "+nf" suffix adds non-finite rows."""
+    if name.endswith("+nf"):
+        x, leaf = giant_case(name[:-3])
+        return with_nonfinite(x, seed=len(name)), leaf
+    kind, arg = name.split(":")
+    if kind == "bits":
+        return key_width_cloud(800 + int(arg), KEY_WIDTH_DIVS[int(arg)]), 1.0
+    if kind == "bin":
+        return bin_boundary_cloud(BIN_WIDTH_DIVS[arg]), 1.0
+    if kind == "A":
+        return lattice_cloud(820, float(arg), n_lattice=30000, n_filler=20000), float(arg)
+    if kind == "C":
+        return offset_cloud(821, float(arg), n=60000), float(arg)
+    if kind == "Z":
+        return signed_zero_subnormal_cloud(822, n_random=3000), float(arg)
+    if kind == "origin":   # ok+ / ok- / beyond+ / beyond-
+        o = {"ok+": ORIGIN_OK, "ok-": -ORIGIN_OK, "beyond+": ORIGIN_BEYOND, "beyond-": -ORIGIN_BEYOND}[arg]
+        return grid_cloud(823, (4, 5, 6), n_filler=5000, origin=(o, 0.0, 0.0)), 1.0
+    if kind == "axis":     # 2^21 cells on x (accepted) and one more (the key range)
+        return grid_cloud(824, ((1 << 21) + (arg == "2p21+"), 3, 2), n_filler=5000), 1.0
+    if kind == "deg":
+        return degenerate_cloud(arg, 825), 0.5
+    raise ValueError(name)
+
+
+GIANT_CASES = (["bits:%d" % b for b in KEY_WIDTH_DIVS] + ["bin:%s" % w for w in BIN_WIDTH_DIVS] +
+               ["A:0.1", "A:0.035", "C:0.05", "Z:0.05", "origin:ok+", "origin:ok-", "axis:2p21"] +
+               ["deg:%s" % k for k in DEGENERATE_KINDS])
+GIANT_RANGE_CASES = ("origin:beyond+", "origin:beyond-", "axis:2p21+")

@@ -144,23 +144,28 @@ def test_giant_dry_routing_four_virtual_ranks(gpu_ok):
     assert max(sizes) < 1.3 * n / world, "splitters balance the point counts (%r)" % sizes
 
 
-@pytest.mark.parametrize("exchange", ["peer", "nccl"])
+@pytest.mark.parametrize("exchange", ["peer", "nccl", "peer-nonfinite"])
 def test_giant_cloud_two_ranks_nccl(gpu_ok, exchange):
     """Two ranks, both exchanges: the grouping kernel storing into the peer's receive buffer over NVLink (the default
     where CUDA IPC maps the peers) and the grouped ncclSend / ncclRecv (CM_GIANT_NO_P2P=1); the merged voxels of both are
-    checked against the oracle on the whole cloud."""
+    checked against the oracle on the whole cloud. The non-finite case puts a NaN in every 997th point: at leaf 0.1 this
+    cloud's index is 32 bits wide, so the sentinel frame of those points makes every rank's local key 33 bits."""
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
     env = dict(os.environ, CM_GIANT_NO_P2P="1" if exchange == "nccl" else "0")
+    port = {"peer": "29617", "nccl": "29619", "peer-nonfinite": "29621"}[exchange]
+    extra = ["--nan-every", "997"] if exchange.endswith("nonfinite") else []
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-                        "--master-addr", "127.0.0.1", "--master-port", "29617" if exchange == "peer" else "29619",
+                        "--master-addr", "127.0.0.1", "--master-port", port,
                         os.path.join(ROOT, "scripts", "giant_cloud.py"),
-                        "--points", "2000000", "--leaf", "0.1", "--check"], capture_output=True, text=True, timeout=600, cwd=ROOT,
-                       env=env)
+                        "--points", "2000000", "--leaf", "0.1", "--check"] + extra, capture_output=True, text=True,
+                       timeout=600, cwd=ROOT, env=env)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
     line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
     assert line["check"] == "ok" and line["n_gpus"] == 2
+    if exchange.endswith("nonfinite"):
+        assert line["key_bits"] == 33
     if exchange == "nccl":
         assert line["exchange"] == "nccl"
     else:
