@@ -20,6 +20,14 @@ class CmPass(C.Structure):
     _fields_ = [("axis", C.c_int32), ("lo", C.c_float), ("hi", C.c_float), ("negative", C.c_int32)]
 
 
+CM_MAX_CROP_BOXES = 8
+
+
+class CmCropBox(C.Structure):
+    _fields_ = [("min", C.c_float * 3), ("max", C.c_float * 3), ("translation", C.c_float * 3), ("rotation", C.c_float * 3),
+                ("transform", C.c_float * 12), ("negative", C.c_int32), ("reserved", C.c_int32)]
+
+
 CM_MAX_ZONES = 16
 CM_MAX_ZONE_PASSES = 4
 
@@ -151,6 +159,7 @@ SYMBOLS = {
     "cm_set_extrinsic_tf": (C.c_int, [_H, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "cm_get_extrinsic": (C.c_int, [_H, C.c_int, C.POINTER(C.c_float)]),
     "cm_set_crop": (C.c_int, [_H, C.c_int, C.POINTER(CmPass)]),
+    "cm_set_crop_boxes": (C.c_int, [_H, C.c_int, C.POINTER(CmCropBox)]),
     "cm_set_voxel": (C.c_int, [_H, C.POINTER(C.c_float), C.c_int, C.c_int]),
     "cm_set_voxel_bounds": (C.c_int, [_H, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "cm_set_overflow_mode": (C.c_int, [_H, C.c_int]),

@@ -12,8 +12,8 @@ from typing import Iterable, List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (CM_MAX_ZONES, CM_MAX_ZONE_PASSES, CmConfig, CmDeviceOut, CmFrameInfo, CmFrameOut, CmLayout, CmPass,
-                   CmSegment, CmStats, CmZone, CmZoneOut)
+from ._lib import (CM_MAX_ZONES, CM_MAX_ZONE_PASSES, CmConfig, CmCropBox, CmDeviceOut, CmFrameInfo, CmFrameOut, CmLayout,
+                   CmPass, CmSegment, CmStats, CmZone, CmZoneOut)
 
 # ---- layouts the reference's sensors produce (SURVEY.md section 8b) ------------------------------------------------------
 LAYOUT_PACKED16 = dict(point_step=16, off_x=0, off_y=4, off_z=8, off_intensity=12)   # float4 x y z intensity
@@ -23,6 +23,24 @@ LAYOUT_LIVOX18 = dict(point_step=18, off_x=0, off_y=4, off_z=8, off_intensity=12
 
 # getROI defaults, pcl_preprocessing/src/Parameter.h:31-35 (axis, lo, hi, negative)
 ROI_PASSES = [(2, -0.5, 3.0, 0), (1, -5.0, 5.0, 0), (0, -15.0, 60.0, 0)]
+
+
+IDENTITY_3X4 = (1.0, 0.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 0.0, 1.0, 0.0)
+
+
+def make_crop_box(min_pt, max_pt, translation=(0.0, 0.0, 0.0), rotation=(0.0, 0.0, 0.0), transform=IDENTITY_3X4,
+                  negative: bool = False) -> CmCropBox:
+    """One pcl::CropBox stage: setMin / setMax, setTranslation, setRotation (roll, pitch, yaw in rad), setTransform (3x4 or
+    4x4 row-major; the identity is PCL's default) and setNegative."""
+    t = np.asarray(transform, np.float32).reshape(-1)[:12]
+    b = CmCropBox()
+    for k in range(3):
+        b.min[k] = float(np.float32(min_pt[k])); b.max[k] = float(np.float32(max_pt[k]))
+        b.translation[k] = float(np.float32(translation[k])); b.rotation[k] = float(np.float32(rotation[k]))
+    for k in range(12):
+        b.transform[k] = float(t[k])
+    b.negative = int(bool(negative))
+    return b
 
 
 class CloudMergerError(RuntimeError):
@@ -158,6 +176,13 @@ class CloudMerger:
         for i, (axis, lo, hi, neg) in enumerate(passes):
             arr[i] = CmPass(int(axis), float(np.float32(lo)), float(np.float32(hi)), int(neg))
         self._check(self._lib.cm_set_crop(self._h, len(passes), arr))
+
+    def set_crop_boxes(self, boxes: Sequence[CmCropBox]):
+        """pcl::CropBox stages after the PassThrough chain, in order (<= 8; see make_crop_box); [] switches them off. The
+        usual one removes the vehicle's own body: make_crop_box(lo, hi, negative=True)."""
+        boxes = list(boxes)
+        arr = (CmCropBox * max(len(boxes), 1))(*boxes)
+        self._check(self._lib.cm_set_crop_boxes(self._h, len(boxes), arr))
 
     # -- zone slicing: getCloudPart x5 + the z windows of removeGround in one pass (pc_preprocessing_main.cpp:49-92, 228-312)
     def set_zones(self, zones: Sequence[Sequence[Tuple[int, float, float, int]]]):

@@ -78,6 +78,8 @@ struct Workspace {
   std::vector<SegDev> segs_host;  // what is currently uploaded
   DevPtr<uint32_t> tile_seg;
   std::vector<uint32_t> tile_seg_host;
+  DevPtr<OrientedBoxDev> obox;               // CropBox stages (allocated on first use)
+  std::vector<OrientedBoxDev> obox_host;     // what is currently uploaded
   DevPtr<float4> surv_xyzi;
   DevPtr<uint32_t> surv_src;
   DevPtr<uint32_t> surv_key;             // box-grid voxel keys written by K1 (fused-key runs)
@@ -169,6 +171,8 @@ struct cm_handle_s {
   // configuration
   float mats_host[CM_MAX_SENSORS * 12];
   CropDev crop{};
+  OrientedBoxDev obox[CM_MAX_CROP_BOXES]{};  // cm_set_crop_boxes
+  int n_obox = 0;
   float leaf[3] = {0.1f, 0.1f, 0.1f};
   float inv_leaf[3] = {10.f, 10.f, 10.f};
   uint32_t min_points = 2;
@@ -753,6 +757,16 @@ int run_pipeline(cm_handle_t h, Workspace& w, const cm_segment_t* segs, int n_se
   kp.surv_key = fused ? w.surv_key.get() : nullptr;
   kp.hist = reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_hist);
   kp.box = box;
+  kp.obox = nullptr; kp.n_obox = 0;
+  if (h->n_obox > 0) {  // the stage table travels like the segment table: uploaded on the run's stream when it changed
+    const std::vector<OrientedBoxDev> ob(h->obox, h->obox + h->n_obox);
+    if (!w.obox) CM_CUDA(h, dev_alloc(w.obox, CM_MAX_CROP_BOXES));
+    if (ob.size() != w.obox_host.size() || memcmp(ob.data(), w.obox_host.data(), ob.size() * sizeof(OrientedBoxDev)) != 0) {
+      CM_CUDA(h, cudaMemcpyAsync(w.obox.get(), ob.data(), ob.size() * sizeof(OrientedBoxDev), cudaMemcpyHostToDevice, st));
+      w.obox_host = ob;
+    }
+    kp.obox = w.obox.get(); kp.n_obox = (uint32_t)h->n_obox;
+  }
   w.n_k1_tiles = plan.n_tiles;
   w.dense_valid = false;
   CM_CUDA(h, launch_transform_crop(kp, plan.tile_points, plan.mode, plan.staged_smem, st));
@@ -978,6 +992,8 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
     key.assign(reinterpret_cast<const char*>(segs.data()), segs.size() * sizeof(cm_segment_t));
     for (const cm_segment_t& g : segs) key.append(reinterpret_cast<const char*>(h->mats_host + g.sensor * 12), 12 * sizeof(float));
     key.append(reinterpret_cast<const char*>(&h->crop), sizeof(h->crop));
+    key.append(reinterpret_cast<const char*>(&h->n_obox), sizeof(h->n_obox));  // the graph reads the stage table uploaded
+    key.append(reinterpret_cast<const char*>(h->obox), h->n_obox * sizeof(OrientedBoxDev));  // by the run it was captured in
     key.append(reinterpret_cast<const char*>(h->inv_leaf), sizeof(h->inv_leaf));
     key.append(reinterpret_cast<const char*>(&h->min_points), sizeof(h->min_points));
     key.append(reinterpret_cast<const char*>(&h->downsample_all), sizeof(h->downsample_all));
@@ -1273,6 +1289,66 @@ int cm_set_crop(cm_handle_t h, int n_pass, const cm_pass_t* passes) {
   h->crop.n_pass = n_pass;
   for (int k = 0; k < n_pass; ++k) h->crop.pass[k] = PassDev{passes[k].axis, passes[k].lo, passes[k].hi, passes[k].negative ? 1 : 0};
   derive_crop_box(h->crop);
+  return CM_OK;
+}
+
+namespace {
+// Eigen 3.3 MatrixBase::isIdentity() with dummy_precision<float>() = 1e-5 on an Affine3f's matrix (its fourth row is exactly
+// 0 0 0 1): relative on the diagonal (isApprox), absolute off it (isMuchSmallerThan).
+bool eigen_is_identity(const float* m12) {
+  const float prec = 1e-5f;
+  for (int r = 0; r < 3; ++r)
+    for (int c = 0; c < 4; ++c) {
+      const float v = m12[r * 4 + c];
+      if (r == c ? !(std::fabs(v - 1.0f) <= std::min(std::fabs(v), 1.0f) * prec) : !(std::fabs(v) <= prec)) return false;
+    }
+  return true;
+}
+
+// What pcl::CropBox<PointT>::applyFilter (PCL 1.8.1) derives from its settings before the point loop, in float as it does.
+void derive_obox(const cm_crop_box_t& b, OrientedBoxDev& d) {
+  memset(&d, 0, sizeof(d));
+  memcpy(d.t, b.transform, sizeof(d.t));
+  memcpy(d.tr, b.translation, sizeof(d.tr));
+  memcpy(d.mn, b.min, sizeof(d.mn));
+  memcpy(d.mx, b.max, sizeof(d.mx));
+  d.flags = b.negative ? OBOX_NEGATIVE : 0u;
+  if (!eigen_is_identity(b.transform)) d.flags |= OBOX_TRANSFORM;
+  if (b.translation[0] != 0.f || b.translation[1] != 0.f || b.translation[2] != 0.f) d.flags |= OBOX_TRANSLATE;
+  const float roll = b.rotation[0], pitch = b.rotation[1], yaw = b.rotation[2];
+  if (roll != 0.f || pitch != 0.f || yaw != 0.f) {
+    // pcl::getTransformation(0, 0, 0, roll, pitch, yaw): float cos / sin
+    const float A = std::cos(yaw), B = std::sin(yaw), C = std::cos(pitch), D = std::sin(pitch), E = std::cos(roll),
+                F = std::sin(roll), DE = D * E, DF = D * F;
+    const float m[3][3] = {{A * C, A * DF - B * E, B * F + A * DE}, {B * C, A * E + B * DF, B * DE - A * F}, {-D, C * F, C * E}};
+    // Transform::inverse() (Affine): the linear part by Eigen's 3x3 cofactor inverse, then translation = -linear * (0, 0, 0)
+    auto cof = [&](int i, int j) {
+      const int i1 = (i + 1) % 3, i2 = (i + 2) % 3, j1 = (j + 1) % 3, j2 = (j + 2) % 3;
+      return m[i1][j1] * m[i2][j2] - m[i1][j2] * m[i2][j1];
+    };
+    const float det = (cof(0, 0) * m[0][0] + cof(1, 0) * m[1][0]) + cof(2, 0) * m[2][0];
+    const float invdet = 1.0f / det;
+    for (int i = 0; i < 3; ++i) {
+      for (int j = 0; j < 3; ++j) d.r[i * 4 + j] = cof(j, i) * invdet;
+      d.r[i * 4 + 3] = ((-d.r[i * 4 + 0]) * 0.0f + (-d.r[i * 4 + 1]) * 0.0f) + (-d.r[i * 4 + 2]) * 0.0f;
+    }
+    if (!eigen_is_identity(d.r)) d.flags |= OBOX_ROTATE;
+  }
+}
+}  // namespace
+
+int cm_set_crop_boxes(cm_handle_t h, int n_boxes, const cm_crop_box_t* boxes) {
+  if (!h) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  if (n_boxes < 0 || n_boxes > CM_MAX_CROP_BOXES || (n_boxes > 0 && !boxes))
+    return fail(h, CM_E_INVALID, "0..%d crop boxes", CM_MAX_CROP_BOXES);
+  for (int k = 0; k < n_boxes; ++k)
+    for (int a = 0; a < 3; ++a)
+      if (std::isnan(boxes[k].min[a]) || std::isnan(boxes[k].max[a])) return fail(h, CM_E_INVALID, "crop box %d: NaN limit", k);
+  OrientedBoxDev d[CM_MAX_CROP_BOXES]{};
+  for (int k = 0; k < n_boxes; ++k) derive_obox(boxes[k], d[k]);
+  memcpy(h->obox, d, sizeof(d));
+  h->n_obox = n_boxes;
   return CM_OK;
 }
 

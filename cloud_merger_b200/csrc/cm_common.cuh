@@ -70,6 +70,25 @@ struct CropDev {
   float lo[4], hi[4];
 };
 
+// ---- pcl::CropBox stages after the PassThrough chain (cm_set_crop_boxes) ---------------------------------------------
+// One stage with everything PCL derives per filter() call precomputed on the host: the three skip decisions (Eigen's fuzzy
+// isIdentity / the exact zero compares) and the float inverse of the rotation. Not the collapsed axis-aligned chain
+// (CropDev::is_box / BoxGrid): these boxes are oriented and may be negative.
+#define CM_MAX_CROP_BOXES 8
+#define OBOX_TRANSFORM 1u    // local = transform * p
+#define OBOX_TRANSLATE 2u    // local -= translation
+#define OBOX_ROTATE 4u       // local = inverse rotation * local
+#define OBOX_NEGATIVE 8u
+struct OrientedBoxDev {  // 144 bytes: nine 16-byte loads
+  float t[12];           // setTransform, rows 0..2 row-major
+  float r[12];           // inverse of the rotation (an Affine3f: its translation column is +-0)
+  float tr[3];           // setTranslation
+  float mn[3], mx[3];
+  uint32_t flags;        // OBOX_*
+  uint32_t pad_[2];
+};
+static_assert(sizeof(OrientedBoxDev) == 144, "OrientedBoxDev is loaded as 16-byte words");
+
 // ---- zone slicing (cm_zones.cu): several PassThrough chains evaluated in one pass ---------------------------------------
 #define CM_MAX_ZONES 16
 #define CM_MAX_ZONE_PASSES 4

@@ -40,6 +40,8 @@ struct K1Params {
   BoxGrid box;
   TileRec* tile_rec;           // [n_tiles] out: count / slot0 / frame of every tile
   unsigned long long* trace;   // debug: 8 clock64 stamps per tile, or null
+  const OrientedBoxDev* obox;  // [n_obox] CropBox stages after the crop chain (device memory, loaded into shared memory)
+  uint32_t n_obox;             // 0: the box-free kernels run
 };
 uint32_t k1_tile_points(int64_t total_points);
 uint32_t k1_min_tile_points();

@@ -6,6 +6,7 @@
 //   * pcl_ros::transformPointCloud                      pc_preprocessing_main.cpp:322,348,373,399,426,465
 //   * the pcl::PassThrough chains getROI/getCloudPart   pc_preprocessing_main.cpp:20-59 (and CloudFusionNode.h:145-216)
 //   * the operator+= concatenation in fusePointclouds   pc_preprocessing_main.cpp:137-149
+//   * pcl::CropBox stages after the chain (vehicle body) (PCL 1.8.1 crop_box.hpp; cm_set_crop_boxes)
 //   * pcl::getMinMax3D, the first step of VoxelGrid     (PCL 1.8.1 voxel_grid.hpp)
 //
 // Roofline: HBM. Algorithmic bytes per launch = sum(n_points * point_step) + survivors * (16 + 4).
@@ -17,7 +18,8 @@
 // counts into dense offsets (frame starts, totals), and the VoxelGrid kernels address survivors by slot. A dense copy of
 // the merged cloud is produced by k_compact_survivors only when a caller asks for it. The kernel is specialised at
 // compile time on the record layout (16-byte packed, 32-byte PCL, generic) and on the crop kind (one
-// box vs. a general chain), which keeps the per-point instruction count low enough to stay memory-bound.
+// box vs. a general chain) and on whether CropBox stages follow (OBOX; without them the kernels are what they were before
+// those stages existed), which keeps the per-point instruction count low enough to stay memory-bound.
 #include <cstdlib>
 
 #include "cm_kernels.h"
@@ -75,6 +77,31 @@ __device__ __forceinline__ bool pass_keeps(const PassDev& ps, float x, float y, 
   return !(v >= ps.lo && v <= ps.hi);
 }
 
+// One row of pcl::transformPoint: ((m0*x + m1*y) + m2*z) + m3, every operation rounded on its own.
+__device__ __forceinline__ float affine_row(const float* m, float x, float y, float z) {
+  return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], x), __fmul_rn(m[1], y)), __fmul_rn(m[2], z)), m[3]);
+}
+
+// One pcl::CropBox stage (PCL 1.8.1 CropBox::applyFilter) on a point that reached it; true = kept. The three steps are
+// applied one after another, as PCL does: composing them into one matrix would round differently.
+__device__ __forceinline__ bool obox_keeps(const OrientedBoxDev& b, float x, float y, float z) {
+  const uint32_t f = b.flags;
+  if (f & OBOX_TRANSFORM) {
+    const float u = affine_row(b.t, x, y, z), v = affine_row(b.t + 4, x, y, z), w = affine_row(b.t + 8, x, y, z);
+    x = u; y = v; z = w;
+  }
+  if (f & OBOX_TRANSLATE) {
+    x = __fsub_rn(x, b.tr[0]); y = __fsub_rn(y, b.tr[1]); z = __fsub_rn(z, b.tr[2]);
+  }
+  if (f & OBOX_ROTATE) {
+    const float u = affine_row(b.r, x, y, z), v = affine_row(b.r + 4, x, y, z), w = affine_row(b.r + 8, x, y, z);
+    x = u; y = v; z = w;
+  }
+  // a NaN coordinate fails every compare: it counts as inside
+  const bool outside = (x < b.mn[0]) | (y < b.mn[1]) | (z < b.mn[2]) | (x > b.mx[0]) | (y > b.mx[1]) | (z > b.mx[2]);
+  return outside == ((f & OBOX_NEGATIVE) != 0u);
+}
+
 // BOX: 0 = general PassThrough chain, 1 = one x/y/z box, 2 = box that also windows the intensity
 // min/max folded only when `on` (predicated instructions, no branch, no select)
 __device__ __forceinline__ void minmax_if(bool on, float v, float& mn, float& mx) {
@@ -83,7 +110,7 @@ __device__ __forceinline__ void minmax_if(bool on, float v, float& mn, float& mx
       : "r"((int)on), "f"(v));
 }
 
-template <int THREADS, int IPT, int MODE, int BOX, bool KEYS>
+template <int THREADS, int IPT, int MODE, int BOX, bool KEYS, bool OBOX>
 __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform_crop(const K1Params p) {
   constexpr int TILE = THREADS * IPT;
   constexpr int WARPS = THREADS / 32;
@@ -101,6 +128,17 @@ __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform
   const long long tr0 = clock64();
   if (KEYS && tid < CM_RADIX) s_hist[tid] = 0u;  // ordered by the barrier further down
 #define K1_TRACE(i) do { if (p.trace && tid == 0) p.trace[(size_t)tile * 8 + (i)] = (unsigned long long)(clock64() - tr0); } while (0)
+  // CropBox stages: the table goes to shared memory once per CTA in 16-byte words (ordered by the barrier after the unpack)
+  const OrientedBoxDev* sbox = nullptr;
+  uint32_t n_obox = 0;
+  if constexpr (OBOX) {
+    __shared__ __align__(16) OrientedBoxDev s_obox[CM_MAX_CROP_BOXES];
+    n_obox = p.n_obox;
+    const uint4* src = reinterpret_cast<const uint4*>(p.obox);
+    for (uint32_t k = tid; k < n_obox * (uint32_t)(sizeof(OrientedBoxDev) / 16); k += THREADS)
+      reinterpret_cast<uint4*>(s_obox)[k] = __ldg(src + k);
+    sbox = s_obox;
+  }
 
   // which segment owns this tile: uniform batches by division, others through the host-built table
   const uint32_t seg_id = p.tiles_per_seg ? (tile / p.tiles_per_seg) : __ldg(p.tile_seg + tile);
@@ -238,6 +276,7 @@ __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform
     }
   }
   K1_TRACE(0);
+  if (OBOX) __syncthreads();
 
   float m[12];
 #pragma unroll
@@ -265,6 +304,10 @@ __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform
       z[i] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[8], a), __fmul_rn(m[9], b)), __fmul_rn(m[10], c)), m[11]);
       keep = in_range & (x[i] >= lo0) & (x[i] <= hi0) & (y[i] >= lo1) & (y[i] <= hi1) & (z[i] >= lo2) & (z[i] <= hi2);
       if (BOX == 2) keep = keep & (it[i] >= lo3) & (it[i] <= hi3);
+      // CropBox stages: their input is dense (PassThrough output) and every survivor of the box is finite; a warp whose
+      // item the box already rejected everywhere skips them
+      if (OBOX && __any_sync(0xFFFFFFFFu, keep))
+        for (uint32_t k = 0; k < n_obox; ++k) keep = keep & obox_keeps(sbox[k], x[i], y[i], z[i]);
       fold = keep;
     } else {
       const bool fin_in = finite_f32(a) && finite_f32(b) && finite_f32(c);
@@ -279,6 +322,13 @@ __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform
       if (n_pass > 0) {
         keep = keep && fin;
         for (int k = 0; k < n_pass; ++k) keep = keep && pass_keeps(p.crop.pass[k], x[i], y[i], z[i], it[i]);
+      }
+      if (OBOX) {
+        // the first CropBox stage removes non-finite points when its input is not dense: with no pass in front, that is
+        // the segment's own flag (PCL marks every filter output dense)
+        if (n_pass == 0 && !dense) keep = keep && fin;
+        if (__any_sync(0xFFFFFFFFu, keep))
+          for (uint32_t k = 0; k < n_obox; ++k) keep = keep & obox_keeps(sbox[k], x[i], y[i], z[i]);
       }
       fold = keep && fin;
       inv_run += __popc(__ballot_sync(0xFFFFFFFFu, keep && !fin));
@@ -378,10 +428,10 @@ __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform
   K1_TRACE(5);
 }
 
-template <int THREADS, int IPT>
+template <int THREADS, int IPT, bool OBOX>
 cudaError_t launch_cfg(const K1Params& p, int mode, int box, uint32_t smem, cudaStream_t stream) {
   const bool keys = p.surv_key != nullptr && box != 0;
-#define CM_K1_LAUNCH(MODE, BOX, KEYS) k_transform_crop<THREADS, IPT, MODE, BOX, KEYS><<<p.n_tiles, THREADS, smem, stream>>>(p)
+#define CM_K1_LAUNCH(MODE, BOX, KEYS) k_transform_crop<THREADS, IPT, MODE, BOX, KEYS, OBOX><<<p.n_tiles, THREADS, smem, stream>>>(p)
 #define CM_K1_BOX(MODE) do { if (box == 1) { if (keys) CM_K1_LAUNCH(MODE, 1, true); else CM_K1_LAUNCH(MODE, 1, false); } \
                              else if (box == 2) { if (keys) CM_K1_LAUNCH(MODE, 2, true); else CM_K1_LAUNCH(MODE, 2, false); } \
                              else CM_K1_LAUNCH(MODE, 0, false); } while (0)
@@ -409,8 +459,10 @@ cudaError_t configure_device_kernels() {
   const int big = 200 * 1024;  // the host falls back to 1024-point tiles when a staged layout needs more
   const int small = (int)k1_staged_smem(1024u, CM_MAX_STAGED_STEP);
   cudaError_t e;
-#define CM_K1_ATTR(T, I, B, K, BYTES)                                                                                      \
-  e = cudaFuncSetAttribute(k_transform_crop<T, I, MODE_GENERIC, B, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES); \
+#define CM_K1_ATTR(T, I, B, K, BYTES)                                                                                            \
+  e = cudaFuncSetAttribute(k_transform_crop<T, I, MODE_GENERIC, B, K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES); \
+  if (e != cudaSuccess) return e;                                                                                                  \
+  e = cudaFuncSetAttribute(k_transform_crop<T, I, MODE_GENERIC, B, K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BYTES);  \
   if (e != cudaSuccess) return e;
   CM_K1_ATTR(512, 8, 0, false, big) CM_K1_ATTR(512, 8, 1, false, big) CM_K1_ATTR(512, 8, 2, false, big)
   CM_K1_ATTR(512, 8, 1, true, big) CM_K1_ATTR(512, 8, 2, true, big)
@@ -424,8 +476,12 @@ cudaError_t launch_transform_crop(const K1Params& p, uint32_t tile_points, int m
                                   cudaStream_t stream) {
   if (p.n_tiles == 0) return cudaSuccess;
   const int box = p.crop.is_box ? (p.crop.use_i ? 2 : 1) : 0;
-  if (tile_points == 4096u) return launch_cfg<512, 8>(p, mode, box, staged_smem_bytes, stream);
-  return launch_cfg<256, 4>(p, mode, box, staged_smem_bytes, stream);
+  if (p.n_obox) {
+    if (tile_points == 4096u) return launch_cfg<512, 8, true>(p, mode, box, staged_smem_bytes, stream);
+    return launch_cfg<256, 4, true>(p, mode, box, staged_smem_bytes, stream);
+  }
+  if (tile_points == 4096u) return launch_cfg<512, 8, false>(p, mode, box, staged_smem_bytes, stream);
+  return launch_cfg<256, 4, false>(p, mode, box, staged_smem_bytes, stream);
 }
 
 }  // namespace cm

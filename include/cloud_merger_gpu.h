@@ -63,6 +63,29 @@ typedef struct {
   int32_t negative;
 } cm_pass_t;
 
+/* ---- crop: pcl::CropBox stages after the PassThrough chain ----
+ * Replaces pcl::CropBox<pcl::PointXYZI> with setMin / setMax / setTranslation / setRotation / setTransform / setNegative
+ * (PCL 1.8.1 filters/impl/crop_box.hpp): most often a negative box that removes the vehicle's own body (or a mirror, a roof
+ * rack) from the merged cloud, which an AND-ed PassThrough chain cannot express. The boxes run in the given order after the
+ * PassThrough chain, each on the previous stage's output, and test the extrinsic-transformed coordinates; survivors keep
+ * those coordinates and their input order. Per point and box, as PCL does it: a non-finite x, y or z is removed when the
+ * stage's input is not dense (only the first box of a chain without passes sees a non-dense input: the segment's
+ * is_dense); then local = transform * p (skipped when transform is the identity within Eigen's 1e-5), local -= translation
+ * (when it is not exactly zero), local = inverse(rotation) * local (rotation = roll, pitch, yaw about x, y, z; skipped when
+ * it is exactly zero or its inverse is the identity within 1e-5). The point is outside when any local coordinate is below
+ * min or above max; negative keeps the outside, otherwise the inside is kept (a NaN coordinate counts as inside). Applies
+ * to cm_merge_frame[_async], cm_run_batch and cm_dev_transform_crop; not to zone slicing or the giant-cloud mode.
+ * cm_set_crop_boxes with 0 boxes switches them off (the default); NaN limits are refused (CM_E_INVALID). */
+#define CM_MAX_CROP_BOXES 8
+typedef struct {
+  float min[3], max[3];   /* setMin / setMax (PCL's 4th component is not tested) */
+  float translation[3];   /* setTranslation */
+  float rotation[3];      /* setRotation: roll, pitch, yaw (rad) */
+  float transform[12];    /* setTransform: row-major 3x4 of the Eigen::Affine3f; identity = PCL's default */
+  int32_t negative;       /* setNegative */
+  int32_t reserved;
+} cm_crop_box_t;
+
 /* ---- zone slicing: several PassThrough chains over ONE cloud, one ordered output per chain ----
  * Replaces the getCloudPart x5 + z-window sequences the reference runs per sensor cloud in proceedFront / proceedRear /
  * proceedTop / proceedLivox (pc_preprocessing_main.cpp:49-59, 80-92, 228-312: one PassThrough on "x" for
@@ -249,6 +272,8 @@ CM_API int cm_set_extrinsic_tf(cm_handle_t h, int sensor, const double* quat_xyz
 CM_API int cm_get_extrinsic(cm_handle_t h, int sensor, float* m12_row_major);
 /* cm_set_crop replaces the PassThrough chains (see cm_pass_t). Defaults = getROI with Parameter.h:31-35. */
 CM_API int cm_set_crop(cm_handle_t h, int n_pass, const cm_pass_t* passes);
+/* cm_set_crop_boxes replaces the pcl::CropBox stages that follow the PassThrough chain (see cm_crop_box_t). */
+CM_API int cm_set_crop_boxes(cm_handle_t h, int n_boxes, const cm_crop_box_t* boxes);
 /* cm_set_voxel replaces voxel_grid.setLeafSize / setDownsampleAllData / setMinimumPointsNumberPerVoxel
  * (pc_preprocessing_main.cpp:171-175). Defaults: leaf 0.1, min_points 2, downsample_all 1 (Parameter.h:27-28). */
 CM_API int cm_set_voxel(cm_handle_t h, const float* leaf3, int min_points, int downsample_all);
