@@ -1222,7 +1222,11 @@ int cm_create(const cm_config_t* cfg, cm_handle_t* out) {
   if (c.max_batch_points > 0xFFFFFFF0ll) { delete h; return CM_E_CAPACITY; }
   h->device = c.device;
   if (cudaSetDevice(h->device) != cudaSuccess) { delete h; return CM_E_CUDA; }
-  if (configure_device_kernels() != cudaSuccess || configure_sort_kernels() != cudaSuccess) { delete h; return CM_E_CUDA; }
+  if (configure_device_kernels() != cudaSuccess || configure_sort_kernels() != cudaSuccess ||
+      configure_centroid_kernels() != cudaSuccess) {
+    delete h;
+    return CM_E_CUDA;
+  }
   if (getenv("CM_NO_GRAPH")) h->use_graph = false;
   for (int s = 0; s < CM_MAX_SENSORS; ++s) {
     float* m = h->mats_host + s * 12;

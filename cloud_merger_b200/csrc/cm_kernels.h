@@ -276,5 +276,6 @@ uint32_t centroid_tile_items();
 // per-device one-time kernel attribute setup (opt-in shared memory sizes)
 cudaError_t configure_device_kernels();
 cudaError_t configure_sort_kernels();
+cudaError_t configure_centroid_kernels();
 
 }  // namespace cm

@@ -27,12 +27,16 @@ constexpr int SCAN_THREADS = 1024;
 #ifndef KH_UNROLL
 #define KH_UNROLL 8
 #endif
+#ifndef CE_ASYNC_GATHER
+#define CE_ASYNC_GATHER 1  // the count sweep of the next tile gathers its points by cp.async into a second buffer (0: the
+#endif                     // tile's item phase reads its records again and gathers synchronously -- the round-2 kernel)
 #ifndef CE_MIN_CTAS
-#define CE_MIN_CTAS 4
+#define CE_MIN_CTAS (CE_ASYNC_GATHER ? 3 : 4)  // two 32 KB point buffers: 70 KB per CTA, 3 CTAs per SM
 #endif
 #ifndef CE_PREFETCH
 #define CE_PREFETCH 0   // tried: L2 prefetch of the next tile's points from the count sweep. cfg3 batch: no change (0.148 vs 0.146 ms);
 #endif                  // cfg5 sweep: 17 % SLOWER (every point is gathered there and the prefetch only adds requests). Off.
+                        // (CE_ASYNC_GATHER 0 only: the asynchronous gather replaces it)
 #ifndef CE_LB_POLL_ONE
 #define CE_LB_POLL_ONE 0
 #endif
@@ -41,6 +45,17 @@ constexpr int SCAN_THREADS = 1024;
 #endif
 constexpr int CE_IPT = 8;
 constexpr int CE_TILE = VX_THREADS * CE_IPT;  // 2048 sorted items per centroid tile
+constexpr int CE_PT_BUFS = CE_ASYNC_GATHER ? 2 : 1;
+constexpr size_t CE_DYN_SMEM = (size_t)CE_PT_BUFS * CE_TILE * sizeof(float4);  // the point buffers (dynamic shared memory)
+
+// 16-byte global -> shared copy that completes asynchronously (LDGSTS; .cg: cached in L2 only), and its group fences
+__device__ __forceinline__ void cp_async_16(void* smem_dst, const void* gmem_src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src)
+               : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int PENDING>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(PENDING) : "memory"); }
 
 // Exclusive scan of one value per thread over a 1024-thread block. Returns the exclusive prefix; *total = block sum.
 __device__ __forceinline__ uint32_t block_excl_scan_1024(uint32_t v, uint32_t* scratch /* 33 words */, uint32_t* total) {
@@ -565,8 +580,8 @@ __global__ void __launch_bounds__(VX_THREADS) k_seg_keys64(const uint2* __restri
 //
 // Two phases per 2048-item tile, both with every lane busy:
 //   per item  (thread t owns items 8t .. 8t+7): records in with 16-byte loads, neighbour keys by shuffle, head-of-run
-//             and min-points flags as bit masks, the points of surviving runs gathered into shared memory (independent
-//             loads, all in flight together), one head bit per item into a shared bit array;
+//             and min-points flags as bit masks, the points of surviving runs gathered into shared memory (asynchronous
+//             copies issued one tile ahead, in the count sweep below), one head bit per item into a shared bit array;
 //   per voxel (thread r owns the r-th surviving run of the tile, found through the block scan of the per-thread
 //             counts): end of run from the head bit array, sequential sum over shared memory (the part of a run that
 //             continues past the tile is read from global memory), division, coalesced tile-local output.
@@ -690,7 +705,7 @@ __global__ void __launch_bounds__(VX_THREADS, CE_MIN_CTAS) k_voxel_centroid(cons
   constexpr bool REC = SEG || sizeof(KeyT) == 4;  // 8-byte (key, value) records
   __shared__ uint32_t s_fss[SEG ? CE_SEG_SMEM_FRAMES + 1 : 1];
   __shared__ uint32_t s_scan[9];
-  __shared__ __align__(16) float4 s_pts[CE_TILE];
+  extern __shared__ __align__(16) float4 s_pts_buf[];  // CE_PT_BUFS point buffers of CE_TILE (CE_DYN_SMEM bytes)
   __shared__ uint32_t s_headw[CE_TILE / 32 + 1];  // bit i: item i starts a run; bit tile_n: sentinel
   __shared__ unsigned short s_start[CE_TILE];     // tile-local position of the r-th surviving run
   __shared__ uint32_t s_tile, s_base;
@@ -759,6 +774,15 @@ __global__ void __launch_bounds__(VX_THREADS, CE_MIN_CTAS) k_voxel_centroid(cons
 
   const uint32_t loc = tid * CE_IPT;  // tile-local index of this thread's first item
 
+  // SEG: the frames of the tile at tile_base (k_grid_setup's seg_cent_range), for frame_of
+  auto frame_range = [&](uint32_t tile_base) {
+    rng_b = tile_base;
+    rng_e = min(tile_base + (uint32_t)CE_TILE, M);
+    const uint2 fr = __ldg(p.seg_cent_range + tile_base / CE_TILE);  // the same in every thread
+    rng_lo = fr.x;
+    rng_hi = fr.y;
+  };
+
   // keys (and point slots) of this thread's eight items of the tile at tile_base, and what they say about runs:
   //   head bit j: item j starts a run; pass bit j: ... a run that survives the min-points filter; need bit j: its point is summed
   auto item_flags = [&](uint32_t tile_base, KeyT (&k)[CE_IPT], uint32_t (&v)[CE_IPT], bool want_vals, uint32_t& head, uint32_t& pass,
@@ -798,11 +822,7 @@ __global__ void __launch_bounds__(VX_THREADS, CE_MIN_CTAS) k_voxel_centroid(cons
       }
     }
     if constexpr (SEG) {  // frame bits from the position
-      rng_b = tile_base;
-      rng_e = min(tile_base + (uint32_t)CE_TILE, M);
-      const uint2 fr = __ldg(p.seg_cent_range + tile_base / CE_TILE);  // the same in every thread
-      rng_lo = fr.x;
-      rng_hi = fr.y;
+      frame_range(tile_base);
       if (rng_lo == rng_hi) {
         const KeyT fb = (KeyT)rng_lo << idx_bits;
 #pragma unroll
@@ -859,14 +879,21 @@ __global__ void __launch_bounds__(VX_THREADS, CE_MIN_CTAS) k_voxel_centroid(cons
   // it: the CTA counts its NEXT tile (keys only: one coalesced sweep, no point gathers) before it works on the current one.
   // With the counts that early, the look-back further down never waits for a tile that is still busy; without this, every tile
   // stalled for the slowest of its ~600 co-resident predecessors and the launch took 0.18 ms instead of 0.12 (measured).
-  // (CE_PREFETCH: the count sweep can also ask L2 for the points the tile will gather one tile-time later; measured, it does
-  // not pay -- see the macro.)
-  auto count_and_publish = [&](uint32_t t) {
+  // The sweep keeps the tile's head and pass bits (registers of the same thread, which owns the same items then) and starts
+  // the copies of its needed points into the tile's point buffer, one cp.async group per tile: they land while the CTA works
+  // on the current tile, and the tile's own item phase reads neither records nor points from global memory.
+  // (CE_PREFETCH, synchronous gathers only: the sweep asks L2 for the points instead; measured, it does not pay -- see the macro.)
+  auto count_and_publish = [&](uint32_t t, float4* pts_dst, uint32_t& head, uint32_t& pass) {
     KeyT k[CE_IPT];
     uint32_t v[CE_IPT];
-    uint32_t head, pass, need;
-    item_flags(t * CE_TILE, k, v, CE_PREFETCH != 0, head, pass, need);
-#if CE_PREFETCH
+    uint32_t need;
+    item_flags(t * CE_TILE, k, v, CE_ASYNC_GATHER || CE_PREFETCH, head, pass, need);
+#if CE_ASYNC_GATHER
+#pragma unroll
+    for (int j = 0; j < CE_IPT; ++j)
+      if (need & (1u << j)) cp_async_16(pts_dst + loc + j, p.pts + v[j]);
+    cp_async_commit();
+#elif CE_PREFETCH
 #pragma unroll
     for (int j = 0; j < CE_IPT; ++j)
       if (need & (1u << j)) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.pts + v[j]));
@@ -883,25 +910,40 @@ __global__ void __launch_bounds__(VX_THREADS, CE_MIN_CTAS) k_voxel_centroid(cons
     }
   };
 
-  count_and_publish(tile);
+  uint32_t head, pass;  // this thread's flags of `tile`, from its count sweep
+  uint32_t buf = 0;     // which point buffer holds `tile`'s points
+  count_and_publish(tile, s_pts_buf, head, pass);
   while (true) {
   // claim and count the next tile first
   if (tid == 0) s_tile = atomicAdd(&p.ctrl->cent_ticket, 1u);
-  __syncthreads();
+  __syncthreads();  // also: the last reads of the other point buffer (the previous tile) are done
   const uint32_t next_tile = s_tile;
-  if (next_tile < n_tiles) count_and_publish(next_tile);
+  const uint32_t next_buf = (buf + 1u) % CE_PT_BUFS;
+  uint32_t next_head = 0, next_pass = 0;
+  if (next_tile < n_tiles) count_and_publish(next_tile, s_pts_buf + next_buf * CE_TILE, next_head, next_pass);
 
   const uint32_t tile_base = tile * CE_TILE;
   const uint32_t tile_n = min((uint32_t)CE_TILE, M - tile_base);
+  float4* const s_pts = s_pts_buf + buf * CE_TILE;
 
   // ---- per item -----------------------------------------------------------------------------------------------------
-  KeyT k[CE_IPT];
-  uint32_t v[CE_IPT];
-  uint32_t head, pass, need;
-  item_flags(tile_base, k, v, true, head, pass, need);
+#if CE_ASYNC_GATHER
+  // this thread's copies of the tile are in (the next tile's group may still fly); the scan's barrier shows them to the CTA.
+  // Without a next tile nothing is left in flight.
+  if (next_tile < n_tiles) cp_async_wait<1>();
+  else cp_async_wait<0>();
+  if constexpr (SEG) frame_range(tile_base);  // the sweep left the next tile's frames behind
+#else
+  {
+    KeyT k[CE_IPT];
+    uint32_t v[CE_IPT];
+    uint32_t need;
+    item_flags(tile_base, k, v, true, head, pass, need);
 #pragma unroll
-  for (int j = 0; j < CE_IPT; ++j)
-    if (need & (1u << j)) s_pts[loc + j] = __ldg(p.pts + v[j]);
+    for (int j = 0; j < CE_IPT; ++j)
+      if (need & (1u << j)) s_pts[loc + j] = __ldg(p.pts + v[j]);
+  }
+#endif
   reinterpret_cast<unsigned char*>(s_headw)[tid] = (unsigned char)head;  // bit position 8*tid + j == item loc + j
   if (tid == 0) { s_headw[CE_TILE / 32] = 0u; s_tail_r = 0xFFFFFFFFu; }
   const uint32_t cnt = (uint32_t)__popc(pass);
@@ -1083,10 +1125,13 @@ __global__ void __launch_bounds__(VX_THREADS, CE_MIN_CTAS) k_voxel_centroid(cons
       s_tail.count_frame = per_voxel_count ? 1u : 0u;
     }
     __syncthreads();
-    finish_tail_run<KeyT, SEG>(&s_params, &s_tail, s_pts, s_tail_lead);
+    finish_tail_run<KeyT, SEG>(&s_params, &s_tail, s_pts, s_tail_lead);  // scratch: this tile's buffer, not the one in flight
     __syncthreads();
   }
   tile = next_tile;
+  head = next_head;
+  pass = next_pass;
+  buf = next_buf;
   if (tile >= n_tiles) break;
   }  // while (true): next tile
 }
@@ -1183,12 +1228,22 @@ cudaError_t launch_centroid(const VoxelParams& p, cudaStream_t stream) {
   // persistent: what the device holds at once (tiles are handed out by a ticket)
   const uint32_t grid = std::min<uint32_t>(tiles, 148u * (uint32_t)CE_MIN_CTAS);
   if (p.key_bytes == 4 && p.segmented)
-    k_voxel_centroid<unsigned long long, true><<<grid, VX_THREADS, 0, stream>>>(p);
+    k_voxel_centroid<unsigned long long, true><<<grid, VX_THREADS, CE_DYN_SMEM, stream>>>(p);
   else if (p.key_bytes == 4)
-    k_voxel_centroid<uint32_t><<<grid, VX_THREADS, 0, stream>>>(p);
+    k_voxel_centroid<uint32_t><<<grid, VX_THREADS, CE_DYN_SMEM, stream>>>(p);
   else
-    k_voxel_centroid<unsigned long long><<<grid, VX_THREADS, 0, stream>>>(p);
+    k_voxel_centroid<unsigned long long><<<grid, VX_THREADS, CE_DYN_SMEM, stream>>>(p);
   return cudaGetLastError();
+}
+
+cudaError_t configure_centroid_kernels() {
+  cudaError_t e = cudaFuncSetAttribute(k_voxel_centroid<unsigned long long, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)CE_DYN_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(k_voxel_centroid<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CE_DYN_SMEM);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(k_voxel_centroid<unsigned long long>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CE_DYN_SMEM);
+  return e;
 }
 
 cudaError_t launch_export_voxels(const VoxelParams& p, void* host_xyzi, uint32_t* host_count, unsigned long long* host_idx,
