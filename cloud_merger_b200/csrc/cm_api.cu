@@ -180,6 +180,7 @@ struct cm_handle_s {
   int overflow_mode = 0;
   bool profiling = false;
   bool have_bounds = false;   // externally supplied bounding box for cm_dev_voxelgrid (partitioned giant cloud)
+  uint32_t epoch_start = 0;   // first run epoch of every workspace's look-back words (CM_EPOCH_START, read by cm_create)
   float bounds_min[3] = {0, 0, 0}, bounds_max[3] = {0, 0, 0};
   // run bookkeeping
   uint32_t run_counter = 0;
@@ -368,7 +369,7 @@ int ws_alloc(cm_handle_t h, Workspace& w, uint32_t points, uint32_t frames, uint
   CM_CUDA(h, cudaMemset(w.cent_status.get(), 0, w.lb_cent_n * 8));
   CM_CUDA(h, cudaMemset(w.lb_sort.get(), 0, w.lb_sort_n * 8));
   CM_CUDA(h, dev_alloc(w.epoch_dev, (size_t)1));
-  CM_CUDA(h, cudaMemset(w.epoch_dev.get(), 0, sizeof(uint32_t)));
+  CM_CUDA(h, cudaMemcpy(w.epoch_dev.get(), &h->epoch_start, sizeof(uint32_t), cudaMemcpyHostToDevice));
   CM_CUDA(h, dev_alloc(w.out_xyzi, np * (size_t)out_step, 0));
   CM_CUDA(h, dev_alloc(w.out_count, np));
   CM_CUDA(h, dev_alloc(w.out_idx, np));
@@ -1228,6 +1229,14 @@ int cm_create(const cm_config_t* cfg, cm_handle_t* out) {
     return CM_E_CUDA;
   }
   if (getenv("CM_NO_GRAPH")) h->use_graph = false;
+  // debug: start the run epochs just below their wrap-around (k_grid_setup clears the look-back words and restarts at 16
+  // once *epoch_dev + 64 reaches 2^30, about 67 M runs into the life of a handle), so that tests reach it
+  if (const char* es = getenv("CM_EPOCH_START")) {
+    char* end = nullptr;
+    const unsigned long long v = strtoull(es, &end, 10);
+    if (end == es || *end != '\0' || v % 16ull != 0ull || v >= (1ull << 30) - 64ull) { delete h; return CM_E_INVALID; }
+    h->epoch_start = (uint32_t)v;
+  }
   for (int s = 0; s < CM_MAX_SENSORS; ++s) {
     float* m = h->mats_host + s * 12;
     for (int k = 0; k < 12; ++k) m[k] = (k % 5 == 0) ? 1.f : 0.f;  // identity rows

@@ -372,3 +372,302 @@ GIANT_CASES = (["bits:%d" % b for b in KEY_WIDTH_DIVS] + ["bin:%s" % w for w in 
                ["A:0.1", "A:0.035", "C:0.05", "Z:0.05", "origin:ok+", "origin:ok-", "axis:2p21"] +
                ["deg:%s" % k for k in DEGENERATE_KINDS])
 GIANT_RANGE_CASES = ("origin:beyond+", "origin:beyond-", "axis:2p21+")
+
+
+# ---- R: run layouts for the centroid pass --------------------------------------------------------------------------------
+# k_voxel_centroid (cloud_merger_b200/csrc/cm_voxel.cu) decides most things by where a run of equal keys sits relative to
+# its own fixed structures: threads of CE_IPT items, warps, tiles of CE_TILE items, the inline walk of CE_TAIL_INLINE points
+# past a tile and the rounds of CE_TAIL_ITEMS items of finish_tail_run. Its constants are mirrored here so that the layouts
+# can aim at them; test_edge_inputs.py reads them out of the source, so a retune fails there instead of missing the edges.
+VX_THREADS = 256
+CE_IPT = 8
+CE_TILE = VX_THREADS * CE_IPT            # sorted items per centroid tile
+CE_TAIL_INLINE = 24                      # points past its tile a run is summed by one thread before it is handed over
+CE_TAIL_U = 4
+CE_TAIL_ITEMS = CE_TAIL_U * VX_THREADS   # sorted items per round of finish_tail_run
+CE_SEG_SMEM_FRAMES = 256                 # frame-segmented runs: frame starts staged in shared memory up to this many frames
+CE_MIN_CTAS = 3                          # resident centroid CTAs per SM (the persistent grid is 148 * CE_MIN_CTAS)
+B200_SMS = 148
+RUN_ROW = 1024                           # cells per row of a run-layout cloud: run r sits in cell (r % RUN_ROW, r // RUN_ROW, 0)
+
+R_BOUND_OFFSETS = (-9, -8, -7, -1, 0, 1, 7, 8, 9)
+# how far a run continues past the end of the tile its head is in: the inline walk (up to 24), the hand-over at the 25th
+# point, and long runs ...
+LEAVE_PAST = (0, 1, 2, 23, 24, 25, 26, 1023, 1024, 1025, 2047, 2048, 2049, 3071, 3072, 3073)
+# ... among them those whose tail rounds (they start after the 24 inline points) end one short of, on and one past a round
+LEAVE_ROUND = tuple(CE_TAIL_INLINE + k * CE_TAIL_ITEMS + d for k in (1, 2, 3) for d in (-1, 0, 1))
+LEAVE_BACK = (1, 7, 8, 9, 255, 256, 257, 1000, 2047, 2048)   # the head of such a run: this many items before its tile's end
+MINPTS_M = (2, 3, 24, 25, 26, 1025)
+
+
+class RunList:
+    """Run lengths in sorted order, appended at the current sorted position `pos`; `marks` names the positions a layout
+    aims at (run starts) so that the CPU test can check them against the oracle's own runs."""
+
+    def __init__(self, seed: int):
+        self.rng = np.random.default_rng(seed)
+        self.runs, self.pos, self.marks = [], 0, {}
+
+    def run(self, n: int, mark: str = None):
+        assert n > 0, n
+        if mark:
+            self.marks.setdefault(mark, []).append((self.pos, self.pos + int(n)))
+        self.runs.append(int(n))
+        self.pos += int(n)
+        return self
+
+    def fill(self, to: int, lo: int = 1, hi: int = 9):
+        """Runs of lo..hi points up to sorted position `to`; the last one ends exactly there."""
+        assert to >= self.pos, (to, self.pos)
+        while self.pos < to:
+            self.run(min(int(self.rng.integers(lo, hi + 1)), to - self.pos))
+        return self
+
+    def to_tile_edge(self):
+        return self.fill(-(-self.pos // CE_TILE) * CE_TILE)
+
+
+def next_edge(pos: int, step: int, skip: int = 0) -> int:
+    """The first multiple of `step` above pos that is not a multiple of `skip`."""
+    e = (pos // step + 1) * step
+    while skip and e % skip == 0:
+        e += step
+    return e
+
+
+def bounds_block(rl: RunList, tiles=(0, 1, 3, 6)):
+    """R-bounds: runs of 1 to 9 points ending at every offset of R_BOUND_OFFSETS around a thread edge, a warp edge and the tile
+    edge of each of the given tiles (counted from the next tile edge)."""
+    t0 = -(-rl.pos // CE_TILE)
+    for t in tiles:
+        b = (t0 + t) * CE_TILE
+        for e in (b + 5 * CE_IPT, b + 3 * VX_THREADS, b + CE_TILE):
+            rl.fill(e + R_BOUND_OFFSETS[0])
+            rl.marks.setdefault("bounds", []).append(e)
+            for d in R_BOUND_OFFSETS[1:]:
+                rl.run(e + d - rl.pos)
+    return rl
+
+
+def leave_block(rl: RunList):
+    """R-leave: for every distance of LEAVE_PAST + LEAVE_ROUND a run whose head lies LEAVE_BACK items before the end of its
+    tile and which continues that far past it; then runs from a tile's first item over exactly 1, 2 and 3 whole tiles."""
+    for n, past in enumerate(LEAVE_PAST + LEAVE_ROUND):
+        back = LEAVE_BACK[n % len(LEAVE_BACK)]
+        end = next_edge(rl.pos, CE_TILE)
+        if end - back < rl.pos:
+            end += CE_TILE
+        rl.fill(end - back).run(back + past, "leave")
+        rl.fill(rl.pos + 1 + n % 13)
+    for k in (1, 2, 3):
+        rl.fill(next_edge(rl.pos, CE_TILE)).run(k * CE_TILE, "whole")
+    return rl.fill(rl.pos + 37)
+
+
+def dense_block(rl: RunList):
+    """R-dense: a tile of 2048 one-point voxels; one of 2047 whose last run is handed over; tiles of exactly 256 and 257
+    runs; and one of 257 runs whose last (the second voxel of thread 0) is handed over."""
+    rl.to_tile_edge()
+    for _ in range(CE_TILE):
+        rl.run(1)
+    for _ in range(CE_TILE - 1):
+        rl.run(1)
+    rl.run(1 + 600, "dense-last")
+    rl.to_tile_edge()
+    for _ in range(256):
+        rl.run(8)
+    for _ in range(255):
+        rl.run(8)
+    rl.run(4).run(4)
+    for _ in range(256):
+        rl.run(7)
+    rl.run(256 + 600, "dense-last")
+    return rl.fill(rl.pos + 50)
+
+
+def layout(name: str, seed: int = 0):
+    """(run lengths, marks) of a named layout: bounds, leave, dense, persist, end:<kind>, minpts:<m>:<length of the last run>."""
+    rl = RunList(seed)
+    if name == "bounds":
+        bounds_block(rl).fill(rl.pos + 100)
+    elif name == "leave":
+        leave_block(rl)
+    elif name == "dense":
+        dense_block(rl)
+    elif name == "persist":   # more than three tiles per CTA of the persistent grid
+        while rl.pos < 3 << 20:
+            bounds_block(rl)
+            leave_block(rl)
+    elif name.startswith("end:"):
+        kind = name[4:]
+        T = CE_TILE
+        small = {"M1": [1], "M3": [3], "M7": [1, 2, 4]}
+        if kind in small:
+            for n in small[kind]:
+                rl.run(n)
+        elif kind in ("2T-1", "2T", "2T+1"):
+            m_end = 2 * T + {"2T-1": -1, "2T": 0, "2T+1": 1}[kind]
+            rl.fill(m_end - 12).run(12, "end")
+        elif kind == "handover-round":   # handed over, and the second round starts exactly at M: the limit ends it
+            rl.fill(2 * T - 5).run(5 + CE_TAIL_INLINE + CE_TAIL_ITEMS, "end")
+        elif kind == "handover-partial":   # crosses into a final partial tile, handed over, ends at M
+            rl.fill(3 * T - 100).run(100 + 700, "end")
+        else:
+            raise ValueError(name)
+    elif name.startswith("minpts:"):
+        _, m, last = name.split(":")
+        m, last = int(m), int(last)
+        for n in (m - 1, m, m + 1):
+            for step, skip in ((CE_IPT, VX_THREADS), (VX_THREADS, CE_TILE), (CE_TILE, 0)):
+                e = next_edge(rl.pos + n, step, skip)
+                rl.fill(e - max(1, n // 2)).run(n, "straddle")
+        rl.fill(rl.pos + 20).run(last, "end")
+    else:
+        raise ValueError(name)
+    return rl.runs, rl.marks
+
+
+R_LAYOUTS = ("bounds", "leave", "dense", "end:M1", "end:M3", "end:M7", "end:2T-1", "end:2T", "end:2T+1",
+             "end:handover-round", "end:handover-partial")
+R_MINPTS = tuple("minpts:%d:%d" % (m, last) for m in MINPTS_M for last in (m - 1, m, m + 1))
+
+
+def _intensities(rng, n):
+    return (rng.uniform(0.0, 255.0, size=n) * 2.0 ** rng.integers(-12, 1, size=n)).astype(F32)
+
+
+def _make_order_sensitive(x, keys, rng):
+    """Redraws the intensities of every run of 3 or more points whose float32 sequential sum in ascending row order equals
+    the reversed sum in all four components (a few per cent of the short runs), until there is none."""
+    order = np.argsort(keys, kind="stable")
+    order = order[keys[order] >= 0]
+    k = keys[order]
+    starts = np.nonzero(np.r_[True, k[1:] != k[:-1]])[0] if len(k) else np.zeros(0, np.int64)
+    lens = np.diff(np.r_[starts, len(k)])
+    todo = np.nonzero(lens >= 3)[0]
+    for _ in range(100):
+        bad = []
+        for n in np.unique(lens[todo]):
+            rs = todo[lens[todo] == n]
+            p = x[order[starts[rs][:, None] + np.arange(n)]]
+            fwd = np.zeros((len(rs), 4), F32)
+            rev = np.zeros((len(rs), 4), F32)
+            for j in range(n):
+                fwd += p[:, j]
+                rev += p[:, n - 1 - j]
+            bad.append(rs[(fwd.view(np.uint32) == rev.view(np.uint32)).all(axis=1)])
+        todo = np.concatenate(bad) if bad else todo[:0]
+        if not len(todo):
+            return
+        rows = order[np.concatenate([np.arange(starts[r], starts[r] + lens[r]) for r in todo])]
+        x[rows, 3] = _intensities(rng, len(rows))
+    raise AssertionError("runs whose sum does not depend on the order")
+
+
+def run_layout_cloud(runs, seed: int, n_nonfinite: int = 0, far: bool = False, shift=(0, 0, 0)) -> np.ndarray:
+    """Family R: a cloud (leaf 1.0) whose VoxelGrid has exactly the given runs in sorted order -- run r is cell r of rows of
+    RUN_ROW cells (origin 0). Every point is jittered inside its cell, at least 0.1 from its planes; the coordinates of a run
+    differ in their fraction bits (z and intensity in their exponents too), so its float32 sum depends on every point, and
+    from 3 points on on their order (intensities are drawn again where it would not). The rows are permuted: the gather is
+    scattered, and the ascending-index order inside a run is not the order of generation. n_nonfinite: rows with a NaN or an
+    infinity (they sort last, into the sentinel frame); far: a point in the far corner cell of the grid DIV_2P32_PLUS (the
+    keys need 33 index bits; one more run at the end); shift: whole cells added to every coordinate (another grid origin)."""
+    rng = np.random.default_rng(seed)
+    runs = np.asarray(runs, np.int64)
+    keys = np.repeat(np.arange(len(runs), dtype=np.int64), runs)
+    out = key_cell_cloud((RUN_ROW, 1 << 21, 1), keys)
+    out[:, :3] = (np.floor(out[:, :3]).astype(np.float64) + rng.uniform(0.1, 0.9, size=(len(keys), 3))
+                  + np.asarray(shift, np.float64)).astype(F32)
+    out[:, 3] = _intensities(rng, len(keys))
+    if far:
+        out = np.concatenate([out, key_cell_cloud(DIV_2P32_PLUS, grid_corner_keys(DIV_2P32_PLUS)[-1:])])
+        keys = np.r_[keys, len(runs)]
+    if n_nonfinite:
+        bad = out[rng.integers(0, len(out), size=n_nonfinite)].copy()
+        bad[np.arange(n_nonfinite), np.arange(n_nonfinite) % 3] = np.array([np.nan, np.inf, -np.inf], F32)[np.arange(n_nonfinite) % 3]
+        out = np.concatenate([out, bad])
+        keys = np.r_[keys, np.full(n_nonfinite, -1, np.int64)]
+    perm = rng.permutation(len(out))
+    out, keys = out[perm], keys[perm]
+    _make_order_sensitive(out, keys, rng)
+    return out
+
+
+def split_runs(runs, cuts):
+    """The runs of each frame when the sorted sequence is cut at the given positions (a run that a cut passes through goes on,
+    as a run of its own, in the next frame; equal cuts make empty frames)."""
+    ends = np.cumsum(runs)
+    starts = ends - np.asarray(runs)
+    frames, lo = [], 0
+    for hi in list(cuts) + [int(ends[-1]) if len(ends) else 0]:
+        f = []
+        for s, e in zip(starts, ends):
+            a, b = max(int(s), lo), min(int(e), hi)
+            if a < b:
+                f.append(b - a)
+        frames.append(f)
+        lo = hi
+    return frames
+
+
+def centroid_walk(starts, m_items: int, frame_starts=(0,)):
+    """How k_voxel_centroid meets each run [starts[r], starts[r+1]) of a sorted array of m_items items: the tile of its head,
+    how far it continues past that tile, whether it is handed over to the CTA and how many items its tail rounds cover, and
+    whether its tile straddles frames (frame_starts: the first position of every frame)."""
+    starts = np.asarray(starts, np.int64)
+    ends = np.append(starts[1:], m_items)
+    tile = starts // CE_TILE
+    tile_end = np.minimum((tile + 1) * CE_TILE, m_items)
+    past = np.maximum(ends - tile_end, 0)
+    fs = np.asarray(frame_starts, np.int64)
+    first_frame = np.searchsorted(fs, tile * CE_TILE, side="right") - 1
+    last_frame = np.searchsorted(fs, tile_end - 1, side="right") - 1
+    return dict(start=starts, end=ends, tile=tile, past=past, handed=past > CE_TAIL_INLINE,
+                tail_items=np.maximum(past - CE_TAIL_INLINE, 0), straddles=first_frame != last_frame)
+
+
+def batch_layout(name: str, seed: int = 0):
+    """(runs, cuts, marks) of a frame-split run layout (split_runs gives each frame's runs).
+    seg3: frame 0 is one run from item 0 to 10 past the first tile, frame 1 one run from there to 500 past the third tile
+    (handed over; its tile straddles frames 0 and 1), frame 2 starts with a run -- the same voxel index 0 as the end of
+    frames 0 and 1, so only the frame tells the runs apart, inside the inline walk and inside a tail round -- and goes on
+    with the R-bounds and R-leave blocks (tail runs in tiles of one frame).
+    seg300: the R-bounds and R-leave blocks cut into 300 frames: at every R-bounds offset, around single-run frames that end
+    inside an inline walk or a tail round, with empty frames, and at further random positions among the R-bounds runs."""
+    T = CE_TILE
+    if name == "seg3":
+        rl = RunList(seed)
+        rl.run(T + 10).run(2 * T + 490, "tail-straddle").run(30)
+        bounds_block(rl)
+        leave_block(rl)
+        return rl.runs, [T + 10, 3 * T + 500], rl.marks
+    if name == "seg300":
+        rl = RunList(seed)
+        bounds_block(rl)
+        split = rl.pos
+        leave_block(rl)
+        cuts = [e + d for e in rl.marks["bounds"] for d in R_BOUND_OFFSETS]
+        leave = rl.marks["leave"]
+        for k, past in ((7, 10), (10, 300), (16, 700)):   # single-run frames ending inline / in a tail round
+            s, e = leave[k]
+            t_end = (s // T + 1) * T
+            assert e - t_end > past
+            cuts += [s + 1, t_end + past]
+        cuts += [cuts[0]] * 2 + [cuts[50]] + [split] * 2   # empty frames
+        rng = np.random.default_rng(seed + 1)
+        while len(cuts) < 299:
+            cuts.append(int(rng.integers(1, split)))
+        return rl.runs, sorted(cuts), rl.marks
+    raise ValueError(name)
+
+
+def run_layout_frames(runs, cuts, seed: int, n_nonfinite: int = 0, shift=(0, 0, 0)) -> list:
+    """One run-layout cloud per frame of split_runs(runs, cuts); frame f is shifted by f * shift cells, and frames with points
+    get n_nonfinite non-finite rows each."""
+    out = []
+    for f, fr in enumerate(split_runs(runs, cuts)):
+        if not fr:
+            out.append(np.zeros((0, 4), F32))
+            continue
+        out.append(run_layout_cloud(fr, seed + f, n_nonfinite=n_nonfinite, shift=tuple(f * s for s in shift)))
+    return out

@@ -1,5 +1,8 @@
 """The edge-case generators (tests/edge_inputs.py) on the CPU: their inputs reach the fragile spots they are meant to reach,
 and the two CPU references -- the C++ oracle and the numpy restatement -- agree on every one of them."""
+import os
+import re
+
 import numpy as np
 import pytest
 
@@ -128,3 +131,226 @@ def test_oracles_agree_on_edge_inputs(oracle, case, min_points):
     assert (c["idx"] == v["idx"]).all() and (c["count"] == v["count"]).all()
     np.testing.assert_allclose(c["centroid_f64"], v["centroid_f64"], rtol=1e-12, atol=1e-12)
     assert c["n_voxels"] > 0
+
+
+# ---- R: run layouts of the centroid pass ---------------------------------------------------------------------------------
+VOXEL_CU = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "cloud_merger_b200", "csrc", "cm_voxel.cu")
+
+
+def test_mirrored_centroid_constants_match_the_source():
+    """The layouts aim at k_voxel_centroid's tiles, threads, hand-over point and tail rounds through constants mirrored in
+    edge_inputs.py: a retune of the kernel must fail here, not quietly move the edges away from the layouts."""
+    src = open(VOXEL_CU).read()
+
+    def const(name):
+        m = re.search(r"constexpr\s+\w+\s+%s\s*=\s*([^;]+);" % name, src)
+        assert m, name
+        return m.group(1).strip()
+
+    def define(name):
+        m = re.search(r"#define\s+%s\s+(.+?)\s*(?://.*)?$" % name, src, re.M)
+        assert m, name
+        return m.group(1).strip()
+    assert int(const("VX_THREADS")) == E.VX_THREADS
+    assert int(const("CE_IPT")) == E.CE_IPT
+    assert const("CE_TILE") == "VX_THREADS * CE_IPT" and E.CE_TILE == E.VX_THREADS * E.CE_IPT == 2048
+    assert int(const("CE_TAIL_INLINE").rstrip("u")) == E.CE_TAIL_INLINE
+    assert int(const("CE_TAIL_U")) == E.CE_TAIL_U
+    assert const("CE_TAIL_ITEMS") == "CE_TAIL_U * VX_THREADS" and E.CE_TAIL_ITEMS == E.CE_TAIL_U * E.VX_THREADS
+    assert int(const("CE_SEG_SMEM_FRAMES").rstrip("u")) == E.CE_SEG_SMEM_FRAMES
+    assert int(define("CE_ASYNC_GATHER")) == 1
+    assert define("CE_MIN_CTAS") == "(CE_ASYNC_GATHER ? %d : 4)" % E.CE_MIN_CTAS
+    assert "std::min<uint32_t>(tiles, %du * (uint32_t)CE_MIN_CTAS)" % E.B200_SMS in src
+    # the persistent grid holds fewer tiles than R-persist has: every CTA takes several and alternates its point buffers
+    runs, _ = E.layout("persist")
+    assert sum(runs) / E.CE_TILE > 3 * E.B200_SMS * E.CE_MIN_CTAS
+
+
+def _runs_of(x, min_points=1):
+    """From the numpy oracle alone: the finite rows in sorted order (stable: ascending row index inside a voxel), their voxel
+    indices, and the sorted positions where runs start."""
+    o = np_oracle.voxelgrid(x, [1.0] * 3, min_points, True, True)
+    pidx = o["point_idx"]
+    fin = np.nonzero(pidx >= 0)[0]
+    order = fin[np.argsort(pidx[fin], kind="stable")]
+    keys = pidx[order]
+    starts = np.nonzero(np.r_[True, keys[1:] != keys[:-1]])[0] if len(keys) else np.zeros(0, np.int64)
+    return order, keys, starts, o
+
+
+def _check_marks(name, runs, marks, starts, m_items):
+    w = E.centroid_walk(starts, m_items)
+    at = {int(s): i for i, s in enumerate(starts)}
+    bounds = set(int(s) for s in starts) | {m_items}
+
+    def run_at(s, e):
+        assert s in at and e in bounds and (at[s] + 1 == len(starts) or int(starts[at[s] + 1]) == e), (name, s, e)
+        return at[s]
+    for e in marks.get("bounds", []):
+        for d in E.R_BOUND_OFFSETS:
+            assert e + d in bounds, (name, e, d)
+    if "leave" in marks:
+        idx = [run_at(s, e) for s, e in marks["leave"]]
+        reps = len(idx) // len(E.LEAVE_PAST + E.LEAVE_ROUND)   # R-persist repeats the block
+        assert reps and sorted(int(w["past"][i]) for i in idx) == sorted((E.LEAVE_PAST + E.LEAVE_ROUND) * reps)
+        inline = [i for i in idx if 0 < w["past"][i] <= E.CE_TAIL_INLINE]
+        handed = [i for i in idx if w["handed"][i]]
+        assert any(w["past"][i] == E.CE_TAIL_INLINE for i in inline), "a run that fills the inline walk exactly"
+        assert any(w["past"][i] == E.CE_TAIL_INLINE + 1 for i in handed), "a run handed over at its 25th point past the tile"
+        tails = w["tail_items"][handed]
+        for d in (-1, 0, 1):   # tail rounds that end one short of, on and one past a round boundary
+            for k in (1, 2, 3):
+                assert (tails == k * E.CE_TAIL_ITEMS + d).any(), (k, d)
+        assert {(-s) % E.CE_TILE or E.CE_TILE for s, _ in marks["leave"]} == set(E.LEAVE_BACK)   # where the heads sit
+    for s, e in marks.get("whole", []):
+        i = run_at(s, e)
+        assert s % E.CE_TILE == 0 and (e - s) % E.CE_TILE == 0
+        k = (e - s) // E.CE_TILE
+        assert w["past"][i] == (k - 1) * E.CE_TILE   # the k - 1 tiles after the first have no head: they publish 0 voxels
+    if "dense-last" in marks:
+        per_tile = np.bincount(w["tile"])
+        assert (per_tile == E.CE_TILE).any() and (per_tile == 256).any() and (per_tile == 257).any()
+        for s, e in marks["dense-last"]:
+            i = run_at(s, e)
+            assert w["handed"][i] and per_tile[w["tile"][i]] > 256
+            assert i + 1 == len(starts) or w["tile"][i + 1] != w["tile"][i], "the handed-over run is its tile's last"
+    if name.startswith("end:"):
+        assert m_items == sum(runs)
+        kind = name[4:]
+        if kind in ("2T-1", "2T", "2T+1"):
+            assert m_items == 2 * E.CE_TILE + {"2T-1": -1, "2T": 0, "2T+1": 1}[kind]
+        if kind == "M7":
+            assert m_items < E.CE_IPT
+        if kind.startswith("handover"):
+            (s, e), = marks["end"]
+            i = run_at(s, e)
+            assert e == m_items and w["handed"][i]
+            if kind == "handover-round":
+                assert w["tail_items"][i] == E.CE_TAIL_ITEMS   # the second round starts at M: only the limit ends it
+            else:
+                assert m_items % E.CE_TILE and w["tile"][i] + 1 == m_items // E.CE_TILE
+    if name.startswith("minpts:"):
+        m, last = (int(v) for v in name.split(":")[1:])
+        crossed = set()
+        for s, e in marks["straddle"]:
+            run_at(s, e)
+            ahead = s + m - 1                      # the item the min-points test of the head looks at
+            for step in (E.CE_IPT, E.VX_THREADS, E.CE_TILE):
+                if ahead // step != s // step:
+                    crossed.add(step)
+        assert crossed == {E.CE_IPT, E.VX_THREADS, E.CE_TILE}
+        (s, e), = marks["end"]
+        assert e == m_items and e - s == last and ((s + m - 1 >= m_items) == (last < m))
+
+
+@pytest.mark.parametrize("name", E.R_LAYOUTS + E.R_MINPTS + ("persist",))
+def test_run_layout_positions(name):
+    """The oracle's own runs of every R layout (recomputed from its keys and its stable order) are exactly the intended
+    ones, and they sit where the layout aims: R-bounds offsets, the inline walk and the hand-over at the 25th point, tail
+    rounds ending one short of, on and one past a round, whole tiles without a head, dense tiles, the end of the cloud, the
+    min-points look-ahead across thread, warp and tile edges and past M."""
+    runs, marks = E.layout(name, seed=7)
+    x = E.run_layout_cloud(runs, seed=len(name))
+    order, keys, starts, _ = _runs_of(x)
+    assert np.diff(np.r_[starts, len(keys)]).tolist() == list(runs)
+    assert (keys[starts] == np.arange(len(runs))).all(), "run r is cell r"
+    assert len(order) < 8 or not (order[1:] > order[:-1]).all(), "the gather must be scattered"
+    _check_marks(name, runs, marks, starts, len(keys))
+
+
+@pytest.mark.parametrize("name", ["seg3", "seg300"])
+def test_batch_layout_positions(name):
+    """The frame-split layouts: every frame's runs are the intended ones; seg3 puts voxel index 0 on both sides of a frame
+    edge inside an inline walk and inside a tail round, and has handed-over runs in a tile that straddles frames and in one
+    that does not; seg300 has more frames than are staged in shared memory, empty frames, and frame edges at every R-bounds
+    offset."""
+    runs, cuts, marks = E.batch_layout(name, seed=3)
+    frames = E.split_runs(runs, cuts)
+    clouds = E.run_layout_frames(runs, cuts, seed=11)
+    fs = np.r_[0, cuts]
+    assert len(frames) == len(cuts) + 1 and np.diff(np.r_[fs, sum(runs)]).tolist() == [len(c) for c in clouds]
+    first_last = []
+    for f, (fr, x) in enumerate(zip(frames, clouds)):
+        if not fr:
+            first_last.append(None)
+            continue
+        _, keys, starts, _ = _runs_of(x)
+        assert np.diff(np.r_[starts, len(keys)]).tolist() == fr, f
+        first_last.append((int(keys[0]), int(keys[-1])))
+    # the kernel's view: runs of equal (frame, index) over the concatenated frames
+    starts = np.unique(np.r_[fs, np.cumsum(runs)[:-1]])
+    starts = starts[starts < sum(runs)]
+    w = E.centroid_walk(starts, sum(runs), fs)
+    assert (w["handed"] & w["straddles"]).any() and (w["handed"] & ~w["straddles"]).any()
+    same = [(f, c) for f, c in enumerate(cuts) if first_last[f] and first_last[f + 1] and first_last[f][1] == first_last[f + 1][0]]
+    kinds = set()
+    for f, c in same:
+        i = int(np.searchsorted(starts, c)) - 1          # the run that ends at the frame edge
+        edge = min((int(w["tile"][i]) + 1) * E.CE_TILE, sum(runs))
+        if w["start"][i] < edge < c:
+            kinds.add("tail" if c - edge > E.CE_TAIL_INLINE else "inline")
+    assert kinds == {"inline", "tail"}, kinds
+    if name == "seg300":
+        assert len(frames) == 300 > E.CE_SEG_SMEM_FRAMES and sum(1 for f in frames if not f) >= 3
+        for e in marks["bounds"]:
+            for d in E.R_BOUND_OFFSETS:
+                assert e + d in cuts
+
+
+def _seq_sum(p):
+    return np.cumsum(np.asarray(p, F32), axis=0, dtype=F32)[-1] if len(p) else np.zeros(4, F32)
+
+
+@pytest.mark.parametrize("name", ["bounds", "leave", "dense", "end:handover-round", "end:handover-partial",
+                                  "minpts:1025:1024", "persist"])
+def test_run_layout_sums_see_every_point_and_their_order(name):
+    """Every run that leaves its tile, and every run at an R-bounds edge, has a float32 sequential sum (ascending row order,
+    as the kernel and the float oracle add) that differs bitwise from the same sum without the point at the tile edge, with
+    that point counted twice, and -- from 3 points on -- from the reversed sum: a kernel that drops, repeats or re-orders a
+    point there cannot match the oracle bit for bit."""
+    runs, marks = E.layout(name, seed=7)
+    x = E.run_layout_cloud(runs, seed=len(name))
+    order, keys, starts, _ = _runs_of(x)
+    m_items = len(keys)
+    w = E.centroid_walk(starts, m_items)
+    ends = w["end"]
+    target = set(np.nonzero(w["past"] > 0)[0].tolist())
+    for e in marks.get("bounds", []):
+        target |= set((np.searchsorted(starts, [e + d for d in E.R_BOUND_OFFSETS], side="right") - 1).tolist())
+    assert target
+    reversed_checked = 0
+    for i in sorted(target):
+        s, e = int(starts[i]), int(ends[i])
+        pts = x[order[s:e]]
+        edge = min(max((s // E.CE_TILE + 1) * E.CE_TILE, s), e - 1) - s   # the first point past the tile, else the last
+        ref = _seq_sum(pts)
+        drop = _seq_sum(np.delete(pts, edge, axis=0))
+        dup = _seq_sum(np.insert(pts, edge, pts[edge], axis=0))
+        assert (ref.view(np.uint32) != drop.view(np.uint32)).any(), (name, s, e, "drop")
+        assert (ref.view(np.uint32) != dup.view(np.uint32)).any(), (name, s, e, "twice")
+        if e - s >= 3:   # (a + b == b + a)
+            assert (ref.view(np.uint32) != _seq_sum(pts[::-1]).view(np.uint32)).any(), (name, s, e, "reversed")
+            reversed_checked += 1
+    assert reversed_checked
+
+
+R_ORACLE_CASES = [(n, 1, 0, False) for n in E.R_LAYOUTS] + [(n, int(n.split(":")[1]), 0, False) for n in E.R_MINPTS] + \
+    [("leave", 2, 0, True), ("bounds", 3, 0, True), ("leave", 1, 5000, False), ("dense", 2, 300, True), ("persist", 2, 0, False)]
+
+
+@pytest.mark.parametrize("case", R_ORACLE_CASES, ids=["%s-mp%d-nf%d-far%d" % c for c in R_ORACLE_CASES])
+def test_oracles_agree_on_run_layouts(oracle, case):
+    """The C++ oracle and the numpy restatement agree on every R layout (with non-finite rows and far corners too): the
+    number of voxels, their indices and counts, and the membership of every point."""
+    name, min_points, n_nf, far = case
+    runs, _ = E.layout(name, seed=7)
+    x = E.run_layout_cloud(runs, seed=len(name), n_nonfinite=n_nf, far=far)
+    c = oracle.voxelgrid(x, [1.0] * 3, min_points, True, force64=True, is_dense=n_nf == 0)
+    n = np_oracle.voxelgrid(x, [1.0] * 3, min_points, True, True)
+    assert c["n"] == len(n["idx"]) and (c["idx"] == n["idx"]).all() and (c["count"] == n["count"]).all()
+    assert (c["point_idx"] == n["point_idx"]).all()
+    np.testing.assert_allclose(c["centroid_f64"], n["centroid_f64"], rtol=1e-12, atol=1e-12)
+    if far:
+        assert E.bits_for(int(np.prod(c["div_b"].astype(np.int64)))) == 33
+    else:
+        assert c["min_b"].tolist() == [0, 0, 0] and c["n"] == sum(1 for r in runs if r >= min_points)
