@@ -70,6 +70,7 @@ struct Workspace {
   bool ready = false;
   uint32_t cap_points = 0, cap_frames = 0, cap_segs = 0;
   uint32_t plan_idx_bits = 0, plan_total_bits = 0;  // key plan of the last unbounded run (fetched from the device)
+  uint32_t plan_error = 0;                          // Ctrl.error when that plan was fetched (k_grid_setup's verdict)
   int out_step = 16;
   MetaLayout ml{};
   DevPtr<uint8_t> meta;
@@ -199,12 +200,14 @@ struct cm_handle_s {
     DevPtr<float4> out_xyzi;
     DevPtr<uint32_t> out_src;
     DevPtr<float4> in_stage;      // host-buffer form: the uploaded cloud
-    HostPtr<uint32_t> report;     // pinned: zone_begin[CM_MAX_ZONES + 1] + overflow
+    HostPtr<uint32_t> report;     // pinned: zone_begin[CM_MAX_ZONES + 1] + overflow + a radius run's device error word
     cudaStream_t stream = nullptr;
     bool ran = false;
     int64_t launches = 0;
     ZoneParams last{};           // the last split, so that its scatter can be repeated after the outputs grew
     int n_zones_run = 0;         // zones of the last split (1 for a radius outlier removal)
+    bool ror_run = false;        // the last split compacted a radius outlier removal: report[CM_MAX_ZONES + 2] holds the
+                                 // error word of its count kernel (the 2^14-cell bound of the cell margin)
   } zw;
   // radius outlier removal: first sorted position of every cell key (allocated on first use, grows)
   DevPtr<uint32_t> ror_table;
@@ -579,14 +582,17 @@ int run_voxel(cm_handle_t h, Workspace& w, VoxelParams& vp, cudaStream_t st, boo
     return CM_OK;
   }
   if (!bounded) {
-    // the key width is only known on the device: fetch the plan (one small round trip), then size the sort to it
+    // the key width is only known on the device: fetch the plan (one small round trip), then size the sort to it. The
+    // control block comes along in the same copy: its error word says whether every frame's grid was usable.
     SortInfo si;
-    CM_CUDA(h, cudaMemcpyAsync(w.report.get() + w.ml.off_info, w.meta.get() + w.ml.off_info, sizeof(SortInfo), cudaMemcpyDeviceToHost, st));
+    Ctrl ctrl;
+    CM_CUDA(h, cudaMemcpyAsync(w.report.get(), w.meta.get(), w.ml.off_info + sizeof(SortInfo), cudaMemcpyDeviceToHost, st));
     CM_CUDA(h, cudaStreamSynchronize(st));
     memcpy(&si, w.report.get() + w.ml.off_info, sizeof(si));
+    memcpy(&ctrl, w.report.get() + w.ml.off_ctrl, sizeof(ctrl));
     vp.key_bytes = si.total_bits <= 32 ? 4 : 8;
     vp.max_passes = si.num_passes;
-    w.plan_idx_bits = si.idx_bits; w.plan_total_bits = si.total_bits;
+    w.plan_idx_bits = si.idx_bits; w.plan_total_bits = si.total_bits; w.plan_error = ctrl.error;
   }
   w.key_bytes = vp.key_bytes;
   w.max_passes = vp.max_passes;
@@ -1654,7 +1660,7 @@ int zone_ws_ensure(cm_handle_t h, size_t points) {
   z.cap_out = 2 * want;
   CM_CUDA(h, dev_alloc(z.out_xyzi, z.cap_out));
   CM_CUDA(h, dev_alloc(z.out_src, z.cap_out));
-  CM_CUDA(h, pinned_alloc(z.report, sizeof(uint32_t) * (CM_MAX_ZONES + 2), cudaHostAllocDefault));
+  CM_CUDA(h, pinned_alloc(z.report, sizeof(uint32_t) * (CM_MAX_ZONES + 3), cudaHostAllocDefault));
   CM_CUDA(h, cudaDeviceSynchronize());  // the clear above ran on the default stream (see ws_alloc)
   z.cap_points = want;
   return CM_OK;
@@ -1709,7 +1715,7 @@ int zone_run(cm_handle_t h, const float4* pts, int64_t n_points, cudaStream_t st
   CM_CUDA(h, launch_zone_split(zp, st));
   CM_CUDA(h, cudaMemcpyAsync(z.report.get(), z.zone_begin.get(), sizeof(uint32_t) * (CM_MAX_ZONES + 1), cudaMemcpyDeviceToHost, st));
   CM_CUDA(h, cudaMemcpyAsync(z.report.get() + CM_MAX_ZONES + 1, z.overflow.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-  z.stream = st; z.ran = true; z.launches = zp.n_tiles ? CM_ZONE_LAUNCHES : 1; z.last = zp;
+  z.stream = st; z.ran = true; z.launches = zp.n_tiles ? CM_ZONE_LAUNCHES : 1; z.last = zp; z.ror_run = false;
   return CM_OK;
 }
 }  // namespace
@@ -1771,6 +1777,9 @@ int zone_out_locked(cm_handle_t h, cm_zone_out_t* out) {
   out->src = z.out_src.get();
   if (report[CM_MAX_ZONES + 1])
     return fail(h, CM_E_CAPACITY, "the zones hold %u points together, capacity is %zu", report[CM_MAX_ZONES + 1], z.cap_out);
+  if (z.ror_run && report[CM_MAX_ZONES + 2] == CM_DEV_E_KEY_RANGE)
+    return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (more than 2^14 cells from the origin)");
+  if (z.ror_run && report[CM_MAX_ZONES + 2]) return fail(h, CM_E_INTERNAL, "device error %u", report[CM_MAX_ZONES + 2]);
   return CM_OK;
 }
 }  // namespace
@@ -1948,6 +1957,11 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
   rc = run_voxel(h, w, vp, st, false, false);  // keys + sort only
   if (rc != CM_OK) return rc;
+  // A cloud whose grid k_grid_setup could not key (more than 2^21 cells on an axis, a coordinate beyond 2^30 cells) has
+  // all its keys at 0 but keeps its real div_b: the cell table would be sized without it and the row walk would leave it.
+  // The plan fetch above brought the verdict along, so such a call stops here, before the table and the count.
+  if (w.plan_error == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (cell grid exceeds the key range)");
+  if (w.plan_error) return fail(h, CM_E_INTERNAL, "device error %u", w.plan_error);
   vp.key_bytes = w.key_bytes;
   RorParams rp;
   rp.r2 = (float)(radius * radius);
@@ -1974,7 +1988,12 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   CM_CUDA(h, launch_radius_count(vp, rp, st));
   ++w.launches;
   CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
-  return zone_run(h, pts, n_points, st, true, n_clouds);
+  rc = zone_run(h, pts, n_points, st, true, n_clouds);
+  if (rc != CM_OK) return rc;
+  // the count kernel's verdict on the 2^14-cell bound rides along with the zone sizes: cm_get_zone_out reports it
+  CM_CUDA(h, cudaMemcpyAsync(h->zw.report.get() + CM_MAX_ZONES + 2, &vp.ctrl->error, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  h->zw.ror_run = true;
+  return CM_OK;
 }
 }  // namespace
 
@@ -2025,12 +2044,6 @@ int cm_radius_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t
   if (rc != CM_OK) return rc;
   {
     std::lock_guard<std::mutex> lk(h->mu);
-    // device-side errors of the key / sort stage (e.g. the radius is too small for the extent of the cloud)
-    uint32_t dev_err = 0;
-    Workspace& w = h->batch;
-    CM_CUDA(h, cudaMemcpy(&dev_err, &reinterpret_cast<Ctrl*>(w.meta.get() + w.ml.off_ctrl)->error, sizeof(dev_err), cudaMemcpyDeviceToHost));
-    if (dev_err == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of the cloud (cell grid exceeds the key range)");
-    if (dev_err) return fail(h, CM_E_INTERNAL, "device error %u", dev_err);
     const int64_t total = zo.begin[n_clouds];
     if (total > capacity) return fail(h, CM_E_CAPACITY, "%lld points kept, caller capacity %lld", (long long)total, (long long)capacity);
     if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
@@ -2533,11 +2546,6 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
     if (rc != CM_OK) return rc;
     for (int c = 0; c <= G; ++c) kb[c] = zo.begin[c];
     kept = reinterpret_cast<const float4*>(zo.xyzi);
-    uint32_t dev_err = 0;  // key-range / watchdog errors of the cell sort
-    CM_CUDA(h, cudaMemcpyAsync(&dev_err, &reinterpret_cast<Ctrl*>(h->batch.meta.get() + h->batch.ml.off_ctrl)->error, sizeof(dev_err), cudaMemcpyDeviceToHost, st));
-    CM_CUDA(h, cudaStreamSynchronize(st));
-    if (dev_err == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a zone (cell grid exceeds the key range)");
-    if (dev_err) return fail(h, CM_E_INTERNAL, "device error %u", dev_err);
   }
   // ---- the appends, in part order
   int64_t n_ng = 0, n_g = 0;

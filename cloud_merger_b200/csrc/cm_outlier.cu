@@ -122,6 +122,9 @@ __global__ void __launch_bounds__(ROR_THREADS) k_ror_count(const VoxelParams p, 
     }
     if (worst >= (1 << 14)) atomicExch(&p.ctrl->error, (uint32_t)CM_DEV_E_KEY_RANGE);
   }
+  // a frame k_grid_setup could not key has every key at 0 but its real div_b: its rows would lie outside the cell table.
+  // The host refuses such a call before this kernel is enqueued; its points stay unmarked here all the same.
+  if (g.zero_keys) return;
   const unsigned long long d0 = (unsigned long long)g.div_b[0], d1 = (unsigned long long)g.div_b[1],
                            d2 = (unsigned long long)g.div_b[2];
   const unsigned long long c0 = key % d0, t = key / d0, c1 = t % d1, c2 = t / d1;

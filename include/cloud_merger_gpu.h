@@ -379,7 +379,10 @@ CM_API int cm_zone_split(cm_handle_t h, const float* xyzi_host, int64_t n_points
  * the others. Non-finite points are never kept. Survivors keep their input order.
  *  cm_dev_radius_outlier: n packed float4 xyzi points on the device; results through cm_get_zone_out (one zone: xyzi +
  *      the index of every survivor in the input). Uses the handle's batch workspace (the previous run's device outputs
- *      are overwritten).
+ *      are overwritten). CM_E_KEY_RANGE when the radius is too small for the extent of the cloud: the call itself returns
+ *      it when the cell grid exceeds the key range (more than 2^21 cells on an axis, a coordinate beyond 2^30 cells);
+ *      cm_get_zone_out returns it when a point lies 2^14 cells or more from the origin (the cell margin only covers
+ *      less, so the neighbour counts are not guaranteed). The next call on the handle is not affected.
  *  cm_radius_outlier: host buffers in and out; *n_out receives the number of survivors (also on CM_E_CAPACITY). */
 CM_API int cm_dev_radius_outlier(cm_handle_t h, const float* xyzi_dev, int64_t n_points, double radius,
                                  int min_neighbors, int negative, void* stream);
@@ -388,7 +391,8 @@ CM_API int cm_radius_outlier(cm_handle_t h, const float* xyzi_host, int64_t n_po
 /* Several independent clouds in one pass (the per-zone outlierRemoval calls of one proceedX): cloud k = the points
  * [begin[k], begin[k+1]) of the array (begin[0] == 0, n_clouds <= CM_MAX_ZONES and <= the handle's max_batch_frames).
  * Every cloud has its own cell grid and neighbours are never counted across clouds. Results: zone k of cm_get_zone_out =
- * the survivors of cloud k (src = index in the whole array); the host form writes n_clouds + 1 offsets to out_begin. */
+ * the survivors of cloud k (src = index in the whole array); the host form writes n_clouds + 1 offsets to out_begin.
+ * CM_E_KEY_RANGE as for one cloud, when any of the clouds is too large for the radius. */
 CM_API int cm_dev_radius_outlier_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
                                        double radius, int min_neighbors, int negative, void* stream);
 CM_API int cm_radius_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds, double radius,

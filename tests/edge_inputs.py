@@ -9,6 +9,8 @@ Random clouds almost never put a coordinate where the float32 formulas are fragi
   C  large offsets: map-frame clouds kilometres from the origin (coarsest float32 cells and centroid sums);
   D  grid-size boundaries: clouds whose extent puts the cell count, the key width or PCL's INT32 guard exactly on or one
      cell past a threshold.
+  N  radius outlier removal: neighbour pairs across computed cell planes up to the 2^14-cell bound, the cell table's gaps
+     and bounds, every key width and pass count, the count's early exit, and grids the plan must refuse.
 
 Every generator is deterministic in its seed and returns (n, 4) float32 xyzi rows.
 """
@@ -671,3 +673,426 @@ def run_layout_frames(runs, cuts, seed: int, n_nonfinite: int = 0, shift=(0, 0, 
             continue
         out.append(run_layout_cloud(fr, seed + f, n_nonfinite=n_nonfinite, shift=tuple(f * s for s in shift)))
     return out
+
+
+# ---- N: radius outlier removal (cloud_merger_b200/csrc/cm_outlier.cu) -----------------------------------------------------
+# The radius outlier removal keys every point on a grid of cells a little wider than the radius, sorts the keys and lets
+# every point count inside the 3 x 3 rows of cells around its own, through a direct-address table of the cells' first
+# sorted positions (k_ror_table) or binary searches. ror_plan restates that plan in numpy: the cell, the grid of every
+# cloud (k_grid_setup), the keys and the sort plan, the table, and the nine rows each point searches with the table
+# entries they read. Its constants mirror the source; test_edge_inputs.py reads them out of it.
+ROR_MARGIN = 1.00390625                  # cell = f32(f32(radius) * (1 + 2^-8))
+ROR_BOUND = 1 << 14                      # |cell index| the margin covers; k_ror_count refuses from here on
+ROR_TABLE_LOG2 = 25                      # the table is used while n_clouds << idx_bits <= 2^25
+ROR_THREADS = 256                        # CTA of k_ror_table
+ROR_LONG_GAP = 2048                      # k_ror_table: a gap with to - from >= this goes to the CTA's shared list ...
+ROR_LIST = 32                            # ... of this many entries; more fall back to the warp that found them
+ROR_ROW_DZ, ROR_ROW_DY = 0x28215, 0x22161   # (dz + 1, dy + 1) of row rr in bits 2rr, 2rr + 1
+GRID_RANGE_CELLS = 1 << 21               # k_grid_setup: more cells on an axis, or a coordinate beyond 2^30 cells, is
+GRID_RANGE_ORIGIN = 1 << 30              # out of range and the frame is keyed as one cell (zero_keys)
+ROR_RADII = (float(F32(0.15)), 0.15, 1e-3, 0.5, 3.0)   # 0.15 as the float the reference holds, and as a double
+# a radius whose float32 cell is below it (f32(0.45) < 0.45): there the computed planes 2^k and 2^k + 1 (k = 1, 5, 9, 13)
+# are closer than the radius, so that without the margin two neighbours can sit two cells apart
+ROR_RADIUS_TIGHT = 0.45
+
+
+def ror_rows():
+    """(dz, dy) of the nine rows in the order k_ror_count visits them."""
+    return [(((ROR_ROW_DZ >> (2 * rr)) & 3) - 1, ((ROR_ROW_DY >> (2 * rr)) & 3) - 1) for rr in range(9)]
+
+
+def ror_cell(radius, margin: bool = True) -> np.float32:
+    r = F32(radius)
+    return F32(r * F32(ROR_MARGIN)) if margin else r
+
+
+def ror_r2(radius) -> np.float32:
+    return F32(float(radius) * float(radius))
+
+
+def ror_cells(x, cell) -> np.ndarray:
+    """floor(f32(x * (1 / cell))) per coordinate, as int64 (the cell of every point before min_b is taken off)."""
+    inv = F32(F32(1.0) / F32(cell))
+    with np.errstate(invalid="ignore", over="ignore"):
+        return np.floor((np.asarray(x, F32)[:, :3] * inv).astype(F32)).astype(np.float64)
+
+
+def _bits(cells: int) -> int:
+    return 0 if cells <= 1 else int(cells - 1).bit_length()
+
+
+def ror_grid(x, cell) -> dict:
+    """k_grid_setup of one cloud on the cell grid: min_b, max_b, div_b (kept at the real width even when out of range, as
+    the kernel leaves it), whether the grid is out of range (zero_keys: every key 0) and its index bits."""
+    x = np.asarray(x, F32)
+    fin = np.isfinite(x[:, :3]).all(axis=1)
+    if not fin.any():
+        return dict(empty=True, min_b=np.zeros(3, np.int64), max_b=np.zeros(3, np.int64), div=np.zeros(3, np.int64),
+                    zero_keys=False, bits=0)
+    fc = ror_cells(x[fin], cell)
+    fmn, fmx = fc.min(axis=0), fc.max(axis=0)
+    err = bool((np.abs(fmn) >= GRID_RANGE_ORIGIN).any() or (np.abs(fmx) >= GRID_RANGE_ORIGIN).any())
+    lim = float(2 ** 31 - 1)
+    mn = np.clip(fmn, -lim - 1, lim).astype(np.int64)      # (int) of the float saturates on the device
+    mx = np.clip(fmx, -lim - 1, lim).astype(np.int64)
+    div = mx - mn + 1
+    err = err or bool((div > GRID_RANGE_CELLS).any())
+    cells = 1 if err else int(div[0]) * int(div[1]) * int(div[2])
+    return dict(empty=False, min_b=mn, max_b=mx, div=div, zero_keys=err, bits=_bits(cells))
+
+
+def ror_plan(clouds, radius, table: bool = True, fixed: bool = True, margin: bool = True) -> dict:
+    """The whole plan of one radius_outlier_multi call (a single cloud is a list of one).
+    fixed=False restates the library before the host refused out-of-range grids: such a frame is then counted with key 0
+    and its real div_b. Returns the grids, the sort plan (idx_bits, key bytes, passes, table keys), whether the call is
+    refused (plan_error: before the table; bound_error: by the count kernel), and per point of every cloud its cells, key,
+    the nine row segments [k_lo, k_hi] it searches (-1 where a clamp skips the row) and the largest table entry it reads."""
+    cell = ror_cell(radius, margin)
+    clouds = [np.asarray(c, F32).reshape(-1, 4) for c in clouds]
+    n = len(clouds)
+    grids = [ror_grid(c, cell) for c in clouds]
+    has_invalid = any((~np.isfinite(c[:, :3]).all(axis=1)).any() for c in clouds)
+    key_frames = n + (1 if has_invalid else 0)
+    frame_bits = _bits(key_frames)
+    idx_bits = max([g["bits"] for g in grids if not g["empty"]] + [0])
+    total = frame_bits + idx_bits
+    plan_error = any(g["zero_keys"] for g in grids) or total > 64
+    total = min(total, 64)
+    idx_bits = total - frame_bits
+    passes = max(1, -(-total // 8))
+    n_points = sum(len(c) for c in clouds)
+    use_table = (table and n_points > 0 and idx_bits <= ROR_TABLE_LOG2 and (n << idx_bits) <= (1 << ROR_TABLE_LOG2))
+    table_keys = (n << idx_bits) if use_table else 0
+    worst = max([int(max(np.abs(g["min_b"]).max(), np.abs(g["max_b"]).max())) for g in grids if not g["empty"]] + [0])
+    refused = fixed and plan_error
+    rows = ror_rows()
+    per = []
+    for f, (c, g) in enumerate(zip(clouds, grids)):
+        fin = np.isfinite(c[:, :3]).all(axis=1)
+        m = len(c)
+        d = g["div"].astype(np.int64)
+        cc = np.zeros((m, 3), np.int64)
+        key = np.full(m, key_frames - 1 if has_invalid else n, np.int64) << idx_bits   # non-finite: the sentinel frame
+        if fin.any() and not g["empty"]:
+            if not g["zero_keys"]:
+                cc[fin] = ror_cells(c[fin], cell).astype(np.int64) - g["min_b"]
+            idx = cc[:, 0] + cc[:, 1] * d[0] + cc[:, 2] * d[0] * d[1]
+            key[fin] = (f << idx_bits) + (0 if g["zero_keys"] else idx[fin])
+        seg = np.full((m, 9, 2), -1, np.int64)
+        reads = np.full(m, -1, np.int64)
+        counted = fin & (not g["zero_keys"] or not fixed) & (not refused)
+        if counted.any():
+            c0, c1, c2 = cc[:, 0], cc[:, 1], cc[:, 2]
+            x_lo, x_hi = np.maximum(c0 - 1, 0), np.minimum(c0 + 1, d[0] - 1)
+            for rr, (dz, dy) in enumerate(rows):
+                ok = counted.copy()
+                if dz < 0: ok &= c2 > 0
+                if dz > 0: ok &= c2 + 1 < d[2]
+                if dy < 0: ok &= c1 > 0
+                if dy > 0: ok &= c1 + 1 < d[1]
+                row = ((c2 + dz) * d[1] + (c1 + dy)) * d[0]
+                seg[ok, rr, 0] = (f << idx_bits) + row[ok] + x_lo[ok]
+                seg[ok, rr, 1] = (f << idx_bits) + row[ok] + x_hi[ok]
+            hi = np.where(seg[:, :, 1] >= 0, seg[:, :, 1] + 1, -1).max(axis=1)
+            reads = np.where(counted, hi, -1)
+        per.append(dict(cells=cc, key=key, fin=fin, seg=seg, max_read=reads))
+    return dict(cell=cell, grids=grids, idx_bits=idx_bits, frame_bits=frame_bits, total_bits=total, passes=passes,
+                key_bytes=4 if total <= 32 else 8, table=use_table, table_keys=table_keys, plan_error=plan_error,
+                bound_error=worst >= ROR_BOUND, worst=worst, refused=refused, points=per)
+
+
+def ror_launches(plan, clouds) -> int:
+    """Kernel launches of the call as cm_launch_count reports them: a bounding box per non-empty cloud, the grid setup,
+    the key kernel, the radix passes, the table when it is used, the count."""
+    return sum(1 for c in clouds if len(c)) + 3 + plan["passes"] + (1 if plan["table"] else 0)
+
+
+def ror_pairs(x, radius) -> np.ndarray:
+    """(i, j), i < j, of the finite points of one cloud strictly inside the radius in the count's float order."""
+    from scipy.spatial import cKDTree
+    x = np.asarray(x, F32)
+    fin = np.nonzero(np.isfinite(x[:, :3]).all(axis=1))[0]
+    if len(fin) < 2:
+        return np.zeros((0, 2), np.int64)
+    p = cKDTree(x[fin, :3].astype(np.float64)).query_pairs(float(radius) * (1 + 1e-5) + 1e-30, output_type="ndarray")
+    p = fin[p]
+    d = x[p[:, 0], :3] - x[p[:, 1], :3]
+    acc = ((d[:, 0] * d[:, 0]).astype(F32) + (d[:, 1] * d[:, 1]).astype(F32)).astype(F32)
+    acc = (acc + (d[:, 2] * d[:, 2]).astype(F32)).astype(F32)
+    return p[acc < ror_r2(radius)]
+
+
+def ror_brute_count(x, radius) -> np.ndarray:
+    """O(n^2) count per point (itself included) in the count's float order; 0 for non-finite points."""
+    x = np.asarray(x, F32)
+    fin = np.isfinite(x[:, :3]).all(axis=1)
+    r2 = ror_r2(radius)
+    out = np.zeros(len(x), np.int64)
+    for s in range(0, len(x), 512):
+        with np.errstate(invalid="ignore", over="ignore"):
+            d = x[s:s + 512, None, :3] - x[None, :, :3]
+            acc = ((d[..., 0] * d[..., 0]).astype(F32) + (d[..., 1] * d[..., 1]).astype(F32)).astype(F32)
+            acc = (acc + (d[..., 2] * d[..., 2]).astype(F32)).astype(F32)
+            inside = (acc < r2) & fin[None, :] & fin[s:s + 512, None]
+        out[s:s + 512] = inside.sum(axis=1)
+    return out
+
+
+def cell_plane(p, cell) -> np.ndarray:
+    """The computed plane of cell index p (scalar or array): the smallest float32 x with floor(f32(x * inv)) >= p."""
+    inv = F32(F32(1.0) / F32(cell))
+    p = np.asarray(p, np.float64)
+    x = (p * float(cell)).astype(F32)
+    for _ in range(64):
+        up = np.floor((x * inv).astype(F32)) >= p
+        below = np.nextafter(x, F32(-np.inf))
+        down = np.floor((below * inv).astype(F32)) >= p
+        if not (~up).any() and not down.any():
+            return x
+        x = np.where(~up, np.nextafter(x, F32(np.inf)), np.where(down, below, x)).astype(F32)
+    raise AssertionError("cell plane search did not converge")
+
+
+def _directions():
+    out = []
+    for v in np.ndindex(3, 3, 3):
+        u = np.array(v, np.float64) - 1
+        if u.any():
+            out.append(u / np.linalg.norm(u))
+    return np.array(out)   # 6 axes, 12 face diagonals, 8 space diagonals
+
+
+MARGIN_PLANES = (0, 1000, 2500, 4000, 6000, 8000, 10000, 12000, 14000, ROR_BOUND - 2 - 3 * (26 * 9 - 1))
+
+
+def margin_cloud(radius, sign: int = 1) -> np.ndarray:
+    """N-margin: pairs at radius * (1 + k * 2^-23), k = -4..4, along the 26 axis and diagonal directions, centred on a corner
+    of computed cell planes (every coordinate on a plane), one corner every third cell from the MARGIN_PLANES indices on
+    (sign -1: mirrored), so that the cells of the pairs reach |index| 2^14 - 1 on every axis. Along the axes a second set
+    aims at the planes of a margin-free cell (cell = radius): the first point is the last float below such a plane, the
+    second the last float still inside the radius and up to 4 floats back from it -- where a grid without the margin can
+    put two neighbours two cells apart."""
+    cell, cell0 = ror_cell(radius), ror_cell(radius, margin=False)
+    r2 = ror_r2(radius)
+    dirs = _directions()
+    ks = np.arange(-4, 5)
+    J = len(dirs) * len(ks)
+    j = np.arange(J)
+    u, k = dirs[j // len(ks)], ks[j % len(ks)]
+    p = sign * (np.asarray(MARGIN_PLANES)[:, None] + 3 * j[None, :]).reshape(-1)
+    u, k = np.tile(u, (len(MARGIN_PLANES), 1)), np.tile(k, len(MARGIN_PLANES))
+    s = float(radius) * (1 + k * 2.0 ** -23)
+    c = np.column_stack([cell_plane(p, cell), cell_plane(p + 1, cell), cell_plane(-p, cell)]).astype(np.float64)
+    pairs = np.stack([c - u * s[:, None] / 2, c + u * s[:, None] / 2], axis=1).reshape(-1, 3).astype(F32)
+    # the aimed set: 6 axis directions x 5 steps back, at the planes 2^k (where the computed plane spacing is shortest) and
+    # spread over the range; every pair at its own place on the other two axes
+    Q = np.array([1 << k for k in range(1, 14)] + [m + 1 for m in MARGIN_PLANES[1:]], np.int64)
+    q = sign * np.repeat(Q, 30)
+    j = np.arange(len(q))
+    axis, neg, k = (j // 5) % 3, (j // 15) % 2 == 1, j % 5
+    keep = np.abs(q) < int((ROR_BOUND - 2) * float(cell0) / float(cell))
+    q, axis, neg, k, j = q[keep], axis[keep], neg[keep], k[keep], j[keep]
+    a = np.nextafter(cell_plane(q, cell0), F32(-np.inf))
+    b = (a + F32(float(radius))).astype(F32)
+    for _ in range(64):
+        out = ((b - a) * (b - a)).astype(F32) >= r2
+        if not out.any():
+            break
+        b = np.where(out, np.nextafter(b, F32(-np.inf)), b).astype(F32)
+    for step in range(4):
+        b = np.where(k > step, np.nextafter(b, F32(-np.inf)), b).astype(F32)
+    base = np.column_stack([cell_plane(sign * (5 + 3 * j), cell), cell_plane(sign * (7 + 3 * j), cell),
+                            cell_plane(sign * (11 + 3 * j), cell)]).astype(F32)
+    q1, q2 = base.copy(), base.copy()
+    rows = np.arange(len(q))
+    q1[rows, axis] = np.where(neg, b, a)
+    q2[rows, axis] = np.where(neg, a, b)
+    aimed = np.stack([q1, q2], axis=1).reshape(-1, 3)
+    out = np.concatenate([pairs, aimed])
+    return np.column_stack([out, np.arange(len(out), dtype=F32)]).astype(F32)
+
+
+def bound_cloud(radius, axis: int, index: int) -> np.ndarray:
+    """N-bound: a small cluster near the origin plus a pair of neighbours whose cells reach `index` on one axis, so that
+    the largest |cell index| of the grid is exactly |index| (2^14 - 1 passes, 2^14 is refused)."""
+    cell = ror_cell(radius)
+    rng = np.random.default_rng(abs(index) * 3 + axis + (index < 0))
+    near = rng.uniform(-3, 3, (200, 3)) * float(cell)
+    far = np.zeros((2, 3))
+    lo, hi = float(cell_plane(index, cell)), float(cell_plane(index + 1, cell))
+    far[:, axis] = [lo + 0.25 * (hi - lo), lo + 0.6 * (hi - lo)]
+    x = np.concatenate([near, far]).astype(F32)
+    assert np.abs(ror_cells(x, cell)).max() == max(abs(index), 3) or np.abs(ror_cells(x, cell)).max() == abs(index)
+    return np.column_stack([x, np.arange(len(x), dtype=F32)]).astype(F32)
+
+
+def range_clouds(radius=float(F32(0.15))) -> dict:
+    """N-range: clouds whose cell grid k_grid_setup cannot key: more than 2^21 cells on x and y (the two-point example
+    {(0,0,0), (4e5,4e5,0)}), and a cloud beyond 2^30 cells from the origin (spread over thousands of cells on x and y)."""
+    cell = float(ror_cell(radius))
+    wide = np.array([[0, 0, 0, 0], [4e5, 4e5, 0, 1]], F32)
+    x0 = 1.01 * GRID_RANGE_ORIGIN * cell
+    rng = np.random.default_rng(5)
+    far = np.column_stack([x0 + 16.0 * rng.integers(0, 60, 40), rng.uniform(0, 2000, 40), np.zeros(40),
+                           np.arange(40)]).astype(F32)
+    return {"wide": wide, "far": far}
+
+
+def gap_cloud(radius, steps, seed: int = 0) -> np.ndarray:
+    """N-gap: one point per cell, at exactly the cell keys cumsum([0] + steps). The rows are as long as the last key below
+    2^15 - 1 plus one (so the first row spans it and the keys come out as designed), centred on the origin. A point sits
+    close to the face it shares with the next cell of its row when the key step to that cell is 1, so neighbours are in
+    key-adjacent cells and a wrong table entry changes a count."""
+    cell = float(ror_cell(radius))
+    keys = np.concatenate([[0], np.cumsum(steps)]).astype(np.int64)
+    row = int(keys[keys < (1 << 15) - 2].max()) + 1
+    c0, c1 = keys % row, keys // row
+    rng = np.random.default_rng(seed)
+    frac = np.full(len(keys), 0.5)
+    nxt = np.r_[np.diff(keys) == 1, False]
+    prv = np.r_[False, np.diff(keys) == 1]
+    frac[nxt & ~prv] = 0.97                 # the first of a pair: at its high face ...
+    frac[prv & ~nxt] = 0.03                 # ... the second at its low face
+    frac[nxt & prv] = 0.5 + rng.choice([-0.47, 0.47], size=int((nxt & prv).sum()))
+    x = np.column_stack([(c0 - row // 2 + frac) * cell, (c1 + 0.5) * cell, np.full(len(keys), 0.5 * cell)]).astype(F32)
+    cells = ror_cells(x, ror_cell(radius)).astype(np.int64)
+    assert (cells[:, 0] == c0 - row // 2).all() and (cells[:, 1] == c1).all()
+    perm = rng.permutation(len(x))
+    return np.column_stack([x[perm], perm.astype(F32)]).astype(F32)
+
+
+def gap_steps(kind: str) -> list:
+    """Key steps of the N-gap layouts (k_ror_table: thread i fills (key[i-1], key[i]]; long means to - from >= 2048)."""
+    short = lambda n, rng: list(rng.choice([1, 1, 1, 2, 3], size=n))
+    rng = np.random.default_rng(len(kind))
+    if kind == "edge":           # gaps of 2047, 2048, 2049, 2050 entries (to - from = 2046 .. 2049) among short ones
+        s = short(300, rng)
+        for j, g in enumerate((2047, 2048, 2049, 2050, 2048, 2049)):
+            s[40 + 37 * j] = g
+        return s
+    if kind.startswith("cta"):   # L long gaps in the second CTA of 256 elements: list full, exactly full, one past
+        L = int(kind[3:])
+        s = short(700, rng)
+        for j in range(L):
+            s[300 + 6 * j] = 2049 + 17 * j
+        return s
+    if kind.startswith("m"):     # M % 256 in {0, 1, 255}: the gap above the largest key is thread M's
+        m = int(kind[1:])
+        s = short(m - 1, rng)
+        s[m // 2] = 5000
+        return s
+    raise ValueError(kind)
+
+
+GAP_KINDS = ("edge", "cta31", "cta32", "cta33", "m512", "m513", "m767")
+
+
+def width_cloud(radius, bits: int, seed: int = 0, n: int = 3000) -> np.ndarray:
+    """N-width: a cloud whose cell grid has exactly 2^bits cells (idx_bits = bits): its corner cells plus clusters of
+    neighbours and loose points in between, centred on the origin so that no cell index reaches 2^14."""
+    cell = float(ror_cell(radius))
+    b = [bits // 3 + (1 if k < bits % 3 else 0) for k in range(3)]
+    div = np.array([(1 << v) - (1 if v == 15 else 0) for v in b], np.int64)   # 2^15 - 1: cells -16383 .. 16383
+    assert _bits(int(np.prod(div))) == bits and (div < 1 << 15).all()
+    lo = -(div // 2)
+    rng = np.random.default_rng(seed + bits)
+    corners = np.array([[lo[k] + (div[k] - 1) * ((m >> k) & 1) for k in range(3)] for m in range(8)], np.float64)
+    centres = lo + rng.random((n // 6, 3)) * (div - 1)
+    pts = [corners + 0.5]
+    pts += [centres + rng.normal(0, 0.4, centres.shape) for _ in range(3)]
+    pts += [lo + rng.random((n // 2, 3)) * div]
+    x = np.concatenate(pts)
+    x = np.clip(x, lo + 0.01, lo + div - 0.01) * cell
+    x = x.astype(F32)
+    c = ror_cells(x, cell)
+    assert (c.min(axis=0) == lo).all() and (c.max(axis=0) == lo + div - 1).all()
+    return np.column_stack([x, rng.uniform(0, 255, len(x))]).astype(F32)
+
+
+def count_cloud(radius, kind: str, seed: int = 0) -> np.ndarray:
+    """N-count: hot: a cell of 2500 points (400 of them exact duplicates) amid loose ones -- the early exit decides in the
+    middle of a row; flat1 / flat2: d = 1 on one / two axes; single: one cell; nonfinite: a hot cloud with NaN / inf rows."""
+    cell = float(ror_cell(radius))
+    rng = np.random.default_rng(seed)
+    if kind in ("hot", "nonfinite"):
+        hot = rng.uniform(0.02, 0.98, (2100, 3)) * cell + 5 * cell
+        dup = np.repeat(hot[:4], 100, axis=0)
+        loose = rng.uniform(0, 12 * cell, (1500, 3))
+        x = np.concatenate([hot, dup, loose])
+    elif kind == "flat1":
+        x = np.column_stack([rng.uniform(0, 40 * cell, 3000), rng.uniform(0, 40 * cell, 3000), np.full(3000, 0.5 * cell)])
+    elif kind == "flat2":
+        x = np.column_stack([rng.uniform(0, 300 * cell, 3000), np.full(3000, 0.5 * cell), np.full(3000, 0.5 * cell)])
+    elif kind == "single":
+        x = rng.uniform(0.01, 0.99, (800, 3)) * cell + 2 * cell
+    else:
+        raise ValueError(kind)
+    x = x.astype(F32)
+    out = np.column_stack([x, rng.uniform(0, 255, len(x))]).astype(F32)
+    if kind == "nonfinite":
+        bad = out[rng.integers(0, len(out), 60)].copy()
+        bad[np.arange(60), np.arange(60) % 3] = np.array([np.nan, np.inf, -np.inf], F32)[np.arange(60) % 3]
+        out = np.concatenate([out, bad])
+    return out[rng.permutation(len(out))]
+
+
+COUNT_KINDS = ("hot", "flat1", "flat2", "single", "nonfinite")
+COUNT_MIN_PTS = (0, 1, 2, 100, 5000, 2 ** 31 - 1)
+
+
+def row_end_clouds(radius) -> list:
+    """N-count, frame edges: three clouds on the same 8 x 4 x 2 cell grid, each with neighbours in the first and the last
+    cell of its rows and in its first and last key cell, so that frame f's last cell and frame f + 1's first one are next
+    to each other in key order (and the same place in space: counting across clouds would change the result)."""
+    cell = float(ror_cell(radius))
+    out = []
+    for f in range(3):
+        rng = np.random.default_rng(40 + f)
+        pts = []
+        for cy in range(4):
+            for cz in range(2):
+                for cx in (0, 7):
+                    base = np.array([cx, cy, cz], np.float64)
+                    pts.append(base + rng.uniform(0.05, 0.95, (3, 3)))
+        pts.append(np.array([[0.02, 0.02, 0.02], [7.98, 3.98, 1.98]]))
+        x = (np.concatenate(pts) * cell).astype(F32)
+        out.append(np.column_stack([x, rng.uniform(0, 255, len(x))]).astype(F32))
+    return out
+
+
+def ror_cases() -> dict:
+    """name -> (clouds, radius, min_pts values) of every N family the GPU runs bit-exact (N-range and the refused N-bound
+    clouds are in ror_refused_cases)."""
+    r15 = float(F32(0.15))
+    cases = {}
+    for r in ROR_RADII + (ROR_RADIUS_TIGHT,):
+        for sign in (1, -1):
+            cases["margin:%g%s:%+d" % (r, "f" if r == r15 else "", sign)] = ([margin_cloud(r, sign)], r, (1, 2))
+    for axis in range(3):
+        for sign in (1, -1):
+            cases["bound:ok:%d%+d" % (axis, sign)] = ([bound_cloud(r15, axis, sign * (ROR_BOUND - 1))], r15, (1,))
+    for kind in GAP_KINDS:
+        cases["gap:" + kind] = ([gap_cloud(r15, gap_steps(kind))], r15, (0, 1, 2))
+    for bits in (4, 12, 20, 28, 36, 44):
+        cases["width:%d" % bits] = ([width_cloud(r15, bits)], r15, (1, 3))
+    cases["width:25"] = ([width_cloud(r15, 25)], r15, (1,))
+    cases["width:26"] = ([width_cloud(r15, 26)], r15, (1,))
+    cases["width:2x24"] = ([width_cloud(r15, 24, 1), width_cloud(r15, 20, 2)], r15, (1,))
+    cases["width:2x25"] = ([width_cloud(r15, 25, 1), width_cloud(r15, 12, 2)], r15, (1,))
+    cases["width:3x12+36"] = ([width_cloud(r15, 12, 3), width_cloud(r15, 36, 4), width_cloud(r15, 8, 5)], r15, (2,))
+    for kind in COUNT_KINDS:
+        cases["count:" + kind] = ([count_cloud(r15, kind)], r15, COUNT_MIN_PTS)
+    cases["count:row-ends"] = (row_end_clouds(r15), r15, (0, 1, 2, 3))
+    return cases
+
+
+def ror_refused_cases() -> dict:
+    """name -> (clouds, radius): calls the library must refuse with CM_E_KEY_RANGE."""
+    r15 = float(F32(0.15))
+    rc = range_clouds(r15)
+    normal = width_cloud(r15, 12, 7)
+    cases = {"bound:over:%d%+d" % (a, s): ([bound_cloud(r15, a, s * ROR_BOUND)], r15) for a in range(3) for s in (1, -1)}
+    cases["range:wide"] = ([rc["wide"]], r15)
+    cases["range:far"] = ([rc["far"]], r15)
+    cases["range:multi"] = ([normal, rc["wide"], normal[:100], rc["far"]], r15)
+    return cases

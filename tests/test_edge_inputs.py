@@ -354,3 +354,181 @@ def test_oracles_agree_on_run_layouts(oracle, case):
         assert E.bits_for(int(np.prod(c["div_b"].astype(np.int64)))) == 33
     else:
         assert c["min_b"].tolist() == [0, 0, 0] and c["n"] == sum(1 for r in runs if r >= min_points)
+
+
+# ---- N: radius outlier removal ------------------------------------------------------------------------------------------
+def _src(name):
+    with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "cloud_merger_b200", "csrc", name)) as f:
+        return f.read()
+
+
+def test_ror_constants_match_the_source():
+    """The N-family restatement mirrors the kernels' constants; a retune must fail here rather than miss the edges."""
+    ror, api, vox = _src("cm_outlier.cu"), _src("cm_api.cu"), _src("cm_voxel.cu")
+    assert "(float)radius * 1.00390625f" in api and E.ROR_MARGIN == 1.00390625
+    assert "worst >= (1 << 14)" in ror and E.ROR_BOUND == 1 << 14
+    assert "w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25)" in api and E.ROR_TABLE_LOG2 == 25
+    assert "constexpr int ROR_THREADS = 256;" in ror and E.ROR_THREADS == 256
+    assert "constexpr unsigned long long LONG_GAP = 2048;" in ror and "to - from >= LONG_GAP" in ror and E.ROR_LONG_GAP == 2048
+    assert "constexpr int LIST = 32;" in ror and E.ROR_LIST == 32
+    assert "0x28215u" in ror and "0x22161u" in ror and (E.ROR_ROW_DZ, E.ROR_ROW_DY) == (0x28215, 0x22161)
+    assert E.ror_rows() == [(0, 0), (0, -1), (0, 1), (-1, 0), (1, 0), (-1, -1), (-1, 1), (1, -1), (1, 1)]
+    assert "dv > (1ll << 21)" in vox and "1073741824.f" in vox
+    assert "if (g.zero_keys) return;" in ror and "w.plan_error == CM_DEV_E_KEY_RANGE" in api
+
+
+def _two_apart(x, pairs, cell):
+    c = E.ror_cells(x, cell)
+    return (np.abs(c[pairs[:, 0]] - c[pairs[:, 1]]) >= 2).any(axis=1)
+
+
+@pytest.mark.parametrize("radius", E.ROR_RADII + (E.ROR_RADIUS_TIGHT,))
+def test_margin_pairs_stay_one_cell_apart(radius):
+    """N-margin: with the shipped margin no neighbour pair is two cells apart on any axis, up to |cell index| 2^14 - 1 on
+    both signs, on both sides of the strict rule. Without the margin (cell = radius) the radius 0.45 puts more than 1 % of
+    the neighbour pairs two cells apart -- pairs the nine rows would not see. For the other radii the float32 cell is not
+    below the radius and the computed planes are never closer than it: there the margin is not what keeps them apart."""
+    for sign in (1, -1):
+        x = E.margin_cloud(radius, sign)
+        pairs = E.ror_pairs(x, radius)
+        designed = pairs[(pairs[:, 1] - pairs[:, 0] == 1) & (pairs[:, 0] % 2 == 0)]
+        assert 0.4 * len(x) / 2 < len(designed) < len(x) / 2   # some designed pairs fall just outside the radius
+        assert not _two_apart(x, pairs, E.ror_cell(radius)).any()
+        without = _two_apart(x, pairs, E.ror_cell(radius, margin=False)).mean()
+        if radius == E.ROR_RADIUS_TIGHT and sign > 0:
+            assert without >= 0.01, without
+        elif radius != E.ROR_RADIUS_TIGHT:
+            assert without == 0.0
+        c = E.ror_cells(x, E.ror_cell(radius))
+        assert (c.max() if sign > 0 else -c.min()) == E.ROR_BOUND - 1 and np.abs(c).max() == E.ROR_BOUND - 1
+        assert (c == 0).any()
+        plan = E.ror_plan([x], radius)
+        assert not plan["bound_error"] and not plan["plan_error"]
+
+
+def _assert_neighbours_searched(clouds, radius):
+    plan = E.ror_plan(clouds, radius)
+    for c, pt in zip(clouds, plan["points"]):
+        pairs = E.ror_pairs(c, radius)
+        for a, b in ((0, 1), (1, 0)):
+            seg = pt["seg"][pairs[:, a]]
+            kb = pt["key"][pairs[:, b]][:, None]
+            assert ((seg[:, :, 0] <= kb) & (kb <= seg[:, :, 1])).any(axis=1).all()
+    return plan
+
+
+@pytest.mark.parametrize("name", sorted(E.ror_cases()))
+def test_every_counted_neighbour_lies_in_the_searched_rows(name):
+    """For every edge cloud the run must succeed: each neighbour the oracle counts has its key in one of the nine row
+    segments the point searches, and with the table no read leaves it ([k_lo, k_hi + 1] <= table_keys)."""
+    clouds, radius, _ = E.ror_cases()[name]
+    plan = _assert_neighbours_searched(clouds, radius)
+    assert not plan["plan_error"] and not plan["bound_error"]
+    if plan["table"]:
+        assert max(int(p["max_read"].max(initial=-1)) for p in plan["points"]) <= plan["table_keys"]
+
+
+def test_bound_clouds_sit_on_the_bound():
+    """N-bound: the largest |cell index| is exactly 2^14 - 1 (accepted) or 2^14 (refused by the count kernel), on each axis
+    and sign; the grid itself stays in range."""
+    r = float(np.float32(0.15))
+    for axis in range(3):
+        for sign in (1, -1):
+            for idx, refused in ((E.ROR_BOUND - 1, False), (E.ROR_BOUND, True)):
+                x = E.bound_cloud(r, axis, sign * idx)
+                c = E.ror_cells(x, E.ror_cell(r))
+                assert (c[:, axis].max() if sign > 0 else -c[:, axis].min()) == idx
+                assert np.abs(np.delete(c, axis, axis=1)).max() < 4
+                plan = E.ror_plan([x], r)
+                assert plan["worst"] == idx and plan["bound_error"] == refused and not plan["plan_error"]
+
+
+@pytest.mark.parametrize("name", ["range:wide", "range:far", "range:multi"])
+def test_out_of_range_grids_read_past_the_table_unless_refused(name):
+    """N-range: the grid of an out-of-range cloud is keyed as one cell but keeps its real div_b. The count as it was
+    before the host check (fixed=False) then reads table entries far past table_keys -- the defect. The fixed library
+    refuses the call before the table and the count, and would not count such a frame at all."""
+    clouds, r = E.ror_refused_cases()[name]
+    before = E.ror_plan(clouds, r, fixed=False)
+    assert before["plan_error"] and before["table"]
+    worst_read = max(int(p["max_read"].max(initial=-1)) for p in before["points"])
+    assert worst_read > before["table_keys"], (worst_read, before["table_keys"])
+    if name == "range:wide":
+        g = before["grids"][0]
+        assert g["zero_keys"] and tuple(g["div"]) == (2656291, 2656291, 1) and before["idx_bits"] == 0
+        assert before["table_keys"] == 1 and worst_read == 2656293
+    after = E.ror_plan(clouds, r)
+    assert after["refused"] and all((p["max_read"] < 0).all() for p in after["points"])
+
+
+def test_gap_layouts_hit_the_table_edges():
+    """N-gap: the sorted keys give the gap lengths around LONG_GAP, 31 / 32 / 33 long gaps in one CTA of k_ror_table,
+    M % 256 in {0, 1, 255} (thread M fills the top gap, alone in its CTA when M % 256 == 0) and a long empty range above
+    the largest key."""
+    r = float(np.float32(0.15))
+    for kind in E.GAP_KINDS:
+        x = E.gap_cloud(r, E.gap_steps(kind))
+        plan = E.ror_plan([x], r)
+        keys = np.sort(plan["points"][0]["key"])
+        assert len(np.unique(keys)) == len(keys) and plan["table"]
+        to_minus_from = np.diff(keys) - 1
+        long_at = np.nonzero(to_minus_from >= E.ROR_LONG_GAP)[0] + 1        # element that fills it
+        if kind == "edge":
+            assert {2046, 2047, 2048, 2049} <= set(to_minus_from.tolist())
+        if kind.startswith("cta"):
+            per_cta = np.bincount(long_at // E.ROR_THREADS)
+            assert per_cta[1] == int(kind[3:]) and (np.delete(per_cta, 1) <= E.ROR_LIST).all()
+        if kind.startswith("m"):
+            assert len(keys) == int(kind[1:]) and len(keys) % 256 in (0, 1, 255)
+        assert plan["table_keys"] - keys[-1] >= 1000
+
+
+def test_width_layouts_hit_every_pass_count_and_the_table_bound():
+    """N-width: 1-4 radix passes with 32-bit keys and 5-6 with 64-bit ones (both parities on both widths), and the
+    table / binary-search boundary at idx_bits 25 / 26 for one cloud and 24 / 25 for two."""
+    cases = E.ror_cases()
+    got = {}
+    for name in [n for n in cases if n.startswith("width:")]:
+        clouds, r, _ = cases[name]
+        p = E.ror_plan(clouds, r)
+        got[name] = (p["idx_bits"], p["key_bytes"], p["passes"], p["table"])
+    assert {(b, p) for (_, b, p, _) in got.values()} >= {(4, 1), (4, 2), (4, 3), (4, 4), (8, 5), (8, 6)}
+    assert got["width:25"][::3] == (25, True) and got["width:26"][::3] == (26, False)
+    assert got["width:2x24"][::3] == (24, True) and got["width:2x25"][::3] == (25, False)
+
+
+def test_count_layouts():
+    """N-count: a hot cell of 2000+ points with exact duplicates, flat grids (d = 1 on one and two axes), a single-cell
+    cloud, non-finite rows, and frames whose last and first key cells are next to each other in key order."""
+    r = float(np.float32(0.15))
+    cell = E.ror_cell(r)
+    hot = E.count_cloud(r, "hot")
+    _, counts = np.unique(E.ror_cells(hot, cell), axis=0, return_counts=True)
+    assert counts.max() >= 2000 and len(np.unique(hot[:, :3], axis=0)) < len(hot)
+    assert (E.ror_grid(E.count_cloud(r, "flat1"), cell)["div"] == 1).sum() == 1
+    assert (E.ror_grid(E.count_cloud(r, "flat2"), cell)["div"] == 1).sum() == 2
+    assert (E.ror_grid(E.count_cloud(r, "single"), cell)["div"] == 1).all()
+    assert (~np.isfinite(E.count_cloud(r, "nonfinite")[:, :3]).all(axis=1)).sum() == 60
+    clouds = E.row_end_clouds(r)
+    plan = E.ror_plan(clouds, r)
+    cells = 8 * 4 * 2
+    for f, pt in enumerate(plan["points"]):
+        k = pt["key"] - (f << plan["idx_bits"])
+        assert k.min() == 0 and k.max() == cells - 1 and E.ror_grid(clouds[f], cell)["div"].tolist() == [8, 4, 2]
+        c0 = pt["cells"][:, 0]
+        assert (c0 == 0).sum() >= 3 and (c0 == 7).sum() >= 3
+    assert plan["idx_bits"] == 6 and cells == 1 << plan["idx_bits"]   # the last cell of frame f is key (f + 1) << 6 minus 1
+
+
+@pytest.mark.parametrize("name", [n for n in sorted(E.ror_cases()) if not n.startswith("margin:") or n.startswith("margin:0.15f")])
+def test_ror_oracle_agrees_with_the_brute_force_count(oracle, name):
+    """The C++ oracle (cmo_radius_outlier) against the O(n^2) numpy count on every N cloud small enough."""
+    clouds, r, min_pts = E.ror_cases()[name]
+    for c in clouds:
+        k = E.ror_brute_count(c, r)
+        fin = np.isfinite(c[:, :3]).all(axis=1)
+        for m in min_pts:
+            for neg in (False, True):
+                want = np.nonzero(fin & ((k <= m) if neg else (k > m)))[0]
+                got = oracle.radius_outlier(c, r, m, neg)
+                assert len(got) == len(want) and (got == want).all(), (m, neg)
