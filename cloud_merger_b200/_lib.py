@@ -53,6 +53,25 @@ class CmPlane(C.Structure):
 
 
 CM_SUM4_SSE2, CM_SUM4_SSE3, CM_SUM4_SCALAR = 0, 1, 2
+
+CM_SOR_MAX_K = 127
+CM_SOR_SQRT_FLOAT, CM_SOR_SQRT_DOUBLE = 0, 1
+CM_SOR_SUM_SERIAL, CM_SOR_SQ_SUM_SERIAL = 1, 2
+
+
+class CmSorCfg(C.Structure):
+    _fields_ = [("mean_k", C.c_int32), ("negative", C.c_int32), ("sqrt_mode", C.c_int32), ("reserved", C.c_int32),
+                ("std_mul", C.c_double)]
+
+
+class CmSorStats(C.Structure):
+    _fields_ = [("mean", C.c_double), ("stddev", C.c_double), ("threshold", C.c_double), ("n_valid", C.c_int64),
+                ("too_few", C.c_int32), ("sum_path", C.c_int32)]
+
+
+class CmSorOut(C.Structure):
+    _fields_ = [("distances", C.c_void_p), ("n_points", C.c_int64), ("n_clouds", C.c_int32), ("reserved", C.c_int32),
+                ("knn_ms", C.c_float), ("sums_ms", C.c_float), ("cloud", CmSorStats * CM_MAX_ZONES)]
 CM_MAX_PROCEED_PARTS = 8
 
 
@@ -188,6 +207,14 @@ SYMBOLS = {
                                               C.c_void_p]),
     "cm_radius_outlier_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.c_double, C.c_int, C.c_int,
                                           C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
+    "cm_dev_statistical_outlier": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmSorCfg), C.c_void_p]),
+    "cm_dev_statistical_outlier_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmSorCfg),
+                                                   C.c_void_p]),
+    "cm_statistical_outlier": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmSorCfg), C.c_void_p, C.c_void_p, C.c_int64,
+                                         C.POINTER(C.c_int64)]),
+    "cm_statistical_outlier_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmSorCfg),
+                                               C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
+    "cm_get_statistical_out": (C.c_int, [_H, C.POINTER(CmSorOut)]),
     "cm_dev_plane_ransac": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmPlaneCfg), C.POINTER(CmPlane), C.c_void_p]),
     "cm_dev_plane_ransac_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmPlaneCfg),
                                             C.POINTER(CmPlane), C.c_void_p]),

@@ -275,6 +275,70 @@ class CloudMerger:
                                                       oi.ctypes.data_as(C.c_void_p), C.c_int64(n), ob))
         return [(ox[ob[c]:ob[c + 1]].copy(), (oi[ob[c]:ob[c + 1]].astype(np.int64) - begin[c]).astype(np.uint32)) for c in range(k)]
 
+    # -- statistical outlier removal (pcl::StatisticalOutlierRemoval) --------------------------------------------------------
+    @staticmethod
+    def _sor_cfg(mean_k, std_mul, negative, sqrt_mode):
+        return _lib.CmSorCfg(int(mean_k), int(bool(negative)), int(sqrt_mode), 0, float(std_mul))
+
+    def dev_statistical_outlier(self, xyzi_ptr: int, n_points: int, mean_k: int, std_mul: float, negative: bool = False,
+                                sqrt_mode: int = 0, stream: int = 0):
+        """Device form; fetch the survivors with radius_outlier_out() / zone_out() and the per-point mean distances and
+        per-cloud statistics with statistical_outlier_out()."""
+        cfg = self._sor_cfg(mean_k, std_mul, negative, sqrt_mode)
+        self._check(self._lib.cm_dev_statistical_outlier(self._h, C.c_void_p(xyzi_ptr or None), C.c_int64(n_points),
+                                                         C.byref(cfg), C.c_void_p(stream or None)))
+
+    def dev_statistical_outlier_multi(self, xyzi_ptr: int, begin, mean_k: int, std_mul: float, negative: bool = False,
+                                      sqrt_mode: int = 0, stream: int = 0):
+        """Independent clouds [begin[k], begin[k+1]) of one device array in one pass; zone k of zone_out() = survivors of
+        cloud k (needs max_batch_frames >= number of clouds)."""
+        b = (C.c_int64 * len(begin))(*[int(v) for v in begin])
+        cfg = self._sor_cfg(mean_k, std_mul, negative, sqrt_mode)
+        self._check(self._lib.cm_dev_statistical_outlier_multi(self._h, C.c_void_p(xyzi_ptr or None), b, len(begin) - 1,
+                                                               C.byref(cfg), C.c_void_p(stream or None)))
+
+    def statistical_outlier_out(self) -> dict:
+        """Of the last statistical outlier removal: "distances" (float32 [n], input order) and "clouds", one dict per cloud
+        (mean, stddev, threshold, n_valid, too_few, sum_path), plus "knn_ms" / "sums_ms" (-1 unless profiling)."""
+        so = _lib.CmSorOut()
+        self._check(self._lib.cm_get_statistical_out(self._h, C.byref(so)))
+        n = int(so.n_points)
+        dist = self.download(so.distances, np.float32, n) if n else np.zeros(0, np.float32)
+        clouds = [{"mean": c.mean, "stddev": c.stddev, "threshold": c.threshold, "n_valid": int(c.n_valid),
+                   "too_few": bool(c.too_few), "sum_path": int(c.sum_path)} for c in so.cloud[:so.n_clouds]]
+        return {"distances": dist, "clouds": clouds, "knn_ms": float(so.knn_ms), "sums_ms": float(so.sums_ms)}
+
+    def statistical_outlier(self, xyzi: np.ndarray, mean_k: int, std_mul: float, negative: bool = False, sqrt_mode: int = 0):
+        """Host-buffer form: (xyzi [k,4] float32, idx [k] uint32 indices into the input, ascending)."""
+        a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
+        n = len(a)
+        ox = np.empty((max(n, 1), 4), np.float32)
+        oi = np.empty(max(n, 1), np.uint32)
+        k = C.c_int64()
+        cfg = self._sor_cfg(mean_k, std_mul, negative, sqrt_mode)
+        self._check(self._lib.cm_statistical_outlier(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(n), C.byref(cfg),
+                                                     ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p),
+                                                     C.c_int64(n), C.byref(k)))
+        return ox[:k.value].copy(), oi[:k.value].copy()
+
+    def statistical_outlier_multi(self, clouds, mean_k: int, std_mul: float, negative: bool = False,
+                                  sqrt_mode: int = 0) -> list:
+        """Host-buffer form: per cloud (xyzi [k,4], idx [k] into that cloud)."""
+        arrs = [np.ascontiguousarray(c, np.float32).reshape(-1, 4) for c in clouds]
+        k = len(arrs)
+        begin = np.concatenate([[0], np.cumsum([len(a) for a in arrs])]).astype(np.int64)
+        n = int(begin[-1])
+        allpts = np.ascontiguousarray(np.concatenate(arrs)) if n else np.zeros((0, 4), np.float32)
+        ox = np.empty((max(n, 1), 4), np.float32)
+        oi = np.empty(max(n, 1), np.uint32)
+        ob = (C.c_int64 * (k + 1))()
+        b = (C.c_int64 * (k + 1))(*[int(v) for v in begin])
+        cfg = self._sor_cfg(mean_k, std_mul, negative, sqrt_mode)
+        self._check(self._lib.cm_statistical_outlier_multi(self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.byref(cfg),
+                                                           ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p),
+                                                           C.c_int64(n), ob))
+        return [(ox[ob[c]:ob[c + 1]].copy(), (oi[ob[c]:ob[c + 1]].astype(np.int64) - begin[c]).astype(np.uint32)) for c in range(k)]
+
     # -- RANSAC ground plane (pcl::SACSegmentation of removeGround, pc_preprocessing_main.cpp:95-117) ------------------------
     @staticmethod
     def _plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order):

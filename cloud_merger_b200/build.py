@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libcloud_merger_gpu.so")
-SOURCES = ["cm_transform_crop.cu", "cm_voxel.cu", "cm_radix_sort.cu", "cm_zones.cu", "cm_outlier.cu", "cm_route.cu", "cm_plane.cu", "cm_api.cu"]
+SOURCES = ["cm_transform_crop.cu", "cm_voxel.cu", "cm_radix_sort.cu", "cm_zones.cu", "cm_outlier.cu", "cm_route.cu", "cm_plane.cu", "cm_statistical.cu", "cm_api.cu"]
 HEADERS = ["cm_common.cuh", "cm_kernels.h", os.path.join("..", "..", "include", "cloud_merger_gpu.h")]
 
 NVCC_FLAGS = [

@@ -212,6 +212,21 @@ struct cm_handle_s {
   // radius outlier removal: first sorted position of every cell key (allocated on first use, grows)
   DevPtr<uint32_t> ror_table;
   size_t ror_table_cap = 0;
+  // statistical outlier removal (allocated on first use, grows)
+  struct SorWs {
+    size_t cap = 0;
+    DevPtr<float4> sorted_pts;     // [cap] the points in sorted key order
+    DevPtr<float> dist;            // [cap] mean distance per input point
+    DevPtr<SorStats> stats;        // [CM_MAX_ZONES]
+    HostPtr<SorStats> stats_host;  // pinned mirror, copied at the end of every run
+    Event ev[3];                   // profiling: before the search, after it, after the sums
+    cudaStream_t stream = nullptr;
+    bool ran = false, profiled = false;
+    int n_clouds = 0;
+    int64_t n_points = 0;
+    uint32_t n_valid[CM_MAX_ZONES] = {};
+    uint32_t too_few = 0;
+  } sw;
   // RANSAC ground plane (allocated on first use): one batch of draws and its scores, device + pinned mirrors
   struct PlaneWs {
     size_t cap_draws = 0;
@@ -2060,6 +2075,271 @@ int cm_radius_outlier(cm_handle_t h, const float* xyzi_host, int64_t n_points, d
   const int rc = cm_radius_outlier_multi(h, xyzi_host, begin, 1, radius, min_neighbors, negative, out_xyzi, out_idx, capacity, ob);
   *n_out = ob[1];
   return rc;
+}
+
+// ---- statistical outlier removal ----------------------------------------------------------------------------------------
+namespace {
+int sor_ws_ensure(cm_handle_t h, size_t points) {
+  cm_handle_s::SorWs& s = h->sw;
+  if (s.cap >= std::max<size_t>(points, 1) && s.stats) return CM_OK;
+  const size_t want = std::max<size_t>(points, 1);
+  s.sorted_pts.reset(); s.dist.reset(); s.cap = 0;  // the old buffers go before the larger ones are allocated
+  CM_CUDA(h, dev_alloc(s.sorted_pts, want));
+  CM_CUDA(h, dev_alloc(s.dist, want));
+  if (!s.stats) {
+    CM_CUDA(h, dev_alloc(s.stats, (size_t)CM_MAX_ZONES));
+    CM_CUDA(h, pinned_alloc(s.stats_host, sizeof(SorStats) * CM_MAX_ZONES, cudaHostAllocDefault));
+    for (auto& e : s.ev) CM_CUDA(h, create(e, cudaEventCreateWithFlags, cudaEventDefault));
+  }
+  s.cap = want;
+  return CM_OK;
+}
+
+// The cell edge of a statistical outlier removal. The result does not depend on it -- the search grows until its bound
+// holds -- but the cost does: cells about as wide as the radius that holds mean_k + 1 neighbours of an average point of
+// the largest cloud, its points taken as spread over the two largest extents of its bounding box (a LiDAR cloud is a
+// surface), so that most searches end after the cube of half-width 1. Never below what keeps every cloud inside the key
+// range: at most 2^19 cells across an axis and |x| / edge <= 2^20, which also keeps the float rounding of x * inv below
+// 1/8 cell. CM_SOR_CELL=<metres> overrides the estimate (not the key-range floor): tests force tiny and huge cells with it.
+double sor_cell_edge(const float (*mn)[3], const float (*mx)[3], const int64_t* n_fin, int n_clouds, int mean_k) {
+  double floor_edge = 0.0, edge = 1.0;
+  int64_t biggest = 0;
+  for (int c = 0; c < n_clouds; ++c) {
+    if (n_fin[c] <= 0) continue;
+    double e[3];
+    for (int a = 0; a < 3; ++a) {
+      e[a] = (double)mx[c][a] - (double)mn[c][a];
+      const double mag = std::max(std::fabs((double)mn[c][a]), std::fabs((double)mx[c][a]));
+      floor_edge = std::max(floor_edge, std::max(mag / 1048576.0, e[a] / 524288.0));
+    }
+    std::sort(e, e + 3, [](double x, double y) { return x > y; });
+    double ec = 1.0;
+    if (e[1] > 0.0) ec = std::sqrt((mean_k + 1.0) * e[0] * e[1] / (3.141592653589793 * (double)n_fin[c]));
+    else if (e[0] > 0.0) ec = (mean_k + 1.0) * e[0] / (2.0 * (double)n_fin[c]);
+    if (n_fin[c] > biggest) { biggest = n_fin[c]; edge = ec; }
+  }
+  const char* forced = getenv("CM_SOR_CELL");
+  if (forced && atof(forced) > 0.0) edge = atof(forced);
+  edge = std::max(edge, floor_edge * (1.0 + 1.0 / 1024.0));
+  return std::min(std::max(edge, 1e-30), 1e36);  // 1 / edge stays a normal float
+}
+
+// clouds = the ranges [begin[k], begin[k+1]) of pts (frames of the cell key: no neighbours across clouds); output zone k =
+// the survivors of cloud k
+int statistical_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, const cm_sor_cfg_t* cfg,
+                            cudaStream_t st) {
+  if (!cfg) return fail(h, CM_E_INVALID, "cfg is NULL");
+  if (cfg->mean_k < 1 || cfg->mean_k > CM_SOR_MAX_K) return fail(h, CM_E_INVALID, "mean_k must be 1 .. %d", CM_SOR_MAX_K);
+  if (std::isnan(cfg->std_mul)) return fail(h, CM_E_INVALID, "std_mul is NaN");
+  if (cfg->sqrt_mode != CM_SOR_SQRT_FLOAT && cfg->sqrt_mode != CM_SOR_SQRT_DOUBLE) return fail(h, CM_E_INVALID, "bad sqrt_mode");
+  if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
+  if (begin[0] != 0) return fail(h, CM_E_INVALID, "begin[0] must be 0");
+  for (int c = 0; c < n_clouds; ++c)
+    if (begin[c + 1] < begin[c]) return fail(h, CM_E_INVALID, "begin must not decrease");
+  const int64_t n_points = begin[n_clouds];
+  if (in_zone_outputs(h, pts, n_points)) return fail(h, CM_E_INVALID, "the input cloud lies in this handle's own zone outputs (use another handle or copy it out)");
+  int rc = ensure_batch_ws(h);
+  if (rc != CM_OK) return rc;
+  Workspace& w = h->batch;
+  if (n_points > (int64_t)w.cap_points) return fail(h, CM_E_CAPACITY, "%lld points > capacity %u", (long long)n_points, w.cap_points);
+  if ((uint32_t)n_clouds > w.cap_frames)
+    return fail(h, CM_E_CAPACITY, "%d clouds > max_batch_frames %u of this handle", n_clouds, w.cap_frames);
+  rc = zone_ws_ensure(h, (size_t)n_points);
+  if (rc != CM_OK) return rc;
+  rc = sor_ws_ensure(h, (size_t)n_points);
+  if (rc != CM_OK) return rc;
+  cm_handle_s::SorWs& s = h->sw;
+  s.ran = false;
+  w.has_run = true; w.report_valid = false; w.profiled = false;
+  w.n_frames = (uint32_t)n_clouds; w.n_segs = 0; w.points_in = n_points; w.launches = 0;
+  w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
+  w.voxel_pts = pts; w.fused_keys = false;
+  h->last = &w;
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
+  CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
+  VoxelParams vp;
+  fill_voxel_params(h, w, vp, pts, (uint32_t)n_clouds, (uint32_t)n_points);
+  vp.pcl_refuses = 0;
+  uint32_t* fss = const_cast<uint32_t*>(vp.frame_surv_start);
+  for (int c = 0; c < n_clouds; ++c) {  // bounding box and non-finite count of every cloud
+    const uint32_t n_here = (uint32_t)(begin[c + 1] - begin[c]);
+    if (!n_here) continue;
+    CM_CUDA(h, launch_minmax(pts + begin[c], n_here, vp.ctrl, vp.acc + c, fss + c, st));
+    ++w.launches;
+  }
+  if (n_clouds > 1 || n_points == 0) {  // the cloud ranges (the single-cloud launch above wrote them itself)
+    uint32_t starts[CM_MAX_ZONES + 1];
+    for (int c = 0; c <= n_clouds; ++c) starts[c] = (uint32_t)begin[c];
+    CM_CUDA(h, cudaMemcpyAsync(fss, starts, sizeof(uint32_t) * (size_t)(n_clouds + 1), cudaMemcpyHostToDevice, st));
+  }
+  // one round trip: the bounds choose the cell edge, the finite counts are PCL's valid_distances
+  FrameAcc acc[CM_MAX_ZONES];
+  CM_CUDA(h, cudaMemcpyAsync(acc, vp.acc, sizeof(FrameAcc) * (size_t)n_clouds, cudaMemcpyDeviceToHost, st));
+  CM_CUDA(h, cudaStreamSynchronize(st));
+  float mn[CM_MAX_ZONES][3], mx[CM_MAX_ZONES][3];
+  int64_t n_fin[CM_MAX_ZONES];
+  uint32_t too_few = 0;
+  for (int c = 0; c < n_clouds; ++c) {
+    const int64_t n_here = begin[c + 1] - begin[c];
+    n_fin[c] = n_here ? n_here - (int64_t)acc[c].n_invalid : 0;
+    for (int a = 0; a < 3; ++a) {
+      const uint32_t lo = f32_order_dec(~acc[c].nmin_enc[a]), hi = f32_order_dec(acc[c].max_enc[a]);
+      memcpy(&mn[c][a], &lo, 4);
+      memcpy(&mx[c][a], &hi, 4);
+    }
+    s.n_valid[c] = (uint32_t)n_fin[c];
+    if (n_fin[c] > 0 && n_fin[c] <= cfg->mean_k) too_few |= 1u << c;
+  }
+  const float inv = (float)(1.0 / sor_cell_edge(mn, mx, n_fin, n_clouds, cfg->mean_k));
+  for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = inv;
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
+  rc = run_voxel(h, w, vp, st, false, false);  // keys + sort only
+  if (rc != CM_OK) return rc;
+  if (w.plan_error == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "cell grid exceeds the key range");
+  if (w.plan_error) return fail(h, CM_E_INTERNAL, "device error %u", w.plan_error);
+  vp.key_bytes = w.key_bytes;
+  SorParams sp;
+  sp.mean_k = (uint32_t)cfg->mean_k;
+  sp.sqrt_mode = (uint32_t)cfg->sqrt_mode;
+  sp.too_few = too_few;
+  sp.sorted_pts = s.sorted_pts.get();
+  sp.dist = s.dist.get();
+  sp.cell_start = nullptr;
+  sp.cell = 1.0 / (double)inv;
+  // the radius outlier removal's direct-address table of the cells' first sorted positions when the key space is small
+  // (CM_SOR_NO_TABLE=1 forces the binary searches: test hook for the large-key-space path)
+  if (n_points > 0 && w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&
+      !getenv("CM_SOR_NO_TABLE")) {
+    const size_t keys = (size_t)n_clouds << w.plan_idx_bits;
+    if (h->ror_table_cap < keys + 1) {
+      h->ror_table.reset(); h->ror_table_cap = 0;  // the old table goes before the larger one is allocated
+      CM_CUDA(h, dev_alloc(h->ror_table, keys + 1));
+      h->ror_table_cap = keys + 1;
+    }
+    RorParams rp{};
+    rp.cell_start = h->ror_table.get(); rp.table_keys = (uint32_t)keys;
+    CM_CUDA(h, launch_radius_table(vp, rp, st));
+    ++w.launches;
+    sp.cell_start = rp.cell_start;
+  }
+  if (n_points) CM_CUDA(h, cudaMemsetAsync(s.dist.get(), 0, (size_t)n_points * sizeof(float), st));
+  s.profiled = h->profiling;
+  if (s.profiled) CM_CUDA(h, cudaEventRecord(s.ev[0].get(), st));
+  CM_CUDA(h, launch_sor_knn(vp, sp, s.sorted_pts.get(), st));
+  w.launches += 2;
+  if (s.profiled) CM_CUDA(h, cudaEventRecord(s.ev[1].get(), st));
+  SorSumParams q{};
+  q.dist = s.dist.get();
+  q.n_clouds = (uint32_t)n_clouds;
+  for (int c = 0; c <= n_clouds; ++c) q.begin[c] = (uint32_t)begin[c];
+  for (int c = 0; c < n_clouds; ++c) q.n_valid[c] = s.n_valid[c];
+  q.too_few = too_few;
+  q.force_serial = getenv("CM_SOR_SERIAL_SUMS") ? 1u : 0u;  // test hook: the serial chain for every cloud
+  q.negative = cfg->negative ? 1u : 0u;
+  q.std_mul = cfg->std_mul;
+  q.stats = s.stats.get();
+  q.mask = h->zw.mask.get();
+  CM_CUDA(h, launch_sor_sums(q, st));
+  if (s.profiled) CM_CUDA(h, cudaEventRecord(s.ev[2].get(), st));
+  CM_CUDA(h, launch_sor_select(q, (uint32_t)n_points, st));
+  w.launches += 2;
+  CM_CUDA(h, cudaMemcpyAsync(s.stats_host.get(), s.stats.get(), sizeof(SorStats) * (size_t)n_clouds, cudaMemcpyDeviceToHost, st));
+  CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
+  rc = zone_run(h, pts, n_points, st, true, n_clouds);
+  if (rc != CM_OK) return rc;
+  s.stream = st; s.n_clouds = n_clouds; s.n_points = n_points; s.too_few = too_few; s.ran = true;
+  return CM_OK;
+}
+}  // namespace
+
+int cm_dev_statistical_outlier(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_sor_cfg_t* cfg, void* stream) {
+  if (!h) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
+  if (n_points < 0) return fail(h, CM_E_INVALID, "bad n_points");
+  const int64_t begin[2] = {0, n_points};
+  return statistical_outlier_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, 1, cfg, static_cast<cudaStream_t>(stream));
+}
+
+int cm_dev_statistical_outlier_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
+                                     const cm_sor_cfg_t* cfg, void* stream) {
+  if (!h || !begin) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  if (n_clouds >= 1 && n_clouds <= CM_MAX_ZONES && begin[n_clouds] > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u)))
+    return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
+  return statistical_outlier_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, n_clouds, cfg,
+                                 static_cast<cudaStream_t>(stream));
+}
+
+int cm_statistical_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds,
+                                 const cm_sor_cfg_t* cfg, float* out_xyzi, uint32_t* out_idx, int64_t capacity,
+                                 int64_t* out_begin) {
+  if (!h || !begin || !out_begin) return CM_E_INVALID;
+  if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
+  const int64_t n_points = begin[n_clouds];
+  if (n_points < 0 || (n_points > 0 && !xyzi_host)) return CM_E_INVALID;
+  cm_zone_out_t zo;
+  {
+    std::lock_guard<std::mutex> lk(h->mu);
+    CM_CUDA(h, cudaSetDevice(h->device));
+    int rc = zone_ws_ensure(h, (size_t)n_points);
+    if (rc != CM_OK) return rc;
+    cm_handle_s::ZoneWs& z = h->zw;
+    if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
+    if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
+    rc = statistical_outlier_run(h, z.in_stage.get(), begin, n_clouds, cfg, nullptr);
+    if (rc != CM_OK) return rc;
+  }
+  int rc = cm_get_zone_out(h, &zo);
+  for (int k = 0; k <= n_clouds; ++k) out_begin[k] = zo.begin[k];
+  if (rc != CM_OK) return rc;
+  {
+    std::lock_guard<std::mutex> lk(h->mu);
+    const int64_t total = zo.begin[n_clouds];
+    if (total > capacity) return fail(h, CM_E_CAPACITY, "%lld points kept, caller capacity %lld", (long long)total, (long long)capacity);
+    if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
+    if (out_idx && total) CM_CUDA(h, cudaMemcpy(out_idx, zo.src, (size_t)total * 4, cudaMemcpyDeviceToHost));
+  }
+  return CM_OK;
+}
+
+int cm_statistical_outlier(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_sor_cfg_t* cfg,
+                           float* out_xyzi, uint32_t* out_idx, int64_t capacity, int64_t* n_out) {
+  if (!h || !n_out || n_points < 0) return CM_E_INVALID;
+  const int64_t begin[2] = {0, n_points};
+  int64_t ob[2] = {0, 0};
+  const int rc = cm_statistical_outlier_multi(h, xyzi_host, begin, 1, cfg, out_xyzi, out_idx, capacity, ob);
+  *n_out = ob[1];
+  return rc;
+}
+
+int cm_get_statistical_out(cm_handle_t h, cm_sor_out_t* out) {
+  if (!h || !out) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  cm_handle_s::SorWs& s = h->sw;
+  if (!s.ran) return fail(h, CM_E_INVALID, "no statistical outlier removal has run on this handle");
+  CM_CUDA(h, cudaSetDevice(h->device));
+  CM_CUDA(h, cudaStreamSynchronize(s.stream));
+  memset(out, 0, sizeof(*out));
+  out->distances = s.dist.get();
+  out->n_points = s.n_points;
+  out->n_clouds = s.n_clouds;
+  out->knn_ms = out->sums_ms = -1.f;
+  if (s.profiled) {
+    if (cudaEventElapsedTime(&out->knn_ms, s.ev[0].get(), s.ev[1].get()) != cudaSuccess) { out->knn_ms = -1.f; cudaGetLastError(); }
+    if (cudaEventElapsedTime(&out->sums_ms, s.ev[1].get(), s.ev[2].get()) != cudaSuccess) { out->sums_ms = -1.f; cudaGetLastError(); }
+  }
+  for (int c = 0; c < s.n_clouds; ++c) {
+    const SorStats& st = s.stats_host.get()[c];
+    cm_sor_stats_t& o = out->cloud[c];
+    o.mean = st.mean; o.stddev = st.stddev; o.threshold = st.threshold;
+    o.n_valid = s.n_valid[c];
+    o.too_few = (s.too_few >> c) & 1u;
+    o.sum_path = (int32_t)st.path;
+  }
+  return CM_OK;
 }
 
 // ---- RANSAC ground plane --------------------------------------------------------------------------------------------------

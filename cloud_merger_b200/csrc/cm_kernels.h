@@ -179,6 +179,38 @@ struct RorParams {
 cudaError_t launch_radius_table(const VoxelParams& p, const RorParams& r, cudaStream_t stream);
 cudaError_t launch_radius_count(const VoxelParams& p, const RorParams& r, cudaStream_t stream);
 
+// ---- statistical outlier removal on the sorted cell keys (cm_statistical.cu) -------------------------------------------------
+struct SorParams {
+  uint32_t mean_k;             // 1 .. CM_SOR_MAX_K
+  uint32_t sqrt_mode;          // 0: (double)sqrtf(d), 1: sqrt((double)d)
+  uint32_t too_few;            // bit c: cloud c has 0 < finite points <= mean_k -- no search, distances stay 0
+  const float4* sorted_pts;    // [M] the points in sorted key order (written by launch_sor_knn's gather)
+  float* dist;                 // [n_points] mean distance per input point (cleared by the caller)
+  const uint32_t* cell_start;  // k_ror_table's table of the cells' first sorted positions, or nullptr: binary searches
+  double cell;                 // 1 / inv_leaf in double: the cell edge the keys were formed with
+};
+struct SorStats {
+  double sum, sq_sum, mean, stddev, threshold;
+  uint32_t path;               // bit 0: sum by the serial chain, bit 1: sq_sum by the serial chain
+  uint32_t pad_;
+};
+struct SorSumParams {
+  const float* dist;
+  uint32_t n_clouds;
+  uint32_t begin[CM_MAX_ZONES + 1];
+  uint32_t n_valid[CM_MAX_ZONES];  // finite points of every cloud
+  uint32_t too_few;
+  uint32_t force_serial;
+  uint32_t negative;
+  double std_mul;
+  SorStats* stats;                 // [n_clouds]
+  unsigned short* mask;            // [n_points] written for every point
+};
+// gathers the points into sorted order (one launch), then one warp per point finds its mean distance (one launch)
+cudaError_t launch_sor_knn(const VoxelParams& p, const SorParams& s, float4* sorted_pts, cudaStream_t stream);
+cudaError_t launch_sor_sums(const SorSumParams& s, cudaStream_t stream);  // one CTA per cloud
+cudaError_t launch_sor_select(const SorSumParams& s, uint32_t n_points, cudaStream_t stream);
+
 // ---- RANSAC ground plane (cm_plane.cu) --------------------------------------------------------------------------------------
 #define CM_MAX_PLANE_CLOUDS (CM_MAX_ZONES / 2)
 struct PlaneParams {  // one batch of draws for up to CM_MAX_PLANE_CLOUDS independent clouds

@@ -398,6 +398,58 @@ CM_API int cm_dev_radius_outlier_multi(cm_handle_t h, const float* xyzi_dev, con
 CM_API int cm_radius_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds, double radius,
                                    int min_neighbors, int negative, float* out_xyzi, uint32_t* out_idx, int64_t capacity,
                                    int64_t* out_begin);
+/* Statistical outlier removal: pcl::StatisticalOutlierRemoval<pcl::PointXYZI> with setMeanK(mean_k),
+ * setStddevMulThresh(std_mul), setNegative(negative), keep_organized false (PCL 1.8.1 applyFilterIndices). Every finite
+ * point gets the mean of the square roots of its mean_k nearest squared distances (exact search, float distances in
+ * FLANN's order, double sum in ascending order, stored as a float); a non-finite point gets 0. Over every cloud, in index
+ * order and in double: mean and stddev of those values over the finite points, threshold = mean + std_mul * stddev; a
+ * point is removed iff its value > threshold (negative != 0: iff <=). Survivors keep their input order.
+ * Documented deviations: the input is always treated as non-dense; a cloud with 0 < finite points <= mean_k (PCL reads
+ * past its neighbour vectors there) keeps every point, whatever negative is, and is flagged too_few.
+ *  cm_dev_statistical_outlier[_multi]: packed float4 xyzi points on the device (clouds as for the radius outlier removal:
+ *      cloud k = [begin[k], begin[k+1]), n_clouds <= CM_MAX_ZONES and <= max_batch_frames, no neighbours across clouds).
+ *      Survivors through cm_get_zone_out (zone k = those of cloud k, src = index in the whole array), the per-point values
+ *      and per-cloud statistics through cm_get_statistical_out. mean_k outside 1 .. CM_SOR_MAX_K, a NaN std_mul or an
+ *      unknown sqrt_mode -> CM_E_INVALID. Uses the handle's batch workspace, like the radius outlier removal.
+ *  cm_statistical_outlier[_multi]: host buffers in and out (CM_E_CAPACITY with the needed size in *n_out /
+ *      out_begin[n_clouds]). */
+#define CM_SOR_MAX_K 127
+#define CM_SOR_SQRT_FLOAT 0   /* the unqualified sqrt of PCL's loop resolves to std::sqrt(float) */
+#define CM_SOR_SQRT_DOUBLE 1  /* ... to ::sqrt(double) on the promoted value */
+typedef struct {
+  int32_t mean_k;     /* setMeanK, 1 .. CM_SOR_MAX_K */
+  int32_t negative;   /* setNegative */
+  int32_t sqrt_mode;  /* CM_SOR_SQRT_* */
+  int32_t reserved;
+  double std_mul;     /* setStddevMulThresh */
+} cm_sor_cfg_t;
+#define CM_SOR_SUM_SERIAL 1     /* sum_path bit: the sum of the values was formed by the serial chain in index order */
+#define CM_SOR_SQ_SUM_SERIAL 2  /* ... the sum of their squares (otherwise: an exact parallel sum, the same bits) */
+typedef struct {
+  double mean, stddev, threshold; /* PCL's distance statistics of the cloud (NaN threshold: every point is kept) */
+  int64_t n_valid;                /* finite points */
+  int32_t too_few;                /* 0 < n_valid <= mean_k: no search, every point kept, values 0 */
+  int32_t sum_path;               /* CM_SOR_*SERIAL bits */
+} cm_sor_stats_t;
+typedef struct {
+  const float* distances;         /* device [n_points]: the value of every input point, in input order */
+  int64_t n_points;
+  int32_t n_clouds;
+  int32_t reserved;
+  float knn_ms, sums_ms;          /* GPU time of the neighbour search and of the sums (cm_set_profiling on; -1 otherwise) */
+  cm_sor_stats_t cloud[CM_MAX_ZONES];
+} cm_sor_out_t;
+CM_API int cm_dev_statistical_outlier(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_sor_cfg_t* cfg,
+                                      void* stream);
+CM_API int cm_dev_statistical_outlier_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
+                                            const cm_sor_cfg_t* cfg, void* stream);
+CM_API int cm_statistical_outlier(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_sor_cfg_t* cfg,
+                                  float* out_xyzi, uint32_t* out_idx, int64_t capacity, int64_t* n_out);
+CM_API int cm_statistical_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds,
+                                        const cm_sor_cfg_t* cfg, float* out_xyzi, uint32_t* out_idx, int64_t capacity,
+                                        int64_t* out_begin);
+/* waits for the last statistical outlier removal on the handle; the device array stays valid until the next one */
+CM_API int cm_get_statistical_out(cm_handle_t h, cm_sor_out_t* out);
 /* RANSAC ground plane. Replaces the pcl::SACSegmentation + pcl::ExtractIndices block of removeGround()
  * (pc_preprocessing_main.cpp:95-117): SACMODEL_PLANE, SAC_RANSAC (setAxis / setEpsAngle are ignored by that model, as in
  * PCL). The three-index draws are PCL 1.8.1's -- boost::mt19937 seeded with cfg->seed, uniform_int<>(0, INT_MAX), the

@@ -245,42 +245,34 @@ class Context {
   // Radius outlier removal of several host clouds in one pass (cm_radius_outlier_multi; at most CM_MAX_ZONES clouds):
   // every cloud is filtered on its own (no neighbours across clouds); out[k] keeps the order of in[k].
   bool radius_outlier_multi(const std::vector<const Cloud*>& in, std::vector<Cloud>& out, double radius, int min_neighbors) {
-    const size_t k = in.size();
-    out.assign(k, Cloud());
-    if (!check(h_ ? CM_OK : CM_E_NO_DEVICE)) return false;
-    std::vector<int64_t> begin(k + 1, 0);
-    for (size_t c = 0; c < k; ++c) begin[c + 1] = begin[c] + static_cast<int64_t>(in[c]->points.size());
-    const int64_t n = begin[k];
-    if (n > max_points_ * max_sensors_) { rc_ = CM_E_CAPACITY; err_ = "clouds larger than the context capacity"; return false; }
-    tmp_.resize(static_cast<size_t>(n) * 4 + 4);
-    for (size_t c = 0; c < k; ++c)
-      for (size_t i = 0; i < in[c]->points.size(); ++i) {
-        const PointXYZI& p = in[c]->points[i];
-        float* o = &tmp_[(static_cast<size_t>(begin[c]) + i) * 4];
-        o[0] = p.x; o[1] = p.y; o[2] = p.z; o[3] = p.intensity;
-      }
-    zone_xyzi_.resize(static_cast<size_t>(n) * 4 + 4);
-    std::vector<int64_t> ob(k + 1, 0);
-    if (!check(cm_radius_outlier_multi(h_, tmp_.data(), begin.data(), static_cast<int>(k), radius, min_neighbors, 0,
-                                       zone_xyzi_.data(), nullptr, n, ob.data())))
-      return false;
-    for (size_t c = 0; c < k; ++c) {
-      Cloud& res = out[c];
-      const size_t b = static_cast<size_t>(ob[c]), e = static_cast<size_t>(ob[c + 1]);
-      res.points.resize(e - b);
-      for (size_t i = b; i < e; ++i) {
-        PointXYZI& p = res.points[i - b];
-        p = PointXYZI();
-        p.x = zone_xyzi_[i * 4 + 0]; p.y = zone_xyzi_[i * 4 + 1]; p.z = zone_xyzi_[i * 4 + 2]; p.intensity = zone_xyzi_[i * 4 + 3];
-      }
-      finish(res, *in[c], true);
-    }
-    return true;
+    return filter_multi(in, out, [&](const int64_t* begin, int k, int64_t n, int64_t* ob) {
+      return cm_radius_outlier_multi(h_, tmp_.data(), begin, k, radius, min_neighbors, 0, zone_xyzi_.data(), nullptr, n, ob);
+    });
   }
   // one cloud
   bool radius_outlier(const Cloud& in, Cloud& out, double radius, int min_neighbors) {
     std::vector<Cloud> res;
     if (!radius_outlier_multi({&in}, res, radius, min_neighbors)) return clear(out);
+    out = res[0];
+    return true;
+  }
+
+  // Statistical outlier removal of several host clouds in one pass (cm_statistical_outlier_multi; at most CM_MAX_ZONES
+  // clouds): pcl::StatisticalOutlierRemoval with setMeanK(mean_k), setStddevMulThresh(std_mul), setNegative(negative) on
+  // every cloud on its own; out[k] keeps the order of in[k]. sqrt_mode: CM_SOR_SQRT_FLOAT / CM_SOR_SQRT_DOUBLE, the
+  // reading of the unqualified sqrt in PCL's loop that the build being replaced makes.
+  bool statistical_outlier_multi(const std::vector<const Cloud*>& in, std::vector<Cloud>& out, int mean_k, double std_mul,
+                                 bool negative = false, int sqrt_mode = CM_SOR_SQRT_FLOAT) {
+    cm_sor_cfg_t cfg{};
+    cfg.mean_k = mean_k; cfg.negative = negative ? 1 : 0; cfg.sqrt_mode = sqrt_mode; cfg.std_mul = std_mul;
+    return filter_multi(in, out, [&](const int64_t* begin, int k, int64_t n, int64_t* ob) {
+      return cm_statistical_outlier_multi(h_, tmp_.data(), begin, k, &cfg, zone_xyzi_.data(), nullptr, n, ob);
+    });
+  }
+  bool statistical_outlier(const Cloud& in, Cloud& out, int mean_k, double std_mul, bool negative = false,
+                           int sqrt_mode = CM_SOR_SQRT_FLOAT) {
+    std::vector<Cloud> res;
+    if (!statistical_outlier_multi({&in}, res, mean_k, std_mul, negative, sqrt_mode)) return clear(out);
     out = res[0];
     return true;
   }
@@ -415,6 +407,41 @@ class Context {
   }
 
  private:
+  // Packs the clouds into tmp_ (xyzi), runs a multi-cloud filter of the C ABI that writes the survivors of cloud c to
+  // zone_xyzi_[ob[c] .. ob[c+1]) and unpacks them into out[c] (header and layout of in[c]).
+  template <typename Run>
+  bool filter_multi(const std::vector<const Cloud*>& in, std::vector<Cloud>& out, Run run) {
+    const size_t k = in.size();
+    out.assign(k, Cloud());
+    if (!check(h_ ? CM_OK : CM_E_NO_DEVICE)) return false;
+    std::vector<int64_t> begin(k + 1, 0);
+    for (size_t c = 0; c < k; ++c) begin[c + 1] = begin[c] + static_cast<int64_t>(in[c]->points.size());
+    const int64_t n = begin[k];
+    if (n > max_points_ * max_sensors_) { rc_ = CM_E_CAPACITY; err_ = "clouds larger than the context capacity"; return false; }
+    tmp_.resize(static_cast<size_t>(n) * 4 + 4);
+    for (size_t c = 0; c < k; ++c)
+      for (size_t i = 0; i < in[c]->points.size(); ++i) {
+        const PointXYZI& p = in[c]->points[i];
+        float* o = &tmp_[(static_cast<size_t>(begin[c]) + i) * 4];
+        o[0] = p.x; o[1] = p.y; o[2] = p.z; o[3] = p.intensity;
+      }
+    zone_xyzi_.resize(static_cast<size_t>(n) * 4 + 4);
+    std::vector<int64_t> ob(k + 1, 0);
+    if (!check(run(begin.data(), static_cast<int>(k), n, ob.data()))) return false;
+    for (size_t c = 0; c < k; ++c) {
+      Cloud& res = out[c];
+      const size_t b = static_cast<size_t>(ob[c]), e = static_cast<size_t>(ob[c + 1]);
+      res.points.resize(e - b);
+      for (size_t i = b; i < e; ++i) {
+        PointXYZI& p = res.points[i - b];
+        p = PointXYZI();
+        p.x = zone_xyzi_[i * 4 + 0]; p.y = zone_xyzi_[i * 4 + 1]; p.z = zone_xyzi_[i * 4 + 2]; p.intensity = zone_xyzi_[i * 4 + 3];
+      }
+      finish(res, *in[c], true);
+    }
+    return true;
+  }
+
   bool check(int rc) {
     rc_ = rc;
     if (rc != CM_OK) err_ = std::string(cm_strerror(rc)) + ": " + (h_ ? cm_last_error(h_) : "");
@@ -577,6 +604,14 @@ inline void getCloudPartsZSplit(Context& ctx, const Cloud::Ptr& cloud_ROI_ptr, c
 inline void outlierRemoval(Context& ctx, const Cloud::Ptr& cloud_ptr) {
   Cloud tmp;
   ctx.radius_outlier(*cloud_ptr, tmp, static_cast<double>(ctx.params().radius), static_cast<int>(ctx.params().min_neighbor));
+  *cloud_ptr = tmp;
+}
+
+// pcl::StatisticalOutlierRemoval<PointXYZI> (setMeanK, setStddevMulThresh) filtering the cloud in place, next to
+// outlierRemoval for a node that replaces its radius filter by PCL's other standard one.
+inline void statisticalOutlierRemoval(Context& ctx, const Cloud::Ptr& cloud_ptr, int mean_k, double std_mul) {
+  Cloud tmp;
+  ctx.statistical_outlier(*cloud_ptr, tmp, mean_k, std_mul);
   *cloud_ptr = tmp;
 }
 
