@@ -49,6 +49,25 @@ class CloudMergerError(RuntimeError):
         self.code = code
 
 
+def _outputs(n: int):
+    """Host output buffers of a filter for up to n points: (xyzi [n,4] float32, idx [n] uint32)."""
+    return np.empty((max(n, 1), 4), np.float32), np.empty(max(n, 1), np.uint32)
+
+
+def _pack(clouds):
+    """Several [n,4] clouds as one float32 array: (array, begin as numpy int64, begin as ctypes int64[], output buffers)."""
+    arrs = [np.ascontiguousarray(c, np.float32).reshape(-1, 4) for c in clouds]
+    begin = np.concatenate([[0], np.cumsum([len(a) for a in arrs])]).astype(np.int64)
+    n = int(begin[-1])
+    allpts = np.ascontiguousarray(np.concatenate(arrs)) if n else np.zeros((0, 4), np.float32)
+    return allpts, begin, (C.c_int64 * len(begin))(*[int(v) for v in begin]), _outputs(n)
+
+
+def _part(xyzi, idx, a: int, b: int, base: int = 0):
+    """Points [a, b) of host outputs as (xyzi, idx - base): one cloud or zone, its indices relative to its own cloud."""
+    return xyzi[a:b].copy(), (idx[a:b].astype(np.int64) - base).astype(np.uint32)
+
+
 def make_layout(point_step=16, off_x=0, off_y=4, off_z=8, off_intensity=12, is_dense=1) -> CmLayout:
     return CmLayout(point_step, off_x, off_y, off_z, off_intensity, int(is_dense))
 
@@ -217,14 +236,13 @@ class CloudMerger:
         a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
         n = len(a)
         cap = int(capacity if capacity is not None else 2 * max(n, 1))
-        ox = np.empty((max(cap, 1), 4), np.float32)
-        osrc = np.empty(max(cap, 1), np.uint32)
+        ox, osrc = _outputs(cap)
         begin = (C.c_int64 * (CM_MAX_ZONES + 1))()
         self._check(self._lib.cm_zone_split(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(n),
                                             ox.ctypes.data_as(C.c_void_p), osrc.ctypes.data_as(C.c_void_p),
                                             C.c_int64(cap), begin))
         nz = self._n_zones
-        return [(ox[begin[z]:begin[z + 1]].copy(), osrc[begin[z]:begin[z + 1]].copy()) for z in range(nz)]
+        return [_part(ox, osrc, begin[z], begin[z + 1]) for z in range(nz)]
 
     # -- radius outlier removal: outlierRemoval() of the reference (pc_preprocessing_main.cpp:184-192) ----------------------
     def dev_radius_outlier(self, xyzi_ptr: int, n_points: int, radius: float, min_neighbors: int = 1,
@@ -242,13 +260,12 @@ class CloudMerger:
         """Host-buffer form: (xyzi [k,4] float32, idx [k] uint32 indices into the input, ascending)."""
         a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
         n = len(a)
-        ox = np.empty((max(n, 1), 4), np.float32)
-        oi = np.empty(max(n, 1), np.uint32)
+        ox, oi = _outputs(n)
         k = C.c_int64()
         self._check(self._lib.cm_radius_outlier(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(n), C.c_double(radius),
                                                 int(min_neighbors), int(negative), ox.ctypes.data_as(C.c_void_p),
                                                 oi.ctypes.data_as(C.c_void_p), C.c_int64(n), C.byref(k)))
-        return ox[:k.value].copy(), oi[:k.value].copy()
+        return _part(ox, oi, 0, k.value)
 
     def dev_radius_outlier_multi(self, xyzi_ptr: int, begin, radius: float, min_neighbors: int = 1, negative: bool = False,
                                  stream: int = 0):
@@ -261,19 +278,13 @@ class CloudMerger:
 
     def radius_outlier_multi(self, clouds, radius: float, min_neighbors: int = 1, negative: bool = False) -> list:
         """Host-buffer form: per cloud (xyzi [k,4], idx [k] into that cloud)."""
-        arrs = [np.ascontiguousarray(c, np.float32).reshape(-1, 4) for c in clouds]
-        k = len(arrs)
-        begin = np.concatenate([[0], np.cumsum([len(a) for a in arrs])]).astype(np.int64)
-        n = int(begin[-1])
-        allpts = np.ascontiguousarray(np.concatenate(arrs)) if n else np.zeros((0, 4), np.float32)
-        ox = np.empty((max(n, 1), 4), np.float32)
-        oi = np.empty(max(n, 1), np.uint32)
+        allpts, begin, b, (ox, oi) = _pack(clouds)
+        k, n = len(begin) - 1, len(allpts)
         ob = (C.c_int64 * (k + 1))()
-        b = (C.c_int64 * (k + 1))(*[int(v) for v in begin])
         self._check(self._lib.cm_radius_outlier_multi(self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.c_double(radius),
                                                       int(min_neighbors), int(negative), ox.ctypes.data_as(C.c_void_p),
                                                       oi.ctypes.data_as(C.c_void_p), C.c_int64(n), ob))
-        return [(ox[ob[c]:ob[c + 1]].copy(), (oi[ob[c]:ob[c + 1]].astype(np.int64) - begin[c]).astype(np.uint32)) for c in range(k)]
+        return [_part(ox, oi, ob[c], ob[c + 1], begin[c]) for c in range(k)]
 
     # -- statistical outlier removal (pcl::StatisticalOutlierRemoval) --------------------------------------------------------
     @staticmethod
@@ -312,32 +323,25 @@ class CloudMerger:
         """Host-buffer form: (xyzi [k,4] float32, idx [k] uint32 indices into the input, ascending)."""
         a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
         n = len(a)
-        ox = np.empty((max(n, 1), 4), np.float32)
-        oi = np.empty(max(n, 1), np.uint32)
+        ox, oi = _outputs(n)
         k = C.c_int64()
         cfg = self._sor_cfg(mean_k, std_mul, negative, sqrt_mode)
         self._check(self._lib.cm_statistical_outlier(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(n), C.byref(cfg),
                                                      ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p),
                                                      C.c_int64(n), C.byref(k)))
-        return ox[:k.value].copy(), oi[:k.value].copy()
+        return _part(ox, oi, 0, k.value)
 
     def statistical_outlier_multi(self, clouds, mean_k: int, std_mul: float, negative: bool = False,
                                   sqrt_mode: int = 0) -> list:
         """Host-buffer form: per cloud (xyzi [k,4], idx [k] into that cloud)."""
-        arrs = [np.ascontiguousarray(c, np.float32).reshape(-1, 4) for c in clouds]
-        k = len(arrs)
-        begin = np.concatenate([[0], np.cumsum([len(a) for a in arrs])]).astype(np.int64)
-        n = int(begin[-1])
-        allpts = np.ascontiguousarray(np.concatenate(arrs)) if n else np.zeros((0, 4), np.float32)
-        ox = np.empty((max(n, 1), 4), np.float32)
-        oi = np.empty(max(n, 1), np.uint32)
+        allpts, begin, b, (ox, oi) = _pack(clouds)
+        k, n = len(begin) - 1, len(allpts)
         ob = (C.c_int64 * (k + 1))()
-        b = (C.c_int64 * (k + 1))(*[int(v) for v in begin])
         cfg = self._sor_cfg(mean_k, std_mul, negative, sqrt_mode)
         self._check(self._lib.cm_statistical_outlier_multi(self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.byref(cfg),
                                                            ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p),
                                                            C.c_int64(n), ob))
-        return [(ox[ob[c]:ob[c + 1]].copy(), (oi[ob[c]:ob[c + 1]].astype(np.int64) - begin[c]).astype(np.uint32)) for c in range(k)]
+        return [_part(ox, oi, ob[c], ob[c + 1], begin[c]) for c in range(k)]
 
     # -- RANSAC ground plane (pcl::SACSegmentation of removeGround, pc_preprocessing_main.cpp:95-117) ------------------------
     @staticmethod
@@ -379,25 +383,18 @@ class CloudMerger:
                            optimize: bool = True, seed: int = 12345, sum_order: int = 0) -> list:
         """Host-buffer form of dev_plane_ransac_multi: one dict per cloud with "ground" / "rest" as in plane_ransac
         (indices relative to the cloud)."""
-        arrs = [np.ascontiguousarray(c, np.float32).reshape(-1, 4) for c in clouds]
-        k = len(arrs)
-        begin = np.concatenate([[0], np.cumsum([len(a) for a in arrs])]).astype(np.int64)
-        n = int(begin[-1])
-        allpts = np.ascontiguousarray(np.concatenate(arrs)) if n else np.zeros((0, 4), np.float32)
+        allpts, begin, b, (ox, oi) = _pack(clouds)
+        k, n = len(begin) - 1, len(allpts)
         cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
         pl = (_lib.CmPlane * max(k, 1))()
-        ox = np.empty((max(n, 1), 4), np.float32)
-        oi = np.empty(max(n, 1), np.uint32)
         ob = (C.c_int64 * (2 * k + 1))()
-        b = (C.c_int64 * (k + 1))(*[int(v) for v in begin])
         self._check(self._lib.cm_plane_ransac_multi(self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.byref(cfg), pl,
                                                     ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p), C.c_int64(n), ob))
         res = []
         for c in range(k):
             r = self._plane_dict(pl[c])
-            g0, g1, g2 = ob[2 * c], ob[2 * c + 1], ob[2 * c + 2]
-            r["ground"] = (ox[g0:g1].copy(), (oi[g0:g1].astype(np.int64) - begin[c]).astype(np.uint32))
-            r["rest"] = (ox[g1:g2].copy(), (oi[g1:g2].astype(np.int64) - begin[c]).astype(np.uint32))
+            r["ground"] = _part(ox, oi, ob[2 * c], ob[2 * c + 1], begin[c])
+            r["rest"] = _part(ox, oi, ob[2 * c + 1], ob[2 * c + 2], begin[c])
             res.append(r)
         return res
 
@@ -408,16 +405,13 @@ class CloudMerger:
         n = len(a)
         cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
         pl = _lib.CmPlane()
-        ox = np.empty((max(n, 1), 4), np.float32)
-        oi = np.empty(max(n, 1), np.uint32)
+        ox, oi = _outputs(n)
         begin = (C.c_int64 * 3)()
         self._check(self._lib.cm_plane_ransac(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(n), C.byref(cfg), C.byref(pl),
                                               ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p), C.c_int64(n),
                                               begin))
         r = self._plane_dict(pl)
-        b = list(begin)
-        r["ground"] = (ox[b[0]:b[1]].copy(), oi[b[0]:b[1]].copy())
-        r["rest"] = (ox[b[1]:b[2]].copy(), oi[b[1]:b[2]].copy())
+        r["ground"], r["rest"] = _part(ox, oi, begin[0], begin[1]), _part(ox, oi, begin[1], begin[2])
         return r
 
     # -- the body of a proceedX in one call (pc_preprocessing_main.cpp:228-312, :428-446, :474-497) ---------------------------

@@ -199,7 +199,6 @@ struct cm_handle_s {
     DevPtr<uint32_t> zone_total;  // [CM_MAX_ZONES] + the scan ticket behind it
     DevPtr<float4> out_xyzi;
     DevPtr<uint32_t> out_src;
-    DevPtr<float4> in_stage;      // host-buffer form: the uploaded cloud
     HostPtr<uint32_t> report;     // pinned: zone_begin[CM_MAX_ZONES + 1] + overflow + a radius run's device error word
     cudaStream_t stream = nullptr;
     bool ran = false;
@@ -209,9 +208,12 @@ struct cm_handle_s {
     bool ror_run = false;        // the last split compacted a radius outlier removal: report[CM_MAX_ZONES + 2] holds the
                                  // error word of its count kernel (the 2^14-cell bound of the cell margin)
   } zw;
-  // radius outlier removal: first sorted position of every cell key (allocated on first use, grows)
-  DevPtr<uint32_t> ror_table;
-  size_t ror_table_cap = 0;
+  // the outlier removals' cell table: first sorted position of every cell key (allocated on first use, grows)
+  DevPtr<uint32_t> cell_table;
+  size_t cell_table_cap = 0;
+  // host-buffer forms: the caller's cloud uploaded (allocated on first use, grows)
+  DevPtr<float4> stage;
+  size_t stage_cap = 0;
   // statistical outlier removal (allocated on first use, grows)
   struct SorWs {
     size_t cap = 0;
@@ -244,7 +246,6 @@ struct cm_handle_s {
     size_t cap = 0;
     DevPtr<float4> low, high, rest, planes;  // [cap] each
     DevPtr<float4> no_ground, ground;        // [2 cap] (windows share their end points)
-    DevPtr<float4> in_stage;                 // host-buffer form: the uploaded ROI cloud
   } prz;
   // host path: slots and streams are set up together on first use (empty until then)
   std::vector<Slot> slots;
@@ -641,8 +642,9 @@ int run_voxel(cm_handle_t h, Workspace& w, VoxelParams& vp, cudaStream_t st, boo
   return CM_OK;
 }
 
-// Derives the single-box form of the crop chain (see CropDev) whenever the chain allows it.
-void derive_crop_box(CropDev& c) {
+// Derives the single-box form of a PassThrough chain (CropDev, ZoneDev) whenever the chain allows it.
+template <typename Chain>
+void derive_box(Chain& c) {
   const float fmax = std::numeric_limits<float>::max();
   c.is_box = 0; c.use_i = 0;
   for (int a = 0; a < 4; ++a) { c.lo[a] = -fmax; c.hi[a] = fmax; }
@@ -1267,7 +1269,7 @@ int cm_create(const cm_config_t* cfg, cm_handle_t* out) {
   h->crop.pass[0] = PassDev{2, -0.5f, 3.0f, 0};
   h->crop.pass[1] = PassDev{1, -10.0f / 2, 10.0f / 2, 0};
   h->crop.pass[2] = PassDev{0, -15.0f, 75.0f - 15.0f, 0};
-  derive_crop_box(h->crop);
+  derive_box(h->crop);
   *out = h;
   return CM_OK;
 }
@@ -1322,7 +1324,7 @@ int cm_set_crop(cm_handle_t h, int n_pass, const cm_pass_t* passes) {
     if (passes[k].axis < 0 || passes[k].axis > 3) return fail(h, CM_E_INVALID, "pass %d: axis must be 0..3", k);
   h->crop.n_pass = n_pass;
   for (int k = 0; k < n_pass; ++k) h->crop.pass[k] = PassDev{passes[k].axis, passes[k].lo, passes[k].hi, passes[k].negative ? 1 : 0};
-  derive_crop_box(h->crop);
+  derive_box(h->crop);
   return CM_OK;
 }
 
@@ -1579,6 +1581,14 @@ int cm_dev_transform_crop(cm_handle_t h, const cm_segment_t* segments, int n_seg
 }
 
 namespace {
+// The cloud of a cm_dev_* entry point: n_points packed float4 in device memory.
+int check_dev_cloud(cm_handle_t h, const void* xyzi_dev, int64_t n_points) {
+  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u)))
+    return fail(h, CM_E_INVALID, "the device cloud must be a 16-byte aligned pointer");
+  if (n_points < 0) return fail(h, CM_E_INVALID, "bad n_points");
+  return CM_OK;
+}
+
 // VoxelGrid of n packed points on the batch workspace. seed_enc_dev: device-resident bounds (GiantPlan::enc) folded into the
 // local box; known_idx_bits >= 0: the key plan is known on the host, no device round trip.
 int voxelgrid_run(cm_handle_t h, const float4* pts, int64_t n_points, cudaStream_t st, const uint32_t* seed_enc_dev = nullptr,
@@ -1615,45 +1625,41 @@ int cm_dev_voxelgrid(cm_handle_t h, const float* xyzi_dev, int64_t n_points, int
   if (!h) return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
+  const int rc = check_dev_cloud(h, xyzi_dev, n_points);
+  if (rc != CM_OK) return rc;
   return voxelgrid_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, static_cast<cudaStream_t>(stream));
 }
 
 // ---- zone slicing ---------------------------------------------------------------------------------------------------------
-int cm_set_zones(cm_handle_t h, int n_zones, const cm_zone_t* zones) {
-  if (!h || n_zones < 0 || n_zones > CM_MAX_ZONES || (n_zones > 0 && !zones)) return CM_E_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  ZoneSet zs{};
+namespace {
+// The device form of n_zones PassThrough chains, each with its box form where the chain allows it (see ZoneDev).
+int make_zone_set(cm_handle_t h, int n_zones, const cm_zone_t* zones, ZoneSet& zs) {
+  zs = ZoneSet{};
   zs.n_zones = n_zones;
+  zs.all_box = n_zones > 0 ? 1 : 0;
   for (int z = 0; z < n_zones; ++z) {
     if (zones[z].n_pass < 0 || zones[z].n_pass > CM_MAX_ZONE_PASSES) return fail(h, CM_E_INVALID, "zone %d: bad n_pass", z);
-    zs.zone[z].n_pass = zones[z].n_pass;
+    ZoneDev& zd = zs.zone[z];
+    zd.n_pass = zones[z].n_pass;
     for (int k = 0; k < zones[z].n_pass; ++k) {
       const cm_pass_t& ps = zones[z].pass[k];
       if (ps.axis < 0 || ps.axis > 3) return fail(h, CM_E_INVALID, "zone %d pass %d: bad axis", z, k);
-      zs.zone[z].pass[k].axis = ps.axis; zs.zone[z].pass[k].lo = ps.lo; zs.zone[z].pass[k].hi = ps.hi;
-      zs.zone[z].pass[k].negative = ps.negative ? 1 : 0;
+      zd.pass[k] = PassDev{ps.axis, ps.lo, ps.hi, ps.negative ? 1 : 0};
     }
-  }
-  // box form of every chain that allows it (see ZoneDev)
-  const float fmax = std::numeric_limits<float>::max();
-  zs.all_box = n_zones > 0 ? 1 : 0;
-  for (int z = 0; z < n_zones; ++z) {
-    ZoneDev& zd = zs.zone[z];
-    zd.is_box = zd.n_pass > 0 ? 1 : 0;
-    zd.use_i = 0;
-    for (int a = 0; a < 4; ++a) { zd.lo[a] = -fmax; zd.hi[a] = fmax; }
-    for (int k = 0; k < zd.n_pass; ++k) {
-      const PassDev& ps = zd.pass[k];
-      if (ps.negative || !(ps.lo == ps.lo) || !(ps.hi == ps.hi)) { zd.is_box = 0; break; }
-      zd.lo[ps.axis] = std::max(zd.lo[ps.axis], ps.lo);
-      zd.hi[ps.axis] = std::min(zd.hi[ps.axis], ps.hi);
-      if (ps.axis == 3) zd.use_i = 1;
-    }
+    derive_box(zd);
     if (!zd.is_box) zs.all_box = 0;
   }
-  h->zones = zs;
   return CM_OK;
+}
+}  // namespace
+
+int cm_set_zones(cm_handle_t h, int n_zones, const cm_zone_t* zones) {
+  if (!h || n_zones < 0 || n_zones > CM_MAX_ZONES || (n_zones > 0 && !zones)) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  ZoneSet zs;
+  const int rc = make_zone_set(h, n_zones, zones, zs);
+  if (rc == CM_OK) h->zones = zs;
+  return rc;
 }
 
 namespace {
@@ -1689,6 +1695,19 @@ bool in_zone_outputs(cm_handle_t h, const void* p, int64_t n_points) {
   const uintptr_t a = reinterpret_cast<uintptr_t>(p), b = a + (uintptr_t)n_points * 16u;
   const uintptr_t lo = reinterpret_cast<uintptr_t>(z.out_xyzi.get()), hi = lo + (uintptr_t)z.cap_out * 16u;
   return a < hi && b > lo;
+}
+
+// The clouds [begin[k], begin[k+1]) of pts that a multi-cloud filter takes.
+int check_clouds(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, int max_clouds) {
+  if (n_clouds < 1 || n_clouds > max_clouds) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", max_clouds);
+  if (begin[0] != 0) return fail(h, CM_E_INVALID, "begin[0] must be 0");
+  for (int c = 0; c < n_clouds; ++c)
+    if (begin[c + 1] < begin[c]) return fail(h, CM_E_INVALID, "begin must not decrease");
+  const int rc = check_dev_cloud(h, pts, begin[n_clouds]);
+  if (rc != CM_OK) return rc;
+  if (in_zone_outputs(h, pts, begin[n_clouds]))
+    return fail(h, CM_E_INVALID, "the input cloud lies in this handle's own zone outputs (use another handle or copy it out)");
+  return CM_OK;
 }
 
 // the launch parameters of one split of `pts` over the handle's zone workspace (which must hold n_points)
@@ -1741,8 +1760,8 @@ int cm_dev_zone_split(cm_handle_t h, const float* xyzi_dev, int64_t n_points, vo
   CM_CUDA(h, cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (xyzi_dev) {
-    if (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
-    return zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st);
+    const int rc = check_dev_cloud(h, xyzi_dev, n_points);
+    return rc == CM_OK ? zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st) : rc;
   }
   // the merged cropped cloud of the last transform_crop run (what getROI hands to getCloudPart)
   if (!h->last || !h->last->ran_k1) return fail(h, CM_E_INVALID, "no transform_crop result on this handle");
@@ -1797,33 +1816,45 @@ int zone_out_locked(cm_handle_t h, cm_zone_out_t* out) {
   if (z.ror_run && report[CM_MAX_ZONES + 2]) return fail(h, CM_E_INTERNAL, "device error %u", report[CM_MAX_ZONES + 2]);
   return CM_OK;
 }
+
+// The host-buffer forms: the caller's cloud is uploaded on the legacy stream into the handle's staging buffer.
+int stage_host_cloud(cm_handle_t h, const float* xyzi_host, int64_t n_points, const float4** staged) {
+  if (n_points < 0 || (n_points > 0 && !xyzi_host)) return fail(h, CM_E_INVALID, "bad host cloud");
+  if (h->stage_cap < (size_t)n_points || !h->stage) {
+    const size_t want = std::max<size_t>({(size_t)n_points, (size_t)h->cfg.max_batch_points, (size_t)1});
+    h->stage.reset(); h->stage_cap = 0;  // the old buffer goes before the larger one is allocated
+    CM_CUDA(h, dev_alloc(h->stage, want));
+    h->stage_cap = want;
+  }
+  if (n_points) CM_CUDA(h, cudaMemcpyAsync(h->stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
+  *staged = h->stage.get();
+  return CM_OK;
+}
+
+// ... and the zone outputs come back: the first n_offsets offsets of the report (zeros if it was never filled) into
+// out_begin, then the points, or CM_E_CAPACITY (the needed size in out_begin[n_offsets - 1]) when they do not fit.
+int zone_copy_out(cm_handle_t h, int n_offsets, float* out_xyzi, uint32_t* out_idx, int64_t capacity, int64_t* out_begin) {
+  cm_zone_out_t zo{};
+  const int rc = zone_out_locked(h, &zo);
+  for (int k = 0; k < n_offsets; ++k) out_begin[k] = zo.begin[k];
+  if (rc != CM_OK) return rc;
+  const int64_t total = zo.begin[n_offsets - 1];
+  if (total > capacity) return fail(h, CM_E_CAPACITY, "%lld points, caller capacity %lld", (long long)total, (long long)capacity);
+  if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
+  if (out_idx && total) CM_CUDA(h, cudaMemcpy(out_idx, zo.src, (size_t)total * 4, cudaMemcpyDeviceToHost));
+  return CM_OK;
+}
 }  // namespace
 
 int cm_zone_split(cm_handle_t h, const float* xyzi_host, int64_t n_points, float* out_xyzi, uint32_t* out_src,
                   int64_t capacity, int64_t* out_begin) {
   if (!h || !out_begin || n_points < 0 || (n_points > 0 && !xyzi_host)) return CM_E_INVALID;
-  cm_zone_out_t zo;
-  {
-    std::lock_guard<std::mutex> lk(h->mu);
-    CM_CUDA(h, cudaSetDevice(h->device));
-    int rc = zone_ws_ensure(h, (size_t)n_points);
-    if (rc != CM_OK) return rc;
-    cm_handle_s::ZoneWs& z = h->zw;
-    if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
-    CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-    rc = zone_run(h, z.in_stage.get(), n_points, nullptr);
-
-    if (rc != CM_OK) return rc;
-  }
-  int rc = cm_get_zone_out(h, &zo);
-  for (int k = 0; k <= zo.n_zones; ++k) out_begin[k] = zo.begin[k];
-  if (rc != CM_OK) return rc;
-  const int64_t total = zo.begin[zo.n_zones];
-  if (total > capacity) return fail(h, CM_E_CAPACITY, "the zones hold %lld points, caller capacity %lld", (long long)total, (long long)capacity);
   std::lock_guard<std::mutex> lk(h->mu);
-  if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
-  if (out_src && total) CM_CUDA(h, cudaMemcpy(out_src, zo.src, (size_t)total * 4, cudaMemcpyDeviceToHost));
-  return CM_OK;
+  CM_CUDA(h, cudaSetDevice(h->device));
+  const float4* pts = nullptr;
+  int rc = stage_host_cloud(h, xyzi_host, n_points, &pts);
+  if (rc == CM_OK) rc = zone_run(h, pts, n_points, nullptr);
+  return rc == CM_OK ? zone_copy_out(h, h->zones.n_zones + 1, out_xyzi, out_src, capacity, out_begin) : rc;
 }
 
 // ---- giant-cloud mode: bounding box, key histogram, routing by key range ------------------------------------------------
@@ -1901,9 +1932,10 @@ int cm_dev_route_by_key(cm_handle_t h, const float* xyzi_dev, int64_t n_points, 
     return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
+  int rc = check_dev_cloud(h, xyzi_dev, n_points);
+  if (rc != CM_OK) return rc;
   RouteGrid g;
-  int rc = route_grid(h, min3, max3, &g, nullptr);
+  rc = route_grid(h, min3, max3, &g, nullptr);
   if (rc != CM_OK) return rc;
   rc = zone_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
@@ -1922,19 +1954,14 @@ int cm_memcpy_d2d(cm_handle_t h, void* dst_dev, const void* src_dev, size_t byte
   return CM_OK;
 }
 
-// ---- radius outlier removal ---------------------------------------------------------------------------------------------
+// ---- the cell-key front end of the outlier removals ----------------------------------------------------------------------
+// Both removals search neighbours on the points sorted by cell key, clouds = the ranges [begin[k], begin[k+1]) of pts as
+// the frames of the key (no neighbours across clouds), on the batch workspace. The statistical removal picks its cell edge
+// from the bounds, so the front end is three steps: the bounds, the keys and sort on a given cell grid, the cell table.
 namespace {
-// clouds = the ranges [begin[k], begin[k+1]) of pts (frames of the cell key: no neighbours across clouds); output zone k =
-// the survivors of cloud k
-int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, double radius, int min_neighbors,
-                       int negative, cudaStream_t st) {
-  if (!(radius > 0.0) || min_neighbors < 0) return fail(h, CM_E_INVALID, "radius must be > 0 and min_neighbors >= 0");
-  if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
-  if (begin[0] != 0) return fail(h, CM_E_INVALID, "begin[0] must be 0");
-  for (int c = 0; c < n_clouds; ++c)
-    if (begin[c + 1] < begin[c]) return fail(h, CM_E_INVALID, "begin must not decrease");
+// Bounding box and non-finite count of every cloud (FrameAcc), and the cloud starts.
+int cell_keys_begin(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, VoxelParams& vp, cudaStream_t st) {
   const int64_t n_points = begin[n_clouds];
-  if (in_zone_outputs(h, pts, n_points)) return fail(h, CM_E_INVALID, "the input cloud lies in this handle's own zone outputs (use another handle or copy it out)");
   int rc = ensure_batch_ws(h);
   if (rc != CM_OK) return rc;
   Workspace& w = h->batch;
@@ -1943,9 +1970,6 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
     return fail(h, CM_E_CAPACITY, "%d clouds > max_batch_frames %u of this handle", n_clouds, w.cap_frames);
   rc = zone_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
-  // cells a little wider than the radius: two points closer than the radius are then at most one cell apart on every
-  // axis even after the float rounding of x * (1 / cell) (valid below 2^14 cells from the origin, checked on the device)
-  const float cell = (float)radius * 1.00390625f;
   w.has_run = true; w.report_valid = false; w.profiled = false;
   w.n_frames = (uint32_t)n_clouds; w.n_segs = 0; w.points_in = n_points; w.launches = 0;
   w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
@@ -1953,9 +1977,7 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   h->last = &w;
   CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
   CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
-  VoxelParams vp;
   fill_voxel_params(h, w, vp, pts, (uint32_t)n_clouds, (uint32_t)n_points);
-  for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = 1.0f / cell;
   vp.pcl_refuses = 0;  // a cell grid of the neighbour search beyond the key range is always an error
   uint32_t* fss = const_cast<uint32_t*>(vp.frame_surv_start);
   for (int c = 0; c < n_clouds; ++c) {  // bounding box of every cloud (its own cell grid)
@@ -1969,36 +1991,73 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
     for (int c = 0; c <= n_clouds; ++c) starts[c] = (uint32_t)begin[c];
     CM_CUDA(h, cudaMemcpyAsync(fss, starts, sizeof(uint32_t) * (size_t)(n_clouds + 1), cudaMemcpyHostToDevice, st));
   }
+  return CM_OK;
+}
+
+// Cell keys of edge 1 / inv and their sort (no centroids).
+int cell_keys_sort(cm_handle_t h, VoxelParams& vp, float inv, cudaStream_t st) {
+  Workspace& w = h->batch;
+  for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = inv;
   CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
-  rc = run_voxel(h, w, vp, st, false, false);  // keys + sort only
+  int rc = run_voxel(h, w, vp, st, false, false);  // keys + sort only
   if (rc != CM_OK) return rc;
   // A cloud whose grid k_grid_setup could not key (more than 2^21 cells on an axis, a coordinate beyond 2^30 cells) has
   // all its keys at 0 but keeps its real div_b: the cell table would be sized without it and the row walk would leave it.
-  // The plan fetch above brought the verdict along, so such a call stops here, before the table and the count.
-  if (w.plan_error == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (cell grid exceeds the key range)");
+  // The plan fetch above brought the verdict along, so such a call stops here, before the table and the search.
+  if (w.plan_error == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "cell too small for the extent of a cloud (cell grid exceeds the key range)");
   if (w.plan_error) return fail(h, CM_E_INTERNAL, "device error %u", w.plan_error);
   vp.key_bytes = w.key_bytes;
+  return CM_OK;
+}
+
+// A small key space (the usual case: a cropped cloud) gets a direct-address table of the cells' first sorted positions
+// instead of binary searches per point: rp.cell_start, else nullptr. no_table_env names the removal's test hook that forces
+// the binary searches (the large-key-space path).
+int enqueue_cell_table(cm_handle_t h, const VoxelParams& vp, const char* no_table_env, RorParams& rp, cudaStream_t st) {
+  Workspace& w = h->batch;
+  const uint32_t n_clouds = vp.n_frames;
+  rp.cell_start = nullptr; rp.table_keys = 0;
+  if (vp.max_points > 0 && w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&
+      !getenv(no_table_env)) {
+    const size_t keys = (size_t)n_clouds << w.plan_idx_bits;
+    if (h->cell_table_cap < keys + 1) {
+      h->cell_table.reset(); h->cell_table_cap = 0;  // the old table goes before the larger one is allocated
+      CM_CUDA(h, dev_alloc(h->cell_table, keys + 1));
+      h->cell_table_cap = keys + 1;
+    }
+    rp.cell_start = h->cell_table.get(); rp.table_keys = (uint32_t)keys;
+    CM_CUDA(h, launch_radius_table(vp, rp, st));
+    ++w.launches;
+  }
+  return CM_OK;
+}
+}  // namespace
+
+// ---- radius outlier removal ---------------------------------------------------------------------------------------------
+namespace {
+// output zone k = the survivors of cloud k
+int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, double radius, int min_neighbors,
+                       int negative, cudaStream_t st) {
+  if (!(radius > 0.0) || min_neighbors < 0) return fail(h, CM_E_INVALID, "radius must be > 0 and min_neighbors >= 0");
+  int rc = check_clouds(h, pts, begin, n_clouds, CM_MAX_ZONES);
+  if (rc != CM_OK) return rc;
+  const int64_t n_points = begin[n_clouds];
+  VoxelParams vp;
+  rc = cell_keys_begin(h, pts, begin, n_clouds, vp, st);
+  if (rc != CM_OK) return rc;
+  // cells a little wider than the radius: two points closer than the radius are then at most one cell apart on every
+  // axis even after the float rounding of x * (1 / cell) (valid below 2^14 cells from the origin, checked on the device)
+  const float cell = (float)radius * 1.00390625f;
+  rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  if (rc != CM_OK) return rc;
+  Workspace& w = h->batch;
   RorParams rp;
   rp.r2 = (float)(radius * radius);
   rp.min_pts = (uint32_t)min_neighbors;
   rp.negative = negative ? 1u : 0u;
   rp.mask = h->zw.mask.get();
-  rp.cell_start = nullptr; rp.table_keys = 0;
-  // a small key space (the usual case: a cropped cloud) gets a direct-address table of the cells' first sorted positions
-  // instead of nine binary searches per point
-  // (CM_ROR_NO_TABLE=1 forces the binary searches: test hook for the large-key-space path)
-  if (n_points > 0 && w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&
-      !getenv("CM_ROR_NO_TABLE")) {
-    const size_t keys = (size_t)n_clouds << w.plan_idx_bits;
-    if (h->ror_table_cap < keys + 1) {
-      h->ror_table.reset(); h->ror_table_cap = 0;  // the old table goes before the larger one is allocated
-      CM_CUDA(h, dev_alloc(h->ror_table, keys + 1));
-      h->ror_table_cap = keys + 1;
-    }
-    rp.cell_start = h->ror_table.get(); rp.table_keys = (uint32_t)keys;
-    CM_CUDA(h, launch_radius_table(vp, rp, st));
-    ++w.launches;
-  }
+  rc = enqueue_cell_table(h, vp, "CM_ROR_NO_TABLE", rp, st);
+  if (rc != CM_OK) return rc;
   if (n_points) CM_CUDA(h, cudaMemsetAsync(h->zw.mask.get(), 0, (size_t)n_points * sizeof(unsigned short), st));
   CM_CUDA(h, launch_radius_count(vp, rp, st));
   ++w.launches;
@@ -2014,14 +2073,8 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
 
 int cm_dev_radius_outlier(cm_handle_t h, const float* xyzi_dev, int64_t n_points, double radius, int min_neighbors,
                           int negative, void* stream) {
-  if (!h) return CM_E_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
-  if (n_points < 0) return fail(h, CM_E_INVALID, "bad n_points");
   const int64_t begin[2] = {0, n_points};
-  return radius_outlier_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, 1, radius, min_neighbors, negative,
-                            static_cast<cudaStream_t>(stream));
+  return cm_dev_radius_outlier_multi(h, xyzi_dev, begin, 1, radius, min_neighbors, negative, stream);
 }
 
 int cm_dev_radius_outlier_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds, double radius,
@@ -2029,8 +2082,6 @@ int cm_dev_radius_outlier_multi(cm_handle_t h, const float* xyzi_dev, const int6
   if (!h || !begin) return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_clouds >= 1 && n_clouds <= CM_MAX_ZONES && begin[n_clouds] > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u)))
-    return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
   return radius_outlier_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, n_clouds, radius, min_neighbors, negative,
                             static_cast<cudaStream_t>(stream));
 }
@@ -2040,31 +2091,12 @@ int cm_radius_outlier_multi(cm_handle_t h, const float* xyzi_host, const int64_t
                             int64_t* out_begin) {
   if (!h || !begin || !out_begin) return CM_E_INVALID;
   if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
-  const int64_t n_points = begin[n_clouds];
-  if (n_points < 0 || (n_points > 0 && !xyzi_host)) return CM_E_INVALID;
-  cm_zone_out_t zo;
-  {
-    std::lock_guard<std::mutex> lk(h->mu);
-    CM_CUDA(h, cudaSetDevice(h->device));
-    int rc = zone_ws_ensure(h, (size_t)n_points);
-    if (rc != CM_OK) return rc;
-    cm_handle_s::ZoneWs& z = h->zw;
-    if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
-    if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-    rc = radius_outlier_run(h, z.in_stage.get(), begin, n_clouds, radius, min_neighbors, negative, nullptr);
-    if (rc != CM_OK) return rc;
-  }
-  int rc = cm_get_zone_out(h, &zo);
-  for (int k = 0; k <= n_clouds; ++k) out_begin[k] = zo.begin[k];
-  if (rc != CM_OK) return rc;
-  {
-    std::lock_guard<std::mutex> lk(h->mu);
-    const int64_t total = zo.begin[n_clouds];
-    if (total > capacity) return fail(h, CM_E_CAPACITY, "%lld points kept, caller capacity %lld", (long long)total, (long long)capacity);
-    if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
-    if (out_idx && total) CM_CUDA(h, cudaMemcpy(out_idx, zo.src, (size_t)total * 4, cudaMemcpyDeviceToHost));
-  }
-  return CM_OK;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  const float4* pts = nullptr;
+  int rc = stage_host_cloud(h, xyzi_host, begin[n_clouds], &pts);
+  if (rc == CM_OK) rc = radius_outlier_run(h, pts, begin, n_clouds, radius, min_neighbors, negative, nullptr);
+  return rc == CM_OK ? zone_copy_out(h, n_clouds + 1, out_xyzi, out_idx, capacity, out_begin) : rc;
 }
 
 int cm_radius_outlier(cm_handle_t h, const float* xyzi_host, int64_t n_points, double radius, int min_neighbors,
@@ -2124,54 +2156,24 @@ double sor_cell_edge(const float (*mn)[3], const float (*mx)[3], const int64_t* 
   return std::min(std::max(edge, 1e-30), 1e36);  // 1 / edge stays a normal float
 }
 
-// clouds = the ranges [begin[k], begin[k+1]) of pts (frames of the cell key: no neighbours across clouds); output zone k =
-// the survivors of cloud k
+// output zone k = the survivors of cloud k
 int statistical_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, const cm_sor_cfg_t* cfg,
                             cudaStream_t st) {
   if (!cfg) return fail(h, CM_E_INVALID, "cfg is NULL");
   if (cfg->mean_k < 1 || cfg->mean_k > CM_SOR_MAX_K) return fail(h, CM_E_INVALID, "mean_k must be 1 .. %d", CM_SOR_MAX_K);
   if (std::isnan(cfg->std_mul)) return fail(h, CM_E_INVALID, "std_mul is NaN");
   if (cfg->sqrt_mode != CM_SOR_SQRT_FLOAT && cfg->sqrt_mode != CM_SOR_SQRT_DOUBLE) return fail(h, CM_E_INVALID, "bad sqrt_mode");
-  if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
-  if (begin[0] != 0) return fail(h, CM_E_INVALID, "begin[0] must be 0");
-  for (int c = 0; c < n_clouds; ++c)
-    if (begin[c + 1] < begin[c]) return fail(h, CM_E_INVALID, "begin must not decrease");
-  const int64_t n_points = begin[n_clouds];
-  if (in_zone_outputs(h, pts, n_points)) return fail(h, CM_E_INVALID, "the input cloud lies in this handle's own zone outputs (use another handle or copy it out)");
-  int rc = ensure_batch_ws(h);
+  int rc = check_clouds(h, pts, begin, n_clouds, CM_MAX_ZONES);
   if (rc != CM_OK) return rc;
-  Workspace& w = h->batch;
-  if (n_points > (int64_t)w.cap_points) return fail(h, CM_E_CAPACITY, "%lld points > capacity %u", (long long)n_points, w.cap_points);
-  if ((uint32_t)n_clouds > w.cap_frames)
-    return fail(h, CM_E_CAPACITY, "%d clouds > max_batch_frames %u of this handle", n_clouds, w.cap_frames);
-  rc = zone_ws_ensure(h, (size_t)n_points);
+  const int64_t n_points = begin[n_clouds];
+  VoxelParams vp;
+  rc = cell_keys_begin(h, pts, begin, n_clouds, vp, st);
   if (rc != CM_OK) return rc;
   rc = sor_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
+  Workspace& w = h->batch;
   cm_handle_s::SorWs& s = h->sw;
   s.ran = false;
-  w.has_run = true; w.report_valid = false; w.profiled = false;
-  w.n_frames = (uint32_t)n_clouds; w.n_segs = 0; w.points_in = n_points; w.launches = 0;
-  w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
-  w.voxel_pts = pts; w.fused_keys = false;
-  h->last = &w;
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
-  CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
-  VoxelParams vp;
-  fill_voxel_params(h, w, vp, pts, (uint32_t)n_clouds, (uint32_t)n_points);
-  vp.pcl_refuses = 0;
-  uint32_t* fss = const_cast<uint32_t*>(vp.frame_surv_start);
-  for (int c = 0; c < n_clouds; ++c) {  // bounding box and non-finite count of every cloud
-    const uint32_t n_here = (uint32_t)(begin[c + 1] - begin[c]);
-    if (!n_here) continue;
-    CM_CUDA(h, launch_minmax(pts + begin[c], n_here, vp.ctrl, vp.acc + c, fss + c, st));
-    ++w.launches;
-  }
-  if (n_clouds > 1 || n_points == 0) {  // the cloud ranges (the single-cloud launch above wrote them itself)
-    uint32_t starts[CM_MAX_ZONES + 1];
-    for (int c = 0; c <= n_clouds; ++c) starts[c] = (uint32_t)begin[c];
-    CM_CUDA(h, cudaMemcpyAsync(fss, starts, sizeof(uint32_t) * (size_t)(n_clouds + 1), cudaMemcpyHostToDevice, st));
-  }
   // one round trip: the bounds choose the cell edge, the finite counts are PCL's valid_distances
   FrameAcc acc[CM_MAX_ZONES];
   CM_CUDA(h, cudaMemcpyAsync(acc, vp.acc, sizeof(FrameAcc) * (size_t)n_clouds, cudaMemcpyDeviceToHost, st));
@@ -2191,37 +2193,19 @@ int statistical_outlier_run(cm_handle_t h, const float4* pts, const int64_t* beg
     if (n_fin[c] > 0 && n_fin[c] <= cfg->mean_k) too_few |= 1u << c;
   }
   const float inv = (float)(1.0 / sor_cell_edge(mn, mx, n_fin, n_clouds, cfg->mean_k));
-  for (int k = 0; k < 3; ++k) vp.inv_leaf[k] = inv;
-  CM_CUDA(h, cudaEventRecord(w.ev[EV_K1].get(), st));
-  rc = run_voxel(h, w, vp, st, false, false);  // keys + sort only
+  rc = cell_keys_sort(h, vp, inv, st);
   if (rc != CM_OK) return rc;
-  if (w.plan_error == CM_DEV_E_KEY_RANGE) return fail(h, CM_E_KEY_RANGE, "cell grid exceeds the key range");
-  if (w.plan_error) return fail(h, CM_E_INTERNAL, "device error %u", w.plan_error);
-  vp.key_bytes = w.key_bytes;
   SorParams sp;
   sp.mean_k = (uint32_t)cfg->mean_k;
   sp.sqrt_mode = (uint32_t)cfg->sqrt_mode;
   sp.too_few = too_few;
   sp.sorted_pts = s.sorted_pts.get();
   sp.dist = s.dist.get();
-  sp.cell_start = nullptr;
   sp.cell = 1.0 / (double)inv;
-  // the radius outlier removal's direct-address table of the cells' first sorted positions when the key space is small
-  // (CM_SOR_NO_TABLE=1 forces the binary searches: test hook for the large-key-space path)
-  if (n_points > 0 && w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&
-      !getenv("CM_SOR_NO_TABLE")) {
-    const size_t keys = (size_t)n_clouds << w.plan_idx_bits;
-    if (h->ror_table_cap < keys + 1) {
-      h->ror_table.reset(); h->ror_table_cap = 0;  // the old table goes before the larger one is allocated
-      CM_CUDA(h, dev_alloc(h->ror_table, keys + 1));
-      h->ror_table_cap = keys + 1;
-    }
-    RorParams rp{};
-    rp.cell_start = h->ror_table.get(); rp.table_keys = (uint32_t)keys;
-    CM_CUDA(h, launch_radius_table(vp, rp, st));
-    ++w.launches;
-    sp.cell_start = rp.cell_start;
-  }
+  RorParams rp{};
+  rc = enqueue_cell_table(h, vp, "CM_SOR_NO_TABLE", rp, st);
+  if (rc != CM_OK) return rc;
+  sp.cell_start = rp.cell_start;
   if (n_points) CM_CUDA(h, cudaMemsetAsync(s.dist.get(), 0, (size_t)n_points * sizeof(float), st));
   s.profiled = h->profiling;
   if (s.profiled) CM_CUDA(h, cudaEventRecord(s.ev[0].get(), st));
@@ -2253,13 +2237,8 @@ int statistical_outlier_run(cm_handle_t h, const float4* pts, const int64_t* beg
 }  // namespace
 
 int cm_dev_statistical_outlier(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_sor_cfg_t* cfg, void* stream) {
-  if (!h) return CM_E_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
-  if (n_points < 0) return fail(h, CM_E_INVALID, "bad n_points");
   const int64_t begin[2] = {0, n_points};
-  return statistical_outlier_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, 1, cfg, static_cast<cudaStream_t>(stream));
+  return cm_dev_statistical_outlier_multi(h, xyzi_dev, begin, 1, cfg, stream);
 }
 
 int cm_dev_statistical_outlier_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
@@ -2267,8 +2246,6 @@ int cm_dev_statistical_outlier_multi(cm_handle_t h, const float* xyzi_dev, const
   if (!h || !begin) return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_clouds >= 1 && n_clouds <= CM_MAX_ZONES && begin[n_clouds] > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u)))
-    return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
   return statistical_outlier_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, n_clouds, cfg,
                                  static_cast<cudaStream_t>(stream));
 }
@@ -2278,31 +2255,12 @@ int cm_statistical_outlier_multi(cm_handle_t h, const float* xyzi_host, const in
                                  int64_t* out_begin) {
   if (!h || !begin || !out_begin) return CM_E_INVALID;
   if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
-  const int64_t n_points = begin[n_clouds];
-  if (n_points < 0 || (n_points > 0 && !xyzi_host)) return CM_E_INVALID;
-  cm_zone_out_t zo;
-  {
-    std::lock_guard<std::mutex> lk(h->mu);
-    CM_CUDA(h, cudaSetDevice(h->device));
-    int rc = zone_ws_ensure(h, (size_t)n_points);
-    if (rc != CM_OK) return rc;
-    cm_handle_s::ZoneWs& z = h->zw;
-    if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
-    if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-    rc = statistical_outlier_run(h, z.in_stage.get(), begin, n_clouds, cfg, nullptr);
-    if (rc != CM_OK) return rc;
-  }
-  int rc = cm_get_zone_out(h, &zo);
-  for (int k = 0; k <= n_clouds; ++k) out_begin[k] = zo.begin[k];
-  if (rc != CM_OK) return rc;
-  {
-    std::lock_guard<std::mutex> lk(h->mu);
-    const int64_t total = zo.begin[n_clouds];
-    if (total > capacity) return fail(h, CM_E_CAPACITY, "%lld points kept, caller capacity %lld", (long long)total, (long long)capacity);
-    if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
-    if (out_idx && total) CM_CUDA(h, cudaMemcpy(out_idx, zo.src, (size_t)total * 4, cudaMemcpyDeviceToHost));
-  }
-  return CM_OK;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  const float4* pts = nullptr;
+  int rc = stage_host_cloud(h, xyzi_host, begin[n_clouds], &pts);
+  if (rc == CM_OK) rc = statistical_outlier_run(h, pts, begin, n_clouds, cfg, nullptr);
+  return rc == CM_OK ? zone_copy_out(h, n_clouds + 1, out_xyzi, out_idx, capacity, out_begin) : rc;
 }
 
 int cm_statistical_outlier(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_sor_cfg_t* cfg,
@@ -2495,15 +2453,12 @@ struct PlaneSearch {
 // clouds = the ranges [begin[k], begin[k+1]) of pts; out[n_clouds]; output zones 2k = inliers, 2k + 1 = rest of cloud k
 int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, const cm_plane_cfg_t& cfg,
                      cm_plane_t* out, cudaStream_t st) {
-  if (n_clouds < 1 || n_clouds > CM_MAX_PLANE_CLOUDS) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_PLANE_CLOUDS);
-  if (begin[0] != 0) return fail(h, CM_E_INVALID, "begin[0] must be 0");
-  for (int c = 0; c < n_clouds; ++c)
-    if (begin[c + 1] < begin[c]) return fail(h, CM_E_INVALID, "begin must not decrease");
+  int rc = check_clouds(h, pts, begin, n_clouds, CM_MAX_PLANE_CLOUDS);
+  if (rc != CM_OK) return rc;
   const int64_t n_points = begin[n_clouds];
   if (n_points > 0x7FFFFFF0ll) return fail(h, CM_E_INVALID, "bad n_points");
   if (cfg.max_iterations < 0 || cfg.sum_order < 0 || cfg.sum_order > 2) return fail(h, CM_E_INVALID, "bad plane settings");
-  if (in_zone_outputs(h, pts, n_points)) return fail(h, CM_E_INVALID, "the input cloud lies in this handle's own zone outputs (use another handle or copy it out)");
-  int rc = zone_ws_ensure(h, (size_t)n_points);
+  rc = zone_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
   rc = plane_ws_ensure(h);
   if (rc != CM_OK) return rc;
@@ -2665,21 +2620,13 @@ int cm_dev_plane_ransac_multi(cm_handle_t h, const float* xyzi_dev, const int64_
   if (!h || !cfg || !out || !begin) return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_clouds >= 1 && n_clouds <= CM_MAX_PLANE_CLOUDS && begin[n_clouds] > 0 &&
-      (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u)))
-    return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
   return plane_ransac_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, n_clouds, *cfg, out, static_cast<cudaStream_t>(stream));
 }
 
 int cm_dev_plane_ransac(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_plane_cfg_t* cfg, cm_plane_t* out,
                         void* stream) {
-  if (!h || !cfg || !out) return CM_E_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_points > 0 && (!xyzi_dev || (reinterpret_cast<uintptr_t>(xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "xyzi_dev must be 16-byte aligned");
-  if (n_points < 0) return fail(h, CM_E_INVALID, "bad n_points");
   const int64_t begin[2] = {0, n_points};
-  return plane_ransac_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, 1, *cfg, out, static_cast<cudaStream_t>(stream));
+  return cm_dev_plane_ransac_multi(h, xyzi_dev, begin, 1, cfg, out, stream);
 }
 
 int cm_plane_ransac_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds, const cm_plane_cfg_t* cfg,
@@ -2688,24 +2635,10 @@ int cm_plane_ransac_multi(cm_handle_t h, const float* xyzi_host, const int64_t* 
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
   if (n_clouds < 1 || n_clouds > CM_MAX_PLANE_CLOUDS) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_PLANE_CLOUDS);
-  const int64_t n_points = begin[n_clouds];
-  if (n_points < 0 || (n_points > 0 && !xyzi_host)) return fail(h, CM_E_INVALID, "bad input");
-  int rc = zone_ws_ensure(h, (size_t)n_points);
-  if (rc != CM_OK) return rc;
-  cm_handle_s::ZoneWs& z = h->zw;
-  if (!z.in_stage) CM_CUDA(h, dev_alloc(z.in_stage, z.cap_points));
-  if (n_points) CM_CUDA(h, cudaMemcpyAsync(z.in_stage.get(), xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
-  rc = plane_ransac_run(h, z.in_stage.get(), begin, n_clouds, *cfg, out, nullptr);
-  if (rc != CM_OK) return rc;
-  cm_zone_out_t zo;
-  rc = zone_out_locked(h, &zo);
-  for (int k = 0; k <= 2 * n_clouds; ++k) out_begin[k] = zo.begin[k];
-  if (rc != CM_OK) return rc;
-  const int64_t total = zo.begin[2 * n_clouds];
-  if (total > capacity) return fail(h, CM_E_CAPACITY, "%lld points, caller capacity %lld", (long long)total, (long long)capacity);
-  if (out_xyzi && total) CM_CUDA(h, cudaMemcpy(out_xyzi, zo.xyzi, (size_t)total * 16, cudaMemcpyDeviceToHost));
-  if (out_idx && total) CM_CUDA(h, cudaMemcpy(out_idx, zo.src, (size_t)total * 4, cudaMemcpyDeviceToHost));
-  return CM_OK;
+  const float4* pts = nullptr;
+  int rc = stage_host_cloud(h, xyzi_host, begin[n_clouds], &pts);
+  if (rc == CM_OK) rc = plane_ransac_run(h, pts, begin, n_clouds, *cfg, out, nullptr);
+  return rc == CM_OK ? zone_copy_out(h, 2 * n_clouds + 1, out_xyzi, out_idx, capacity, out_begin) : rc;
 }
 
 int cm_plane_ransac(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_plane_cfg_t* cfg, cm_plane_t* out,
@@ -2771,25 +2704,9 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
         pl.n_pass = 1; pl.pass[0] = x;
       }
     }
-    ZoneSet zs{};
-    zs.n_zones = 2 * G + P;
-    zs.all_box = 1;
-    const float fmax = std::numeric_limits<float>::max();
-    for (int z = 0; z < zs.n_zones; ++z) {
-      ZoneDev& zd = zs.zone[z];
-      zd.n_pass = zones[(size_t)z].n_pass; zd.is_box = 1; zd.use_i = 0;
-      for (int a = 0; a < 4; ++a) { zd.lo[a] = -fmax; zd.hi[a] = fmax; }
-      for (int q = 0; q < zd.n_pass; ++q) {
-        const cm_pass_t& ps = zones[(size_t)z].pass[q];
-        zd.pass[q] = PassDev{ps.axis, ps.lo, ps.hi, 0};
-        if (!(ps.lo == ps.lo) || !(ps.hi == ps.hi)) { zd.is_box = 0; zs.all_box = 0; continue; }
-        zd.lo[ps.axis] = std::max(zd.lo[ps.axis], ps.lo);
-        zd.hi[ps.axis] = std::min(zd.hi[ps.axis], ps.hi);
-      }
-    }
-    h->zones = zs;
+    rc = make_zone_set(h, 2 * G + P, zones.data(), h->zones);
   }
-  rc = zone_run(h, roi, n, st);
+  if (rc == CM_OK) rc = zone_run(h, roi, n, st);
   h->zones = saved;
   if (rc != CM_OK) return rc;
   cm_zone_out_t zo;
@@ -2859,7 +2776,8 @@ int cm_dev_proceed_zones(cm_handle_t h, const float* roi_xyzi_dev, int64_t n_poi
   if (!h || !cfg || !out) return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  if (n_points > 0 && (!roi_xyzi_dev || (reinterpret_cast<uintptr_t>(roi_xyzi_dev) & 15u))) return fail(h, CM_E_INVALID, "roi_xyzi_dev must be 16-byte aligned");
+  const int rc = check_dev_cloud(h, roi_xyzi_dev, n_points);
+  if (rc != CM_OK) return rc;
   return proceed_run(h, reinterpret_cast<const float4*>(roi_xyzi_dev), n_points, *cfg, out, static_cast<cudaStream_t>(stream));
 }
 
@@ -2869,13 +2787,11 @@ int cm_proceed_zones(cm_handle_t h, const float* roi_xyzi_host, int64_t n_points
   if (!h || !cfg || !n_no_ground || !n_ground || n_points < 0 || (n_points > 0 && !roi_xyzi_host)) return CM_E_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   CM_CUDA(h, cudaSetDevice(h->device));
-  int rc = proceed_ws_ensure(h, (size_t)n_points);
+  const float4* roi = nullptr;
+  int rc = stage_host_cloud(h, roi_xyzi_host, n_points, &roi);
   if (rc != CM_OK) return rc;
-  cm_handle_s::ProceedWs& w = h->prz;
-  if (!w.in_stage) CM_CUDA(h, dev_alloc(w.in_stage, w.cap));
-  if (n_points) CM_CUDA(h, cudaMemcpyAsync(w.in_stage.get(), roi_xyzi_host, (size_t)n_points * 16, cudaMemcpyHostToDevice, nullptr));
   cm_proceed_out_t po;
-  rc = proceed_run(h, w.in_stage.get(), n_points, *cfg, &po, nullptr);
+  rc = proceed_run(h, roi, n_points, *cfg, &po, nullptr);
   if (rc != CM_OK) return rc;
   *n_no_ground = po.n_no_ground;
   *n_ground = po.n_ground;

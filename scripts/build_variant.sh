@@ -7,7 +7,9 @@ srcs=${@:-cm_radix_sort.cu}
 root=$(cd "$(dirname "$0")/.." && pwd)
 mkdir -p "$root/variants/obj_$name"
 objs=""
-for s in cm_transform_crop.cu cm_voxel.cu cm_radix_sort.cu cm_zones.cu cm_outlier.cu cm_route.cu cm_plane.cu cm_api.cu; do
+# every source the library links, in build.py's order (the other objects come from its build directory)
+all=$(python3 -c "import runpy, sys; print(' '.join(runpy.run_path(sys.argv[1])['SOURCES']))" "$root/cloud_merger_b200/build.py")
+for s in $all; do
   o="$root/cloud_merger_b200/build/${s%.cu}.o"
   for v in $srcs; do
     if [ "$v" == "$s" ]; then

@@ -11,6 +11,14 @@ from cloud_merger_b200 import make_layout, synth
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
+def host_function(name, source="cm_api.cu"):
+    """The text of the host function `int name(...)` in cloud_merger_b200/csrc/<source>, up to its closing brace."""
+    with open(os.path.join(os.path.dirname(HERE), "cloud_merger_b200", "csrc", source)) as f:
+        src = f.read()
+    a = src.index("\nint %s(" % name) + 1
+    return src[a:src.index("\n}\n", a)]
+
+
 def known_answer():
     with open(os.path.join(HERE, "golden", "known_answer.json")) as f:
         d = json.load(f)

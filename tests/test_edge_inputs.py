@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import edge_inputs as E
-from helpers import cloud_dict
+from helpers import cloud_dict, host_function
 from oracle import np_oracle
 
 F32 = np.float32
@@ -364,17 +364,25 @@ def _src(name):
 
 def test_ror_constants_match_the_source():
     """The N-family restatement mirrors the kernels' constants; a retune must fail here rather than miss the edges."""
-    ror, api, vox = _src("cm_outlier.cu"), _src("cm_api.cu"), _src("cm_voxel.cu")
-    assert "(float)radius * 1.00390625f" in api and E.ROR_MARGIN == 1.00390625
+    ror, vox = _src("cm_outlier.cu"), _src("cm_voxel.cu")
+    run, front, keys, table = (host_function(f) for f in ("radius_outlier_run", "cell_keys_begin", "cell_keys_sort",
+                                                          "enqueue_cell_table"))
+    assert "(float)radius * 1.00390625f" in run and E.ROR_MARGIN == 1.00390625
     assert "worst >= (1 << 14)" in ror and E.ROR_BOUND == 1 << 14
-    assert "w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25)" in api and E.ROR_TABLE_LOG2 == 25
+    assert "w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25)" in table and E.ROR_TABLE_LOG2 == 25
+    assert 'enqueue_cell_table(h, vp, "CM_ROR_NO_TABLE", rp, st)' in run
+    # the launches cm_launch_count reports for the call (ror_launches): a bounding box per cloud and the table in the shared
+    # front end, the count in the run
+    assert front.count("++w.launches;") == 1 and table.count("++w.launches;") == 1 and run.count("++w.launches;") == 1
+    assert "w.launches" not in keys and "rc = run_voxel(h, w, vp, st, false, false);" in keys
+    assert "rc = cell_keys_sort(h, vp, 1.0f / cell, st);" in run
     assert "constexpr int ROR_THREADS = 256;" in ror and E.ROR_THREADS == 256
     assert "constexpr unsigned long long LONG_GAP = 2048;" in ror and "to - from >= LONG_GAP" in ror and E.ROR_LONG_GAP == 2048
     assert "constexpr int LIST = 32;" in ror and E.ROR_LIST == 32
     assert "0x28215u" in ror and "0x22161u" in ror and (E.ROR_ROW_DZ, E.ROR_ROW_DY) == (0x28215, 0x22161)
     assert E.ror_rows() == [(0, 0), (0, -1), (0, 1), (-1, 0), (1, 0), (-1, -1), (-1, 1), (1, -1), (1, 1)]
     assert "dv > (1ll << 21)" in vox and "1073741824.f" in vox
-    assert "if (g.zero_keys) return;" in ror and "w.plan_error == CM_DEV_E_KEY_RANGE" in api
+    assert "if (g.zero_keys) return;" in ror and "w.plan_error == CM_DEV_E_KEY_RANGE" in keys
 
 
 def _two_apart(x, pairs, cell):

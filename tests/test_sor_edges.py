@@ -14,6 +14,7 @@ import pytest
 import sor_edges as S
 import sor_np
 import sor_oracle
+from helpers import host_function
 
 SRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "cloud_merger_b200", "csrc")
 CASES = S.sor_cases()
@@ -33,9 +34,11 @@ def _valid(c, mean_k):
     return int(np.isfinite(np.asarray(c, F32)[:, :3]).all(axis=1).sum()) > mean_k
 
 
-def test_sor_constants_match_the_source():
+def test_sor_constants_match_the_shared_front_end():
     """The S-family restatement mirrors the kernels' constants; a retune must fail here rather than miss the edges."""
     sor, api, vox = _src("cm_statistical.cu"), _src("cm_api.cu"), _src("cm_voxel.cu")
+    body, front, keys, table = (host_function(f) for f in ("statistical_outlier_run", "cell_keys_begin", "cell_keys_sort",
+                                                           "enqueue_cell_table"))
     assert "s.mean_k + 1 <= 32 ? 1 : s.mean_k + 1 <= 64 ? 2 : 4" in sor and S.SOR_NS_LIMITS == (32, 64)
     assert re.search(r"constexpr int SOR_WARPS = (\d+);", sor).group(1) == str(S.SOR_WARPS)
     assert re.search(r"constexpr int SUM_THREADS = (\d+);", sor).group(1) == str(S.SUM_THREADS)
@@ -49,14 +52,17 @@ def test_sor_constants_match_the_source():
     assert "mag / 1048576.0, e[a] / 524288.0" in api and (S.FLOOR_MAG, S.FLOOR_EXTENT) == (2.0 ** 20, 2.0 ** 19)
     assert "floor_edge * (1.0 + 1.0 / 1024.0)" in api and S.FLOOR_MARGIN == 1.0 + 1.0 / 1024.0
     assert "std::min(std::max(edge, 1e-30), 1e36)" in api and (S.EDGE_MIN, S.EDGE_MAX) == (1e-30, 1e36)
-    assert "const float inv = (float)(1.0 / sor_cell_edge(" in api
+    assert "const float inv = (float)(1.0 / sor_cell_edge(" in body and "rc = cell_keys_sort(h, vp, inv, st);" in body
     assert ("w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&\n      "
-            "!getenv(\"CM_SOR_NO_TABLE\")") in api and S.TABLE_LOG2 == 25
+            "!getenv(no_table_env)") in table and S.TABLE_LOG2 == 25
+    assert 'enqueue_cell_table(h, vp, "CM_SOR_NO_TABLE", rp, st)' in body
     assert "dv > (1ll << 21)" in vox and "1073741824.f" in vox
-    # the launches cm_launch_count reports for the call (sor_plan's "launches")
-    body = api[api.index("int statistical_outlier_run("):api.index("int cm_dev_statistical_outlier(")]
-    assert body.count("++w.launches;") == 2 and body.count("w.launches += 2;") == 2
-    assert "rc = run_voxel(h, w, vp, st, false, false);" in body and "zone_run(h, pts, n_points, st, true, n_clouds)" in body
+    # the launches cm_launch_count reports for the call (sor_plan's "launches"): a bounding box per cloud and the table in
+    # the shared front end, the search, sums and select in the run
+    assert front.count("++w.launches;") == 1 and table.count("++w.launches;") == 1
+    assert body.count("++w.launches;") == 0 and body.count("w.launches += 2;") == 2
+    assert "w.launches" not in keys and "rc = run_voxel(h, w, vp, st, false, false);" in keys
+    assert "zone_run(h, pts, n_points, st, true, n_clouds)" in body
 
 
 @pytest.mark.parametrize("name", sorted(CASES))
