@@ -187,6 +187,7 @@ struct cm_handle_s {
   uint32_t run_counter = 0;
   Workspace batch;          // device-resident batch path
   Workspace* last = nullptr;  // workspace of the most recent run
+  bool zone_launches = false;  // cm_launch_count reports zw.launches: a zone split or a plane search ran after `last`
   std::vector<cm_frame_info_t> frame_info;
   cm_stats_t stats{};
   float stage_ms[EV_COUNT]{};
@@ -759,7 +760,7 @@ int run_pipeline(cm_handle_t h, Workspace& w, const cm_segment_t* segs, int n_se
   w.n_frames = n_frames; w.n_segs = (uint32_t)n_seg; w.points_in = total; w.launches = 0;
   w.ran_k1 = true; w.ran_voxel = false; w.stream = st;
   w.voxel_pts = w.surv_xyzi.get();
-  h->last = &w;
+  h->last = &w; h->zone_launches = false;
 
   if (!w.capturing) CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
   CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
@@ -1027,7 +1028,7 @@ int merge_async_impl(cm_handle_t h, uint64_t mask, int64_t* ticket) {
   if (graphable && sl.graph && sl.graph_key == key) {
     Workspace& w = sl.ws;  // same configuration as the captured frame: every host-side field of the run is unchanged
     w.has_run = true; w.report_valid = false; w.dense_valid = false; w.stream = st;
-    h->last = &w;
+    h->last = &w; h->zone_launches = false;
     CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
     CM_CUDA(h, cudaGraphLaunch(sl.graph.get(), st));
     CM_CUDA(h, cudaEventRecord(w.ev[EV_CENT].get(), st));
@@ -1087,7 +1088,7 @@ int wait_impl(cm_handle_t h, int64_t ticket, cm_frame_out_t* out, uint64_t* used
   for (auto& s : h->slots) if (s.busy && s.ticket == ticket) sl = &s;
   if (!sl) return fail(h, CM_E_INVALID, "unknown ticket %lld", (long long)ticket);
   Workspace& w = sl->ws;
-  h->last = &w;
+  h->last = &w; h->zone_launches = false;
   int rc = fetch_report(h, w, sl->done.get());
   sl->busy = false;
   if (rc != CM_OK) return rc;
@@ -1601,7 +1602,7 @@ int voxelgrid_run(cm_handle_t h, const float4* pts, int64_t n_points, cudaStream
   w.n_frames = 1; w.n_segs = 0; w.points_in = n_points; w.launches = 0;
   w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
   w.voxel_pts = pts; w.fused_keys = false;
-  h->last = &w;
+  h->last = &w; h->zone_launches = false;
   CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
   CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
   VoxelParams vp;
@@ -1760,8 +1761,10 @@ int cm_dev_zone_split(cm_handle_t h, const float* xyzi_dev, int64_t n_points, vo
   CM_CUDA(h, cudaSetDevice(h->device));
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (xyzi_dev) {
-    const int rc = check_dev_cloud(h, xyzi_dev, n_points);
-    return rc == CM_OK ? zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st) : rc;
+    int rc = check_dev_cloud(h, xyzi_dev, n_points);
+    if (rc == CM_OK) rc = zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st);
+    if (rc == CM_OK) h->zone_launches = true;
+    return rc;
   }
   // the merged cropped cloud of the last transform_crop run (what getROI hands to getCloudPart)
   if (!h->last || !h->last->ran_k1) return fail(h, CM_E_INVALID, "no transform_crop result on this handle");
@@ -1771,7 +1774,9 @@ int cm_dev_zone_split(cm_handle_t h, const float* xyzi_dev, int64_t n_points, vo
   rc = materialize_dense(h, w);
   if (rc != CM_OK) return rc;
   CM_CUDA(h, cudaStreamSynchronize(w.stream));
-  return zone_run(h, w.dense_xyzi.get(), h->stats.survivors, st);
+  rc = zone_run(h, w.dense_xyzi.get(), h->stats.survivors, st);
+  if (rc == CM_OK) h->zone_launches = true;  // h->last stays the crop's workspace: the next split without a cloud needs it
+  return rc;
 }
 
 namespace {
@@ -1810,7 +1815,8 @@ int zone_out_locked(cm_handle_t h, cm_zone_out_t* out) {
   out->xyzi = reinterpret_cast<const float*>(z.out_xyzi.get());
   out->src = z.out_src.get();
   if (report[CM_MAX_ZONES + 1])
-    return fail(h, CM_E_CAPACITY, "the zones hold %u points together, capacity is %zu", report[CM_MAX_ZONES + 1], z.cap_out);
+    return fail(h, CM_E_CAPACITY, "the zones hold %s%u points together, capacity is %zu",
+                report[CM_MAX_ZONES + 1] > 0xFFFFFFF0u ? "more than " : "", std::min(report[CM_MAX_ZONES + 1], 0xFFFFFFF0u), z.cap_out);
   if (z.ror_run && report[CM_MAX_ZONES + 2] == CM_DEV_E_KEY_RANGE)
     return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (more than 2^14 cells from the origin)");
   if (z.ror_run && report[CM_MAX_ZONES + 2]) return fail(h, CM_E_INTERNAL, "device error %u", report[CM_MAX_ZONES + 2]);
@@ -1854,6 +1860,7 @@ int cm_zone_split(cm_handle_t h, const float* xyzi_host, int64_t n_points, float
   const float4* pts = nullptr;
   int rc = stage_host_cloud(h, xyzi_host, n_points, &pts);
   if (rc == CM_OK) rc = zone_run(h, pts, n_points, nullptr);
+  if (rc == CM_OK) h->zone_launches = true;
   return rc == CM_OK ? zone_copy_out(h, h->zones.n_zones + 1, out_xyzi, out_src, capacity, out_begin) : rc;
 }
 
@@ -1944,7 +1951,11 @@ int cm_dev_route_by_key(cm_handle_t h, const float* xyzi_dev, int64_t n_points, 
   for (int k = 0; k + 1 < n_parts; ++k) sp.splitter[k] = splitters[k];
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   CM_CUDA(h, launch_route_mask(reinterpret_cast<const float4*>(xyzi_dev), (uint32_t)n_points, g, sp, h->zw.mask.get(), st));
-  return zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st, true, n_parts);
+  rc = zone_run(h, reinterpret_cast<const float4*>(xyzi_dev), n_points, st, true, n_parts);
+  if (rc != CM_OK) return rc;
+  if (n_points) ++h->zw.launches;  // the mask kernel (launch_route_mask launches nothing without points)
+  h->zone_launches = true;
+  return CM_OK;
 }
 
 int cm_memcpy_d2d(cm_handle_t h, void* dst_dev, const void* src_dev, size_t bytes, void* stream) {
@@ -1974,7 +1985,7 @@ int cell_keys_begin(cm_handle_t h, const float4* pts, const int64_t* begin, int 
   w.n_frames = (uint32_t)n_clouds; w.n_segs = 0; w.points_in = n_points; w.launches = 0;
   w.ran_k1 = false; w.ran_voxel = false; w.stream = st; w.n_k1_tiles = 0; w.dense_valid = false;
   w.voxel_pts = pts; w.fused_keys = false;
-  h->last = &w;
+  h->last = &w; h->zone_launches = false;
   CM_CUDA(h, cudaEventRecord(w.ev[EV_START].get(), st));
   CM_CUDA(h, cudaMemsetAsync(w.meta.get(), 0, w.ml.zero_bytes, st));
   fill_voxel_params(h, w, vp, pts, (uint32_t)n_clouds, (uint32_t)n_points);
@@ -2464,7 +2475,12 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
   if (rc != CM_OK) return rc;
   cm_handle_s::PlaneWs& q = h->pw;
   // PCL compares the float distance with the double threshold: the smallest float >= threshold decides the same way
-  float thr = (float)cfg.distance_threshold;
+  // (beyond +-FLT_MAX the cast itself would be undefined: above it every finite distance is inside, as below +inf, and
+  // below -FLT_MAX nothing is, as below -inf)
+  const double fmax = (double)std::numeric_limits<float>::max();
+  float thr = cfg.distance_threshold > fmax    ? std::numeric_limits<float>::infinity()
+              : cfg.distance_threshold < -fmax ? -std::numeric_limits<float>::infinity()
+                                               : (float)cfg.distance_threshold;
   if ((double)thr < cfg.distance_threshold) thr = std::nextafter(thr, std::numeric_limits<float>::infinity());
   int64_t launches = 0;
 
@@ -2598,19 +2614,19 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
   }
   // selectWithinDistance with the final model + the two ExtractIndices passes
   CM_CUDA(h, launch_plane_select(ps, (uint32_t)cfg.sum_order, st));
-  ++launches;
+  if (n_points) ++launches;  // launch_plane_select launches nothing without points
   rc = zone_run(h, pts, n_points, st, true, 2 * n_clouds);
   if (rc != CM_OK) return rc;
-  launches += h->zw.launches;
   cm_zone_out_t zo;
   rc = zone_out_locked(h, &zo);
+  h->zw.launches += launches;  // cm_launch_count: the whole search, its select and its compaction
+  h->zone_launches = true;
   if (rc != CM_OK) return rc;
-  h->zw.launches = launches;
   for (int c = 0; c < n_clouds; ++c) out[c].n_inliers = zo.begin[2 * c + 1] - zo.begin[2 * c];
   if (trace)
     fprintf(stderr, "[cm plane] clouds %d points %lld: %d scoring rounds (host draws %.1f us, GPU round trips %.1f us, stopping rule %.1f us), "
             "refit + select + compaction %.1f us, total %.1f us, %lld launches\n", n_clouds, (long long)n_points, rounds, t_draw, t_score,
-            t_walk, us(t_search, now()), us(t_begin, now()), (long long)launches);
+            t_walk, us(t_search, now()), us(t_begin, now()), (long long)h->zw.launches);
   return CM_OK;
 }
 }  // namespace
@@ -2709,6 +2725,7 @@ int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cf
   if (rc == CM_OK) rc = zone_run(h, roi, n, st);
   h->zones = saved;
   if (rc != CM_OK) return rc;
+  h->zone_launches = true;  // without a ground part the split is the last filter of the call
   cm_zone_out_t zo;
   rc = zone_out_locked(h, &zo);
   ++out->host_syncs;
@@ -3259,8 +3276,9 @@ int cm_get_frame_info(cm_handle_t h, cm_frame_info_t* out, int capacity, int* n_
 }
 
 int64_t cm_launch_count(cm_handle_t h) {
-  if (!h || !h->last) return 0;
-  return h->last->launches;
+  if (!h) return 0;
+  if (h->zone_launches) return h->zw.launches;
+  return h->last ? h->last->launches : 0;
 }
 
 int cm_stage_ms(cm_handle_t h, const char* stage, float* ms) {

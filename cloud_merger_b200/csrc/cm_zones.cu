@@ -179,13 +179,16 @@ __global__ void __launch_bounds__(1024) k_zone_scan(const ZoneParams p) {
   __syncthreads();
   if (s_last && tid == 0) {
     __threadfence();
-    uint32_t run = 0;
+    // Each zone total is at most n_points, but up to CM_MAX_ZONES of them add up past 2^32: the sum is 64-bit, and a sum
+    // beyond 0xFFFFFFF0 reports the saturated 0xFFFFFFFF (more than any output may hold: the host does not regrow).
+    unsigned long long run = 0;
     for (uint32_t k = 0; k < gridDim.x; ++k) {
-      p.zone_begin[k] = run;
+      p.zone_begin[k] = (uint32_t)min(run, 0xFFFFFFFFull);
       run += reinterpret_cast<volatile uint32_t*>(p.zone_total)[k];
     }
-    p.zone_begin[gridDim.x] = run;
-    if (run > p.out_capacity) *p.overflow = run;  // the scatter kernel then writes nothing
+    const uint32_t total = run > 0xFFFFFFF0ull ? 0xFFFFFFFFu : (uint32_t)run;
+    p.zone_begin[gridDim.x] = total;
+    if (run > p.out_capacity) *p.overflow = total;  // the scatter kernel then writes nothing
     *p.scan_ticket = 0;                           // ready for the next split
   }
 }

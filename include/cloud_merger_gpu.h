@@ -592,7 +592,12 @@ CM_API int cm_sync(cm_handle_t h);
 CM_API int cm_get_stats(cm_handle_t h, cm_stats_t* out);
 CM_API int cm_get_device_out(cm_handle_t h, cm_device_out_t* out);
 CM_API int cm_get_frame_info(cm_handle_t h, cm_frame_info_t* out, int capacity, int* n_frames);
-/* Number of kernel launches the last run enqueued (the caller's "gpu_launches" evidence). */
+/* Number of kernel launches the last run enqueued (the caller's "gpu_launches" evidence). Only launches that happened are
+ * counted. After cm_[dev_]zone_split: the split (3, or 1 without points), plus 1 once cm_get_zone_out has repeated the
+ * scatter into grown outputs. After cm_[dev_]plane_ransac[_multi]: the whole call, scoring rounds, refit sums, select and
+ * compaction. After cm_[dev_]radius_outlier[_multi] and cm_[dev_]statistical_outlier[_multi]: the filter up to its mask,
+ * without the compaction. After cm_dev_route_by_key: the mask kernel and the split. After cm_[dev_]proceed_zones: the
+ * radius outlier removal when a part removes ground, else the zone split. After cm_giant_voxelgrid: its local VoxelGrid. */
 CM_API int64_t cm_launch_count(cm_handle_t h);
 /* Device time (ms) of one named stage of the last run, measured with CUDA events on the run's stream:
  * "transform_crop", "grid", "key_hist", "sort", "centroid", "total", and "sort_pass0" (the first radix pass alone; -1 when

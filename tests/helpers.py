@@ -41,6 +41,12 @@ def bits(a):
     return np.ascontiguousarray(a, np.float32).view(np.uint32)
 
 
+def same_floats(a, b):
+    """Bit equality, except that any NaN equals any NaN (x86 and the GPU produce different NaN payloads)."""
+    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
+    return bool(((a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))).all())
+
+
 def assert_bit_equal(a, b, what=""):
     a = np.ascontiguousarray(a, np.float32)
     b = np.ascontiguousarray(b, np.float32)

@@ -7,7 +7,7 @@ import pytest
 
 from cloud_merger_b200 import CloudMerger
 
-from helpers import assert_bit_equal
+from helpers import assert_bit_equal, same_floats
 
 pytestmark = pytest.mark.gpu
 
@@ -25,12 +25,6 @@ def ground_scene(seed, n, ground_frac=0.7, slope=0.02, noise=0.03):
     pts[g:, 2] = rng.uniform(-1.5, 1.0, n - g)
     pts[:, 3] = rng.uniform(0, 255, n)
     return pts[rng.permutation(n)]
-
-
-def same_floats(a, b):
-    """Bit equality, except that any NaN equals any NaN (x86 and the GPU produce different NaN payloads)."""
-    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
-    return bool(((a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))).all())
 
 
 def check(cm, oracle, cloud, thr=THR, prob=PROB, max_it=1000, optimize=True, seed=12345, order=0, device_form=False):
