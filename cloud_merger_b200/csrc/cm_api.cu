@@ -367,7 +367,7 @@ int ws_alloc(cm_handle_t h, Workspace& w, uint32_t points, uint32_t frames, uint
   CM_CUDA(h, dev_alloc(w.surv_xyzi, np));
   CM_CUDA(h, dev_alloc(w.surv_src, np));
   CM_CUDA(h, dev_alloc(w.surv_key, np));
-  CM_CUDA(h, dev_alloc(w.first_k1, sort_lookback_rows((uint32_t)np)));
+  CM_CUDA(h, dev_alloc(w.first_k1, sort_lookback_rows((uint32_t)np) + frames));
   CM_CUDA(h, dev_alloc(w.keys_a, np, 0));
   CM_CUDA(h, dev_alloc(w.keys_b, np, 0));
   CM_CUDA(h, dev_alloc(w.vals_a, np));
@@ -375,8 +375,9 @@ int ws_alloc(cm_handle_t h, Workspace& w, uint32_t points, uint32_t frames, uint
   // every segment owns at least one K1 tile
   w.lb_k1_n = np / k1_min_tile_points() + segs + 2;
   CM_CUDA(h, dev_alloc(w.tile_seg, w.lb_k1_n));
-  w.lb_sort_n = (sort_lookback_rows((uint32_t)np) + (frames > 1 ? frames : 0u)) * CM_RADIX;  // segmented: a partial tile per frame
-  if (frames > 1) {
+  // frame by frame: a partial tile per frame; a wide top digit (BoxGrid::top_bins) has rows of CM_WIDE_BINS words
+  w.lb_sort_n = (sort_lookback_rows((uint32_t)np) + frames) * CM_WIDE_BINS;
+  {  // a single frame too: a fused-key run with a wide top digit sorts it as one segment
     CM_CUDA(h, dev_alloc(w.seg_tile, sort_lookback_rows((uint32_t)np) + frames));
     CM_CUDA(h, dev_alloc(w.seg_hist, (size_t)frames * CM_SEG_PASSES * CM_RADIX));
     CM_CUDA(h, dev_alloc(w.seg_frame_tile0, (size_t)frames + 1));
@@ -481,6 +482,22 @@ bool crop_box_grid(cm_handle_t h, uint32_t n_frames, BoxGrid* g) {
   g->mul2 = (uint32_t)(div[0] * div[1]);
   g->idx_bits = idx_bits;
   g->n_pass = std::max<uint32_t>(1u, (bits + CM_RADIX_BITS - 1) / CM_RADIX_BITS);
+  // Fewer passes: sort every frame on its own (the frame bits are not ranked) and let the top digit idx >> 8 (P - 1) take up to
+  // CM_WIDE_BINS values. P is the fewest passes that allows; the plan is taken only when it saves a pass. (A grid of at most
+  // CM_WIDE_BINS cells keeps the bit-based plan: its top digit would be pass 0's.) CM_NO_WIDE_TOP=1 keeps it always (A/B).
+  static const bool no_wide = getenv("CM_NO_WIDE_TOP") != nullptr;
+  g->seg_sort = 0;
+  g->top_bins = CM_RADIX;
+  if (!no_wide && cells > CM_WIDE_BINS) {
+    uint32_t p = 2;
+    unsigned long long span = CM_RADIX;  // 256^(p - 1)
+    while ((cells + span - 1) / span > CM_WIDE_BINS) { ++p; span *= CM_RADIX; }
+    if (p < g->n_pass) {
+      g->n_pass = p;
+      g->seg_sort = 1;
+      g->top_bins = (cells + span - 1) / span > CM_RADIX ? CM_WIDE_BINS : CM_RADIX;
+    }
+  }
   return true;
 }
 
@@ -629,6 +646,10 @@ int run_voxel(cm_handle_t h, Workspace& w, VoxelParams& vp, cudaStream_t st, boo
     if (ps == 0 && h->profiling) {  // pass 0 of a fused-key run does the key kernel's histogram work too: timed on its own
       CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT0].get(), st));
       w.timed_pass0 = true;
+    }
+    if (ps == 0 && vp.fused_keys && vp.box.seg_sort && vp.max_passes > 1) {  // pass 0 counted the later passes' digits per frame
+      CM_CUDA(h, launch_seg_base(vp, st));
+      ++w.launches;
     }
   }
   if (h->profiling) CM_CUDA(h, cudaEventRecord(w.ev[EV_SORT].get(), st));
@@ -781,6 +802,12 @@ int run_pipeline(cm_handle_t h, Workspace& w, const cm_segment_t* segs, int n_se
   w.fused_keys = fused; w.box = box;
   kp.surv_key = fused ? w.surv_key.get() : nullptr;
   kp.hist = reinterpret_cast<uint32_t*>(w.meta.get() + w.ml.off_hist);
+  kp.hist_frame_stride = 0;
+  if (fused && box.seg_sort) {  // K1 counts the pass-0 digits frame by frame
+    CM_CUDA(h, cudaMemsetAsync(w.seg_hist.get(), 0, (size_t)n_frames * CM_SEG_PASSES * CM_RADIX * sizeof(uint32_t), st));
+    kp.hist = w.seg_hist.get();
+    kp.hist_frame_stride = CM_SEG_PASSES * CM_RADIX;
+  }
   kp.box = box;
   kp.obox = nullptr; kp.n_obox = 0;
   if (h->n_obox > 0) {  // the stage table travels like the segment table: uploaded on the run's stream when it changed

@@ -157,7 +157,9 @@ struct SortInfo {
   uint32_t width;       // bytes of the keys that travel through the sort: 4 (8-byte records) or 8
   uint32_t segmented;   // frame-segmented sort: the keys are the voxel index alone (no frame bits), every frame is sorted as its
                         // own segment of the frame-ordered input, the frame of a key is known from its position
-  uint32_t n_seg_tiles; // segmented: number of (frame-aligned) radix tiles
+  uint32_t n_seg_tiles; // seg_sort: number of (frame-aligned) radix tiles
+  uint32_t seg_sort;    // the passes sort every frame as a segment of its own: segmented runs, and fused-key runs whose frame
+                        // bits stay in the keys but are not ranked (BoxGrid::seg_sort)
 };
 
 // One radix tile of a frame-segmented sort: tiles never straddle frames.
@@ -169,6 +171,9 @@ struct SegTile {
 };
 constexpr uint32_t CM_SEG_FIRST = 0x80000000u;
 constexpr uint32_t CM_SEG_PASSES = 4;  // a segmented key is 32 bits wide at most
+// Bins of a wide top digit: the last pass of a fused-key run may rank up to 384 values of the box-grid index (BoxGrid::top_bins)
+// instead of 256. A frame's row of seg_hist holds it as long as it is pass 2 or earlier (2 * 256 + 384 <= 4 * 256).
+constexpr uint32_t CM_WIDE_BINS = 384;
 
 // ---- float <-> order-preserving uint -----------------------------------------------------------------------------
 __host__ __device__ __forceinline__ uint32_t f32_order_enc(uint32_t bits) {
@@ -294,27 +299,33 @@ __device__ __forceinline__ uint32_t lb_wait_inclusive(unsigned long long* p, uin
 // Exclusive scan over 256 values held one per thread by threads 0..255 of a block with >= 256 threads.
 // `scratch` is >= 9 uint32 of shared memory. Every thread of the block must call it; returns the exclusive prefix
 // (for threads >= 256 the return value is meaningless). *total receives the sum (valid in all threads).
-__device__ __forceinline__ uint32_t block_excl_scan_256(uint32_t v, uint32_t* scratch, uint32_t* total) {
+// Exclusive scan of one value per thread over the first N threads of the block (N / 32 warps; scratch >= N / 32 + 1 words).
+template <int N>
+__device__ __forceinline__ uint32_t block_excl_scan(uint32_t v, uint32_t* scratch, uint32_t* total) {
+  constexpr int W = N / 32;
   const uint32_t tid = threadIdx.x, lane = tid & 31u, w = tid >> 5;
-  if (tid >= 256) v = 0;
+  if (tid >= (uint32_t)N) v = 0;
   const uint32_t incl = warp_incl_scan_u32(v);
-  if (lane == 31 && w < 8) scratch[w] = incl;
+  if (lane == 31 && w < W) scratch[w] = incl;
   __syncthreads();
   if (tid == 0) {
     uint32_t run = 0;
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < W; ++i) {
       uint32_t t = scratch[i];
       scratch[i] = run;
       run += t;
     }
-    scratch[8] = run;
+    scratch[W] = run;
   }
   __syncthreads();
-  const uint32_t res = incl - v + (w < 8 ? scratch[w] : 0u);
-  *total = scratch[8];
+  const uint32_t res = incl - v + (w < W ? scratch[w] : 0u);
+  *total = scratch[W];
   __syncthreads();
   return res;
+}
+__device__ __forceinline__ uint32_t block_excl_scan_256(uint32_t v, uint32_t* scratch, uint32_t* total) {
+  return block_excl_scan<256>(v, scratch, total);
 }
 
 #endif  // __CUDACC__

@@ -22,6 +22,10 @@ struct BoxGrid {
   uint32_t mul1, mul2;       // div_x, div_x * div_y of the box grid
   uint32_t idx_bits;         // bits of the largest box-grid index: key = (frame << idx_bits) | idx
   uint32_t n_pass;           // radix passes the run will make
+  // Fewer passes for a grid of more than 2^(8k) cells: every frame is sorted as a segment of its own (the frame bits stay in
+  // the keys but are not ranked) and the top digit, idx >> 8 (n_pass - 1), ranks top_bins <= 384 values instead of 256.
+  uint32_t seg_sort;         // 1: the passes run frame by frame; K1 counts the pass-0 digits per frame (seg_hist)
+  uint32_t top_bins;         // seg_sort: bins of the last pass (256, or CM_WIDE_BINS when idx >> 8 (n_pass - 1) exceeds 255)
 };
 struct K1Params {
   const SegDev* segs;
@@ -37,6 +41,7 @@ struct K1Params {
   FrameAcc* acc;
   uint32_t* surv_key;          // [slots] box-grid voxel key of every survivor, or null: keys come from k_voxel_key_hist
   uint32_t* hist;              // [CM_MAX_SORT_PASSES][256] digit histograms of all passes (with surv_key)
+  uint32_t hist_frame_stride;  // 0, or box.seg_sort: hist is seg_hist and frame f counts at hist + f * hist_frame_stride
   BoxGrid box;
   TileRec* tile_rec;           // [n_tiles] out: count / slot0 / frame of every tile
   unsigned long long* trace;   // debug: 8 clock64 stamps per tile, or null
@@ -95,7 +100,7 @@ struct VoxelParams {
                                      // no k_voxel_key_hist; radix pass 0 reads surv_key through the K1 tile records
   const uint32_t* surv_key;          // [slots]
   BoxGrid box;
-  uint32_t* first_k1;                // [sort tiles] K1 tile that holds dense position t * sort_tile (written by k_grid_setup)
+  uint32_t* first_k1;                // [sort tiles] K1 tile that holds the first key of radix tile t (written by k_grid_setup)
   uint32_t sort_tile;                // keys per tile of the radix passes of this run
   uint32_t dual_width;               // the key width is only known on the device (SortInfo.width): the host enqueues the
                                      // 32-bit AND the 64-bit instantiation of every kernel, the one that does not apply exits
@@ -123,7 +128,8 @@ cudaError_t launch_seed_bounds(FrameAcc* acc, const float* mn, const float* mx, 
 cudaError_t launch_grid_setup(const VoxelParams& p, cudaStream_t stream, TileRec* scan_rec = nullptr, uint32_t scan_tiles = 0,
                               const SegDev* segs = nullptr, uint32_t n_seg = 0, uint32_t* seg_surv_start = nullptr);
 cudaError_t launch_key_hist(const VoxelParams& p, cudaStream_t stream);
-cudaError_t launch_seg_base(const VoxelParams& p, cudaStream_t stream);  // segmented runs: between key_hist and the passes
+// segmented runs: between key_hist and the passes; fused-key runs with box.seg_sort: between pass 0 and pass 1 (passes 1..)
+cudaError_t launch_seg_base(const VoxelParams& p, cudaStream_t stream);
 // segmented runs sort bare voxel indices; this hands out (frame << idx_bits | idx) keys and the values as two arrays
 cudaError_t launch_seg_keys64(const void* records, unsigned long long* keys, uint32_t* vals, const VoxelParams& p,
                               cudaStream_t stream);

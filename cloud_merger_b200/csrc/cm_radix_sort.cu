@@ -3,7 +3,8 @@
 // Replaces the std::sort(index_vector) at the heart of pcl::VoxelGrid::applyFilter (PCL 1.8.1 voxel_grid.hpp, reached
 // from the reference's voxelgrid(), pc_preprocessing_main.cpp:168-177). No CUB / Thrust.
 //
-// One launch per 8-bit digit. The digit histograms of all passes were produced up front by k_voxel_key_hist, so a pass
+// One launch per digit (8 bits; the top digit of a fused-key run sorted frame by frame may take up to 384 values, see
+// sort_digit). The digit histograms of all passes were produced up front by k_voxel_key_hist, so a pass
 // is a single sweep: each CTA takes a tile, ranks its keys by digit (ballot-based match, stable), obtains for
 // each of the 256 digits the global position of its first key of that digit (chained scan; see "scanner CTAs"), and
 // scatters keys and values to their final place of this pass through shared memory so that global stores are
@@ -82,23 +83,25 @@ struct SortCfg<unsigned long long> {
 // its life waiting for its row). The running sum starts from the exclusive scan of the pass's global digit histogram
 // (row -1). Scanners are CTAs 0..7 of the grid, i.e. resident before any worker; workers publish their counts before
 // they wait, so the pair cannot deadlock.
-constexpr int RS_SCANNERS = 8;
-constexpr int RS_SCAN_DIGITS = CM_RADIX / RS_SCANNERS;  // 32: one digit per lane
+constexpr int RS_SCAN_DIGITS = 32;                      // one digit per lane
+constexpr int RS_SCANNERS = CM_RADIX / RS_SCAN_DIGITS;  // 8 (a pass of NB bins has NB / 32)
 constexpr int RS_SCAN_ROWS = 32;                        // rows per batch (one warp)
 constexpr int RS_SCAN_GROUP = RS_THREADS >= 512 ? 8 : 16;  // rows polled together (register budget of the CTA shape)
-static_assert(RS_SCAN_DIGITS == 32, "one digit per lane");
+static_assert(RS_THREADS >= (int)CM_WIDE_BINS, "one thread per digit of a wide pass is needed");
 
 //
 // SEG (frame-segmented sort): the tiles are frame-aligned and every frame is a sort of its own, so the running sum restarts
 // at the first tile of a frame from that frame's own first positions (seg_base: frame start + exclusive scan of the frame's
 // digit counts, prepared by k_seg_base); a worker on the first tile of a frame reads them itself and waits for nobody.
-template <bool SEG>
-__device__ __forceinline__ void scanner_cta(uint32_t scanner /* 0 .. RS_SCANNERS-1 */, unsigned long long* rows /* row 0 */,
+// NB: bins of the pass (256; CM_WIDE_BINS for the wide top digit of a SEG run): rows are NB words wide, NB / 32 scanners.
+template <bool SEG, int NB = CM_RADIX>
+__device__ __forceinline__ void scanner_cta(uint32_t scanner /* 0 .. NB/32-1 */, unsigned long long* rows /* row 0 */,
                                             uint32_t n_tiles, uint32_t epoch, const uint32_t* hist /* this pass */,
                                             uint32_t* err, uint32_t* s_scan, uint32_t* s_tmp /* >= 256 words */,
                                             unsigned long long* s_chain /* 32 */, const SegTile* __restrict__ seg_tile,
                                             const uint32_t* __restrict__ seg_base /* [frame][CM_SEG_PASSES][256], at this pass */) {
   const uint32_t tid = threadIdx.x, lane = tid & 31u, q = tid >> 5;
+  static_assert(SEG || NB == CM_RADIX, "a wide top digit is only ranked frame by frame");
   const uint32_t d = scanner * RS_SCAN_DIGITS + lane;  // digit
   if (SEG) {
     if (q == 0) s_chain[lane] = 0ull;  // sequence number 0; the value is never used (tile 0 starts a frame)
@@ -119,7 +122,7 @@ __device__ __forceinline__ void scanner_cta(uint32_t scanner /* 0 .. RS_SCANNERS
   volatile unsigned long long* chain = s_chain + lane;
   for (uint32_t b = q; b < n_batches; b += RS_WARPS) {
     const uint32_t r0 = b * RS_SCAN_ROWS;
-    unsigned long long* const base = rows + (size_t)r0 * CM_RADIX + d;
+    unsigned long long* const base = rows + (size_t)r0 * NB + d;
     uint32_t c[RS_SCAN_ROWS];
 #pragma unroll
     for (int g0 = 0; g0 < RS_SCAN_ROWS; g0 += RS_SCAN_GROUP) {
@@ -129,7 +132,7 @@ __device__ __forceinline__ void scanner_cta(uint32_t scanner /* 0 .. RS_SCANNERS
         unsigned long long w[RS_SCAN_GROUP];
 #pragma unroll
         for (int k = 0; k < RS_SCAN_GROUP; ++k)
-          w[k] = (r0 + g0 + k < n_tiles) ? ld_cg_u64(base + (size_t)(g0 + k) * CM_RADIX) : lb_pack(epoch, CM_LB_AGG, 0u);
+          w[k] = (r0 + g0 + k < n_tiles) ? ld_cg_u64(base + (size_t)(g0 + k) * NB) : lb_pack(epoch, CM_LB_AGG, 0u);
         bool all = true;
 #pragma unroll
         for (int k = 0; k < RS_SCAN_GROUP; ++k) {
@@ -184,18 +187,19 @@ __device__ __forceinline__ void scanner_cta(uint32_t scanner /* 0 .. RS_SCANNERS
 #pragma unroll
       for (int k = 0; k < RS_SCAN_ROWS; ++k)
         if (r0 + k < n_tiles)
-          st_cg_u64(base + (size_t)k * CM_RADIX, lb_pack(epoch, CM_LB_INCL, (uint32_t)k >= abs_from ? c[k] : run + c[k]));
+          st_cg_u64(base + (size_t)k * NB, lb_pack(epoch, CM_LB_INCL, (uint32_t)k >= abs_from ? c[k] : run + c[k]));
     } else {
       *chain = ((unsigned long long)(b + 1u) << 32) | (unsigned long long)(run + sum);
 #pragma unroll
       for (int k = 0; k < RS_SCAN_ROWS; ++k)
-        if (r0 + k < n_tiles) st_cg_u64(base + (size_t)k * CM_RADIX, lb_pack(epoch, CM_LB_INCL, run + c[k]));
+        if (r0 + k < n_tiles) st_cg_u64(base + (size_t)k * NB, lb_pack(epoch, CM_LB_INCL, run + c[k]));
     }
   }
 }
 
 // Which lanes of the warp hold a different value in bits 0..7 of x: bit j of the result is set iff lane j differs.
 // One ballot per bit; a lane whose bit is set complements the ballot, so the OR over bits marks the differing lanes.
+// (warp_diff<8> is this; warp_diff<9> takes one ballot more for a digit of up to 511.)
 __device__ __forceinline__ uint32_t warp_diff8(uint32_t x) {
   uint32_t t[8];
 #pragma unroll
@@ -213,6 +217,32 @@ __device__ __forceinline__ uint32_t warp_diff8(uint32_t x) {
   return a | c;
 }
 
+template <int BITS>
+__device__ __forceinline__ uint32_t warp_diff(uint32_t x) {
+  if constexpr (BITS == 8) {
+    return warp_diff8(x);
+  } else {
+    static_assert(BITS == 9, "8 or 9 digit bits");
+    const uint32_t t8 = warp_diff8(x);
+    uint32_t t;
+    asm volatile(
+        "{\n .reg .pred p;\n .reg .b32 y;\n and.b32 y, %1, %2;\n setp.ne.u32 p, y, 0;\n"
+        " vote.sync.ballot.b32 %0, p, 0xffffffff;\n @p not.b32 %0, %0;\n}"
+        : "=r"(t)
+        : "r"(x), "r"(1u << 8));
+    return t8 | t;
+  }
+}
+
+// The digit a pass ranks. 8-bit passes: bits shift .. shift+7 of the key. Wide top digit (NB = CM_WIDE_BINS, fused-key runs
+// sorted frame by frame): the box-grid index bits from shift up, clamped to NB - 1 -- the all-ones key that pads a partial tile
+// has 9 set index bits there (the plan takes a wide digit only for 9-bit ones), so it ranks last like digit 255 does.
+template <int NB, typename KeyT>
+__device__ __forceinline__ uint32_t sort_digit(KeyT k, uint32_t shift, uint32_t idx_mask) {
+  if constexpr (NB == CM_RADIX) return (uint32_t)(k >> shift) & (CM_RADIX - 1);
+  else return min(((uint32_t)k & idx_mask) >> shift, (uint32_t)NB - 1u);
+}
+
 __device__ __forceinline__ uint32_t lanemask_gt() {
   uint32_t m;
   asm("mov.u32 %0, %%lanemask_gt;" : "=r"(m));
@@ -221,37 +251,45 @@ __device__ __forceinline__ uint32_t lanemask_gt() {
 
 // Shared memory of one worker CTA. The sorted-tile buffers are double: a CTA ranks and places tile B while the scanners
 // are still producing the row that tile A (placed in the other buffer) needs for its scatter -- see the kernel.
-template <typename KeyT, int IPT>
+// NB: bins of the pass. WIDE_LATER: the FUSED0 pass of a run whose last pass ranks a wide digit (its counters overrun row 3).
+template <typename KeyT, int IPT, int NB = CM_RADIX, bool WIDE_LATER = false>
 struct SortSmem {
   static constexpr int TILE = RS_THREADS * IPT;
   static constexpr bool AOS = sizeof(KeyT) == 4;
+  static constexpr int LATER = 3 * CM_RADIX + (WIDE_LATER ? (int)CM_WIDE_BINS - CM_RADIX : 0);
   unsigned long long k[2][TILE];       // AOS: records (value << 32 | key); else keys
   uint32_t v[2][AOS ? 1 : TILE];       // values of 64-bit keys
-  uint32_t hist[RS_WARPS * CM_RADIX];  // per-warp digit counters, then per-warp first positions
-  uint32_t scatter[2][CM_RADIX];       // global position of sorted-tile position 0 of digit d
-  uint32_t scan[12];
-  uint32_t cnt[CM_RADIX];              // RS_EARLY_COUNT: the tile's digit counts, taken before the ranking
-  uint32_t later[3][CM_RADIX];         // FUSED0: digit counts of passes 1..3, taken while pass 0 holds the keys
+  uint32_t hist[RS_WARPS * NB];        // per-warp digit counters, then per-warp first positions
+  uint32_t scatter[2][NB];             // global position of sorted-tile position 0 of digit d
+  uint32_t scan[NB / 32 + 4];
+  uint32_t cnt[NB];                    // RS_EARLY_COUNT: the tile's digit counts, taken before the ranking
+  uint32_t later[LATER];               // FUSED0: digit counts of pass ps = 1..3 at (ps - 1) * 256, taken while pass 0 holds the keys
   uint32_t next_tile[2];               // written by thread 0 one iteration ahead (parity-indexed)
 };
 
 // FUSED0: pass 0 of a run whose keys were written by K1 at the survivors' slots (VoxelParams::fused_keys): the tile's keys
 // are read through the K1 tile records, the value of a key is the slot it was read from.
 // SEG: frame-segmented sort (see scanner_cta): tile t is seg_tile[t] -- a range of one frame -- instead of [t TILE, (t+1) TILE).
-template <typename KeyT, int IPT, bool FUSED0 = false, bool SEG = false>
+// FUSED0 && SEG: pass 0 of a fused-key run sorted frame by frame (BoxGrid::seg_sort); K1 counted the pass-0 digits per frame
+// and the later passes' digits are counted here per frame (seg_hist), turned into first positions by k_seg_base.
+// NB: bins of the pass -- 256, or CM_WIDE_BINS for the wide top digit of a fused-key SEG run (see sort_digit).
+template <typename KeyT, int IPT, bool FUSED0 = false, bool SEG = false, int NB = CM_RADIX>
 __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const VoxelParams p, const int pass) {
-  static_assert(!SEG || (sizeof(KeyT) == 4 && !FUSED0), "segmented keys are 32-bit records written by k_voxel_key_hist");
+  static_assert(!SEG || sizeof(KeyT) == 4, "segmented keys are 32-bit records");
+  static_assert(NB == CM_RADIX || (SEG && !FUSED0 && NB == (int)CM_WIDE_BINS), "a wide digit is the top digit of a SEG run");
   constexpr int TILE = RS_THREADS * IPT;
   constexpr int WARP_ITEMS = 32 * IPT;
   constexpr bool AOS = sizeof(KeyT) == 4;  // (key, value) records of 8 bytes
+  constexpr int SCANNERS = NB / RS_SCAN_DIGITS;
+  using Smem = SortSmem<KeyT, IPT, NB, FUSED0 && SEG>;
   extern __shared__ __align__(16) unsigned char s_raw[];
-  SortSmem<KeyT, IPT>& sm = *reinterpret_cast<SortSmem<KeyT, IPT>*>(s_raw);
+  Smem& sm = *reinterpret_cast<Smem*>(s_raw);
 
   const long long tr0 = clock64();
   const SortInfo si = *p.info;
   if ((uint32_t)pass >= si.num_passes) return;
   if (p.dual_width && ((si.width == 4u) != (sizeof(KeyT) == 4))) return;  // the other key width runs
-  if (SEG != (si.segmented != 0u)) return;
+  if (SEG != (si.seg_sort != 0u)) return;
   const uint32_t M = si.n_keys;
   const uint32_t n_tiles = SEG ? si.n_seg_tiles : (M + TILE - 1) / TILE;
   const uint32_t* const seg_base = SEG ? p.seg_hist + (size_t)pass * CM_RADIX : nullptr;
@@ -259,7 +297,7 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
   const uint32_t tid = threadIdx.x, lane = tid & 31u;
   const uint32_t warp = __shfl_sync(0xFFFFFFFFu, tid >> 5, 0);  // provably warp-uniform
   const uint32_t epoch = *p.epoch_dev + 1u + (uint32_t)pass;
-  unsigned long long* const rows = p.lb_sort + CM_RADIX;  // row -1 lives in front
+  unsigned long long* const rows = p.lb_sort + NB;  // row -1 lives in front
   uint32_t* const err = &p.ctrl->error;
   // Roles go by ARRIVAL, not by block index: the first RS_SCANNERS CTAs of the pass to start running are the scanners, so
   // the scanners are resident by construction whatever order the hardware dispatches CTAs in and whatever else shares the
@@ -269,13 +307,13 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
   if (tid == 0) {
     const uint32_t role = atomicAdd(&p.ctrl->role_counter[pass], 1u);
     sm.next_tile[1] = role;
-    if (role >= (uint32_t)RS_SCANNERS) sm.next_tile[0] = atomicAdd(counter, 1u);
+    if (role >= (uint32_t)SCANNERS) sm.next_tile[0] = atomicAdd(counter, 1u);
   }
   __syncthreads();
   const uint32_t role = sm.next_tile[1];
-  if (role < (uint32_t)RS_SCANNERS) {
+  if (role < (uint32_t)SCANNERS) {
     __syncthreads();  // every thread has read the role before the scanner reuses the shared memory
-    scanner_cta<SEG>(role, rows, n_tiles, epoch, p.hist + pass * CM_RADIX, err, sm.scan, sm.hist, &sm.k[0][0], p.seg_tile, seg_base);
+    scanner_cta<SEG, NB>(role, rows, n_tiles, epoch, p.hist + pass * CM_RADIX, err, sm.scan, sm.hist, &sm.k[0][0], p.seg_tile, seg_base);
     return;
   }
 
@@ -283,16 +321,28 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
   const bool odd = (pass & 1) != 0;
   const uint32_t shift = (uint32_t)pass * CM_RADIX_BITS;
   const uint32_t lt = lanemask_lt(), gt = lanemask_gt();
-  uint32_t* const wh = sm.hist + warp * CM_RADIX;  // the warp's own counter row
+  uint32_t* const wh = sm.hist + warp * NB;  // the warp's own counter row
+  // wide digit / FUSED0 && SEG: the box-grid index bits of the key (the frame bits above them are not ranked)
+  const uint32_t idx_mask = (NB > CM_RADIX || (FUSED0 && SEG)) ? (si.idx_bits >= 32u ? 0xFFFFFFFFu : (1u << si.idx_bits) - 1u) : 0u;
+  uint32_t hist_frame = 0xFFFFFFFFu;  // FUSED0 && SEG: the frame sm.later counts for
+  // FUSED0 && SEG: sm.later -> the frame's rows of seg_hist (passes 1..), fire-and-forget; cleared for the next frame
+  auto flush_later = [&]() {
+    if (hist_frame == 0xFFFFFFFFu) return;
+    uint32_t* dst = p.seg_hist + (size_t)hist_frame * (CM_SEG_PASSES * CM_RADIX) + CM_RADIX;
+    for (uint32_t i = tid; i < (uint32_t)Smem::LATER; i += RS_THREADS) {
+      const uint32_t c = sm.later[i];
+      if (c) { atomicAdd(dst + i, c); sm.later[i] = 0u; }
+    }
+  };
 
   // Tiles are handed out by an atomic counter (forward progress never depends on which CTAs are resident). A CTA works
   // on two tiles at a time, software-pipelined:  front(t1): load, rank, publish counts, place into buffer b1
   //                                              back(t0):  wait for row t0-1 from the scanners, scatter buffer b0
   // so the scanners' latency (poll + chain + store + our poll, ~4-6 thousand cycles) hides behind front(t1) instead of
   // idling a third of the SM's warps as it did when a CTA handled one tile from start to end.
-  if (RS_EARLY_COUNT && tid < CM_RADIX) sm.cnt[tid] = 0;
+  if (RS_EARLY_COUNT && tid < NB) sm.cnt[tid] = 0;
   if (FUSED0)
-    for (uint32_t i = tid; i < 3u * CM_RADIX; i += RS_THREADS) (&sm.later[0][0])[i] = 0u;
+    for (uint32_t i = tid; i < (uint32_t)Smem::LATER; i += RS_THREADS) sm.later[i] = 0u;
   uint32_t cur = sm.next_tile[0];
   __syncthreads();  // next_tile[1] (the role) is rewritten below; sm.cnt is cleared
   uint32_t prev = 0xFFFFFFFFu, prev_n = 0;
@@ -326,6 +376,11 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
         // Dense position d of the merged cropped cloud -> slot: K1 tile e holds positions [dense0_e, dense0_e + count_e) at slots
         // slot0_e + (d - dense0_e). Lane l of every warp holds the record of K1 tile first + l (a radix tile spans a handful
         // of K1 tiles); the tile of a position is the last one whose dense0 does not exceed it.
+        if (SEG && (cur_seg & ~CM_SEG_FIRST) != hist_frame) {  // CTA-uniform; the last tile's increments are done
+          flush_later();
+          hist_frame = cur_seg & ~CM_SEG_FIRST;
+          __syncthreads();
+        }
         const uint32_t k1_first = p.first_k1[cur];
         const uint32_t e = k1_first + lane;
         uint32_t e_dense = 0xFFFFFFFFu, e_slot = 0u, e_end = 0xFFFFFFFFu;
@@ -360,17 +415,33 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
             }
             slot = tdense[lo * 4u + 1u] + (d - tdense[lo * 4u + 3u]);
           }
-          const bool in = d < M;
+          const bool in = SEG ? item0 + 32 * i < n_here : d < M;
           key[i] = in ? (KeyT)p.surv_key[slot] : ~(KeyT)0;
           val[i] = in ? slot : 0u;
         }
         // K1 counted the digits of pass 0 only; the later passes' histograms are taken here, where every key passes once
+        if (SEG) {  // the frame's counts; the last pass ranks a wide digit when the plan says so
+          const uint32_t wide_pass = p.box.top_bins > CM_RADIX ? si.num_passes - 1u : 0u;
 #pragma unroll
-        for (int i = 0; i < IPT; ++i) {
-          if (tile_base + item0 + 32 * i < M) {
+          for (int i = 0; i < IPT; ++i) {
+            if (item0 + 32 * i < n_here) {
 #pragma unroll
-            for (uint32_t ps = 1; ps < 4; ++ps)
-              if (ps < si.num_passes) atomicAdd(&sm.later[ps - 1][((uint32_t)key[i] >> (ps * CM_RADIX_BITS)) & (CM_RADIX - 1)], 1u);
+              for (uint32_t ps = 1; ps < 3; ++ps)
+                if (ps < si.num_passes) {
+                  const uint32_t dg = ps == wide_pass ? sort_digit<(int)CM_WIDE_BINS>((uint32_t)key[i], ps * CM_RADIX_BITS, idx_mask)
+                                                      : sort_digit<CM_RADIX>((uint32_t)key[i], ps * CM_RADIX_BITS, 0u);
+                  atomicAdd(&sm.later[(ps - 1) * CM_RADIX + dg], 1u);
+                }
+            }
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < IPT; ++i) {
+            if (tile_base + item0 + 32 * i < M) {
+#pragma unroll
+              for (uint32_t ps = 1; ps < 4; ++ps)
+                if (ps < si.num_passes) atomicAdd(&sm.later[(ps - 1) * CM_RADIX + (((uint32_t)key[i] >> (ps * CM_RADIX_BITS)) & (CM_RADIX - 1))], 1u);
+            }
           }
         }
       } else if (AOS) {
@@ -407,20 +478,20 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
         }
       }
 #pragma unroll
-      for (int k = 0; k < CM_RADIX / 32; ++k) wh[lane + 32 * k] = 0;
+      for (int k = 0; k < NB / 32; ++k) wh[lane + 32 * k] = 0;
       __syncwarp();
       RS_TRACE(cur, 0, tr_cur);
       if (RS_EARLY_COUNT) {
         // The tile's digit counts go out before the (long) ranking: one hardware-aggregated shared-memory increment per
         // key (ATOMS.POPC.INC). The later a tile publishes, the longer every tile after it waits for its row.
 #pragma unroll
-        for (int i = 0; i < IPT; ++i) atomicAdd(&sm.cnt[(uint32_t)(key[i] >> shift) & (CM_RADIX - 1)], 1u);
+        for (int i = 0; i < IPT; ++i) atomicAdd(&sm.cnt[sort_digit<NB>(key[i], shift, idx_mask)], 1u);
         __syncthreads();
-        if (RS_THREADS == CM_RADIX || tid < CM_RADIX) {
+        if (RS_THREADS == NB || tid < NB) {
           const uint32_t c = sm.cnt[tid];
           sm.cnt[tid] = 0;  // for the next tile (no increments can follow in this iteration)
-          const uint32_t real = (tid == CM_RADIX - 1) ? c - ((uint32_t)TILE - n_here) : c;
-          st_relaxed_u64(rows + (size_t)cur * CM_RADIX + tid, lb_pack(epoch, CM_LB_AGG, real));
+          const uint32_t real = (tid == NB - 1) ? c - ((uint32_t)TILE - n_here) : c;
+          st_relaxed_u64(rows + (size_t)cur * NB + tid, lb_pack(epoch, CM_LB_AGG, real));
         }
       }
 
@@ -432,10 +503,17 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
       uint32_t rank[IPT];
 #pragma unroll
       for (int i = 0; i < IPT; ++i) {
-        const uint32_t ks = (uint32_t)(key[i] >> shift);
-        const uint32_t diff = warp_diff8(ks);
+        uint32_t ks, diff;
+        if constexpr (NB == CM_RADIX) {
+          ks = (uint32_t)(key[i] >> shift);
+          diff = warp_diff<8>(ks);
+          ks &= CM_RADIX - 1;
+        } else {
+          ks = sort_digit<NB>(key[i], shift, idx_mask);
+          diff = warp_diff<9>(ks);
+        }
         const uint32_t below = (uint32_t)__popc(~diff & lt);
-        volatile uint32_t* c = wh + (ks & (CM_RADIX - 1));
+        volatile uint32_t* c = wh + ks;
         const uint32_t r = *c + below;
         rank[i] = r;
         if ((~diff & gt) == 0u) *c = r + 1u;
@@ -446,28 +524,28 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
 
       // ---- per digit (one per thread): tile count -> published; prefix over digits and warps -> first positions -----
       {
-        const bool dt = RS_THREADS == CM_RADIX || tid < CM_RADIX;  // digit threads
+        const bool dt = RS_THREADS == NB || tid < NB;  // digit threads
         uint32_t wc[RS_WARPS];
         uint32_t cnt = 0;
         if (dt) {
 #pragma unroll
           for (int w = 0; w < RS_WARPS; ++w) {
-            wc[w] = sm.hist[w * CM_RADIX + tid];
+            wc[w] = sm.hist[w * NB + tid];
             cnt += wc[w];
           }
           if (!RS_EARLY_COUNT) {
-            const uint32_t real = (tid == CM_RADIX - 1) ? cnt - ((uint32_t)TILE - n_here) : cnt;
-            st_relaxed_u64(rows + (size_t)cur * CM_RADIX + tid, lb_pack(epoch, CM_LB_AGG, real));
+            const uint32_t real = (tid == NB - 1) ? cnt - ((uint32_t)TILE - n_here) : cnt;
+            st_relaxed_u64(rows + (size_t)cur * NB + tid, lb_pack(epoch, CM_LB_AGG, real));
           }
         }
         RS_TRACE(cur, 2, tr_cur);
         uint32_t tot;
-        const uint32_t bin_start = block_excl_scan_256(cnt, sm.scan, &tot);
+        const uint32_t bin_start = block_excl_scan<NB>(cnt, sm.scan, &tot);
         if (dt) {
           uint32_t run = bin_start;
 #pragma unroll
           for (int w = 0; w < RS_WARPS; ++w) {
-            sm.hist[w * CM_RADIX + tid] = run;
+            sm.hist[w * NB + tid] = run;
             run += wc[w];
           }
           sm.scatter[buf][tid] = 0u - bin_start;  // completed in back() once the scanners have delivered the row
@@ -479,8 +557,7 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
       // ---- keys and values into sorted-tile order in shared memory -------------------------------------------------
 #pragma unroll
       for (int i = 0; i < IPT; ++i) {
-        const uint32_t ks = (uint32_t)(key[i] >> shift);
-        const uint32_t pos = wh[ks & (CM_RADIX - 1)] + rank[i];
+        const uint32_t pos = wh[sort_digit<NB>(key[i], shift, idx_mask)] + rank[i];
         if (AOS) {
           sm.k[buf][pos] = ((unsigned long long)val[i] << 32) | (unsigned long long)key[i];
         } else {
@@ -495,12 +572,12 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
       const uint32_t pb = buf ^ 1u;
       RS_TRACE(prev, 7, tr_prev);
       // ---- one row from the scanners: where this tile's keys of digit d start in the output ----------------------
-      if (RS_THREADS == CM_RADIX || tid < CM_RADIX) {
+      if (RS_THREADS == NB || tid < NB) {
         uint32_t first;
         if (SEG && (prev_seg & CM_SEG_FIRST))  // first tile of its frame: the frame's own first positions, nobody to wait for
           first = __ldg(seg_base + (size_t)(prev_seg & ~CM_SEG_FIRST) * (CM_SEG_PASSES * CM_RADIX) + tid);
         else
-          first = lb_wait_inclusive(rows + ((long long)prev - 1) * CM_RADIX + tid, epoch, err);
+          first = lb_wait_inclusive(rows + ((long long)prev - 1) * NB + tid, epoch, err);
         sm.scatter[pb][tid] += first;  // modulo 2^32
       }
       __syncthreads();
@@ -521,13 +598,13 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
           for (int j = 0; j < IPT; ++j) r[j] = sk[j * RS_THREADS + tid];
 #pragma unroll
           for (int j = 0; j < IPT; ++j) {
-            const uint32_t dg = ((uint32_t)r[j] >> shift) & (CM_RADIX - 1);
+            const uint32_t dg = sort_digit<NB>((uint32_t)r[j], shift, idx_mask);
             out[ssc[dg] + (j * RS_THREADS + tid)] = r[j];
           }
         } else {
           for (uint32_t pos = tid; pos < prev_n; pos += RS_THREADS) {
             const unsigned long long r = sk[pos];
-            const uint32_t dg = ((uint32_t)r >> shift) & (CM_RADIX - 1);
+            const uint32_t dg = sort_digit<NB>((uint32_t)r, shift, idx_mask);
             out[ssc[dg] + pos] = r;
           }
         }
@@ -578,11 +655,15 @@ __global__ void __launch_bounds__(RS_THREADS, RS_MIN_CTAS) k_onesweep_pass(const
     __syncthreads();
     cur = sm.next_tile[buf];
   }
-  if (FUSED0) {  // this CTA's share of the histograms of passes 1.. (a persistent CTA flushes once)
+  if (FUSED0) {  // this CTA's share of the histograms of passes 1.. (a persistent CTA flushes once, SEG: per frame)
     __syncthreads();
-    for (uint32_t i = tid; i < 3u * CM_RADIX; i += RS_THREADS) {
-      const uint32_t c = (&sm.later[0][0])[i];
-      if (c && (i >> 8) + 1u < si.num_passes) atomicAdd(p.hist + CM_RADIX + i, c);
+    if (SEG) {
+      flush_later();
+    } else {
+      for (uint32_t i = tid; i < 3u * CM_RADIX; i += RS_THREADS) {
+        const uint32_t c = sm.later[i];
+        if (c && (i >> 8) + 1u < si.num_passes) atomicAdd(p.hist + CM_RADIX + i, c);
+      }
     }
   }
 }
@@ -625,7 +706,7 @@ uint32_t sort_tile_items(uint32_t key_bytes, uint32_t max_points) {
 }
 
 // rows of look-back words a workspace of `capacity` points needs (+1 for row -1, +1 spare)
-// (a frame-segmented sort needs one more row per frame: see ws_alloc)
+// (a frame-segmented sort needs one more row per frame, and a wide top digit rows of CM_WIDE_BINS words: see ws_alloc)
 size_t sort_lookback_rows(uint32_t capacity) {
   const uint32_t small_part = std::min(capacity, RS_SMALL_LIMIT);
   const size_t rows_small = small_part / (RS_THREADS * RS_IPT_SMALL) + 1;
@@ -634,23 +715,25 @@ size_t sort_lookback_rows(uint32_t capacity) {
 }
 
 namespace {
-template <typename KeyT, int IPT, bool FUSED0 = false, bool SEG = false>
+template <typename KeyT, int IPT, bool FUSED0 = false, bool SEG = false, int NB = CM_RADIX>
 struct PassLaunch {
+  using Smem = SortSmem<KeyT, IPT, NB, FUSED0 && SEG>;
+  static constexpr uint32_t SCANNERS = NB / RS_SCAN_DIGITS;
   static inline int ctas_per_sm = 0;
   static cudaError_t configure() {
-    cudaError_t e = cudaFuncSetAttribute(k_onesweep_pass<KeyT, IPT, FUSED0, SEG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)sizeof(SortSmem<KeyT, IPT>));
+    cudaError_t e = cudaFuncSetAttribute(k_onesweep_pass<KeyT, IPT, FUSED0, SEG, NB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)sizeof(Smem));
     if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, k_onesweep_pass<KeyT, IPT, FUSED0, SEG>, RS_THREADS,
-                                                         sizeof(SortSmem<KeyT, IPT>));
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, k_onesweep_pass<KeyT, IPT, FUSED0, SEG, NB>, RS_THREADS,
+                                                         sizeof(Smem));
   }
   static cudaError_t launch(const VoxelParams& p, int pass, int sms, cudaStream_t stream) {
     const uint32_t tile = RS_THREADS * IPT;
     const uint32_t tiles = (p.max_points + tile - 1) / tile + (SEG ? p.n_frames : 0u);  // SEG: a partial tile per frame
     if (tiles == 0) return cudaSuccess;
     // persistent workers: at most what the device holds at once (tiles are handed out by an atomic counter)
-    const uint32_t workers = std::min<uint32_t>(tiles, (uint32_t)(sms * std::max(1, ctas_per_sm)) - RS_SCANNERS);
-    k_onesweep_pass<KeyT, IPT, FUSED0, SEG><<<workers + RS_SCANNERS, RS_THREADS, sizeof(SortSmem<KeyT, IPT>), stream>>>(p, pass);
+    const uint32_t workers = std::min<uint32_t>(tiles, (uint32_t)(sms * std::max(1, ctas_per_sm)) - SCANNERS);
+    k_onesweep_pass<KeyT, IPT, FUSED0, SEG, NB><<<workers + SCANNERS, RS_THREADS, sizeof(Smem), stream>>>(p, pass);
     return cudaGetLastError();
   }
 };
@@ -667,12 +750,18 @@ cudaError_t configure_sort_kernels() {
   if (e == cudaSuccess) e = PassLaunch<uint32_t, RS_IPT_SMALL, true>::configure();
   if (e == cudaSuccess) e = PassLaunch<uint32_t, SortCfg<uint32_t>::IPT, false, true>::configure();
   if (e == cudaSuccess) e = PassLaunch<uint32_t, RS_IPT_SMALL, false, true>::configure();
+  if (e == cudaSuccess) e = PassLaunch<uint32_t, SortCfg<uint32_t>::IPT, true, true>::configure();
+  if (e == cudaSuccess) e = PassLaunch<uint32_t, RS_IPT_SMALL, true, true>::configure();
+  if (e == cudaSuccess) e = PassLaunch<uint32_t, SortCfg<uint32_t>::IPT, false, true, CM_WIDE_BINS>::configure();
+  if (e == cudaSuccess) e = PassLaunch<uint32_t, RS_IPT_SMALL, false, true, CM_WIDE_BINS>::configure();
   if (e != cudaSuccess) return e;
   if (getenv("CM_DEBUG"))
-    fprintf(stderr, "[cm] sort pass CTAs per SM: %d / %d (32 / 64-bit keys), small tile %d / %d\n",
+    fprintf(stderr, "[cm] sort pass CTAs per SM: %d / %d (32 / 64-bit keys), small tile %d / %d, wide top digit %d / %d\n",
             PassLaunch<uint32_t, SortCfg<uint32_t>::IPT>::ctas_per_sm,
             PassLaunch<unsigned long long, SortCfg<unsigned long long>::IPT>::ctas_per_sm,
-            PassLaunch<uint32_t, RS_IPT_SMALL>::ctas_per_sm, PassLaunch<unsigned long long, RS_IPT_SMALL>::ctas_per_sm);
+            PassLaunch<uint32_t, RS_IPT_SMALL>::ctas_per_sm, PassLaunch<unsigned long long, RS_IPT_SMALL>::ctas_per_sm,
+            PassLaunch<uint32_t, SortCfg<uint32_t>::IPT, false, true, CM_WIDE_BINS>::ctas_per_sm,
+            PassLaunch<uint32_t, RS_IPT_SMALL, false, true, CM_WIDE_BINS>::ctas_per_sm);
   g_sort_configured = true;
   return cudaSuccess;
 }
@@ -682,6 +771,17 @@ cudaError_t launch_sort_pass(const VoxelParams& p, int pass, cudaStream_t stream
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const bool small = sort_uses_small_tile(p.max_points);
+  if (p.fused_keys && p.box.seg_sort) {  // frame by frame, 32-bit keys; the last pass may rank a wide digit
+    constexpr int I = SortCfg<uint32_t>::IPT;
+    if (pass == 0)
+      return small ? PassLaunch<uint32_t, RS_IPT_SMALL, true, true>::launch(p, pass, sms, stream)
+                   : PassLaunch<uint32_t, I, true, true>::launch(p, pass, sms, stream);
+    if ((uint32_t)pass + 1u == p.box.n_pass && p.box.top_bins > CM_RADIX)
+      return small ? PassLaunch<uint32_t, RS_IPT_SMALL, false, true, CM_WIDE_BINS>::launch(p, pass, sms, stream)
+                   : PassLaunch<uint32_t, I, false, true, CM_WIDE_BINS>::launch(p, pass, sms, stream);
+    return small ? PassLaunch<uint32_t, RS_IPT_SMALL, false, true>::launch(p, pass, sms, stream)
+                 : PassLaunch<uint32_t, I, false, true>::launch(p, pass, sms, stream);
+  }
   if (p.fused_keys && pass == 0)  // 32-bit keys by construction
     return small ? PassLaunch<uint32_t, RS_IPT_SMALL, true>::launch(p, pass, sms, stream)
                  : PassLaunch<uint32_t, SortCfg<uint32_t>::IPT, true>::launch(p, pass, sms, stream);

@@ -418,11 +418,12 @@ __global__ void __launch_bounds__(THREADS, (THREADS >= 512 ? 2 : 4)) k_transform
     }
     pos += __popc(ballots[i]);
   }
-  if (KEYS) {  // this tile's digit counts -> the run's pass-0 histogram (fire-and-forget reductions; empty bins cost nothing)
+  if (KEYS) {  // this tile's digit counts -> the run's (or, frame by frame, the frame's) pass-0 histogram (fire-and-forget
+               // reductions; empty bins cost nothing)
     __syncthreads();
     if (tid < CM_RADIX) {
       const uint32_t c = s_hist[tid];
-      if (c) atomicAdd(p.hist + tid, c);
+      if (c) atomicAdd(p.hist + sg->frame * p.hist_frame_stride + tid, c);
     }
   }
   K1_TRACE(5);

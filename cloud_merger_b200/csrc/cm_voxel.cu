@@ -238,7 +238,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
   if (ts.rec) tile_scan_body(ts.rec, ts.n_tiles, ts.segs, ts.n_seg, p.n_frames, const_cast<uint32_t*>(p.frame_surv_start),
                              ts.seg_surv_start, s_scr);
   __syncthreads();
-  if (ts.rec && p.fused_keys) {
+  if (ts.rec && p.fused_keys && !p.box.seg_sort) {
     // which K1 tile holds the first key of every radix tile (pass 0 reads the keys where K1 left them): a K1 tile has at
     // most 4096 survivors, fewer than a radix tile, so at most one radix-tile boundary falls into it
     const unsigned long long T = p.sort_tile;
@@ -328,6 +328,8 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
     bool seg = p.segmented == 2u;
     if (p.segmented == 1u) seg = !has_invalid && idx_bits <= 32u;
     if (seg) frame_bits = 0u;
+    // a fused-key run planned frame by frame (BoxGrid::seg_sort) keeps its frame bits in the keys but ranks none of them
+    const bool fused_seg = p.fused_keys && p.box.seg_sort;
     uint32_t width = p.key_bytes;
     if (p.dual_width) width = p.segmented == 1u ? (seg ? 4u : 8u) : (frame_bits + idx_bits <= 32u ? 4u : 8u);
     uint32_t total = frame_bits + idx_bits;
@@ -336,7 +338,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
       total = width * 8u;
       idx_bits = total - frame_bits;
     }
-    uint32_t passes = (total + CM_RADIX_BITS - 1) / CM_RADIX_BITS;
+    uint32_t passes = fused_seg ? p.box.n_pass : (total + CM_RADIX_BITS - 1) / CM_RADIX_BITS;
     if (passes == 0) passes = 1;
     if (passes > p.max_passes) {  // the host enqueued fewer pass launches than the data needs
       atomicExch(&p.ctrl->error, (uint32_t)CM_DEV_E_KEY_RANGE);
@@ -351,10 +353,11 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
     si.width = width;
     si.segmented = seg ? 1u : 0u;
     si.n_seg_tiles = 0;
+    si.seg_sort = (seg || fused_seg) ? 1u : 0u;
     s_si = si;
   }
   __syncthreads();
-  if (s_si.segmented) {
+  if (s_si.seg_sort) {
     // the frame-aligned radix tiles: frame f owns ceil(n_f / T) consecutive tiles
     const uint32_t T = p.sort_tile, F = p.n_frames;
     uint32_t carry = 0;
@@ -381,8 +384,29 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_grid_setup(const VoxelParams p
         p.seg_tile[t0 + t] = st;
       }
     }
+    if (p.fused_keys) {
+      // which K1 tile holds the first key of every radix tile (a K1 tile lies in one frame and has fewer survivors than a
+      // radix tile, so at most one tile start of its frame falls into it) ...
+      for (uint32_t i = tid; i < ts.n_tiles; i += SCAN_THREADS) {
+        const TileRec r = ts.rec[i];
+        if (!r.count) continue;
+        const uint32_t fs = p.frame_surv_start[r.frame];
+        const uint32_t t = (r.dense0 - fs + T - 1u) / T;
+        if (fs + (unsigned long long)t * T < (unsigned long long)r.dense0 + r.count) p.first_k1[p.seg_frame_tile0[r.frame] + t] = i;
+      }
+      // ... and the frames' first positions of pass 0 from the digit counts K1 left in seg_hist (one warp per frame)
+      for (uint32_t f = warp; f < F; f += SCAN_THREADS / 32) {
+        uint32_t* h = p.seg_hist + (size_t)f * (CM_SEG_PASSES * CM_RADIX) + lane * 8u;
+        uint32_t c[8], sum = 0;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) { c[k] = h[k]; sum += c[k]; }
+        uint32_t run = p.frame_surv_start[f] + warp_incl_scan_u32(sum) - sum;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) { h[k] = run; run += c[k]; }
+      }
+    }
     // ... and which frames every tile of the centroid pass touches (nearly always one: no search per item there)
-    const uint32_t M = s_si.n_keys;
+    const uint32_t M = s_si.segmented ? s_si.n_keys : 0u;
     auto frame_from = [&](uint32_t i, uint32_t lo) {  // the last frame that starts at or before position i
       uint32_t hi = F - 1u;
       while (lo < hi) {
@@ -539,15 +563,20 @@ __global__ void __launch_bounds__(VX_THREADS) k_voxel_key_hist(const VoxelParams
 }
 
 // ---- segmented runs: per-frame digit counts -> where the frame's keys of digit d start in the output of pass ps ------------
-__global__ void __launch_bounds__(CM_RADIX) k_seg_base(const VoxelParams p) {
-  __shared__ uint32_t s_scan[12];
+// NB = CM_WIDE_BINS: a fused-key run sorted frame by frame -- passes 1.. only (k_grid_setup did pass 0), the last one of
+// box.top_bins digits.
+template <int NB>
+__global__ void __launch_bounds__(NB) k_seg_base(const VoxelParams p) {
+  __shared__ uint32_t s_scan[NB / 32 + 4];
   const SortInfo si = *p.info;
-  if (!si.segmented || blockIdx.y >= si.num_passes) return;
+  constexpr uint32_t first_pass = NB > CM_RADIX ? 1u : 0u;
+  if (!si.seg_sort || blockIdx.y < first_pass || blockIdx.y >= si.num_passes) return;
   const uint32_t f = blockIdx.x, tid = threadIdx.x;
   uint32_t* h = p.seg_hist + ((size_t)f * CM_SEG_PASSES + blockIdx.y) * CM_RADIX;
+  const uint32_t nb = (NB > CM_RADIX && blockIdx.y + 1u == si.num_passes) ? p.box.top_bins : CM_RADIX;
   uint32_t tot;
-  const uint32_t ex = block_excl_scan_256(h[tid], s_scan, &tot);
-  h[tid] = p.frame_surv_start[f] + ex;
+  const uint32_t ex = block_excl_scan<NB>(tid < nb ? h[tid] : 0u, s_scan, &tot);
+  if (tid < nb) h[tid] = p.frame_surv_start[f] + ex;
 }
 
 // segmented runs sort (idx, slot) records; callers of cm_get_device_out get (frame << idx_bits | idx) and the slots
@@ -1210,7 +1239,10 @@ cudaError_t launch_key_hist(const VoxelParams& p, cudaStream_t stream) {
 
 cudaError_t launch_seg_base(const VoxelParams& p, cudaStream_t stream) {
   if (p.n_frames == 0) return cudaSuccess;
-  k_seg_base<<<dim3(p.n_frames, CM_SEG_PASSES), CM_RADIX, 0, stream>>>(p);
+  if (p.fused_keys && p.box.seg_sort)
+    k_seg_base<CM_WIDE_BINS><<<dim3(p.n_frames, CM_SEG_PASSES), CM_WIDE_BINS, 0, stream>>>(p);
+  else
+    k_seg_base<CM_RADIX><<<dim3(p.n_frames, CM_SEG_PASSES), CM_RADIX, 0, stream>>>(p);
   return cudaGetLastError();
 }
 
