@@ -72,6 +72,16 @@ class CmSorStats(C.Structure):
 class CmSorOut(C.Structure):
     _fields_ = [("distances", C.c_void_p), ("n_points", C.c_int64), ("n_clouds", C.c_int32), ("reserved", C.c_int32),
                 ("knn_ms", C.c_float), ("sums_ms", C.c_float), ("cloud", CmSorStats * CM_MAX_ZONES)]
+
+
+class CmEcCfg(C.Structure):
+    _fields_ = [("tolerance", C.c_double), ("min_size", C.c_int32), ("max_size", C.c_int32)]
+
+
+class CmClusterOut(C.Structure):
+    _fields_ = [("xyzi", C.c_void_p), ("idx", C.c_void_p), ("begin", C.c_void_p), ("n_clusters", C.c_int64),
+                ("n_clustered", C.c_int64), ("n_unclustered", C.c_int64), ("cloud_clusters", C.c_int64 * CM_MAX_ZONES),
+                ("n_clouds", C.c_int32), ("host_syncs", C.c_int32), ("hook_ms", C.c_float), ("reserved", C.c_float)]
 CM_MAX_PROCEED_PARTS = 8
 
 
@@ -215,6 +225,15 @@ SYMBOLS = {
     "cm_statistical_outlier_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmSorCfg),
                                                C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
     "cm_get_statistical_out": (C.c_int, [_H, C.POINTER(CmSorOut)]),
+    "cm_dev_euclidean_clusters": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmEcCfg), C.c_void_p]),
+    "cm_dev_euclidean_clusters_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmEcCfg),
+                                                  C.c_void_p]),
+    "cm_get_cluster_out": (C.c_int, [_H, C.POINTER(CmClusterOut)]),
+    "cm_euclidean_clusters": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmEcCfg), C.c_void_p, C.c_void_p, C.c_int64,
+                                        C.POINTER(C.c_int64), C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "cm_euclidean_clusters_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmEcCfg), C.c_void_p,
+                                              C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.c_int64, C.POINTER(C.c_int64),
+                                              C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "cm_dev_plane_ransac": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmPlaneCfg), C.POINTER(CmPlane), C.c_void_p]),
     "cm_dev_plane_ransac_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmPlaneCfg),
                                             C.POINTER(CmPlane), C.c_void_p]),

@@ -343,6 +343,85 @@ class CloudMerger:
                                                            C.c_int64(n), ob))
         return [_part(ox, oi, ob[c], ob[c + 1], begin[c]) for c in range(k)]
 
+    # -- Euclidean cluster extraction (pcl::EuclideanClusterExtraction) ------------------------------------------------------
+    @staticmethod
+    def _ec_cfg(tolerance, min_size, max_size):
+        return _lib.CmEcCfg(float(tolerance), int(min_size), int(max_size))
+
+    def dev_euclidean_clusters(self, xyzi_ptr: int, n_points: int, tolerance: float, min_size: int = 1,
+                               max_size: int = 2 ** 31 - 1, stream: int = 0):
+        """Device form; fetch the clusters with euclidean_clusters_out()."""
+        cfg = self._ec_cfg(tolerance, min_size, max_size)
+        self._check(self._lib.cm_dev_euclidean_clusters(self._h, C.c_void_p(xyzi_ptr or None), C.c_int64(n_points),
+                                                        C.byref(cfg), C.c_void_p(stream or None)))
+
+    def dev_euclidean_clusters_multi(self, xyzi_ptr: int, begin, tolerance: float, min_size: int = 1,
+                                     max_size: int = 2 ** 31 - 1, stream: int = 0):
+        """Independent clouds [begin[k], begin[k+1]) of one device array in one pass (needs max_batch_frames >= the
+        number of clouds); fetch the clusters with euclidean_clusters_out()."""
+        b = (C.c_int64 * len(begin))(*[int(v) for v in begin])
+        cfg = self._ec_cfg(tolerance, min_size, max_size)
+        self._check(self._lib.cm_dev_euclidean_clusters_multi(self._h, C.c_void_p(xyzi_ptr or None), b, len(begin) - 1,
+                                                              C.byref(cfg), C.c_void_p(stream or None)))
+
+    def euclidean_clusters_out(self) -> dict:
+        """Of the last cluster extraction: "clusters", per cloud a list of index arrays (uint32, indices into the whole
+        input array, PCL's cluster order), "xyzi" (float32 [n_clustered, 4] in the same order), "begin" (int64 cluster
+        offsets), "n_unclustered", "host_syncs" and "hook_ms" (-1 unless profiling)."""
+        co = _lib.CmClusterOut()
+        self._check(self._lib.cm_get_cluster_out(self._h, C.byref(co)))
+        k, m = int(co.n_clusters), int(co.n_clustered)
+        begin = self.download(co.begin, np.int64, k + 1)
+        idx = self.download(co.idx, np.uint32, m) if m else np.zeros(0, np.uint32)
+        xyzi = self.download(co.xyzi, np.float32, 4 * m).reshape(-1, 4) if m else np.zeros((0, 4), np.float32)
+        return {"clusters": self._per_cloud(idx, begin, co.cloud_clusters[:co.n_clouds]), "xyzi": xyzi, "begin": begin,
+                "n_unclustered": int(co.n_unclustered), "host_syncs": int(co.host_syncs), "hook_ms": float(co.hook_ms)}
+
+    @staticmethod
+    def _per_cloud(idx, begin, cloud_clusters) -> list:
+        out, j = [], 0
+        for n in cloud_clusters:
+            out.append([idx[begin[j + q]:begin[j + q + 1]].copy() for q in range(int(n))])
+            j += int(n)
+        return out
+
+    def euclidean_clusters_multi(self, clouds, tolerance: float, min_size: int = 1, max_size: int = 2 ** 31 - 1,
+                                 with_xyzi: bool = False) -> list:
+        """Host-buffer form: per cloud a list of clusters, each an index array (uint32, into that cloud, ascending), in
+        PCL's order. with_xyzi: per cloud a list of (xyzi [m,4], idx) pairs instead."""
+        allpts, begin, b, (ox, oi) = _pack(clouds)
+        k, n = len(begin) - 1, len(allpts)
+        cb = np.zeros(n + 1, np.int64)
+        per = np.zeros(k, np.int64)
+        nc, npo = C.c_int64(), C.c_int64()
+        cfg = self._ec_cfg(tolerance, min_size, max_size)
+        self._check(self._lib.cm_euclidean_clusters_multi(
+            self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.byref(cfg), ox.ctypes.data_as(C.c_void_p),
+            oi.ctypes.data_as(C.c_void_p), C.c_int64(n), cb.ctypes.data_as(C.POINTER(C.c_int64)), C.c_int64(n),
+            per.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(nc), C.byref(npo)))
+        out, j = [], 0
+        for c in range(k):
+            cl = [_part(ox, oi, cb[j + q], cb[j + q + 1], begin[c]) for q in range(int(per[c]))]
+            out.append(cl if with_xyzi else [i for _, i in cl])
+            j += int(per[c])
+        return out
+
+    def euclidean_clusters(self, xyzi: np.ndarray, tolerance: float, min_size: int = 1, max_size: int = 2 ** 31 - 1,
+                           with_xyzi: bool = False) -> list:
+        """Host-buffer form for one cloud: a list of clusters, each an index array (uint32, ascending), in PCL's order."""
+        a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
+        n = len(a)
+        ox, oi = _outputs(n)
+        cb = np.zeros(n + 1, np.int64)
+        nc, npo = C.c_int64(), C.c_int64()
+        cfg = self._ec_cfg(tolerance, min_size, max_size)
+        self._check(self._lib.cm_euclidean_clusters(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(n), C.byref(cfg),
+                                                    ox.ctypes.data_as(C.c_void_p), oi.ctypes.data_as(C.c_void_p),
+                                                    C.c_int64(n), cb.ctypes.data_as(C.POINTER(C.c_int64)), C.c_int64(n),
+                                                    C.byref(nc), C.byref(npo)))
+        cl = [_part(ox, oi, cb[q], cb[q + 1]) for q in range(nc.value)]
+        return cl if with_xyzi else [i for _, i in cl]
+
     # -- RANSAC ground plane (pcl::SACSegmentation of removeGround, pc_preprocessing_main.cpp:95-117) ------------------------
     @staticmethod
     def _plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order):

@@ -230,6 +230,26 @@ struct cm_handle_s {
     uint32_t n_valid[CM_MAX_ZONES] = {};
     uint32_t too_few = 0;
   } sw;
+  // Euclidean cluster extraction (allocated on first use, grows)
+  struct EcWs {
+    size_t cap = 0;
+    DevPtr<float4> pts;            // [cap] the points in sorted key order, then the output coordinates
+    DevPtr<uint32_t> parent;       // [cap] union-find forest
+    DevPtr<uint32_t> label;        // [cap] every point's root
+    DevPtr<uint32_t> size;         // [cap] points per root, then the output rank per kept root
+    DevPtr<uint32_t> keys[2], vals[2];  // [cap] the output sort
+    DevPtr<uint32_t> perm;         // [cap] output rank per seed position, then the kept roots' sizes
+    DevPtr<uint32_t> counts;       // [256 * tiles] digit counts of the output sort
+    DevPtr<int64_t> begin;         // [cap + 1] cluster offsets
+    Event ev[2];                   // profiling: around the hook kernel
+    cudaStream_t stream = nullptr;
+    bool ran = false, profiled = false;
+    const uint32_t* idx = nullptr; // vals[passes & 1] of the last run
+    int n_clouds = 0;
+    int64_t n_clusters = 0, n_clustered = 0, n_points = 0, host_syncs = 0;
+    int64_t cloud_clusters[CM_MAX_ZONES] = {};
+    uint32_t device_error = 0;
+  } ew;
   // RANSAC ground plane (allocated on first use): one batch of draws and its scores, device + pinned mirrors
   struct PlaneWs {
     size_t cap_draws = 0;
@@ -2336,6 +2356,233 @@ int cm_get_statistical_out(cm_handle_t h, cm_sor_out_t* out) {
     o.sum_path = (int32_t)st.path;
   }
   return CM_OK;
+}
+
+// ---- Euclidean cluster extraction -----------------------------------------------------------------------------------------
+namespace {
+int ec_ws_ensure(cm_handle_t h, size_t points) {
+  cm_handle_s::EcWs& e = h->ew;
+  const size_t want = std::max<size_t>(points, 1);
+  if (e.cap >= want) return CM_OK;
+  e = cm_handle_s::EcWs();  // the old buffers go before the larger ones are allocated
+  CM_CUDA(h, dev_alloc(e.pts, want));
+  CM_CUDA(h, dev_alloc(e.parent, want));
+  CM_CUDA(h, dev_alloc(e.label, want));
+  CM_CUDA(h, dev_alloc(e.size, want));
+  for (int k = 0; k < 2; ++k) {
+    CM_CUDA(h, dev_alloc(e.keys[k], want));
+    CM_CUDA(h, dev_alloc(e.vals[k], want));
+  }
+  CM_CUDA(h, dev_alloc(e.perm, want));
+  CM_CUDA(h, dev_alloc(e.counts, (size_t)256 * ec_sort_tiles((uint32_t)want)));
+  CM_CUDA(h, dev_alloc(e.begin, want + 1));
+  for (auto& ev : e.ev) CM_CUDA(h, create(ev, cudaEventCreateWithFlags, cudaEventDefault));
+  e.cap = want;
+  return CM_OK;
+}
+
+// PCL's cluster order: the kept clusters of every cloud in seed order, then std::sort over reverse iterators with
+// comparePointClusters (size <). The sort is unstable; what it does with equal sizes depends only on the sequence of
+// sizes, so sorting (size, seed position) records with the same comparator reproduces it -- for libstdc++, the standard
+// library PCL is built with on Linux. perm[k] = output rank of seed position k; cb = cluster offsets in output order.
+void ec_order(const std::vector<uint32_t>& sizes, const uint32_t* cloud_first, int n_clouds, std::vector<uint32_t>& perm,
+              std::vector<int64_t>& cb) {
+  struct Rec { uint32_t size, pos; };
+  std::vector<Rec> recs(sizes.size());
+  for (size_t k = 0; k < sizes.size(); ++k) recs[k] = Rec{sizes[k], (uint32_t)k};
+  for (int c = 0; c < n_clouds; ++c)
+    std::sort(std::reverse_iterator<std::vector<Rec>::iterator>(recs.begin() + cloud_first[c + 1]),
+              std::reverse_iterator<std::vector<Rec>::iterator>(recs.begin() + cloud_first[c]),
+              [](const Rec& a, const Rec& b) { return a.size < b.size; });
+  perm.assign(recs.size(), 0);
+  cb.assign(recs.size() + 1, 0);
+  for (size_t r = 0; r < recs.size(); ++r) {
+    perm[recs[r].pos] = (uint32_t)r;
+    cb[r + 1] = cb[r] + recs[r].size;
+  }
+}
+
+// The clusters of every cloud [begin[k], begin[k+1]) into the handle's cluster outputs. The zone outputs carry the kept
+// roots on the way (zone k = the seeds of cloud k).
+int euclidean_clusters_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, const cm_ec_cfg_t* cfg,
+                           cudaStream_t st) {
+  if (!cfg) return fail(h, CM_E_INVALID, "cfg is NULL");
+  const float tf = (float)cfg->tolerance;
+  if (!(cfg->tolerance > 0.0) || !std::isfinite(cfg->tolerance) || !(tf > 0.0f) || std::isinf(tf))
+    return fail(h, CM_E_INVALID, "tolerance must be finite and > 0 (also as a float)");
+  if (cfg->min_size < 0 || cfg->max_size < 0) return fail(h, CM_E_INVALID, "min_size and max_size must be >= 0");
+  int rc = check_clouds(h, pts, begin, n_clouds, CM_MAX_ZONES);
+  if (rc != CM_OK) return rc;
+  const int64_t n_points = begin[n_clouds];
+  cm_handle_s::EcWs& e = h->ew;
+  e.ran = false;
+  VoxelParams vp;
+  rc = cell_keys_begin(h, pts, begin, n_clouds, vp, st);
+  if (rc != CM_OK) return rc;
+  rc = ec_ws_ensure(h, (size_t)n_points);
+  if (rc != CM_OK) return rc;
+  // the radius outlier removal's cells: two points closer than the tolerance are at most one cell apart on every axis
+  const float cell = tf * 1.00390625f;
+  rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  if (rc != CM_OK) return rc;
+  Workspace& w = h->batch;
+  RorParams rp{};
+  rc = enqueue_cell_table(h, vp, "CM_EC_NO_TABLE", rp, st);
+  if (rc != CM_OK) return rc;
+  EcParams ep{};
+  ep.pts = pts;
+  ep.sorted_pts = e.pts.get();
+  ep.cell_start = rp.cell_start;
+  // EuclideanClusterExtraction::extract narrows the tolerance to float; KdTreeFLANN::radiusSearch squares it in double
+  ep.r2 = (float)((double)tf * (double)tf);
+  ep.min_size = (uint32_t)cfg->min_size;
+  ep.max_size = (uint32_t)cfg->max_size;
+  ep.parent = e.parent.get();
+  ep.label = e.label.get();
+  ep.size = e.size.get();
+  ep.mask = h->zw.mask.get();
+  for (int c = 0; c <= CM_MAX_ZONES; ++c) ep.begin[c] = (uint32_t)begin[std::min(c, n_clouds)];
+  if (n_points) CM_CUDA(h, cudaMemsetAsync(e.size.get(), 0, (size_t)n_points * sizeof(uint32_t), st));
+  e.profiled = h->profiling;
+  if (e.profiled) CM_CUDA(h, cudaEventRecord(e.ev[0].get(), st));
+  CM_CUDA(h, launch_ec_hook(vp, ep, e.pts.get(), st));
+  if (e.profiled) CM_CUDA(h, cudaEventRecord(e.ev[1].get(), st));
+  CM_CUDA(h, launch_ec_roots(ep, (uint32_t)n_points, st));
+  if (n_points) w.launches += 4;
+  rc = zone_run(h, pts, n_points, st, true, n_clouds);
+  if (rc != CM_OK) return rc;
+  w.launches += h->zw.launches;
+  // round trip 1: the kept roots per cloud and the hook's verdict on the 2^14-cell bound
+  uint32_t* rep = h->zw.report.get();
+  CM_CUDA(h, cudaMemcpyAsync(rep + CM_MAX_ZONES + 2, &vp.ctrl->error, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  CM_CUDA(h, cudaStreamSynchronize(st));
+  e.host_syncs = 1;
+  e.device_error = rep[CM_MAX_ZONES + 2];
+  if (e.device_error == CM_DEV_E_KEY_RANGE)
+    return fail(h, CM_E_KEY_RANGE, "tolerance too small for the extent of a cloud (more than 2^14 cells from the origin)");
+  if (e.device_error) return fail(h, CM_E_INTERNAL, "device error %u", e.device_error);
+  uint32_t first[CM_MAX_ZONES + 1];
+  for (int c = 0; c <= n_clouds; ++c) first[c] = rep[c];
+  const uint32_t K = first[n_clouds];
+  // round trip 2: their sizes
+  std::vector<uint32_t> sizes(K);
+  if (K) {
+    CM_CUDA(h, launch_ec_sizes(ep, h->zw.out_src.get(), K, e.perm.get(), st));
+    ++w.launches;
+    CM_CUDA(h, cudaMemcpyAsync(sizes.data(), e.perm.get(), sizeof(uint32_t) * K, cudaMemcpyDeviceToHost, st));
+    CM_CUDA(h, cudaStreamSynchronize(st));
+    ++e.host_syncs;
+  }
+  std::vector<uint32_t> perm;
+  std::vector<int64_t> cb;
+  ec_order(sizes, first, n_clouds, perm, cb);
+  CM_CUDA(h, cudaMemcpyAsync(e.begin.get(), cb.data(), sizeof(int64_t) * (K + 1), cudaMemcpyHostToDevice, st));
+  EcOrder o{};
+  uint32_t bits = 0;
+  while (bits < 32 && (K >> bits) != 0u) ++bits;
+  o.passes = std::max<uint32_t>(1, (bits + 7) / 8);
+  if (K) {
+    CM_CUDA(h, cudaMemcpyAsync(e.perm.get(), perm.data(), sizeof(uint32_t) * K, cudaMemcpyHostToDevice, st));
+    o.roots = h->zw.out_src.get();
+    o.perm = e.perm.get();
+    o.n_clusters = K;
+    o.n_points_out = (uint32_t)cb[K];
+    o.rank = e.size.get();
+    for (int k = 0; k < 2; ++k) { o.keys[k] = e.keys[k].get(); o.vals[k] = e.vals[k].get(); }
+    o.counts = e.counts.get();
+    o.out_xyzi = e.pts.get();
+    cudaError_t err;
+    w.launches += launch_ec_order(ep, o, (uint32_t)n_points, st, &err);
+    CM_CUDA(h, err);
+  }
+  e.idx = e.vals[o.passes & 1u].get();
+  e.stream = st; e.n_clouds = n_clouds; e.n_points = n_points;
+  e.n_clusters = K; e.n_clustered = cb[K];
+  for (int c = 0; c < CM_MAX_ZONES; ++c) e.cloud_clusters[c] = c < n_clouds ? (int64_t)(first[c + 1] - first[c]) : 0;
+  e.ran = true;
+  return CM_OK;
+}
+
+int cluster_out_locked(cm_handle_t h, cm_cluster_out_t* out) {
+  cm_handle_s::EcWs& e = h->ew;
+  if (!e.ran) return fail(h, CM_E_INVALID, "no Euclidean cluster extraction has run on this handle");
+  CM_CUDA(h, cudaSetDevice(h->device));
+  CM_CUDA(h, cudaStreamSynchronize(e.stream));
+  memset(out, 0, sizeof(*out));
+  out->xyzi = reinterpret_cast<const float*>(e.pts.get());
+  out->idx = e.idx;
+  out->begin = e.begin.get();
+  out->n_clusters = e.n_clusters;
+  out->n_clustered = e.n_clustered;
+  out->n_unclustered = e.n_points - e.n_clustered;
+  out->n_clouds = e.n_clouds;
+  out->host_syncs = (int32_t)e.host_syncs;
+  for (int c = 0; c < CM_MAX_ZONES; ++c) out->cloud_clusters[c] = e.cloud_clusters[c];
+  out->hook_ms = -1.f;
+  if (e.profiled && cudaEventElapsedTime(&out->hook_ms, e.ev[0].get(), e.ev[1].get()) != cudaSuccess) {
+    out->hook_ms = -1.f;
+    cudaGetLastError();
+  }
+  return CM_OK;
+}
+}  // namespace
+
+int cm_dev_euclidean_clusters(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_ec_cfg_t* cfg, void* stream) {
+  const int64_t begin[2] = {0, n_points};
+  return cm_dev_euclidean_clusters_multi(h, xyzi_dev, begin, 1, cfg, stream);
+}
+
+int cm_dev_euclidean_clusters_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
+                                    const cm_ec_cfg_t* cfg, void* stream) {
+  if (!h || !begin) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  return euclidean_clusters_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, n_clouds, cfg,
+                                static_cast<cudaStream_t>(stream));
+}
+
+int cm_get_cluster_out(cm_handle_t h, cm_cluster_out_t* out) {
+  if (!h || !out) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  return cluster_out_locked(h, out);
+}
+
+int cm_euclidean_clusters_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds,
+                                const cm_ec_cfg_t* cfg, float* out_xyzi, uint32_t* out_idx, int64_t point_capacity,
+                                int64_t* out_cluster_begin, int64_t cluster_capacity, int64_t* out_cloud_clusters,
+                                int64_t* n_clusters, int64_t* n_points_out) {
+  if (!h || !begin || !n_clusters || !n_points_out) return CM_E_INVALID;
+  *n_clusters = 0; *n_points_out = 0;
+  if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  const float4* pts = nullptr;
+  int rc = stage_host_cloud(h, xyzi_host, begin[n_clouds], &pts);
+  if (rc == CM_OK) rc = euclidean_clusters_run(h, pts, begin, n_clouds, cfg, nullptr);
+  if (rc != CM_OK) return rc;
+  cm_cluster_out_t co;
+  rc = cluster_out_locked(h, &co);
+  if (rc != CM_OK) return rc;
+  *n_clusters = co.n_clusters; *n_points_out = co.n_clustered;
+  if (out_cloud_clusters)
+    for (int c = 0; c < n_clouds; ++c) out_cloud_clusters[c] = co.cloud_clusters[c];
+  if (co.n_clustered > point_capacity || co.n_clusters > cluster_capacity)
+    return fail(h, CM_E_CAPACITY, "%lld points in %lld clusters, caller capacity %lld points, %lld clusters",
+                (long long)co.n_clustered, (long long)co.n_clusters, (long long)point_capacity, (long long)cluster_capacity);
+  if (out_cluster_begin)
+    CM_CUDA(h, cudaMemcpy(out_cluster_begin, co.begin, sizeof(int64_t) * (size_t)(co.n_clusters + 1), cudaMemcpyDeviceToHost));
+  if (out_xyzi && co.n_clustered) CM_CUDA(h, cudaMemcpy(out_xyzi, co.xyzi, (size_t)co.n_clustered * 16, cudaMemcpyDeviceToHost));
+  if (out_idx && co.n_clustered) CM_CUDA(h, cudaMemcpy(out_idx, co.idx, (size_t)co.n_clustered * 4, cudaMemcpyDeviceToHost));
+  return CM_OK;
+}
+
+int cm_euclidean_clusters(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_ec_cfg_t* cfg, float* out_xyzi,
+                          uint32_t* out_idx, int64_t point_capacity, int64_t* out_cluster_begin, int64_t cluster_capacity,
+                          int64_t* n_clusters, int64_t* n_points_out) {
+  if (!h || n_points < 0) return CM_E_INVALID;
+  const int64_t begin[2] = {0, n_points};
+  return cm_euclidean_clusters_multi(h, xyzi_host, begin, 1, cfg, out_xyzi, out_idx, point_capacity, out_cluster_begin,
+                                     cluster_capacity, nullptr, n_clusters, n_points_out);
 }
 
 // ---- RANSAC ground plane --------------------------------------------------------------------------------------------------

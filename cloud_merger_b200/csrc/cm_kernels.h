@@ -217,6 +217,40 @@ cudaError_t launch_sor_knn(const VoxelParams& p, const SorParams& s, float4* sor
 cudaError_t launch_sor_sums(const SorSumParams& s, cudaStream_t stream);  // one CTA per cloud
 cudaError_t launch_sor_select(const SorSumParams& s, uint32_t n_points, cudaStream_t stream);
 
+// ---- Euclidean cluster extraction on the sorted cell keys (cm_cluster.cu) ----------------------------------------------------
+struct EcParams {
+  const float4* pts;           // [n_points] the input cloud(s)
+  const float4* sorted_pts;    // [M] the points in sorted key order (written by launch_ec_hook's gather)
+  const uint32_t* cell_start;  // k_ror_table's table of the cells' first sorted positions, or nullptr: binary searches
+  float r2;                    // (float)((double)tf * tf), tf = (float)tolerance: neighbours are strictly below it
+  uint32_t min_size, max_size;
+  uint32_t* parent;            // [n_points] union-find forest in input-index space (a root is its own parent)
+  uint32_t* label;             // [n_points] root of every finite point, 0xFFFFFFFF for the others
+  uint32_t* size;              // [n_points] points of every root (cleared by the caller)
+  unsigned short* mask;        // [n_points] zone mask: bit c on the kept roots of cloud c
+  uint32_t begin[CM_MAX_ZONES + 1];
+};
+struct EcOrder {               // the output of the kept clusters, after the host ordered them
+  const uint32_t* roots;       // [n_clusters] the kept roots in seed order
+  const uint32_t* perm;        // [n_clusters] output rank of the cluster at seed position k
+  uint32_t n_clusters;
+  uint32_t n_points_out;       // points of the kept clusters
+  uint32_t passes;             // 8-bit radix passes over the ranks 0 .. n_clusters
+  uint32_t* rank;              // [n_points] scratch: output rank of every kept root
+  uint32_t* keys[2];           // [n_points] ping-pong keys and values of the output sort
+  uint32_t* vals[2];           // vals[passes & 1]: the input indices in output order
+  uint32_t* counts;            // [256 * ec_sort_tiles(n_points)]
+  float4* out_xyzi;            // [n_points_out]
+};
+uint32_t ec_sort_tiles(uint32_t n_points);
+// gathers the points into sorted order and resets the forest (one launch), then unions every pair of neighbours (one launch)
+cudaError_t launch_ec_hook(const VoxelParams& p, const EcParams& e, float4* sorted_pts, cudaStream_t stream);
+// roots and sizes (one launch), then the kept roots' zone mask (one launch)
+cudaError_t launch_ec_roots(const EcParams& e, uint32_t n_points, cudaStream_t stream);
+cudaError_t launch_ec_sizes(const EcParams& e, const uint32_t* roots, uint32_t n_roots, uint32_t* out, cudaStream_t stream);
+// ranks, keys, 3 launches per radix pass, the coordinates; returns the number of launches
+int launch_ec_order(const EcParams& e, const EcOrder& o, uint32_t n_points, cudaStream_t stream, cudaError_t* err);
+
 // ---- RANSAC ground plane (cm_plane.cu) --------------------------------------------------------------------------------------
 #define CM_MAX_PLANE_CLOUDS (CM_MAX_ZONES / 2)
 struct PlaneParams {  // one batch of draws for up to CM_MAX_PLANE_CLOUDS independent clouds

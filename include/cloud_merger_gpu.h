@@ -450,6 +450,59 @@ CM_API int cm_statistical_outlier_multi(cm_handle_t h, const float* xyzi_host, c
                                         int64_t* out_begin);
 /* waits for the last statistical outlier removal on the handle; the device array stays valid until the next one */
 CM_API int cm_get_statistical_out(cm_handle_t h, cm_sor_out_t* out);
+/* Euclidean cluster extraction: pcl::EuclideanClusterExtraction<pcl::PointXYZI> with setClusterTolerance(tolerance),
+ * setMinClusterSize(min_size), setMaxClusterSize(max_size) and a KdTreeFLANN search (PCL 1.8.1 extract() and
+ * extractEuclideanClusters). Two points are neighbours iff their float squared distance (dx*dx + dy*dy) + dz*dz, each
+ * operation rounded on its own, is strictly below r2 = (float)((double)tf * (double)tf) with tf = (float)tolerance. A
+ * cluster is a connected component of that neighbour graph -- which is what PCL's seed-queue loop produces, DESIGN section
+ * 8 -- and is kept when min_size <= size <= max_size (PCL's defaults: 1 and INT_MAX; min_size > max_size keeps none). The
+ * indices inside a cluster are ascending. Cluster order: per cloud, the kept clusters in seed order (ascending smallest
+ * index), then std::sort(clusters.rbegin(), clusters.rend(), size <) as libstdc++ does it -- the order of a GCC-built PCL,
+ * where clusters of equal size come out in whatever order that unstable sort leaves them.
+ * Documented deviations: non-finite points belong to no cluster (a release build of PCL searches from them and may emit
+ * singleton clusters); several clouds in one call never share a cluster.
+ *  cm_dev_euclidean_clusters[_multi]: packed float4 xyzi points on the device, clouds as for the radius outlier removal
+ *      (cloud k = [begin[k], begin[k+1]), n_clouds <= CM_MAX_ZONES and <= max_batch_frames). Results through
+ *      cm_get_cluster_out: cloud 0's clusters, then cloud 1's, ... Uses the handle's batch workspace, and its zone outputs
+ *      (cm_get_zone_out) as scratch. A tolerance <= 0, NaN or infinite (also after the narrowing to float), or a negative
+ *      min_size / max_size -> CM_E_INVALID; CM_E_KEY_RANGE when the tolerance is too small for the extent of a cloud (the
+ *      cell grid exceeds the key range, or a point lies 2^14 cells or more from the origin). The call blocks until the
+ *      cluster sizes are known (two device round trips); the output itself is enqueued on `stream`.
+ *  cm_euclidean_clusters[_multi]: host buffers in and out. out_cluster_begin receives n_clusters + 1 offsets into out_xyzi /
+ *      out_idx (indices into the whole input array), out_cloud_clusters (may be NULL) the clusters of every cloud.
+ *      *n_clusters and *n_points_out always receive the totals; CM_E_CAPACITY when they exceed cluster_capacity or
+ *      point_capacity. */
+typedef struct {
+  double tolerance;   /* setClusterTolerance (metres) */
+  int32_t min_size;   /* setMinClusterSize */
+  int32_t max_size;   /* setMaxClusterSize */
+} cm_ec_cfg_t;
+/* device-resident result of the last cluster extraction on a handle (valid until the next one) */
+typedef struct {
+  const float* xyzi;                     /* device [n_clustered][4]: the points of cluster 0, then cluster 1, ... */
+  const uint32_t* idx;                   /* device [n_clustered]: index of every point in the input array */
+  const int64_t* begin;                  /* device [n_clusters + 1]: cluster j = [begin[j], begin[j+1]) */
+  int64_t n_clusters;
+  int64_t n_clustered;                   /* begin[n_clusters] */
+  int64_t n_unclustered;                 /* points in no kept cluster (non-finite ones included) */
+  int64_t cloud_clusters[CM_MAX_ZONES];  /* clusters of every cloud, in cloud order */
+  int32_t n_clouds;
+  int32_t host_syncs;                    /* device round trips of the call */
+  float hook_ms;                         /* GPU time of the neighbour unions (cm_set_profiling on; -1 otherwise) */
+  float reserved;
+} cm_cluster_out_t;
+CM_API int cm_dev_euclidean_clusters(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_ec_cfg_t* cfg,
+                                     void* stream);
+CM_API int cm_dev_euclidean_clusters_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
+                                           const cm_ec_cfg_t* cfg, void* stream);
+CM_API int cm_get_cluster_out(cm_handle_t h, cm_cluster_out_t* out);
+CM_API int cm_euclidean_clusters(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_ec_cfg_t* cfg,
+                                 float* out_xyzi, uint32_t* out_idx, int64_t point_capacity, int64_t* out_cluster_begin,
+                                 int64_t cluster_capacity, int64_t* n_clusters, int64_t* n_points_out);
+CM_API int cm_euclidean_clusters_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds,
+                                       const cm_ec_cfg_t* cfg, float* out_xyzi, uint32_t* out_idx, int64_t point_capacity,
+                                       int64_t* out_cluster_begin, int64_t cluster_capacity, int64_t* out_cloud_clusters,
+                                       int64_t* n_clusters, int64_t* n_points_out);
 /* RANSAC ground plane. Replaces the pcl::SACSegmentation + pcl::ExtractIndices block of removeGround()
  * (pc_preprocessing_main.cpp:95-117): SACMODEL_PLANE, SAC_RANSAC (setAxis / setEpsAngle are ignored by that model, as in
  * PCL). The three-index draws are PCL 1.8.1's -- boost::mt19937 seeded with cfg->seed, uniform_int<>(0, INT_MAX), the
@@ -596,7 +649,9 @@ CM_API int cm_get_frame_info(cm_handle_t h, cm_frame_info_t* out, int capacity, 
  * counted. After cm_[dev_]zone_split: the split (3, or 1 without points), plus 1 once cm_get_zone_out has repeated the
  * scatter into grown outputs. After cm_[dev_]plane_ransac[_multi]: the whole call, scoring rounds, refit sums, select and
  * compaction. After cm_[dev_]radius_outlier[_multi] and cm_[dev_]statistical_outlier[_multi]: the filter up to its mask,
- * without the compaction. After cm_dev_route_by_key: the mask kernel and the split. After cm_[dev_]proceed_zones: the
+ * without the compaction. After cm_[dev_]euclidean_clusters[_multi]: the whole call -- the cell-key front end, the gather
+ * and the unions, roots and kept-root mask, the compaction of the kept roots, and with kept clusters their sizes, ranks,
+ * keys, 3 launches per radix pass of the output sort and the coordinate gather. After cm_dev_route_by_key: the mask kernel and the split. After cm_[dev_]proceed_zones: the
  * radius outlier removal when a part removes ground, else the zone split. After cm_giant_voxelgrid: its local VoxelGrid. */
 CM_API int64_t cm_launch_count(cm_handle_t h);
 /* Device time (ms) of one named stage of the last run, measured with CUDA events on the run's stream:

@@ -40,6 +40,10 @@
 #include <pcl/point_types.h>
 #define CM_SHIM_HAVE_PCL 1
 #endif
+#if __has_include(<pcl/PointIndices.h>) && !defined(CM_SHIM_NO_PCL)
+#include <pcl/PointIndices.h>
+#define CM_SHIM_HAVE_PCL_INDICES 1
+#endif
 #endif
 
 // Optional adapters for the types either side of the path; each block compiles only where its header exists (ROS Melodic
@@ -274,6 +278,54 @@ class Context {
     std::vector<Cloud> res;
     if (!statistical_outlier_multi({&in}, res, mean_k, std_mul, negative, sqrt_mode)) return clear(out);
     out = res[0];
+    return true;
+  }
+
+  // Euclidean cluster extraction of several host clouds in one pass (cm_euclidean_clusters_multi; at most CM_MAX_ZONES
+  // clouds): pcl::EuclideanClusterExtraction with setClusterTolerance(tolerance), setMinClusterSize(min_size),
+  // setMaxClusterSize(max_size) on every cloud on its own. clusters[k] = the clusters of in[k] in PCL's order, each a list
+  // of ascending indices into in[k]. Non-finite points belong to no cluster.
+  bool euclidean_clusters_multi(const std::vector<const Cloud*>& in, std::vector<std::vector<std::vector<int>>>& clusters,
+                                double tolerance, int min_size, int max_size) {
+    const size_t k = in.size();
+    clusters.assign(k, std::vector<std::vector<int>>());
+    if (!check(h_ ? CM_OK : CM_E_NO_DEVICE)) return false;
+    std::vector<int64_t> begin(k + 1, 0);
+    for (size_t c = 0; c < k; ++c) begin[c + 1] = begin[c] + static_cast<int64_t>(in[c]->points.size());
+    const int64_t n = begin[k];
+    if (n > max_points_ * max_sensors_) { rc_ = CM_E_CAPACITY; err_ = "clouds larger than the context capacity"; return false; }
+    tmp_.resize(static_cast<size_t>(n) * 4 + 4);
+    for (size_t c = 0; c < k; ++c)
+      for (size_t i = 0; i < in[c]->points.size(); ++i) {
+        const PointXYZI& p = in[c]->points[i];
+        float* o = &tmp_[(static_cast<size_t>(begin[c]) + i) * 4];
+        o[0] = p.x; o[1] = p.y; o[2] = p.z; o[3] = p.intensity;
+      }
+    // every kept cluster holds at least one point: n points and n clusters always fit
+    std::vector<uint32_t> idx(static_cast<size_t>(n) + 1);
+    std::vector<int64_t> cb(static_cast<size_t>(n) + 1, 0), per(k, 0);
+    int64_t n_clusters = 0, n_out = 0;
+    cm_ec_cfg_t cfg{};
+    cfg.tolerance = tolerance; cfg.min_size = min_size; cfg.max_size = max_size;
+    if (!check(cm_euclidean_clusters_multi(h_, tmp_.data(), begin.data(), static_cast<int>(k), &cfg, nullptr, idx.data(), n,
+                                           cb.data(), n, per.data(), &n_clusters, &n_out)))
+      return false;
+    int64_t j = 0;
+    for (size_t c = 0; c < k; ++c)
+      for (int64_t q = 0; q < per[c]; ++q, ++j) {
+        std::vector<int> cl;
+        cl.reserve(static_cast<size_t>(cb[j + 1] - cb[j]));
+        for (int64_t t = cb[j]; t < cb[j + 1]; ++t) cl.push_back(static_cast<int>(idx[t] - begin[c]));
+        clusters[c].push_back(std::move(cl));
+      }
+    return true;
+  }
+  bool euclidean_clusters(const Cloud& in, std::vector<std::vector<int>>& clusters, double tolerance, int min_size = 1,
+                          int max_size = 2147483647) {
+    std::vector<std::vector<std::vector<int>>> res;
+    clusters.clear();
+    if (!euclidean_clusters_multi({&in}, res, tolerance, min_size, max_size)) return false;
+    clusters = std::move(res[0]);
     return true;
   }
 
@@ -614,6 +666,26 @@ inline void statisticalOutlierRemoval(Context& ctx, const Cloud::Ptr& cloud_ptr,
   ctx.statistical_outlier(*cloud_ptr, tmp, mean_k, std_mul);
   *cloud_ptr = tmp;
 }
+
+// pcl::EuclideanClusterExtraction<PointXYZI> (setClusterTolerance, setMinClusterSize, setMaxClusterSize; extract) on a cloud,
+// the step a node runs on its no-ground cloud to find objects: clusters in PCL's order, each a list of ascending indices.
+inline void extractEuclideanClusters(Context& ctx, const Cloud::Ptr& cloud_ptr, double tolerance, int min_size, int max_size,
+                                     std::vector<std::vector<int>>& clusters) {
+  ctx.euclidean_clusters(*cloud_ptr, clusters, tolerance, min_size, max_size);
+}
+#ifdef CM_SHIM_HAVE_PCL_INDICES
+// ... with extract()'s own output type
+inline void extractEuclideanClusters(Context& ctx, const Cloud::Ptr& cloud_ptr, double tolerance, int min_size, int max_size,
+                                     std::vector<pcl::PointIndices>& cluster_indices) {
+  std::vector<std::vector<int>> clusters;
+  ctx.euclidean_clusters(*cloud_ptr, clusters, tolerance, min_size, max_size);
+  cluster_indices.assign(clusters.size(), pcl::PointIndices());
+  for (size_t j = 0; j < clusters.size(); ++j) {
+    cluster_indices[j].header = cloud_ptr->header;
+    cluster_indices[j].indices = std::move(clusters[j]);
+  }
+}
+#endif
 
 // void removeGround(cloud, no_ground, ground, z_min_ground, z_max_ground, max_angle) -- :71-122, the whole function: the two
 // z windows (one zone-slicing pass), the RANSAC plane on the lower one + ExtractIndices, outlierRemoval of what is not
