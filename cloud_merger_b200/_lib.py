@@ -43,16 +43,23 @@ class CmZoneOut(C.Structure):
 
 class CmPlaneCfg(C.Structure):
     _fields_ = [("distance_threshold", C.c_double), ("probability", C.c_double), ("max_iterations", C.c_int32),
-                ("optimize", C.c_int32), ("seed", C.c_uint32), ("sum_order", C.c_int32)]
+                ("optimize", C.c_int32), ("seed", C.c_uint32), ("sum_order", C.c_int32), ("model", C.c_int32),
+                ("axis", C.c_float * 3), ("eps_angle", C.c_double)]
 
 
 class CmPlane(C.Structure):
     _fields_ = [("found", C.c_int32), ("iterations", C.c_int32), ("draws", C.c_int32), ("best_count", C.c_int32),
-                ("sample", C.c_int32 * 3), ("reserved", C.c_int32), ("coeff_ransac", C.c_float * 4),
+                ("sample", C.c_int32 * 3), ("rejected", C.c_int32), ("coeff_ransac", C.c_float * 4),
                 ("coeff", C.c_float * 4), ("n_inliers", C.c_int64)]
 
 
 CM_SUM4_SSE2, CM_SUM4_SSE3, CM_SUM4_SCALAR = 0, 1, 2
+CM_SAC_PLANE, CM_SAC_PERPENDICULAR_PLANE, CM_SAC_PARALLEL_PLANE = 0, 1, 2
+
+
+class CmPlaneAxisRule(C.Structure):
+    _fields_ = [("test", C.c_int32), ("c_neg", C.c_float), ("c_pos", C.c_float), ("f_plus", C.c_float),
+                ("axis", C.c_float * 4)]
 
 CM_SOR_MAX_K = 127
 CM_SOR_SQRT_FLOAT, CM_SOR_SQRT_DOUBLE = 0, 1
@@ -241,6 +248,7 @@ SYMBOLS = {
                                         C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
     "cm_plane_ransac": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmPlaneCfg), C.POINTER(CmPlane), C.c_void_p,
                                   C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
+    "cm_plane_axis_rule": (C.c_int, [C.POINTER(CmPlaneCfg), C.POINTER(CmPlaneAxisRule)]),
     "cm_dev_proceed_zones": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmProceedCfg), C.POINTER(CmProceedOut), C.c_void_p]),
     "cm_proceed_zones": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmProceedCfg), C.c_void_p, C.c_int64, C.POINTER(C.c_int64),
                                    C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.POINTER(CmPlane)]),

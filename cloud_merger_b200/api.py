@@ -424,22 +424,38 @@ class CloudMerger:
 
     # -- RANSAC ground plane (pcl::SACSegmentation of removeGround, pc_preprocessing_main.cpp:95-117) ------------------------
     @staticmethod
-    def _plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order):
+    def _plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model=0, axis=(0.0, 0.0, 1.0),
+                   eps_angle=0.0):
+        """model: CM_SAC_PLANE (0, the reference's; axis and eps_angle unused), CM_SAC_PERPENDICULAR_PLANE (1: normal
+        within eps_angle [rad] of axis) or CM_SAC_PARALLEL_PLANE (2: normal within eps_angle of perpendicular to axis)."""
+        ax = (C.c_float * 3)(*[float(np.float32(v)) for v in axis])
         return _lib.CmPlaneCfg(float(distance_threshold), float(probability), int(max_iterations), int(bool(optimize)),
-                               int(seed), int(sum_order))
+                               int(seed), int(sum_order), int(model), ax, float(eps_angle))
+
+    @staticmethod
+    def plane_axis_rule(model: int, axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0, sum_order: int = 0) -> dict:
+        """The float form of the axis test the plane search applies (cm_plane_axis_rule): test (0 none, 1 perpendicular,
+        2 parallel), the cutoffs c_neg / c_pos / f_plus and the normalized axis."""
+        cfg = CloudMerger._plane_cfg(0.3, 0.99, 1000, True, 12345, sum_order, model, axis, eps_angle)
+        r = _lib.CmPlaneAxisRule()
+        rc = _lib.load().cm_plane_axis_rule(C.byref(cfg), C.byref(r))
+        if rc != _lib.CM_OK:
+            raise CloudMergerError(rc, "cm_plane_axis_rule failed")
+        return {"test": int(r.test), "c_neg": np.float32(r.c_neg), "c_pos": np.float32(r.c_pos),
+                "f_plus": np.float32(r.f_plus), "axis": np.array(r.axis, np.float32)}
 
     @staticmethod
     def _plane_dict(pl) -> dict:
         return {"found": bool(pl.found), "iterations": int(pl.iterations), "draws": int(pl.draws),
-                "best_count": int(pl.best_count), "sample": np.array(pl.sample, np.int32),
+                "best_count": int(pl.best_count), "rejected": int(pl.rejected), "sample": np.array(pl.sample, np.int32),
                 "coeff_ransac": np.array(pl.coeff_ransac, np.float32), "coeff": np.array(pl.coeff, np.float32),
                 "n_inliers": int(pl.n_inliers)}
 
     def dev_plane_ransac(self, xyzi_ptr: int, n_points: int, distance_threshold: float, probability: float = 0.99,
                          max_iterations: int = 1000, optimize: bool = True, seed: int = 12345, sum_order: int = 0,
-                         stream: int = 0) -> dict:
+                         stream: int = 0, model: int = 0, axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0) -> dict:
         """Device form; the ground / no-ground clouds are zones 0 / 1 of zone_out()."""
-        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
+        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model, axis, eps_angle)
         pl = _lib.CmPlane()
         self._check(self._lib.cm_dev_plane_ransac(self._h, C.c_void_p(xyzi_ptr or None), C.c_int64(n_points), C.byref(cfg),
                                                   C.byref(pl), C.c_void_p(stream or None)))
@@ -447,24 +463,25 @@ class CloudMerger:
 
     def dev_plane_ransac_multi(self, xyzi_ptr: int, begin, distance_threshold: float, probability: float = 0.99,
                                max_iterations: int = 1000, optimize: bool = True, seed: int = 12345, sum_order: int = 0,
-                               stream: int = 0) -> list:
+                               stream: int = 0, model: int = 0, axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0) -> list:
         """Independent plane searches over the consecutive clouds [begin[k], begin[k+1]) of one device array in one pass;
         zone_out() then holds zone 2k = inliers of cloud k, zone 2k + 1 = its other points."""
         b = (C.c_int64 * len(begin))(*[int(v) for v in begin])
         k = len(begin) - 1
-        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
+        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model, axis, eps_angle)
         pl = (_lib.CmPlane * max(k, 1))()
         self._check(self._lib.cm_dev_plane_ransac_multi(self._h, C.c_void_p(xyzi_ptr or None), b, k, C.byref(cfg), pl,
                                                         C.c_void_p(stream or None)))
         return [self._plane_dict(pl[i]) for i in range(k)]
 
     def plane_ransac_multi(self, clouds, distance_threshold: float, probability: float = 0.99, max_iterations: int = 1000,
-                           optimize: bool = True, seed: int = 12345, sum_order: int = 0) -> list:
+                           optimize: bool = True, seed: int = 12345, sum_order: int = 0, model: int = 0,
+                           axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0) -> list:
         """Host-buffer form of dev_plane_ransac_multi: one dict per cloud with "ground" / "rest" as in plane_ransac
         (indices relative to the cloud)."""
         allpts, begin, b, (ox, oi) = _pack(clouds)
         k, n = len(begin) - 1, len(allpts)
-        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
+        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model, axis, eps_angle)
         pl = (_lib.CmPlane * max(k, 1))()
         ob = (C.c_int64 * (2 * k + 1))()
         self._check(self._lib.cm_plane_ransac_multi(self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.byref(cfg), pl,
@@ -478,11 +495,12 @@ class CloudMerger:
         return res
 
     def plane_ransac(self, xyzi: np.ndarray, distance_threshold: float, probability: float = 0.99,
-                     max_iterations: int = 1000, optimize: bool = True, seed: int = 12345, sum_order: int = 0) -> dict:
+                     max_iterations: int = 1000, optimize: bool = True, seed: int = 12345, sum_order: int = 0,
+                     model: int = 0, axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0) -> dict:
         """Host-buffer form. Adds "ground" and "rest": (xyzi [k,4] float32, idx [k] uint32 into the input, ascending)."""
         a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
         n = len(a)
-        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
+        cfg = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model, axis, eps_angle)
         pl = _lib.CmPlane()
         ox, oi = _outputs(n)
         begin = (C.c_int64 * 3)()
@@ -495,7 +513,7 @@ class CloudMerger:
 
     # -- the body of a proceedX in one call (pc_preprocessing_main.cpp:228-312, :428-446, :474-497) ---------------------------
     def _proceed_cfg(self, parts, roi_z_max, radius, min_neighbors, distance_threshold, probability, max_iterations, optimize,
-                     seed, sum_order):
+                     seed, sum_order, model=0, axis=(0.0, 0.0, 1.0), eps_angle=0.0):
         """parts: (length, deviation, z_max_ground) for a ground-removal part, (length, deviation, None) for a plain one."""
         cfg = _lib.CmProceedCfg()
         cfg.n_parts = len(parts)
@@ -506,16 +524,17 @@ class CloudMerger:
                                              float(np.float32(0.0 if zg is None else zg)), 0 if zg is None else 1)
         cfg.roi_z_max = float(np.float32(roi_z_max))
         cfg.radius = float(radius)
-        cfg.plane = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order)
+        cfg.plane = self._plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model, axis,
+                                    eps_angle)
         return cfg
 
     def dev_proceed_zones(self, roi_ptr: int, n_points: int, parts, roi_z_max: float = 3.0, radius: float = 0.15,
                           min_neighbors: int = 1, distance_threshold: float = 0.3, probability: float = 0.99,
                           max_iterations: int = 1000, optimize: bool = True, seed: int = 12345, sum_order: int = 0,
-                          stream: int = 0) -> dict:
+                          stream: int = 0, model: int = 0, axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0) -> dict:
         """Device form: the ROI cloud at roi_ptr -> no-ground / ground clouds in device memory (pointers + sizes)."""
         cfg = self._proceed_cfg(parts, roi_z_max, radius, min_neighbors, distance_threshold, probability, max_iterations,
-                                optimize, seed, sum_order)
+                                optimize, seed, sum_order, model, axis, eps_angle)
         po = _lib.CmProceedOut()
         self._check(self._lib.cm_dev_proceed_zones(self._h, C.c_void_p(roi_ptr or None), C.c_int64(n_points), C.byref(cfg),
                                                    C.byref(po), C.c_void_p(stream or None)))
@@ -525,12 +544,13 @@ class CloudMerger:
 
     def proceed_zones(self, roi_xyzi: np.ndarray, parts, roi_z_max: float = 3.0, radius: float = 0.15, min_neighbors: int = 1,
                       distance_threshold: float = 0.3, probability: float = 0.99, max_iterations: int = 1000,
-                      optimize: bool = True, seed: int = 12345, sum_order: int = 0) -> dict:
+                      optimize: bool = True, seed: int = 12345, sum_order: int = 0, model: int = 0,
+                      axis=(0.0, 0.0, 1.0), eps_angle: float = 0.0) -> dict:
         """Host-buffer form: (no_ground [n,4], ground [m,4], planes)."""
         a = np.ascontiguousarray(roi_xyzi, np.float32).reshape(-1, 4)
         n = len(a)
         cfg = self._proceed_cfg(parts, roi_z_max, radius, min_neighbors, distance_threshold, probability, max_iterations,
-                                optimize, seed, sum_order)
+                                optimize, seed, sum_order, model, axis, eps_angle)
         cap = 2 * max(n, 1)
         ng, g = np.empty((cap, 4), np.float32), np.empty((cap, 4), np.float32)
         n_ng, n_g = C.c_int64(), C.c_int64()

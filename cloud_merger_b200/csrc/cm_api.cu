@@ -2650,6 +2650,83 @@ float sum4_host(float l0, float l1, float l2, float l3, int order) {
   return ((l0 + l1) + l2) + l3;
 }
 
+// Eigen 3.3 normalize() of a Vector4f: divides only when the squared norm is positive
+void normalize4_host(float* v, int order) {
+  const float z = sum4_host(v[0] * v[0], v[1] * v[1], v[2] * v[2], v[3] * v[3], order);
+  if (z > 0.0f) {
+    const float nrm = std::sqrt(z);
+    for (int i = 0; i < 4; ++i) v[i] = v[i] / nrm;
+  }
+}
+
+float f32_bits(uint32_t u) {
+  float f;
+  memcpy(&f, &u, sizeof(f));
+  return f;
+}
+
+// SampleConsensusModelPerpendicularPlane::isModelValid as PCL 1.8.1 evaluates it on the float d = dot(axis, normal):
+// getAngle3D widens d to double, clamps it to [-1, 1] and takes acos; the model is invalid iff min(angle, pi - angle) > eps
+bool perpendicular_valid_f64(float d, double eps) {
+  double rad = (double)d;
+  if (rad < -1.0) rad = -1.0;
+  else if (rad > 1.0) rad = 1.0;
+  const double angle = std::fabs(std::acos(rad));
+  return !(std::min(angle, M_PI - angle) > eps);
+}
+
+// the first float bit pattern in [lo, hi] (one sign, magnitudes growing with the pattern) that passes, given that hi does
+uint32_t first_valid_bits(uint32_t lo, uint32_t hi, double eps) {
+  if (perpendicular_valid_f64(f32_bits(lo), eps)) return lo;
+  while (hi - lo > 1) {
+    const uint32_t mid = lo + (hi - lo) / 2;
+    if (perpendicular_valid_f64(f32_bits(mid), eps)) hi = mid;
+    else lo = mid;
+  }
+  return hi;
+}
+
+// The axis test of cfg as float cutoffs (PlaneAxisRule), once per call. PERPENDICULAR: the double predicate above is
+// monotone in |d| on each side of 0 (|d| = 1 always passes), so bisecting over the float bit patterns of [0, 1] and
+// [-0, -1] finds the cutoffs; each is checked against its float neighbours. PARALLEL: PCL compares fabs(d) with the double
+// sin_angle_ = |sin(eps)|: |d| > sin_angle_ iff |d| >= the smallest float above it.
+int plane_axis_rule(const cm_plane_cfg_t& cfg, PlaneAxisRule* r) {
+  if (cfg.model < CM_SAC_PLANE || cfg.model > CM_SAC_PARALLEL_PLANE || cfg.sum_order < 0 || cfg.sum_order > 2) return CM_E_INVALID;
+  *r = PlaneAxisRule{};
+  float a[4] = {cfg.axis[0], cfg.axis[1], cfg.axis[2], 0.0f};
+  normalize4_host(a, cfg.sum_order);  // PERPENDICULAR: in getAngle3D; PARALLEL: in setAxis (a zero axis stays zero)
+  r->axis = make_float4(a[0], a[1], a[2], a[3]);
+  if (cfg.model == CM_SAC_PLANE || !(cfg.eps_angle > 0.0)) return CM_OK;  // isModelValid tests only when eps_angle_ > 0
+  if (cfg.model == CM_SAC_PARALLEL_PLANE) {
+    const double sin_angle = std::fabs(std::sin(cfg.eps_angle));
+    float f = (float)sin_angle;
+    if ((double)f <= sin_angle) f = std::nextafter(f, std::numeric_limits<float>::infinity());
+    r->test = CM_SAC_PARALLEL_PLANE;
+    r->f_plus = f;
+    return CM_OK;
+  }
+  const uint32_t pos = first_valid_bits(0x00000000u, 0x3f800000u, cfg.eps_angle);
+  const uint32_t neg = first_valid_bits(0x80000000u, 0xbf800000u, cfg.eps_angle);
+  for (const uint32_t u : {pos, neg}) {
+    const bool edge_ok = perpendicular_valid_f64(f32_bits(u), cfg.eps_angle) && perpendicular_valid_f64(f32_bits(u + 1), cfg.eps_angle) &&
+                         ((u & 0x7fffffffu) == 0 || !perpendicular_valid_f64(f32_bits(u - 1), cfg.eps_angle));
+    if (!edge_ok) return CM_E_INTERNAL;
+  }
+  if (pos == 0x00000000u && neg == 0x80000000u) return CM_OK;  // eps >= pi / 2: every plane passes
+  r->test = CM_SAC_PERPENDICULAR_PLANE;
+  r->c_pos = f32_bits(pos);
+  r->c_neg = f32_bits(neg);
+  return CM_OK;
+}
+
+// d of the axis test for a model on the host (the refitted one), in the operations k_plane_score uses
+float plane_axis_dot(const PlaneAxisRule& r, const float* coeff, int order) {
+  float m[4] = {coeff[0], coeff[1], coeff[2], 0.0f};
+  normalize4_host(m, order);
+  if (r.test == CM_SAC_PERPENDICULAR_PLANE) normalize4_host(m, order);
+  return sum4_host(r.axis.x * m[0], r.axis.y * m[1], r.axis.z * m[2], r.axis.w * m[3], order);
+}
+
 // pcl::computeRoots2 (common/impl/eigen.hpp): roots of x^2 - b x + c, with the zero root in front
 void plane_roots2(float b, float c, float* roots) {
   roots[0] = 0.0f;
@@ -2731,7 +2808,7 @@ struct PlaneSearch {
   int iterations = 0, draws = 0, bad_run = 0;
   long long best = -(long long)std::numeric_limits<int>::max();
   double k = 1.0, one_over_indices = 0.0;
-  bool stop = false, found = false;
+  bool stop = false, found = false, best_valid = false;
   bool running() const { return n >= 3 && !stop && iterations < k; }
 };
 
@@ -2743,6 +2820,10 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
   const int64_t n_points = begin[n_clouds];
   if (n_points > 0x7FFFFFF0ll) return fail(h, CM_E_INVALID, "bad n_points");
   if (cfg.max_iterations < 0 || cfg.sum_order < 0 || cfg.sum_order > 2) return fail(h, CM_E_INVALID, "bad plane settings");
+  PlaneAxisRule axis_rule;
+  rc = plane_axis_rule(cfg, &axis_rule);
+  if (rc == CM_E_INVALID) return fail(h, rc, "unknown plane model %d", cfg.model);
+  if (rc != CM_OK) return fail(h, rc, "no float cutoff for eps_angle %.17g", cfg.eps_angle);
   rc = zone_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
   rc = plane_ws_ensure(h);
@@ -2760,7 +2841,7 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
 
   PlaneParams pp{};
   pp.pts = pts; pp.n_clouds = (uint32_t)n_clouds; pp.draw_stride = (uint32_t)PLANE_BATCH;
-  pp.threshold = thr; pp.sum_order = (uint32_t)cfg.sum_order;
+  pp.threshold = thr; pp.sum_order = (uint32_t)cfg.sum_order; pp.axis_rule = axis_rule;
   pp.samples = q.samples_dev.get(); pp.models = q.models_dev.get(); pp.counts = q.counts_dev.get(); pp.good = q.counts_dev.get() + q.cap_draws;
   std::vector<PlaneSearch> search((size_t)n_clouds);
   // CM_PLANE_TRACE=1: where the wall time of a call goes (host draws / scoring round trips / select + refit), to stderr
@@ -2827,9 +2908,11 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
           continue;
         }
         s.bad_run = 0;
+        if (good[d] == 2) ++out[c].rejected;  // isModelValid failed: an iteration with 0 inliers
         if ((long long)counts[d] > s.best) {
           s.best = counts[d];
           s.found = true;
+          s.best_valid = good[d] == 1;
           out[c].best_count = counts[d];
           for (int i = 0; i < 3; ++i) out[c].sample[i] = q.samples_pin.get()[3 * (off + d) + i];
           const float4 m = q.models_pin.get()[off + d];
@@ -2861,7 +2944,8 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
     out[c].iterations = s.iterations;
     out[c].draws = s.draws;
     memcpy(out[c].coeff, out[c].coeff_ransac, sizeof(out[c].coeff));
-    ps.found[c] = s.found ? 1u : 0u;
+    // a best model that fails the axis test is still PCL's result, but its selectWithinDistance keeps no point
+    ps.found[c] = s.found && s.best_valid ? 1u : 0u;
     ps.coeff[c] = make_float4(out[c].coeff[0], out[c].coeff[1], out[c].coeff[2], out[c].coeff[3]);
     any_found = any_found || s.found;
   }
@@ -2881,9 +2965,11 @@ int plane_ransac_run(cm_handle_t h, const float4* pts, const int64_t* begin, int
         fprintf(stderr, "[cm plane] cloud %d: moments kernel %u cycles, adding warp busy %u cycles, %u inliers\n", c, cyc[0], cyc[1], n_in);
       }
 #endif
-      if (!search[(size_t)c].found || n_in < 4) continue;  // below 4 inliers PCL keeps the RANSAC model
+      if (!ps.found[c] || n_in < 4) continue;  // below 4 inliers PCL keeps the RANSAC model
       plane_refit(q.acc_pin.get() + 16 * c, n_in, cfg.sum_order, out[c].coeff);
       ps.coeff[c] = make_float4(out[c].coeff[0], out[c].coeff[1], out[c].coeff[2], out[c].coeff[3]);
+      // the final selectWithinDistance tests the refitted model again: outside the cone it keeps no point
+      if (!plane_axis_valid(axis_rule, plane_axis_dot(axis_rule, out[c].coeff, cfg.sum_order))) ps.found[c] = 0u;
     }
   }
   // selectWithinDistance with the final model + the two ExtractIndices passes
@@ -2931,6 +3017,17 @@ int cm_plane_ransac_multi(cm_handle_t h, const float* xyzi_host, const int64_t* 
   return rc == CM_OK ? zone_copy_out(h, 2 * n_clouds + 1, out_xyzi, out_idx, capacity, out_begin) : rc;
 }
 
+int cm_plane_axis_rule(const cm_plane_cfg_t* cfg, cm_plane_axis_rule_t* out) {
+  if (!cfg || !out) return CM_E_INVALID;
+  PlaneAxisRule r;
+  const int rc = plane_axis_rule(*cfg, &r);
+  if (rc != CM_OK) return rc;
+  out->test = (int32_t)r.test;
+  out->c_neg = r.c_neg; out->c_pos = r.c_pos; out->f_plus = r.f_plus;
+  out->axis[0] = r.axis.x; out->axis[1] = r.axis.y; out->axis[2] = r.axis.z; out->axis[3] = r.axis.w;
+  return CM_OK;
+}
+
 int cm_plane_ransac(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_plane_cfg_t* cfg, cm_plane_t* out,
                     float* out_xyzi, uint32_t* out_idx, int64_t capacity, int64_t* out_begin) {
   if (n_points < 0) return CM_E_INVALID;
@@ -2958,6 +3055,7 @@ int proceed_ws_ensure(cm_handle_t h, size_t points) {
 int proceed_run(cm_handle_t h, const float4* roi, int64_t n, const cm_proceed_cfg_t& cfg, cm_proceed_out_t* out, cudaStream_t st) {
   if (cfg.n_parts < 1 || cfg.n_parts > CM_MAX_PROCEED_PARTS) return fail(h, CM_E_INVALID, "1 .. %d parts", CM_MAX_PROCEED_PARTS);
   if (n < 0 || n > 0x7FFFFFF0ll) return fail(h, CM_E_INVALID, "bad n_points");
+  if (cfg.plane.model < CM_SAC_PLANE || cfg.plane.model > CM_SAC_PARALLEL_PLANE) return fail(h, CM_E_INVALID, "unknown plane model %d", cfg.plane.model);
   int ground_of[CM_MAX_PROCEED_PARTS], plain_of[CM_MAX_PROCEED_PARTS];
   int G = 0, P = 0;
   for (int k = 0; k < cfg.n_parts; ++k) {

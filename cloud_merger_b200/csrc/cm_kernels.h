@@ -253,6 +253,20 @@ int launch_ec_order(const EcParams& e, const EcOrder& o, uint32_t n_points, cuda
 
 // ---- RANSAC ground plane (cm_plane.cu) --------------------------------------------------------------------------------------
 #define CM_MAX_PLANE_CLOUDS (CM_MAX_ZONES / 2)
+// The axis test of SACMODEL_PERPENDICULAR_PLANE / SACMODEL_PARALLEL_PLANE (isModelValid) on the float
+// d = dot(axis, normal), with the double comparisons of PCL folded into float cutoffs by the host (plane_axis_rule in
+// cm_api.cu). One rule for the scored draws (k_plane_score) and the refitted model (plane_ransac_run).
+struct PlaneAxisRule {
+  uint32_t test;        // 0 none, 1 perpendicular, 2 parallel (the CM_SAC_* values)
+  float c_neg, c_pos;   // perpendicular: valid iff d is NaN, d <= c_neg or d >= c_pos
+  float f_plus;         // parallel: valid iff !(|d| >= f_plus), the smallest float above |sin(eps_angle)|
+  float4 axis;          // (ax, ay, az, 0) normalized as Eigen does it
+};
+__host__ __device__ inline bool plane_axis_valid(const PlaneAxisRule& r, float d) {
+  if (r.test == 1) return d != d || d <= r.c_neg || d >= r.c_pos;
+  if (r.test == 2) return !(fabsf(d) >= r.f_plus);
+  return true;
+}
 struct PlaneParams {  // one batch of draws for up to CM_MAX_PLANE_CLOUDS independent clouds
   const float4* pts;                         // the clouds, one after the other
   uint32_t n_clouds;
@@ -264,7 +278,8 @@ struct PlaneParams {  // one batch of draws for up to CM_MAX_PLANE_CLOUDS indepe
   const int32_t* samples;  // [draw][3] point indices (relative to the cloud's first point)
   float4* models;          // [draw] plane of every draw
   int32_t* counts;         // [draw] inliers of every draw (cleared by the caller)
-  int32_t* good;           // [draw] isSampleGood
+  int32_t* good;           // [draw] 0: not isSampleGood; 1: a model that passes the axis test; 2: one that fails it
+  PlaneAxisRule axis_rule;
 };
 struct PlaneSelect {
   const float4* pts;

@@ -1,4 +1,5 @@
-// cm_plane.cu -- RANSAC ground plane (pcl::SACSegmentation, SACMODEL_PLANE + SAC_RANSAC) for sm_100a.
+// cm_plane.cu -- RANSAC ground plane (pcl::SACSegmentation, SACMODEL_PLANE / PERPENDICULAR_PLANE / PARALLEL_PLANE +
+// SAC_RANSAC) for sm_100a.
 //
 // Replaces the plane search of removeGround() in the reference (pcl_preprocessing/src/pc_preprocessing_main.cpp:95-117;
 // parameters Parameter.h:38-42: 1000 iterations, threshold 0.3 m, probability 0.99, optimize on). PCL 1.8.1 evaluates one
@@ -9,7 +10,8 @@
 //   k_plane_score   fits and scores a whole batch of draws at once, for up to eight independent clouds (blockIdx.z; the
 //                   zones of one sensor cloud): blockIdx.y picks 128 draws (one per thread), blockIdx.x a chunk of
 //                   512 points staged in shared memory and broadcast to the 128 threads; per draw the kernel
-//                   writes the sample test (isSampleGood), the model and the inlier count. The host then walks the batch
+//                   writes the sample test (isSampleGood) and the axis test of the constrained models (isModelValid;
+//                   a model that fails it skips the point loop: 0 inliers), the model and the inlier count. The host then walks the batch
 //                   in draw order with PCL's stopping rule -- the result is the model PCL's sequential loop ends on.
 //   k_plane_select  selectWithinDistance with the final model of every cloud: inlier / rest flags of every point (bits 2k /
 //                   2k + 1 of the zone-slicing mask for cloud k; its scan + scatter kernels produce the ground and
@@ -44,6 +46,17 @@ __device__ __forceinline__ float sum4(float l0, float l1, float l2, float l3) {
   else return __fadd_rn(__fadd_rn(__fadd_rn(l0, l1), l2), l3);
 }
 
+// Eigen 3.3 normalize(): only when the squared norm is positive
+template <int ORDER>
+__device__ __forceinline__ float4 normalized(float4 c) {
+  const float z = sum4<ORDER>(__fmul_rn(c.x, c.x), __fmul_rn(c.y, c.y), __fmul_rn(c.z, c.z), __fmul_rn(c.w, c.w));
+  if (z > 0.f) {
+    const float nrm = __fsqrt_rn(z);
+    c.x = __fdiv_rn(c.x, nrm); c.y = __fdiv_rn(c.y, nrm); c.z = __fdiv_rn(c.z, nrm); c.w = __fdiv_rn(c.w, nrm);
+  }
+  return c;
+}
+
 template <int ORDER>
 __device__ __forceinline__ float plane_abs_dist(const float4 c, const float4 q) {
   return fabsf(sum4<ORDER>(__fmul_rn(c.x, q.x), __fmul_rn(c.y, q.y), __fmul_rn(c.z, q.z), c.w));
@@ -64,7 +77,7 @@ __global__ void __launch_bounds__(PL_THREADS) k_plane_score(const PlaneParams p)
   }
   const uint32_t h = blockIdx.y * PL_THREADS + threadIdx.x;
   const uint32_t slot = cloud * p.draw_stride + h;
-  bool good = false;
+  bool good = false, valid = true;
   float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
   if (h < n_draws) {
     const int32_t* smp = p.samples + 3 * (size_t)slot;
@@ -78,20 +91,24 @@ __global__ void __launch_bounds__(PL_THREADS) k_plane_score(const PlaneParams p)
     c.y = __fsub_rn(__fmul_rn(uz, vx), __fmul_rn(ux, vz));
     c.z = __fsub_rn(__fmul_rn(ux, vy), __fmul_rn(uy, vx));
     c.w = 0.f;
-    // Eigen 3.3 normalize(): only when the squared norm is positive
-    const float z = sum4<ORDER>(__fmul_rn(c.x, c.x), __fmul_rn(c.y, c.y), __fmul_rn(c.z, c.z), __fmul_rn(c.w, c.w));
-    if (z > 0.f) {
-      const float nrm = __fsqrt_rn(z);
-      c.x = __fdiv_rn(c.x, nrm); c.y = __fdiv_rn(c.y, nrm); c.z = __fdiv_rn(c.z, nrm); c.w = __fdiv_rn(c.w, nrm);
-    }
+    c = normalized<ORDER>(c);
     c.w = __fmul_rn(-1.0f, sum4<ORDER>(__fmul_rn(c.x, p0.x), __fmul_rn(c.y, p0.y), __fmul_rn(c.z, p0.z), __fmul_rn(c.w, 1.0f)));
+    if (p.axis_rule.test) {
+      // isModelValid of the axis-constrained models: (a, b, c, 0) normalized once more -- and a second time inside
+      // getAngle3D for PERPENDICULAR -- dotted with the pre-normalized axis
+      float4 m = normalized<ORDER>(make_float4(c.x, c.y, c.z, 0.f));
+      if (p.axis_rule.test == 1) m = normalized<ORDER>(m);
+      const float4 a = p.axis_rule.axis;
+      const float d = sum4<ORDER>(__fmul_rn(a.x, m.x), __fmul_rn(a.y, m.y), __fmul_rn(a.z, m.z), __fmul_rn(a.w, m.w));
+      valid = plane_axis_valid(p.axis_rule, d);
+    }
     if (blockIdx.x == 0) {
       p.models[slot] = c;
-      p.good[slot] = good ? 1 : 0;
+      p.good[slot] = !good ? 0 : valid ? 1 : 2;
     }
   }
   __syncthreads();
-  if (!good) return;
+  if (!good || !valid) return;  // an invalid model counts 0 inliers (countWithinDistance)
   int cnt = 0;
 #pragma unroll 8
   for (int i = 0; i < PL_CHUNK; ++i) cnt += plane_abs_dist<ORDER>(c, s_pts[i]) < p.threshold ? 1 : 0;

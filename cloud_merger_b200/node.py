@@ -57,6 +57,11 @@ class NodeParams:
     distance_threshold: float = float(np.float32(0.3))
     prob: float = float(np.float32(0.99))
     sum_order: int = 0
+    # seg.setModelType / setAxis / setEpsAngle: the reference's SACMODEL_PLANE ignores the other two; with
+    # CM_SAC_PERPENDICULAR_PLANE (1) only planes within eps_angle [rad] of horizontal count as ground
+    sac_model: int = 0
+    axis: Tuple[float, float, float] = (0.0, 0.0, 1.0)
+    eps_angle: float = 0.0
     parts: Sequence[Sequence[Tuple[float, float, float]]] = field(default_factory=lambda: [FRONT_PARTS])  # per sensor (cycled)
 
 
@@ -81,7 +86,8 @@ class _SensorLane:
     def run(self, roi_ptr: int, n: int):
         p = self.p
         r = self.h.dev_proceed_zones(roi_ptr, n, self.parts, p.roi_z_max, p.radius, p.min_neighbor, p.distance_threshold, p.prob,
-                                     p.max_iterations, True, 12345, p.sum_order, stream=self.stream)
+                                     p.max_iterations, True, 12345, p.sum_order, stream=self.stream, model=p.sac_model,
+                                     axis=p.axis, eps_angle=p.eps_angle)
         self.h.stream_sync(self.stream)
         self.n_ng, self.n_g = r["n_no_ground"], r["n_ground"]
         self.no_ground_ptr, self.ground_ptr = r["no_ground_ptr"], r["ground_ptr"]

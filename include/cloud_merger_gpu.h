@@ -113,6 +113,9 @@ typedef struct {
 #define CM_SUM4_SSE2 0   /* Eigen packet reductions as an SSE2 build does them: (l0+l2)+(l1+l3) */
 #define CM_SUM4_SSE3 1   /* SSE3 and later (haddps): (l0+l1)+(l2+l3) */
 #define CM_SUM4_SCALAR 2 /* no vectorisation: ((l0+l1)+l2)+l3 */
+#define CM_SAC_PLANE 0              /* SACMODEL_PLANE: any plane (the reference's model) */
+#define CM_SAC_PERPENDICULAR_PLANE 1 /* SACMODEL_PERPENDICULAR_PLANE: normal within eps_angle of the axis (ground) */
+#define CM_SAC_PARALLEL_PLANE 2     /* SACMODEL_PARALLEL_PLANE: normal within eps_angle of perpendicular to the axis (walls) */
 typedef struct {
   double distance_threshold; /* seg.setDistanceThreshold (Parameter.h:40: 0.3f) */
   double probability;        /* seg.setProbability (Parameter.h:41: 0.99f) */
@@ -120,6 +123,10 @@ typedef struct {
   int32_t optimize;          /* seg.setOptimizeCoefficients (true in the reference) */
   uint32_t seed;             /* 12345 = PCL's sampler (SampleConsensusModel with random == false) */
   int32_t sum_order;         /* CM_SUM4_* */
+  /* seg.setModelType / setAxis / setEpsAngle. A zero-filled tail is SACMODEL_PLANE, which ignores axis and eps_angle. */
+  int32_t model;             /* CM_SAC_* */
+  float axis[3];             /* setAxis (the reference: 0, 0, 1); a zero axis is never set, as in SACSegmentation */
+  double eps_angle;          /* setEpsAngle [rad]; no constraint unless > 0 (and, for PERPENDICULAR, < pi/2) */
 } cm_plane_cfg_t;
 typedef struct {
   int32_t found;        /* 0: segment() failed (fewer than 3 points / no good sample): no inliers */
@@ -127,7 +134,7 @@ typedef struct {
   int32_t draws;        /* three-index draws taken from the sampler (>= iterations: bad samples are redrawn) */
   int32_t best_count;   /* inliers of the RANSAC model */
   int32_t sample[3];    /* the three point indices it was fitted through */
-  int32_t reserved;
+  int32_t rejected;     /* iterations whose model failed the axis test (counted with 0 inliers, as PCL does) */
   float coeff_ransac[4]; /* sac_->getModelCoefficients */
   float coeff[4];        /* what segment() returns: the least-squares refit when optimize != 0 */
   int64_t n_inliers;     /* inliers->indices.size() */
@@ -504,8 +511,13 @@ CM_API int cm_euclidean_clusters_multi(cm_handle_t h, const float* xyzi_host, co
                                        int64_t* out_cluster_begin, int64_t cluster_capacity, int64_t* out_cloud_clusters,
                                        int64_t* n_clusters, int64_t* n_points_out);
 /* RANSAC ground plane. Replaces the pcl::SACSegmentation + pcl::ExtractIndices block of removeGround()
- * (pc_preprocessing_main.cpp:95-117): SACMODEL_PLANE, SAC_RANSAC (setAxis / setEpsAngle are ignored by that model, as in
- * PCL). The three-index draws are PCL 1.8.1's -- boost::mt19937 seeded with cfg->seed, uniform_int<>(0, INT_MAX), the
+ * (pc_preprocessing_main.cpp:95-117): SAC_RANSAC with cfg->model = SACMODEL_PLANE (the reference's model, which ignores
+ * setAxis / setEpsAngle, as in PCL), SACMODEL_PERPENDICULAR_PLANE (only planes whose normal lies within eps_angle of the
+ * axis: the ground, not a wall or a car side that holds more points) or SACMODEL_PARALLEL_PLANE (normal within eps_angle
+ * of perpendicular to the axis: walls and facades with axis z). The axis test is PCL 1.8.1's isModelValid: a model that
+ * fails it counts 0 inliers but is still an iteration (out->rejected counts them), may still become the best model (then
+ * found = 1 with 0 inliers), and a refit that leaves the cone selects no inliers. A NaN model passes it. Unknown model ->
+ * CM_E_INVALID. The three-index draws are PCL 1.8.1's -- boost::mt19937 seeded with cfg->seed, uniform_int<>(0, INT_MAX), the
  * partial shuffle of drawIndexSample -- and are scored on the GPU a batch at a time; the host applies PCL's stopping rule
  * to the batch in draw order, so model, iteration count and inliers are those of PCL's sequential loop. With optimize the
  * least-squares refit follows (float running sums in inlier order as computeMeanAndCovarianceMatrix forms them, pcl::eigen33
@@ -531,6 +543,18 @@ CM_API int cm_plane_ransac_multi(cm_handle_t h, const float* xyzi_host, const in
                                  int64_t capacity, int64_t* out_begin);
 CM_API int cm_plane_ransac(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_plane_cfg_t* cfg,
                            cm_plane_t* out, float* out_xyzi, uint32_t* out_idx, int64_t capacity, int64_t* out_begin);
+/* The axis test the plane search applies, for inspection (host only, no handle). PCL's double-precision predicate on the
+ * float d = dot(axis, normal) is replaced by float cutoffs computed once per call:
+ *   test 0: none (SACMODEL_PLANE, eps_angle <= 0 or NaN);
+ *   test CM_SAC_PERPENDICULAR_PLANE: valid iff d is NaN or d <= c_neg or d >= c_pos;
+ *   test CM_SAC_PARALLEL_PLANE:      valid iff !(|d| >= f_plus), f_plus = the smallest float above |sin(eps_angle)|.
+ * axis = (ax, ay, az, 0) normalized as Eigen does it in cfg->sum_order. Unknown model -> CM_E_INVALID. */
+typedef struct {
+  int32_t test;
+  float c_neg, c_pos, f_plus;
+  float axis[4];
+} cm_plane_axis_rule_t;
+CM_API int cm_plane_axis_rule(const cm_plane_cfg_t* cfg, cm_plane_axis_rule_t* out);
 /* ---- the body of a proceedX in ONE call ----
  * Replaces what proceedFront / proceedRear / callbackTopMiddle / callbackFrontMiddle do after getROI
  * (pc_preprocessing_main.cpp:228-312, :428-446, :474-497): for every part of the sensor's zone table

@@ -122,6 +122,11 @@ struct Params {
   float distance_threshold = 0.3f;
   float prob = 0.99f;
   int sum_order = CM_SUM4_SSE2;
+  // seg.setModelType / setAxis / setEpsAngle: the reference keeps SACMODEL_PLANE, which ignores the other two; with
+  // CM_SAC_PERPENDICULAR_PLANE only planes within max_angle [rad] of horizontal are ground (a wall with more points is not)
+  int sac_model = CM_SAC_PLANE;
+  double max_angle = 0.0;
+  float axis[3] = {0.0f, 0.0f, 1.0f};
   // per-sensor zone tables (Parameter.h:45-81): zone lengths along x and the ground window |z| <= z_max_ground of each zone
   float vf_front_length = 30.0f, vf_mid_length = 15.0f, vf_mid_length2 = 11.0f, vf_veh_length = 8.0f, vf_rear_length = 11.0f;
   float vf_z_max_ground_front = 2.5f, vf_z_max_ground_mid2 = 2.0f, vf_z_max_ground_mid = 1.5f, vf_z_max_ground_veh = 0.3f,
@@ -132,6 +137,22 @@ struct Params {
   float l_front_length = 26.0f, l_mid_length = 10.0f, l_mid2_length = 10.0f, l_rear_length = 10.0f, l_deviation_mid_point = 4.0f;
   float l_z_max_ground_front = 1.5f, l_z_max_ground_mid2 = 1.2f, l_z_max_ground_mid = 0.8f, l_z_max_ground_rear = 0.5f;
 };
+
+// The pcl::SACSegmentation settings of removeGround() (pc_preprocessing_main.cpp:95-108); eps_angle = setEpsAngle's argument
+inline cm_plane_cfg_t planeConfig(const Params& p, double eps_angle) {
+  cm_plane_cfg_t cfg;
+  std::memset(&cfg, 0, sizeof(cfg));
+  cfg.distance_threshold = static_cast<double>(p.distance_threshold);
+  cfg.probability = static_cast<double>(p.prob);
+  cfg.max_iterations = p.max_iterations;
+  cfg.optimize = 1;
+  cfg.seed = 12345u;
+  cfg.sum_order = p.sum_order;
+  cfg.model = p.sac_model;
+  for (int a = 0; a < 3; ++a) cfg.axis[a] = p.axis[a];
+  cfg.eps_angle = eps_angle;
+  return cfg;
+}
 
 // my_cloud_fusion/src/Parameter.h:15-110 -- that package's constants are `double` (narrowed to float where PCL takes them)
 struct FusionParams {
@@ -334,6 +355,11 @@ class Context {
   // ground[k] = the inliers of in[k], no_ground[k] = its other points, both in input order.
   bool plane_ransac_multi(const std::vector<const Cloud*>& in, std::vector<Cloud>& ground, std::vector<Cloud>& no_ground,
                           std::vector<cm_plane_t>* models = nullptr) {
+    return plane_ransac_multi(in, ground, no_ground, planeConfig(params_, params_.max_angle), models);
+  }
+  // with explicit SACSegmentation settings (removeGround passes its max_angle as eps_angle)
+  bool plane_ransac_multi(const std::vector<const Cloud*>& in, std::vector<Cloud>& ground, std::vector<Cloud>& no_ground,
+                          const cm_plane_cfg_t& cfg, std::vector<cm_plane_t>* models = nullptr) {
     const size_t k = in.size();
     ground.assign(k, Cloud()); no_ground.assign(k, Cloud());
     if (!check(h_ ? CM_OK : CM_E_NO_DEVICE)) return false;
@@ -348,13 +374,6 @@ class Context {
         float* o = &tmp_[(static_cast<size_t>(begin[c]) + i) * 4];
         o[0] = p.x; o[1] = p.y; o[2] = p.z; o[3] = p.intensity;
       }
-    cm_plane_cfg_t cfg;
-    cfg.distance_threshold = static_cast<double>(params_.distance_threshold);
-    cfg.probability = static_cast<double>(params_.prob);
-    cfg.max_iterations = params_.max_iterations;
-    cfg.optimize = 1;
-    cfg.seed = 12345u;
-    cfg.sum_order = params_.sum_order;
     std::vector<cm_plane_t> pl(k);
     std::vector<int64_t> ob(2 * k + 1, 0);
     zone_xyzi_.resize(static_cast<size_t>(n) * 4 + 4);
@@ -377,9 +396,12 @@ class Context {
   }
   // one cloud
   bool plane_ransac(const Cloud& in, Cloud& ground, Cloud& no_ground, cm_plane_t* model = nullptr) {
+    return plane_ransac(in, ground, no_ground, planeConfig(params_, params_.max_angle), model);
+  }
+  bool plane_ransac(const Cloud& in, Cloud& ground, Cloud& no_ground, const cm_plane_cfg_t& cfg, cm_plane_t* model = nullptr) {
     std::vector<Cloud> g, r;
     std::vector<cm_plane_t> m;
-    const bool ok = plane_ransac_multi({&in}, g, r, &m);
+    const bool ok = plane_ransac_multi({&in}, g, r, cfg, &m);
     if (ok) { ground = g[0]; no_ground = r[0]; if (model) *model = m[0]; }
     else { clear(ground); clear(no_ground); }
     return ok;
@@ -689,18 +711,18 @@ inline void extractEuclideanClusters(Context& ctx, const Cloud::Ptr& cloud_ptr, 
 
 // void removeGround(cloud, no_ground, ground, z_min_ground, z_max_ground, max_angle) -- :71-122, the whole function: the two
 // z windows (one zone-slicing pass), the RANSAC plane on the lower one + ExtractIndices, outlierRemoval of what is not
-// ground, and the points above the window appended. max_angle is accepted and unused, as in the reference (SACMODEL_PLANE
-// ignores setAxis / setEpsAngle).
+// ground, and the points above the window appended. max_angle is setEpsAngle's argument (widened to double as that call
+// does); it matters only when Params::sac_model is not CM_SAC_PLANE (the reference's model ignores it).
 inline void removeGround(Context& ctx, const Cloud::Ptr& cloud_ptr, const Cloud::Ptr& no_ground_cloud_ptr,
                          const Cloud::Ptr& ground_cloud_ptr, const float z_min_ground, const float z_max_ground,
-                         const float /*max_angle*/) {
+                         const float max_angle) {
   std::vector<cm_zone_t> zones(2);
   zones[0].n_pass = 1; zones[0].pass[0] = cm_pass_t{2, z_min_ground, z_max_ground, 0};
   zones[1].n_pass = 1; zones[1].pass[0] = cm_pass_t{2, static_cast<float>(z_max_ground + 0.01), ctx.params().roi_z_max, 0};
   std::vector<Cloud> parts;
   ctx.zone_split(*cloud_ptr, zones, parts);
   Cloud ground, no_ground;
-  ctx.plane_ransac(parts[0], ground, no_ground);
+  ctx.plane_ransac(parts[0], ground, no_ground, planeConfig(ctx.params(), static_cast<double>(max_angle)));
   *ground_cloud_ptr = ground;
   *no_ground_cloud_ptr = no_ground;
   outlierRemoval(ctx, no_ground_cloud_ptr);
@@ -725,12 +747,7 @@ inline cm_proceed_cfg_t proceedConfig(const Params& p, const std::vector<ZonePar
   cfg.roi_z_max = p.roi_z_max;
   cfg.radius = static_cast<double>(p.radius);
   cfg.min_neighbors = static_cast<int>(p.min_neighbor);
-  cfg.plane.distance_threshold = static_cast<double>(p.distance_threshold);
-  cfg.plane.probability = static_cast<double>(p.prob);
-  cfg.plane.max_iterations = p.max_iterations;
-  cfg.plane.optimize = 1;
-  cfg.plane.seed = 12345u;
-  cfg.plane.sum_order = p.sum_order;
+  cfg.plane = planeConfig(p, p.max_angle);
   return cfg;
 }
 inline void proceedZones(Context& ctx, const Cloud::Ptr& cloud_ROI_ptr, const std::vector<ZonePart>& parts,
