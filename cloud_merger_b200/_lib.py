@@ -89,6 +89,20 @@ class CmClusterOut(C.Structure):
     _fields_ = [("xyzi", C.c_void_p), ("idx", C.c_void_p), ("begin", C.c_void_p), ("n_clusters", C.c_int64),
                 ("n_clustered", C.c_int64), ("n_unclustered", C.c_int64), ("cloud_clusters", C.c_int64 * CM_MAX_ZONES),
                 ("n_clouds", C.c_int32), ("host_syncs", C.c_int32), ("hook_ms", C.c_float), ("reserved", C.c_float)]
+CM_NE_WARP_CAP = 512   # include/cloud_merger_gpu.h: the largest neighbourhood a warp solves
+CM_NE_CTA_CAP = 7936   # the largest one a CTA collects in a single walk
+
+
+class CmNeCfg(C.Structure):
+    _fields_ = [("radius", C.c_double), ("viewpoint", C.c_float * 3), ("reserved", C.c_int32)]
+
+
+class CmNormalOut(C.Structure):
+    _fields_ = [("normals", C.c_void_p), ("n_points", C.c_int64), ("n_nan", C.c_int64 * CM_MAX_ZONES),
+                ("max_neighbors", C.c_int64), ("n_warp", C.c_int64), ("n_cta", C.c_int64), ("n_multi", C.c_int64),
+                ("n_clouds", C.c_int32), ("host_syncs", C.c_int32), ("warp_ms", C.c_float), ("cta_ms", C.c_float)]
+
+
 CM_MAX_PROCEED_PARTS = 8
 
 
@@ -241,6 +255,11 @@ SYMBOLS = {
     "cm_euclidean_clusters_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmEcCfg), C.c_void_p,
                                               C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.c_int64, C.POINTER(C.c_int64),
                                               C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "cm_dev_normals": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmNeCfg), C.c_void_p]),
+    "cm_dev_normals_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmNeCfg), C.c_void_p]),
+    "cm_get_normal_out": (C.c_int, [_H, C.POINTER(CmNormalOut)]),
+    "cm_normals": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmNeCfg), C.c_void_p]),
+    "cm_normals_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmNeCfg), C.c_void_p]),
     "cm_dev_plane_ransac": (C.c_int, [_H, C.c_void_p, C.c_int64, C.POINTER(CmPlaneCfg), C.POINTER(CmPlane), C.c_void_p]),
     "cm_dev_plane_ransac_multi": (C.c_int, [_H, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.POINTER(CmPlaneCfg),
                                             C.POINTER(CmPlane), C.c_void_p]),

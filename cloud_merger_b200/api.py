@@ -422,6 +422,57 @@ class CloudMerger:
         cl = [_part(ox, oi, cb[q], cb[q + 1]) for q in range(nc.value)]
         return cl if with_xyzi else [i for _, i in cl]
 
+    # -- normal estimation (pcl::NormalEstimation with a radius search) -------------------------------------------------------
+    @staticmethod
+    def _ne_cfg(radius, viewpoint):
+        return _lib.CmNeCfg(float(radius), (C.c_float * 3)(*[float(np.float32(v)) for v in viewpoint]), 0)
+
+    def dev_normals(self, xyzi_ptr: int, n_points: int, radius: float, viewpoint=(0.0, 0.0, 0.0), stream: int = 0):
+        """Device form; fetch the normals with normals_out()."""
+        cfg = self._ne_cfg(radius, viewpoint)
+        self._check(self._lib.cm_dev_normals(self._h, C.c_void_p(xyzi_ptr or None), C.c_int64(n_points), C.byref(cfg),
+                                             C.c_void_p(stream or None)))
+
+    def dev_normals_multi(self, xyzi_ptr: int, begin, radius: float, viewpoint=(0.0, 0.0, 0.0), stream: int = 0):
+        """Independent clouds [begin[k], begin[k+1]) of one device array in one pass (needs max_batch_frames >= the number
+        of clouds); fetch the normals with normals_out()."""
+        b = (C.c_int64 * len(begin))(*[int(v) for v in begin])
+        cfg = self._ne_cfg(radius, viewpoint)
+        self._check(self._lib.cm_dev_normals_multi(self._h, C.c_void_p(xyzi_ptr or None), b, len(begin) - 1, C.byref(cfg),
+                                                   C.c_void_p(stream or None)))
+
+    def normals_out(self) -> dict:
+        """Of the last normal estimation: "normals" (float32 [n, 4]: nx ny nz curvature, input order), "n_nan" per cloud,
+        "max_neighbors", the queries per path ("n_warp", "n_cta", "n_multi"), "host_syncs", and "warp_ms" (the
+        sorted-order gather and the warp kernel) / "cta_ms" (-1 unless profiling)."""
+        no = _lib.CmNormalOut()
+        self._check(self._lib.cm_get_normal_out(self._h, C.byref(no)))
+        n = int(no.n_points)
+        nrm = self.download(no.normals, np.float32, 4 * n).reshape(-1, 4) if n else np.zeros((0, 4), np.float32)
+        return {"normals": nrm, "n_nan": [int(v) for v in no.n_nan[:no.n_clouds]], "max_neighbors": int(no.max_neighbors),
+                "n_warp": int(no.n_warp), "n_cta": int(no.n_cta), "n_multi": int(no.n_multi),
+                "host_syncs": int(no.host_syncs), "warp_ms": float(no.warp_ms), "cta_ms": float(no.cta_ms)}
+
+    def normals_multi(self, clouds, radius: float, viewpoint=(0.0, 0.0, 0.0)) -> list:
+        """Host-buffer form: per cloud a float32 [n, 4] array (nx ny nz curvature of every point, input order)."""
+        allpts, begin, b, _ = _pack(clouds)
+        k = len(begin) - 1
+        out = np.zeros((max(len(allpts), 1), 4), np.float32)
+        cfg = self._ne_cfg(radius, viewpoint)
+        self._check(self._lib.cm_normals_multi(self._h, allpts.ctypes.data_as(C.c_void_p), b, k, C.byref(cfg),
+                                               out.ctypes.data_as(C.c_void_p)))
+        return [out[begin[c]:begin[c + 1]].copy() for c in range(k)]
+
+    def normals(self, xyzi: np.ndarray, radius: float, viewpoint=(0.0, 0.0, 0.0)) -> np.ndarray:
+        """Host-buffer form for one cloud: float32 [n, 4], nx ny nz curvature of every point in input order (NaN x4
+        where PCL gives no normal)."""
+        a = np.ascontiguousarray(xyzi, np.float32).reshape(-1, 4)
+        out = np.zeros((max(len(a), 1), 4), np.float32)
+        cfg = self._ne_cfg(radius, viewpoint)
+        self._check(self._lib.cm_normals(self._h, a.ctypes.data_as(C.c_void_p), C.c_int64(len(a)), C.byref(cfg),
+                                         out.ctypes.data_as(C.c_void_p)))
+        return out[:len(a)]
+
     # -- RANSAC ground plane (pcl::SACSegmentation of removeGround, pc_preprocessing_main.cpp:95-117) ------------------------
     @staticmethod
     def _plane_cfg(distance_threshold, probability, max_iterations, optimize, seed, sum_order, model=0, axis=(0.0, 0.0, 1.0),

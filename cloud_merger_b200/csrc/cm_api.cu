@@ -250,6 +250,20 @@ struct cm_handle_s {
     int64_t cloud_clusters[CM_MAX_ZONES] = {};
     uint32_t device_error = 0;
   } ew;
+  // normal estimation (allocated on first use)
+  struct NeWs {
+    size_t cap = 0;
+    DevPtr<float4> out;            // [cap] nx ny nz curvature, input order
+    DevPtr<float4> sorted_pts;     // [cap] the points in sorted key order
+    DevPtr<uint32_t> queue;        // [cap] the CTA kernel's queries
+    DevPtr<NeStats> stats;
+    HostPtr<NeStats> stats_host;   // pinned mirror of stats; its `error` receives Ctrl.error of the run
+    Event ev[3];                   // profiling: before the warp kernel, between the two, behind the CTA kernel
+    cudaStream_t stream = nullptr;
+    bool ran = false, profiled = false;
+    int n_clouds = 0;
+    int64_t n_points = 0;
+  } nw;
   // RANSAC ground plane (allocated on first use): one batch of draws and its scores, device + pinned mirrors
   struct PlaneWs {
     size_t cap_draws = 0;
@@ -1295,7 +1309,7 @@ int cm_create(const cm_config_t* cfg, cm_handle_t* out) {
   h->device = c.device;
   if (cudaSetDevice(h->device) != cudaSuccess) { delete h; return CM_E_CUDA; }
   if (configure_device_kernels() != cudaSuccess || configure_sort_kernels() != cudaSuccess ||
-      configure_centroid_kernels() != cudaSuccess) {
+      configure_centroid_kernels() != cudaSuccess || configure_normal_kernels() != cudaSuccess) {
     delete h;
     return CM_E_CUDA;
   }
@@ -2583,6 +2597,141 @@ int cm_euclidean_clusters(cm_handle_t h, const float* xyzi_host, int64_t n_point
   const int64_t begin[2] = {0, n_points};
   return cm_euclidean_clusters_multi(h, xyzi_host, begin, 1, cfg, out_xyzi, out_idx, point_capacity, out_cluster_begin,
                                      cluster_capacity, nullptr, n_clusters, n_points_out);
+}
+
+// ---- normal estimation ----------------------------------------------------------------------------------------------------
+namespace {
+int ne_ws_ensure(cm_handle_t h, size_t points) {
+  cm_handle_s::NeWs& e = h->nw;
+  const size_t want = std::max<size_t>(points, 1);
+  if (e.cap >= want) return CM_OK;
+  e = cm_handle_s::NeWs();  // the old buffers go before the larger ones are allocated
+  CM_CUDA(h, dev_alloc(e.out, want));
+  CM_CUDA(h, dev_alloc(e.sorted_pts, want));
+  CM_CUDA(h, dev_alloc(e.queue, want));
+  CM_CUDA(h, dev_alloc(e.stats, 1));
+  CM_CUDA(h, pinned_alloc(e.stats_host, sizeof(NeStats), cudaHostAllocDefault));
+  for (auto& ev : e.ev) CM_CUDA(h, create(ev, cudaEventCreateWithFlags, cudaEventDefault));
+  e.cap = want;
+  return CM_OK;
+}
+
+// the normals of every cloud [begin[k], begin[k+1]) into the handle's normal output; the statistics and the search's
+// verdict on the cell bound follow into pinned memory, read by cm_get_normal_out
+int normals_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_clouds, const cm_ne_cfg_t* cfg, cudaStream_t st) {
+  if (!cfg) return fail(h, CM_E_INVALID, "cfg is NULL");
+  if (!(cfg->radius > 0.0) || !std::isfinite(cfg->radius)) return fail(h, CM_E_INVALID, "radius must be finite and > 0");
+  int rc = check_clouds(h, pts, begin, n_clouds, CM_MAX_ZONES);
+  if (rc != CM_OK) return rc;
+  const int64_t n_points = begin[n_clouds];
+  cm_handle_s::NeWs& e = h->nw;
+  e.ran = false;
+  VoxelParams vp;
+  rc = cell_keys_begin(h, pts, begin, n_clouds, vp, st);
+  if (rc != CM_OK) return rc;
+  rc = ne_ws_ensure(h, (size_t)n_points);
+  if (rc != CM_OK) return rc;
+  // the radius outlier removal's cells: two neighbours are at most one cell apart on every axis
+  const float cell = (float)cfg->radius * 1.00390625f;
+  rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  if (rc != CM_OK) return rc;
+  Workspace& w = h->batch;
+  RorParams rp{};
+  rc = enqueue_cell_table(h, vp, "CM_NE_NO_TABLE", rp, st);
+  if (rc != CM_OK) return rc;
+  NeParams np{};
+  np.pts = pts;
+  np.sorted_pts = e.sorted_pts.get();
+  np.cell_start = rp.cell_start;
+  np.r2 = (float)(cfg->radius * cfg->radius);  // KdTreeFLANN::radiusSearch: the double square, narrowed
+  for (int k = 0; k < 3; ++k) np.vp[k] = cfg->viewpoint[k];
+  np.out = e.out.get();
+  np.queue = e.queue.get();
+  np.stats = e.stats.get();
+  for (int c = 0; c <= CM_MAX_ZONES; ++c) np.begin[c] = (uint32_t)begin[std::min(c, n_clouds)];
+  CM_CUDA(h, cudaMemsetAsync(e.stats.get(), 0, sizeof(NeStats), st));
+  e.profiled = h->profiling;
+  if (e.profiled) CM_CUDA(h, cudaEventRecord(e.ev[0].get(), st));
+  cudaError_t err;
+  w.launches += launch_normals(vp, np, e.sorted_pts.get(), st, e.profiled ? e.ev[1].get() : nullptr, &err);
+  CM_CUDA(h, err);
+  if (e.profiled) CM_CUDA(h, cudaEventRecord(e.ev[2].get(), st));
+  CM_CUDA(h, cudaMemcpyAsync(e.stats_host.get(), e.stats.get(), sizeof(NeStats), cudaMemcpyDeviceToHost, st));
+  // the warp kernel's verdict on the 2^14-cell bound
+  CM_CUDA(h, cudaMemcpyAsync(&e.stats_host.get()->error, &vp.ctrl->error, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  e.stream = st; e.n_clouds = n_clouds; e.n_points = n_points;
+  e.ran = true;
+  return CM_OK;
+}
+
+int normal_out_locked(cm_handle_t h, cm_normal_out_t* out) {
+  cm_handle_s::NeWs& e = h->nw;
+  if (!e.ran) return fail(h, CM_E_INVALID, "no normal estimation has run on this handle");
+  CM_CUDA(h, cudaSetDevice(h->device));
+  CM_CUDA(h, cudaStreamSynchronize(e.stream));
+  const uint32_t dev_error = e.stats_host.get()->error;
+  if (dev_error == CM_DEV_E_KEY_RANGE)
+    return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (more than 2^14 cells from the origin)");
+  if (dev_error) return fail(h, CM_E_INTERNAL, "device error %u", dev_error);
+  memset(out, 0, sizeof(*out));
+  const NeStats& s = *e.stats_host.get();
+  out->normals = reinterpret_cast<const float*>(e.out.get());
+  out->n_points = e.n_points;
+  for (int c = 0; c < e.n_clouds; ++c) out->n_nan[c] = s.n_nan[c];
+  out->max_neighbors = s.max_neighbors;
+  out->n_warp = s.n_warp; out->n_cta = s.n_cta; out->n_multi = s.n_multi;
+  out->n_clouds = e.n_clouds;
+  out->host_syncs = 1;  // the key plan (cell_keys_sort)
+  out->warp_ms = out->cta_ms = -1.f;
+  if (e.profiled) {
+    if (cudaEventElapsedTime(&out->warp_ms, e.ev[0].get(), e.ev[1].get()) != cudaSuccess) { out->warp_ms = -1.f; cudaGetLastError(); }
+    if (cudaEventElapsedTime(&out->cta_ms, e.ev[1].get(), e.ev[2].get()) != cudaSuccess) { out->cta_ms = -1.f; cudaGetLastError(); }
+  }
+  return CM_OK;
+}
+}  // namespace
+
+int cm_dev_normals(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_ne_cfg_t* cfg, void* stream) {
+  const int64_t begin[2] = {0, n_points};
+  return cm_dev_normals_multi(h, xyzi_dev, begin, 1, cfg, stream);
+}
+
+int cm_dev_normals_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds, const cm_ne_cfg_t* cfg,
+                         void* stream) {
+  if (!h || !begin) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  return normals_run(h, reinterpret_cast<const float4*>(xyzi_dev), begin, n_clouds, cfg, static_cast<cudaStream_t>(stream));
+}
+
+int cm_get_normal_out(cm_handle_t h, cm_normal_out_t* out) {
+  if (!h || !out) return CM_E_INVALID;
+  std::lock_guard<std::mutex> lk(h->mu);
+  return normal_out_locked(h, out);
+}
+
+int cm_normals_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds, const cm_ne_cfg_t* cfg,
+                     float* out_normals) {
+  if (!h || !begin) return CM_E_INVALID;
+  if (n_clouds < 1 || n_clouds > CM_MAX_ZONES) return fail(h, CM_E_INVALID, "1 .. %d clouds per call", CM_MAX_ZONES);
+  if (begin[n_clouds] > 0 && !out_normals) return fail(h, CM_E_INVALID, "out_normals is NULL");
+  std::lock_guard<std::mutex> lk(h->mu);
+  CM_CUDA(h, cudaSetDevice(h->device));
+  const float4* pts = nullptr;
+  int rc = stage_host_cloud(h, xyzi_host, begin[n_clouds], &pts);
+  if (rc == CM_OK) rc = normals_run(h, pts, begin, n_clouds, cfg, nullptr);
+  if (rc != CM_OK) return rc;
+  cm_normal_out_t no;
+  rc = normal_out_locked(h, &no);
+  if (rc != CM_OK) return rc;
+  if (no.n_points) CM_CUDA(h, cudaMemcpy(out_normals, no.normals, (size_t)no.n_points * 16, cudaMemcpyDeviceToHost));
+  return CM_OK;
+}
+
+int cm_normals(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_ne_cfg_t* cfg, float* out_normals) {
+  if (!h || n_points < 0) return CM_E_INVALID;
+  const int64_t begin[2] = {0, n_points};
+  return cm_normals_multi(h, xyzi_host, begin, 1, cfg, out_normals);
 }
 
 // ---- RANSAC ground plane --------------------------------------------------------------------------------------------------

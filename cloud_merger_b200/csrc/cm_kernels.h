@@ -217,6 +217,33 @@ cudaError_t launch_sor_knn(const VoxelParams& p, const SorParams& s, float4* sor
 cudaError_t launch_sor_sums(const SorSumParams& s, cudaStream_t stream);  // one CTA per cloud
 cudaError_t launch_sor_select(const SorSumParams& s, uint32_t n_points, cudaStream_t stream);
 
+// the points in sorted key order (one launch): sorted_pts[i] = pts[value of sorted position i]
+cudaError_t launch_sorted_gather(const VoxelParams& p, float4* sorted_pts, cudaStream_t stream);
+
+// ---- normal estimation on the sorted cell keys (cm_normals.cu) ------------------------------------------------------------
+struct NeStats {                     // device counters of one call (cleared by the caller)
+  uint32_t n_queue;                  // queries whose neighbourhood exceeds CM_NE_WARP_CAP (the CTA kernel's queue)
+  uint32_t max_neighbors;            // the largest neighbourhood (the query itself included)
+  uint32_t n_warp, n_cta, n_multi;   // queries solved by the warp kernel, the CTA kernel in one walk, in several walks
+  uint32_t n_nan[CM_MAX_ZONES];      // points of every cloud whose normal is NaN
+  uint32_t error;                    // host mirror only: Ctrl.error of the run
+};
+struct NeParams {
+  const float4* pts;                 // [n_points] the input cloud(s)
+  const float4* sorted_pts;          // [M] the points in sorted key order
+  const uint32_t* cell_start;        // k_ror_table's table of the cells' first sorted positions, or nullptr: binary searches
+  float r2;                          // (float)(radius * radius): neighbours are strictly below it
+  float vp[3];                       // the viewpoint
+  float4* out;                       // [n_points] nx ny nz curvature, input order
+  uint32_t* queue;                   // [n_points] sorted positions of the queries for the CTA kernel
+  NeStats* stats;
+  uint32_t begin[CM_MAX_ZONES + 1];  // cloud k = input indices [begin[k], begin[k+1])
+};
+cudaError_t configure_normal_kernels();
+// the sorted-order gather, the warp kernel (event `mid` recorded behind it when given), the CTA kernel; returns the launches
+int launch_normals(const VoxelParams& p, const NeParams& e, float4* sorted_pts, cudaStream_t stream, cudaEvent_t mid,
+                   cudaError_t* err);
+
 // ---- Euclidean cluster extraction on the sorted cell keys (cm_cluster.cu) ----------------------------------------------------
 struct EcParams {
   const float4* pts;           // [n_points] the input cloud(s)

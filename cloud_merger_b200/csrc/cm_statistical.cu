@@ -347,11 +347,18 @@ __global__ void __launch_bounds__(256) k_sor_select(const SorSumParams s, uint32
 
 }  // namespace
 
-cudaError_t launch_sor_knn(const VoxelParams& p, const SorParams& s, float4* sorted_pts, cudaStream_t stream) {
+cudaError_t launch_sorted_gather(const VoxelParams& p, float4* sorted_pts, cudaStream_t stream) {
   if (p.max_points == 0) return cudaSuccess;
   const uint32_t gb = (p.max_points + 255) / 256;
   if (p.key_bytes == 4) k_sor_gather<uint32_t><<<gb, 256, 0, stream>>>(p, sorted_pts);
   else k_sor_gather<unsigned long long><<<gb, 256, 0, stream>>>(p, sorted_pts);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_sor_knn(const VoxelParams& p, const SorParams& s, float4* sorted_pts, cudaStream_t stream) {
+  if (p.max_points == 0) return cudaSuccess;
+  const cudaError_t ge = launch_sorted_gather(p, sorted_pts, stream);
+  if (ge != cudaSuccess) return ge;
   const uint32_t blocks = (p.max_points + SOR_WARPS - 1) / SOR_WARPS;
   const int ns = s.mean_k + 1 <= 32 ? 1 : s.mean_k + 1 <= 64 ? 2 : 4;
 #define CM_SOR_LAUNCH(KT, TB, NS) k_sor_knn<KT, TB, NS><<<blocks, SOR_THREADS, 0, stream>>>(p, s)

@@ -510,6 +510,53 @@ CM_API int cm_euclidean_clusters_multi(cm_handle_t h, const float* xyzi_host, co
                                        const cm_ec_cfg_t* cfg, float* out_xyzi, uint32_t* out_idx, int64_t point_capacity,
                                        int64_t* out_cluster_begin, int64_t cluster_capacity, int64_t* out_cloud_clusters,
                                        int64_t* n_clusters, int64_t* n_points_out);
+/* Normal estimation: pcl::NormalEstimation<pcl::PointXYZI, pcl::Normal> with setRadiusSearch(radius), a KdTreeFLANN search
+ * and setViewPoint(viewpoint) (PCL 1.8.1 computeFeature). The neighbours of a finite query are the finite points of its
+ * cloud whose float squared distance (dx*dx + dy*dy) + dz*dz, each operation rounded on its own, is strictly below
+ * r2 = (float)(radius * radius) -- the radius outlier removal's rule; the query itself included -- in FLANN's order,
+ * ascending (squared distance, index). Their float mean and covariance (nine running sums in that order), pcl::eigen33's
+ * eigenvector of the smallest eigenvalue, the curvature |lambda0 / trace| and the flip towards the viewpoint follow PCL
+ * operation by operation (DESIGN section 8). Fewer than 3 neighbours or a non-finite query: quiet NaN x4.
+ * Documented deviations: the transcendental functions of computeRoots are this library's rule (correctly rounded except
+ * within ~2^-50 of a float midpoint), not the host libm's, which differs from build to build; the cloud is always treated
+ * as non-dense; several clouds in one call never see each other's points; a covariance with a non-finite entry gives
+ * quiet NaN x4; every NaN is written as quiet_NaN (0x7fc00000).
+ *  cm_dev_normals[_multi]: packed float4 xyzi points on the device, clouds as for the radius outlier removal (cloud k =
+ *      [begin[k], begin[k+1]), n_clouds <= CM_MAX_ZONES and <= max_batch_frames). The normals go to a device array of the
+ *      handle (cm_get_normal_out), in input order; the call returns after one round trip (the key plan) with the search
+ *      enqueued on `stream`. A radius <= 0, NaN or infinite -> CM_E_INVALID; CM_E_KEY_RANGE when the radius is too small
+ *      for the extent of a cloud: from the call when the cell grid exceeds the key range, from cm_get_normal_out when a
+ *      point lies 2^14 cells or more from the origin (as cm_get_zone_out reports it for the radius outlier removal).
+ *  cm_normals[_multi]: host buffers; out_normals receives n_points x 4 floats (nx ny nz curvature) in input order.
+ * Neighbourhoods of up to CM_NE_WARP_CAP points are solved by one warp each, larger ones by one CTA each: in one walk up
+ * to CM_NE_CTA_CAP, beyond that in one walk per ~4096 neighbours. Memory: 36 bytes per point of the handle's batch
+ * capacity, allocated on first use. */
+#define CM_NE_WARP_CAP 512
+#define CM_NE_CTA_CAP 7936
+typedef struct {
+  double radius;        /* setRadiusSearch (metres) */
+  float viewpoint[3];   /* setViewPoint */
+  int32_t reserved;     /* 0 */
+} cm_ne_cfg_t;
+/* device-resident result of the last normal estimation on a handle (valid until the next one) */
+typedef struct {
+  const float* normals;                  /* device [n_points][4]: nx ny nz curvature of every input point, input order */
+  int64_t n_points;
+  int64_t n_nan[CM_MAX_ZONES];           /* points of every cloud whose normal is NaN (non-finite ones included) */
+  int64_t max_neighbors;                 /* the largest neighbourhood of the call */
+  int64_t n_warp, n_cta, n_multi;        /* queries solved by a warp, by a CTA in one walk, by a CTA in several walks */
+  int32_t n_clouds;
+  int32_t host_syncs;                    /* device round trips of the call */
+  float warp_ms, cta_ms;                 /* GPU time of the sorted-order gather + warp kernel and of the CTA kernel, search
+                                            and solve (cm_set_profiling on; -1 otherwise) */
+} cm_normal_out_t;
+CM_API int cm_dev_normals(cm_handle_t h, const float* xyzi_dev, int64_t n_points, const cm_ne_cfg_t* cfg, void* stream);
+CM_API int cm_dev_normals_multi(cm_handle_t h, const float* xyzi_dev, const int64_t* begin, int n_clouds,
+                                const cm_ne_cfg_t* cfg, void* stream);
+CM_API int cm_get_normal_out(cm_handle_t h, cm_normal_out_t* out);
+CM_API int cm_normals(cm_handle_t h, const float* xyzi_host, int64_t n_points, const cm_ne_cfg_t* cfg, float* out_normals);
+CM_API int cm_normals_multi(cm_handle_t h, const float* xyzi_host, const int64_t* begin, int n_clouds, const cm_ne_cfg_t* cfg,
+                            float* out_normals);
 /* RANSAC ground plane. Replaces the pcl::SACSegmentation + pcl::ExtractIndices block of removeGround()
  * (pc_preprocessing_main.cpp:95-117): SAC_RANSAC with cfg->model = SACMODEL_PLANE (the reference's model, which ignores
  * setAxis / setEpsAngle, as in PCL), SACMODEL_PERPENDICULAR_PLANE (only planes whose normal lies within eps_angle of the

@@ -24,6 +24,7 @@
 #ifndef CLOUD_MERGER_SHIM_HPP_
 #define CLOUD_MERGER_SHIM_HPP_
 
+#include <array>
 #include <atomic>
 #include <cstdint>
 #include <cstring>
@@ -347,6 +348,42 @@ class Context {
     clusters.clear();
     if (!euclidean_clusters_multi({&in}, res, tolerance, min_size, max_size)) return false;
     clusters = std::move(res[0]);
+    return true;
+  }
+
+  // Normal estimation of several host clouds in one pass (cm_normals_multi; at most CM_MAX_ZONES clouds):
+  // pcl::NormalEstimation with setRadiusSearch(radius) and setViewPoint(vp) on every cloud on its own. normals[k] holds
+  // 4 floats per point of in[k] -- normal_x normal_y normal_z curvature, input order, quiet NaN x4 where PCL gives none.
+  bool normals_multi(const std::vector<const Cloud*>& in, std::vector<std::vector<float>>& normals, double radius,
+                     const std::array<float, 3>& vp = {0.f, 0.f, 0.f}) {
+    const size_t k = in.size();
+    normals.assign(k, std::vector<float>());
+    if (!check(h_ ? CM_OK : CM_E_NO_DEVICE)) return false;
+    std::vector<int64_t> begin(k + 1, 0);
+    for (size_t c = 0; c < k; ++c) begin[c + 1] = begin[c] + static_cast<int64_t>(in[c]->points.size());
+    const int64_t n = begin[k];
+    if (n > max_points_ * max_sensors_) { rc_ = CM_E_CAPACITY; err_ = "clouds larger than the context capacity"; return false; }
+    tmp_.resize(static_cast<size_t>(n) * 4 + 4);
+    for (size_t c = 0; c < k; ++c)
+      for (size_t i = 0; i < in[c]->points.size(); ++i) {
+        const PointXYZI& p = in[c]->points[i];
+        float* o = &tmp_[(static_cast<size_t>(begin[c]) + i) * 4];
+        o[0] = p.x; o[1] = p.y; o[2] = p.z; o[3] = p.intensity;
+      }
+    std::vector<float> out(static_cast<size_t>(n) * 4 + 4);
+    cm_ne_cfg_t cfg{};
+    cfg.radius = radius;
+    for (int a = 0; a < 3; ++a) cfg.viewpoint[a] = vp[a];
+    if (!check(cm_normals_multi(h_, tmp_.data(), begin.data(), static_cast<int>(k), &cfg, out.data()))) return false;
+    for (size_t c = 0; c < k; ++c)
+      normals[c].assign(out.begin() + begin[c] * 4, out.begin() + begin[c + 1] * 4);
+    return true;
+  }
+  bool normals(const Cloud& in, std::vector<float>& out, double radius, const std::array<float, 3>& vp = {0.f, 0.f, 0.f}) {
+    std::vector<std::vector<float>> res;
+    out.clear();
+    if (!normals_multi({&in}, res, radius, vp)) return false;
+    out = std::move(res[0]);
     return true;
   }
 
@@ -706,6 +743,28 @@ inline void extractEuclideanClusters(Context& ctx, const Cloud::Ptr& cloud_ptr, 
     cluster_indices[j].header = cloud_ptr->header;
     cluster_indices[j].indices = std::move(clusters[j]);
   }
+}
+#endif
+
+// pcl::NormalEstimation<PointXYZI, Normal> (setRadiusSearch, setViewPoint; compute) on a cloud: 4 floats per point,
+// normal_x normal_y normal_z curvature in input order
+inline void estimateNormals(Context& ctx, const Cloud::Ptr& cloud_ptr, double radius, const std::array<float, 3>& vp,
+                            std::vector<float>& out) {
+  ctx.normals(*cloud_ptr, out, radius, vp);
+}
+#ifdef CM_SHIM_HAVE_PCL
+// ... with compute()'s own output type
+inline void estimateNormals(Context& ctx, const Cloud::Ptr& cloud_ptr, double radius, const std::array<float, 3>& vp,
+                            pcl::PointCloud<pcl::Normal>& out) {
+  std::vector<float> v;
+  ctx.normals(*cloud_ptr, v, radius, vp);
+  out.header = cloud_ptr->header;
+  out.points.resize(v.size() / 4);
+  for (size_t i = 0; i < out.points.size(); ++i) {
+    out.points[i].normal_x = v[4 * i]; out.points[i].normal_y = v[4 * i + 1];
+    out.points[i].normal_z = v[4 * i + 2]; out.points[i].curvature = v[4 * i + 3];
+  }
+  out.width = static_cast<uint32_t>(out.points.size()); out.height = 1; out.is_dense = false;
 }
 #endif
 
