@@ -12,7 +12,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libcloud_merger_gpu.so")
 SOURCES = ["cm_transform_crop.cu", "cm_voxel.cu", "cm_radix_sort.cu", "cm_zones.cu", "cm_outlier.cu", "cm_route.cu", "cm_plane.cu", "cm_statistical.cu", "cm_cluster.cu", "cm_normals.cu", "cm_api.cu"]
-HEADERS = ["cm_common.cuh", "cm_kernels.h", "cm_ne_math.h", os.path.join("..", "..", "include", "cloud_merger_gpu.h")]
+HEADERS = ["cm_common.cuh", "cm_kernels.h", "cm_cells.cuh", "cm_ne_math.h", os.path.join("..", "..", "include", "cloud_merger_gpu.h")]
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

@@ -311,6 +311,24 @@ int fail(cm_handle_t h, int code, const char* fmt, ...) {
                                         __FILE__, __LINE__);                                          \
   } while (0)
 
+// The search's verdict on the 2^14-cell bound (Ctrl.error of the run) as a return code; `what` names the radius parameter.
+int cell_margin_verdict(cm_handle_t h, uint32_t dev_error, const char* what) {
+  if (dev_error == CM_DEV_E_KEY_RANGE)
+    return fail(h, CM_E_KEY_RANGE, "%s too small for the extent of a cloud (more than 2^14 cells from the origin)", what);
+  if (dev_error) return fail(h, CM_E_INTERNAL, "device error %u", dev_error);
+  return CM_OK;
+}
+
+// The time between two recorded events, or -1 when it cannot be read (the error is cleared).
+float elapsed_ms(cudaEvent_t a, cudaEvent_t b) {
+  float ms = -1.f;
+  if (cudaEventElapsedTime(&ms, a, b) != cudaSuccess) {
+    cudaGetLastError();
+    return -1.f;
+  }
+  return ms;
+}
+
 // ---- page-locked host memory next to the GPU ---------------------------------------------------------------------------------
 // A frame travels host -> device at PCIe speed only if its pages sit on the NUMA node the GPU hangs off: with one process per
 // GPU and eight GPUs copying at once, arenas that all landed on one node share that node's memory controllers and the
@@ -1878,10 +1896,7 @@ int zone_out_locked(cm_handle_t h, cm_zone_out_t* out) {
   if (report[CM_MAX_ZONES + 1])
     return fail(h, CM_E_CAPACITY, "the zones hold %s%u points together, capacity is %zu",
                 report[CM_MAX_ZONES + 1] > 0xFFFFFFF0u ? "more than " : "", std::min(report[CM_MAX_ZONES + 1], 0xFFFFFFF0u), z.cap_out);
-  if (z.ror_run && report[CM_MAX_ZONES + 2] == CM_DEV_E_KEY_RANGE)
-    return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (more than 2^14 cells from the origin)");
-  if (z.ror_run && report[CM_MAX_ZONES + 2]) return fail(h, CM_E_INTERNAL, "device error %u", report[CM_MAX_ZONES + 2]);
-  return CM_OK;
+  return z.ror_run ? cell_margin_verdict(h, report[CM_MAX_ZONES + 2], "radius") : CM_OK;
 }
 
 // The host-buffer forms: the caller's cloud is uploaded on the legacy stream into the handle's staging buffer.
@@ -2083,12 +2098,12 @@ int cell_keys_sort(cm_handle_t h, VoxelParams& vp, float inv, cudaStream_t st) {
 }
 
 // A small key space (the usual case: a cropped cloud) gets a direct-address table of the cells' first sorted positions
-// instead of binary searches per point: rp.cell_start, else nullptr. no_table_env names the removal's test hook that forces
-// the binary searches (the large-key-space path).
-int enqueue_cell_table(cm_handle_t h, const VoxelParams& vp, const char* no_table_env, RorParams& rp, cudaStream_t st) {
+// instead of binary searches per point: table.cell_start, else nullptr. no_table_env names the filter's test hook that
+// forces the binary searches (the large-key-space path).
+int enqueue_cell_table(cm_handle_t h, const VoxelParams& vp, const char* no_table_env, CellTable& table, cudaStream_t st) {
   Workspace& w = h->batch;
   const uint32_t n_clouds = vp.n_frames;
-  rp.cell_start = nullptr; rp.table_keys = 0;
+  table.cell_start = nullptr; table.table_keys = 0;
   if (vp.max_points > 0 && w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&
       !getenv(no_table_env)) {
     const size_t keys = (size_t)n_clouds << w.plan_idx_bits;
@@ -2097,11 +2112,22 @@ int enqueue_cell_table(cm_handle_t h, const VoxelParams& vp, const char* no_tabl
       CM_CUDA(h, dev_alloc(h->cell_table, keys + 1));
       h->cell_table_cap = keys + 1;
     }
-    rp.cell_start = h->cell_table.get(); rp.table_keys = (uint32_t)keys;
-    CM_CUDA(h, launch_radius_table(vp, rp, st));
+    table.cell_start = h->cell_table.get(); table.table_keys = (uint32_t)keys;
+    CM_CUDA(h, launch_radius_table(vp, table, st));
     ++w.launches;
   }
   return CM_OK;
+}
+
+// The cells of a radius search (cm_cells.cuh): a little wider than the radius, so that two points closer than it are at
+// most one cell apart on every axis even after the float rounding of x * (1 / cell) (valid below 2^14 cells from the
+// origin, checked on the device), their sorted keys and the cell table.
+int radius_cell_keys(cm_handle_t h, VoxelParams& vp, float radius_f, const char* no_table_env, CellTable& table,
+                     cudaStream_t st) {
+  const float cell = radius_f * 1.00390625f;
+  const int rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  if (rc != CM_OK) return rc;
+  return enqueue_cell_table(h, vp, no_table_env, table, st);
 }
 }  // namespace
 
@@ -2117,10 +2143,8 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   VoxelParams vp;
   rc = cell_keys_begin(h, pts, begin, n_clouds, vp, st);
   if (rc != CM_OK) return rc;
-  // cells a little wider than the radius: two points closer than the radius are then at most one cell apart on every
-  // axis even after the float rounding of x * (1 / cell) (valid below 2^14 cells from the origin, checked on the device)
-  const float cell = (float)radius * 1.00390625f;
-  rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  CellTable table;
+  rc = radius_cell_keys(h, vp, (float)radius, "CM_ROR_NO_TABLE", table, st);
   if (rc != CM_OK) return rc;
   Workspace& w = h->batch;
   RorParams rp;
@@ -2128,8 +2152,7 @@ int radius_outlier_run(cm_handle_t h, const float4* pts, const int64_t* begin, i
   rp.min_pts = (uint32_t)min_neighbors;
   rp.negative = negative ? 1u : 0u;
   rp.mask = h->zw.mask.get();
-  rc = enqueue_cell_table(h, vp, "CM_ROR_NO_TABLE", rp, st);
-  if (rc != CM_OK) return rc;
+  rp.cell_start = table.cell_start;
   if (n_points) CM_CUDA(h, cudaMemsetAsync(h->zw.mask.get(), 0, (size_t)n_points * sizeof(unsigned short), st));
   CM_CUDA(h, launch_radius_count(vp, rp, st));
   ++w.launches;
@@ -2274,10 +2297,10 @@ int statistical_outlier_run(cm_handle_t h, const float4* pts, const int64_t* beg
   sp.sorted_pts = s.sorted_pts.get();
   sp.dist = s.dist.get();
   sp.cell = 1.0 / (double)inv;
-  RorParams rp{};
-  rc = enqueue_cell_table(h, vp, "CM_SOR_NO_TABLE", rp, st);
+  CellTable table;
+  rc = enqueue_cell_table(h, vp, "CM_SOR_NO_TABLE", table, st);
   if (rc != CM_OK) return rc;
-  sp.cell_start = rp.cell_start;
+  sp.cell_start = table.cell_start;
   if (n_points) CM_CUDA(h, cudaMemsetAsync(s.dist.get(), 0, (size_t)n_points * sizeof(float), st));
   s.profiled = h->profiling;
   if (s.profiled) CM_CUDA(h, cudaEventRecord(s.ev[0].get(), st));
@@ -2356,11 +2379,8 @@ int cm_get_statistical_out(cm_handle_t h, cm_sor_out_t* out) {
   out->distances = s.dist.get();
   out->n_points = s.n_points;
   out->n_clouds = s.n_clouds;
-  out->knn_ms = out->sums_ms = -1.f;
-  if (s.profiled) {
-    if (cudaEventElapsedTime(&out->knn_ms, s.ev[0].get(), s.ev[1].get()) != cudaSuccess) { out->knn_ms = -1.f; cudaGetLastError(); }
-    if (cudaEventElapsedTime(&out->sums_ms, s.ev[1].get(), s.ev[2].get()) != cudaSuccess) { out->sums_ms = -1.f; cudaGetLastError(); }
-  }
+  out->knn_ms = s.profiled ? elapsed_ms(s.ev[0].get(), s.ev[1].get()) : -1.f;
+  out->sums_ms = s.profiled ? elapsed_ms(s.ev[1].get(), s.ev[2].get()) : -1.f;
   for (int c = 0; c < s.n_clouds; ++c) {
     const SorStats& st = s.stats_host.get()[c];
     cm_sor_stats_t& o = out->cloud[c];
@@ -2435,18 +2455,14 @@ int euclidean_clusters_run(cm_handle_t h, const float4* pts, const int64_t* begi
   if (rc != CM_OK) return rc;
   rc = ec_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
-  // the radius outlier removal's cells: two points closer than the tolerance are at most one cell apart on every axis
-  const float cell = tf * 1.00390625f;
-  rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  CellTable table;
+  rc = radius_cell_keys(h, vp, tf, "CM_EC_NO_TABLE", table, st);
   if (rc != CM_OK) return rc;
   Workspace& w = h->batch;
-  RorParams rp{};
-  rc = enqueue_cell_table(h, vp, "CM_EC_NO_TABLE", rp, st);
-  if (rc != CM_OK) return rc;
   EcParams ep{};
   ep.pts = pts;
   ep.sorted_pts = e.pts.get();
-  ep.cell_start = rp.cell_start;
+  ep.cell_start = table.cell_start;
   // EuclideanClusterExtraction::extract narrows the tolerance to float; KdTreeFLANN::radiusSearch squares it in double
   ep.r2 = (float)((double)tf * (double)tf);
   ep.min_size = (uint32_t)cfg->min_size;
@@ -2472,9 +2488,8 @@ int euclidean_clusters_run(cm_handle_t h, const float4* pts, const int64_t* begi
   CM_CUDA(h, cudaStreamSynchronize(st));
   e.host_syncs = 1;
   e.device_error = rep[CM_MAX_ZONES + 2];
-  if (e.device_error == CM_DEV_E_KEY_RANGE)
-    return fail(h, CM_E_KEY_RANGE, "tolerance too small for the extent of a cloud (more than 2^14 cells from the origin)");
-  if (e.device_error) return fail(h, CM_E_INTERNAL, "device error %u", e.device_error);
+  rc = cell_margin_verdict(h, e.device_error, "tolerance");
+  if (rc != CM_OK) return rc;
   uint32_t first[CM_MAX_ZONES + 1];
   for (int c = 0; c <= n_clouds; ++c) first[c] = rep[c];
   const uint32_t K = first[n_clouds];
@@ -2532,11 +2547,7 @@ int cluster_out_locked(cm_handle_t h, cm_cluster_out_t* out) {
   out->n_clouds = e.n_clouds;
   out->host_syncs = (int32_t)e.host_syncs;
   for (int c = 0; c < CM_MAX_ZONES; ++c) out->cloud_clusters[c] = e.cloud_clusters[c];
-  out->hook_ms = -1.f;
-  if (e.profiled && cudaEventElapsedTime(&out->hook_ms, e.ev[0].get(), e.ev[1].get()) != cudaSuccess) {
-    out->hook_ms = -1.f;
-    cudaGetLastError();
-  }
+  out->hook_ms = e.profiled ? elapsed_ms(e.ev[0].get(), e.ev[1].get()) : -1.f;
   return CM_OK;
 }
 }  // namespace
@@ -2631,18 +2642,14 @@ int normals_run(cm_handle_t h, const float4* pts, const int64_t* begin, int n_cl
   if (rc != CM_OK) return rc;
   rc = ne_ws_ensure(h, (size_t)n_points);
   if (rc != CM_OK) return rc;
-  // the radius outlier removal's cells: two neighbours are at most one cell apart on every axis
-  const float cell = (float)cfg->radius * 1.00390625f;
-  rc = cell_keys_sort(h, vp, 1.0f / cell, st);
+  CellTable table;
+  rc = radius_cell_keys(h, vp, (float)cfg->radius, "CM_NE_NO_TABLE", table, st);
   if (rc != CM_OK) return rc;
   Workspace& w = h->batch;
-  RorParams rp{};
-  rc = enqueue_cell_table(h, vp, "CM_NE_NO_TABLE", rp, st);
-  if (rc != CM_OK) return rc;
   NeParams np{};
   np.pts = pts;
   np.sorted_pts = e.sorted_pts.get();
-  np.cell_start = rp.cell_start;
+  np.cell_start = table.cell_start;
   np.r2 = (float)(cfg->radius * cfg->radius);  // KdTreeFLANN::radiusSearch: the double square, narrowed
   for (int k = 0; k < 3; ++k) np.vp[k] = cfg->viewpoint[k];
   np.out = e.out.get();
@@ -2669,10 +2676,8 @@ int normal_out_locked(cm_handle_t h, cm_normal_out_t* out) {
   if (!e.ran) return fail(h, CM_E_INVALID, "no normal estimation has run on this handle");
   CM_CUDA(h, cudaSetDevice(h->device));
   CM_CUDA(h, cudaStreamSynchronize(e.stream));
-  const uint32_t dev_error = e.stats_host.get()->error;
-  if (dev_error == CM_DEV_E_KEY_RANGE)
-    return fail(h, CM_E_KEY_RANGE, "radius too small for the extent of a cloud (more than 2^14 cells from the origin)");
-  if (dev_error) return fail(h, CM_E_INTERNAL, "device error %u", dev_error);
+  const int rc = cell_margin_verdict(h, e.stats_host.get()->error, "radius");
+  if (rc != CM_OK) return rc;
   memset(out, 0, sizeof(*out));
   const NeStats& s = *e.stats_host.get();
   out->normals = reinterpret_cast<const float*>(e.out.get());
@@ -2682,11 +2687,8 @@ int normal_out_locked(cm_handle_t h, cm_normal_out_t* out) {
   out->n_warp = s.n_warp; out->n_cta = s.n_cta; out->n_multi = s.n_multi;
   out->n_clouds = e.n_clouds;
   out->host_syncs = 1;  // the key plan (cell_keys_sort)
-  out->warp_ms = out->cta_ms = -1.f;
-  if (e.profiled) {
-    if (cudaEventElapsedTime(&out->warp_ms, e.ev[0].get(), e.ev[1].get()) != cudaSuccess) { out->warp_ms = -1.f; cudaGetLastError(); }
-    if (cudaEventElapsedTime(&out->cta_ms, e.ev[1].get(), e.ev[2].get()) != cudaSuccess) { out->cta_ms = -1.f; cudaGetLastError(); }
-  }
+  out->warp_ms = e.profiled ? elapsed_ms(e.ev[0].get(), e.ev[1].get()) : -1.f;
+  out->cta_ms = e.profiled ? elapsed_ms(e.ev[1].get(), e.ev[2].get()) : -1.f;
   return CM_OK;
 }
 }  // namespace

@@ -8,8 +8,8 @@
 //  * the cloud goes through the radius outlier removal's front end with cell edge tf * (1 + 2^-8) (keys + onesweep sort +
 //    cell table): two neighbours are at most one cell apart on every axis;
 //  * k_ec_gather puts the points into sorted order and sets every point's parent to itself;
-//  * k_ec_hook walks the 3 x 3 rows of cells of k_ror_count from every sorted position i, tests the candidates behind i
-//    (one direction per pair) with the same float operations, and unions the two points' trees: a parallel union-find in
+//  * k_ec_hook walks the 3 x 3 rows of cells of cm_cells.cuh from every sorted position i, tests the candidates behind i
+//    (one direction per pair) with FLANN's float distance, and unions the two points' trees: a parallel union-find in
 //    input-index space in the style of ECL-CC, the larger root hooked under the smaller one with atomicCAS, path halving in
 //    find. A root only ever gets a smaller parent, so the final root of a component is its smallest index -- PCL's seed --
 //    whatever the thread timing;
@@ -19,7 +19,7 @@
 //  * k_ec_keys keys every point by its cluster's output rank (the points of no kept cluster by the largest key), and a
 //    stable LSD radix sort of (rank, input index) (k_ec_digits / k_ec_offsets / k_ec_scatter, 8 bits a pass) leaves every
 //    cluster's indices ascending; k_ec_gather_out copies the coordinates.
-#include "cm_kernels.h"
+#include "cm_cells.cuh"
 
 namespace cm {
 
@@ -35,15 +35,10 @@ constexpr uint32_t FULL = 0xFFFFFFFFu;
 template <typename KeyT>
 __global__ void __launch_bounds__(EC_THREADS) k_ec_gather(const VoxelParams p, float4* __restrict__ sorted_pts,
                                                           uint32_t* __restrict__ parent) {
-  constexpr bool REC = sizeof(KeyT) == 4;
   const uint32_t M = p.frame_surv_start[p.n_frames];
   const uint32_t i = blockIdx.x * EC_THREADS + threadIdx.x;
   if (i >= M) return;
-  const bool odd = (p.info->num_passes & 1u) != 0u;
-  uint32_t v;
-  if constexpr (REC) v = reinterpret_cast<const uint2*>(odd ? p.keys_b : p.keys_a)[i].y;
-  else v = (odd ? p.vals_b : p.vals_a)[i];
-  sorted_pts[i] = __ldg(p.pts + v);
+  sorted_pts[i] = __ldg(p.pts + sorted_of<KeyT>(p).val(i));
   parent[i] = i;
 }
 
@@ -78,73 +73,38 @@ __device__ __forceinline__ void ec_union(uint32_t* parent, uint32_t a, uint32_t 
 
 template <typename KeyT, bool TABLE>
 __global__ void __launch_bounds__(EC_THREADS) k_ec_hook(const VoxelParams p, const EcParams e) {
-  constexpr bool REC = sizeof(KeyT) == 4;
   const uint32_t M = p.frame_surv_start[p.n_frames];
   const uint32_t i = blockIdx.x * EC_THREADS + threadIdx.x;
   if (i >= M) return;
-  const SortInfo si = *p.info;
-  const bool odd = (si.num_passes & 1u) != 0u;
-  const void* __restrict__ sorted = odd ? p.keys_b : p.keys_a;
-  const uint32_t* __restrict__ vals = odd ? p.vals_b : p.vals_a;
-  auto key_at = [&](uint32_t j) -> unsigned long long {
-    if constexpr (REC) return reinterpret_cast<const uint2*>(sorted)[j].x;
-    else return reinterpret_cast<const unsigned long long*>(sorted)[j];
-  };
-  auto val_at = [&](uint32_t j) -> uint32_t {
-    if constexpr (REC) return reinterpret_cast<const uint2*>(sorted)[j].y;
-    else return vals[j];
-  };
-  const uint32_t idx_bits = si.idx_bits;
-  const unsigned long long full_key = key_at(i);
-  // clouds are frames of the key; keys of frame >= n_frames are the non-finite points, which belong to no cluster
-  const unsigned long long frame = idx_bits >= 64 ? 0ull : (full_key >> idx_bits);
-  if (frame >= p.n_frames) return;
-  const unsigned long long fbits = idx_bits >= 64 ? 0ull : (frame << idx_bits);
-  const unsigned long long key = full_key - fbits;
-  const GridDev g = p.grid[frame];
-  // the cell margin only covers |coordinate / cell| < 2^14 (as in k_ror_count)
-  if (i == 0) {
-    int worst = 0;
-    for (uint32_t f = 0; f < p.n_frames; ++f) {
-      if (p.frame_surv_start[f + 1] == p.frame_surv_start[f]) continue;
-      const GridDev gf = p.grid[f];
-      for (int a = 0; a < 3; ++a) worst = max(worst, max(abs(gf.min_b[a]), abs(gf.max_b[a])));
-    }
-    if (worst >= (1 << 14)) atomicExch(&p.ctrl->error, (uint32_t)CM_DEV_E_KEY_RANGE);
-  }
+  const Sorted<KeyT> s = sorted_of<KeyT>(p);
+  // query_cell written out, so that the margin check sits between the frame and the cell decode: next to a query_cell
+  // call ptxas gives 40 registers to the three instantiations that get 32 here (DESIGN section 4)
+  const uint32_t idx_bits = p.info->idx_bits;
+  const unsigned long long full_key = s.key(i);
+  QueryCell qc;
+  qc.frame = idx_bits >= 64 ? 0ull : (full_key >> idx_bits);
+  if (qc.frame >= p.n_frames) return;  // a non-finite point belongs to no cluster
+  qc.fbits = idx_bits >= 64 ? 0ull : (qc.frame << idx_bits);
+  const unsigned long long key = full_key - qc.fbits;
+  const GridDev g = p.grid[qc.frame];
+  if (i == 0) check_cell_margin(p);
   if (g.zero_keys) return;  // the host refuses such a call before this kernel is enqueued
-  const unsigned long long d0 = (unsigned long long)g.div_b[0], d1 = (unsigned long long)g.div_b[1],
-                           d2 = (unsigned long long)g.div_b[2];
-  const unsigned long long c0 = key % d0, t = key / d0, c1 = t % d1, c2 = t / d1;
+  qc.d0 = (unsigned long long)g.div_b[0]; qc.d1 = (unsigned long long)g.div_b[1]; qc.d2 = (unsigned long long)g.div_b[2];
+  qc.c0 = key % qc.d0;
+  const unsigned long long t = key / qc.d0;
+  qc.c1 = t % qc.d1; qc.c2 = t / qc.d1;
   const float4 q = e.sorted_pts[i];
   uint32_t me = NONE;
-  const unsigned long long x_lo = c0 > 0 ? c0 - 1 : 0, x_hi = c0 + 1 < d0 ? c0 + 1 : d0 - 1;
   for (int rr = 0; rr < 9; ++rr) {
-    const int dz = (int)((0x28215u >> (2 * rr)) & 3u) - 1, dy = (int)((0x22161u >> (2 * rr)) & 3u) - 1;
-    if ((dz < 0 && c2 == 0) || (dz > 0 && c2 + 1 >= d2)) continue;
-    if ((dy < 0 && c1 == 0) || (dy > 0 && c1 + 1 >= d1)) continue;
-    const unsigned long long row = ((c2 + dz) * d1 + (c1 + dy)) * d0;
-    const unsigned long long k_lo = fbits + row + x_lo, k_hi = fbits + row + x_hi;
-    uint32_t lo = 0, hi = M;
-    if constexpr (TABLE) {
-      lo = __ldg(e.cell_start + k_lo);
-      hi = __ldg(e.cell_start + k_hi + 1);
-    } else {
-      while (lo < hi) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (key_at(mid) < k_lo) lo = mid + 1; else hi = mid;
-      }
-      hi = M;
-    }
+    uint32_t lo, hi;
+    unsigned long long k_hi;
+    if (!row_segment<KeyT, TABLE>(s, e.cell_start, M, qc, rr, lo, hi, k_hi)) continue;
     // only the candidates behind i: every pair is tested once, from its earlier sorted position
     for (uint32_t j = max(lo, i + 1); j < hi; ++j) {
-      if (!TABLE && key_at(j) > k_hi) break;
-      const float4 d = e.sorted_pts[j];
-      const float ex = __fsub_rn(q.x, d.x), ey = __fsub_rn(q.y, d.y), ez = __fsub_rn(q.z, d.z);
-      const float acc = __fadd_rn(__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)), __fmul_rn(ez, ez));
-      if (acc < e.r2) {
-        if (me == NONE) me = val_at(i);
-        ec_union(e.parent, me, val_at(j));
+      if (!TABLE && s.key(j) > k_hi) break;
+      if (flann_d2(q, e.sorted_pts[j]) < e.r2) {
+        if (me == NONE) me = s.val(i);
+        ec_union(e.parent, me, s.val(j));
       }
     }
   }
@@ -298,15 +258,12 @@ uint32_t ec_sort_tiles(uint32_t n) { return (n + RS_TILE - 1) / RS_TILE; }
 cudaError_t launch_ec_hook(const VoxelParams& p, const EcParams& e, float4* sorted_pts, cudaStream_t stream) {
   if (p.max_points == 0) return cudaSuccess;
   const uint32_t blocks = blocks_of(p.max_points);
-  if (p.key_bytes == 4) k_ec_gather<uint32_t><<<blocks, EC_THREADS, 0, stream>>>(p, sorted_pts, e.parent);
-  else k_ec_gather<unsigned long long><<<blocks, EC_THREADS, 0, stream>>>(p, sorted_pts, e.parent);
-  if (e.cell_start) {
-    if (p.key_bytes == 4) k_ec_hook<uint32_t, true><<<blocks, EC_THREADS, 0, stream>>>(p, e);
-    else k_ec_hook<unsigned long long, true><<<blocks, EC_THREADS, 0, stream>>>(p, e);
-  } else {
-    if (p.key_bytes == 4) k_ec_hook<uint32_t, false><<<blocks, EC_THREADS, 0, stream>>>(p, e);
-    else k_ec_hook<unsigned long long, false><<<blocks, EC_THREADS, 0, stream>>>(p, e);
-  }
+  with_key_type(p, [&](auto key) {
+    k_ec_gather<decltype(key)><<<blocks, EC_THREADS, 0, stream>>>(p, sorted_pts, e.parent);
+  });
+  with_cells(p, e.cell_start, [&](auto key, auto table) {
+    k_ec_hook<decltype(key), decltype(table)::value><<<blocks, EC_THREADS, 0, stream>>>(p, e);
+  });
   return cudaGetLastError();
 }
 

@@ -177,12 +177,16 @@ struct RorParams {
   float r2;              // (float)(radius * radius): FLANN counts squared distances strictly below it
   uint32_t min_pts;      // keep iff count (the point itself included) > min_pts
   uint32_t negative;
-  unsigned short* mask;  // [n_points] keep flag per input point (cleared by the caller)
+  unsigned short* mask;        // [n_points] keep flag per input point (cleared by the caller)
+  const uint32_t* cell_start;  // k_ror_table's table of the cells' first sorted positions, or nullptr: binary searches
+};
+// the direct-address table of the cells' first sorted positions, shared by the searches on the sorted cell keys
+struct CellTable {
   uint32_t* cell_start;  // [table_keys + 1] first sorted position with key >= k, or nullptr: binary searches instead
   uint32_t table_keys;   // n_frames << idx_bits: every valid key is below it
 };
 // fills cell_start from the sorted keys (one launch), then counts (one launch)
-cudaError_t launch_radius_table(const VoxelParams& p, const RorParams& r, cudaStream_t stream);
+cudaError_t launch_radius_table(const VoxelParams& p, const CellTable& t, cudaStream_t stream);
 cudaError_t launch_radius_count(const VoxelParams& p, const RorParams& r, cudaStream_t stream);
 
 // ---- statistical outlier removal on the sorted cell keys (cm_statistical.cu) -------------------------------------------------

@@ -7,7 +7,7 @@
 // shared with the C++ statement of the tests. Here:
 //  * the cloud goes through the radius outlier removal's front end with cell edge radius * (1 + 2^-8) (keys + onesweep
 //    sort + cell table) and the statistical removal's sorted-order gather;
-//  * k_ne_warp: one warp per query, in sorted order. It walks the nine row segments of k_ror_count 32 candidates at a time
+//  * k_ne_warp: one warp per query, in sorted order. It walks the nine row segments of cm_cells.cuh 32 candidates at a time
 //    and ballot-compacts the hits as keys (bits(d2) << 32) | input index -- for non-negative floats the integer order of
 //    that key is exactly FLANN's (distance, index) order -- into a list of CM_NE_WARP_CAP keys in shared memory, sorts the
 //    list (bitonic), runs the nine running sums (lanes 0..8, each a serial chain in list order: reassociating them would
@@ -21,7 +21,7 @@
 // Both kernels are launched every call (the CTA grid exits at once on an empty queue): the launch plan does not depend on
 // the data and nothing waits for the host.
 #include "../../include/cloud_merger_gpu.h"  // CM_NE_WARP_CAP, CM_NE_CTA_CAP
-#include "cm_kernels.h"
+#include "cm_cells.cuh"
 #include "cm_ne_math.h"
 
 namespace cm {
@@ -39,78 +39,9 @@ constexpr uint32_t FULL = 0xFFFFFFFFu;
 constexpr unsigned long long NO_KEY = ~0ull;
 static_assert(NE_CTA_CAP == CM_NE_CTA_CAP, "CM_NE_CTA_CAP");
 
-template <typename KeyT>
-struct Sorted {
-  const void* keys;
-  const uint32_t* vals;
-  __device__ __forceinline__ unsigned long long key(uint32_t j) const {
-    if constexpr (sizeof(KeyT) == 4) return reinterpret_cast<const uint2*>(keys)[j].x;
-    else return reinterpret_cast<const unsigned long long*>(keys)[j];
-  }
-  __device__ __forceinline__ uint32_t val(uint32_t j) const {
-    if constexpr (sizeof(KeyT) == 4) return reinterpret_cast<const uint2*>(keys)[j].y;
-    else return vals[j];
-  }
-};
-
-template <typename KeyT>
-__device__ __forceinline__ Sorted<KeyT> sorted_of(const VoxelParams& p) {
-  const bool odd = (p.info->num_passes & 1u) != 0u;
-  return Sorted<KeyT>{odd ? p.keys_b : p.keys_a, odd ? p.vals_b : p.vals_a};
-}
-
-// the cell of sorted position i and its frame; false for a non-finite point (keys of frame >= n_frames)
-struct QueryCell {
-  unsigned long long fbits, c0, c1, c2, d0, d1, d2;
-};
-template <typename KeyT>
-__device__ __forceinline__ bool query_cell(const VoxelParams& p, const Sorted<KeyT>& s, uint32_t i, QueryCell& qc, bool& skip) {
-  const uint32_t idx_bits = p.info->idx_bits;
-  const unsigned long long full_key = s.key(i);
-  const unsigned long long frame = idx_bits >= 64 ? 0ull : (full_key >> idx_bits);
-  skip = false;
-  if (frame >= p.n_frames) return false;
-  qc.fbits = idx_bits >= 64 ? 0ull : (frame << idx_bits);
-  const unsigned long long key = full_key - qc.fbits;
-  const GridDev g = p.grid[frame];
-  if (g.zero_keys) { skip = true; return true; }  // the host refuses such a call before the search is enqueued
-  qc.d0 = (unsigned long long)g.div_b[0]; qc.d1 = (unsigned long long)g.div_b[1]; qc.d2 = (unsigned long long)g.div_b[2];
-  qc.c0 = key % qc.d0;
-  const unsigned long long t = key / qc.d0;
-  qc.c1 = t % qc.d1; qc.c2 = t / qc.d1;
-  return true;
-}
-
-// row segment rr (of k_ror_count's nine) of a query: [lo, hi) of sorted positions (hi = M without the table: the walk
-// then stops at the first key above k_hi); false when a clamp skips the row
-template <typename KeyT, bool TABLE>
-__device__ __forceinline__ bool row_segment(const Sorted<KeyT>& s, const uint32_t* cell_start, uint32_t M, const QueryCell& qc,
-                                            int rr, uint32_t& lo, uint32_t& hi, unsigned long long& k_hi) {
-  const int dz = (int)((0x28215u >> (2 * rr)) & 3u) - 1, dy = (int)((0x22161u >> (2 * rr)) & 3u) - 1;
-  if ((dz < 0 && qc.c2 == 0) || (dz > 0 && qc.c2 + 1 >= qc.d2)) return false;
-  if ((dy < 0 && qc.c1 == 0) || (dy > 0 && qc.c1 + 1 >= qc.d1)) return false;
-  const unsigned long long x_lo = qc.c0 > 0 ? qc.c0 - 1 : 0, x_hi = qc.c0 + 1 < qc.d0 ? qc.c0 + 1 : qc.d0 - 1;
-  const unsigned long long row = ((qc.c2 + dz) * qc.d1 + (qc.c1 + dy)) * qc.d0;
-  const unsigned long long k_lo = qc.fbits + row + x_lo;
-  k_hi = qc.fbits + row + x_hi;
-  if constexpr (TABLE) {
-    lo = __ldg(cell_start + k_lo);
-    hi = __ldg(cell_start + k_hi + 1);
-  } else {
-    lo = 0; hi = M;
-    while (lo < hi) {
-      const uint32_t mid = (lo + hi) >> 1;
-      if (s.key(mid) < k_lo) lo = mid + 1; else hi = mid;
-    }
-    hi = M;
-  }
-  return true;
-}
-
 // FLANN's float squared distance of candidate j to the query, as a list key; NO_KEY when it is not below r2
 __device__ __forceinline__ unsigned long long hit_key(const float4& q, const float4& d, float r2, uint32_t idx) {
-  const float ex = __fsub_rn(q.x, d.x), ey = __fsub_rn(q.y, d.y), ez = __fsub_rn(q.z, d.z);
-  const float acc = __fadd_rn(__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)), __fmul_rn(ez, ez));
+  const float acc = flann_d2(q, d);
   return acc < r2 ? ((unsigned long long)__float_as_uint(acc) << 32) | idx : NO_KEY;
 }
 
@@ -186,15 +117,7 @@ __global__ void __launch_bounds__(NE_WARPS * 32) k_ne_warp(const VoxelParams p, 
   if (i < M) do {
     const Sorted<KeyT> s = sorted_of<KeyT>(p);
     const uint32_t me = s.val(i);
-    if (i == 0 && lane == 0) {  // the cell margin only covers |coordinate / cell| < 2^14 (as in k_ror_count)
-      int worst = 0;
-      for (uint32_t f = 0; f < p.n_frames; ++f) {
-        if (p.frame_surv_start[f + 1] == p.frame_surv_start[f]) continue;
-        const GridDev gf = p.grid[f];
-        for (int a = 0; a < 3; ++a) worst = max(worst, max(abs(gf.min_b[a]), abs(gf.max_b[a])));
-      }
-      if (worst >= (1 << 14)) atomicExch(&p.ctrl->error, (uint32_t)CM_DEV_E_KEY_RANGE);
-    }
+    if (i == 0 && lane == 0) check_cell_margin(p);
     QueryCell qc;
     bool skip;
     if (!query_cell<KeyT>(p, s, i, qc, skip)) {  // a non-finite query
@@ -339,20 +262,13 @@ int launch_normals(const VoxelParams& p, const NeParams& e, float4* sorted_pts, 
   const uint32_t wb = (p.max_points + NE_WARPS - 1) / NE_WARPS;
   const uint32_t cb = std::min<uint32_t>(p.max_points, NE_CTA_GRID);
   const size_t smem = NE_CTA_BUF * sizeof(unsigned long long);
-  const bool k4 = p.key_bytes == 4;
-  if (e.cell_start) {
-    if (k4) k_ne_warp<uint32_t, true><<<wb, NE_WARPS * 32, 0, stream>>>(p, e);
-    else k_ne_warp<unsigned long long, true><<<wb, NE_WARPS * 32, 0, stream>>>(p, e);
+  with_cells(p, e.cell_start, [&](auto key, auto table) {
+    using KeyT = decltype(key);
+    constexpr bool TABLE = decltype(table)::value;
+    k_ne_warp<KeyT, TABLE><<<wb, NE_WARPS * 32, 0, stream>>>(p, e);
     if (mid) cudaEventRecord(mid, stream);
-    if (k4) k_ne_cta<uint32_t, true><<<cb, NE_CTA_THREADS, smem, stream>>>(p, e);
-    else k_ne_cta<unsigned long long, true><<<cb, NE_CTA_THREADS, smem, stream>>>(p, e);
-  } else {
-    if (k4) k_ne_warp<uint32_t, false><<<wb, NE_WARPS * 32, 0, stream>>>(p, e);
-    else k_ne_warp<unsigned long long, false><<<wb, NE_WARPS * 32, 0, stream>>>(p, e);
-    if (mid) cudaEventRecord(mid, stream);
-    if (k4) k_ne_cta<uint32_t, false><<<cb, NE_CTA_THREADS, smem, stream>>>(p, e);
-    else k_ne_cta<unsigned long long, false><<<cb, NE_CTA_THREADS, smem, stream>>>(p, e);
-  }
+    k_ne_cta<KeyT, TABLE><<<cb, NE_CTA_THREADS, smem, stream>>>(p, e);
+  });
   *err = cudaGetLastError();
   return 3;
 }

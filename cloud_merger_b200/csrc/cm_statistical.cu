@@ -23,7 +23,7 @@
 // scan + scatter kernels compact the survivors in input order (cm_zones.cu).
 #include <climits>
 
-#include "cm_kernels.h"
+#include "cm_cells.cuh"
 
 namespace cm {
 
@@ -37,15 +37,10 @@ constexpr uint32_t FULL = 0xFFFFFFFFu;
 
 template <typename KeyT>
 __global__ void __launch_bounds__(256) k_sor_gather(const VoxelParams p, float4* __restrict__ sorted_pts) {
-  constexpr bool REC = sizeof(KeyT) == 4;
   const uint32_t M = p.frame_surv_start[p.n_frames];
   const uint32_t i = blockIdx.x * 256 + threadIdx.x;
   if (i >= M) return;
-  const bool odd = (p.info->num_passes & 1u) != 0u;
-  uint32_t v;
-  if constexpr (REC) v = reinterpret_cast<const uint2*>(odd ? p.keys_b : p.keys_a)[i].y;
-  else v = (odd ? p.vals_b : p.vals_a)[i];
-  sorted_pts[i] = __ldg(p.pts + v);
+  sorted_pts[i] = __ldg(p.pts + sorted_of<KeyT>(p).val(i));
 }
 
 // largest kept value and its slot (j * 32 + lane), the same in every lane; ties go to the lowest slot
@@ -68,37 +63,23 @@ __device__ __forceinline__ float warp_argmax(const float (&v)[NS], uint32_t lane
 
 template <typename KeyT, bool TABLE, int NS>
 __global__ void __launch_bounds__(SOR_THREADS, 2) k_sor_knn(const VoxelParams p, const SorParams s) {
-  constexpr bool REC = sizeof(KeyT) == 4;
   __shared__ float s_val[SOR_WARPS][32 * NS];
   __shared__ double s_root[SOR_WARPS][32 * NS];
   const uint32_t wib = threadIdx.x >> 5, lane = threadIdx.x & 31u;
   const uint32_t M = p.frame_surv_start[p.n_frames];
   const uint32_t i = blockIdx.x * SOR_WARPS + wib;  // one warp per sorted position
   if (i >= M) return;
-  const SortInfo si = *p.info;
-  const bool odd = (si.num_passes & 1u) != 0u;
-  const void* __restrict__ sorted = odd ? p.keys_b : p.keys_a;
-  const uint32_t* __restrict__ vals = odd ? p.vals_b : p.vals_a;
-  auto key_at = [&](uint32_t j) -> unsigned long long {
-    if constexpr (REC) return reinterpret_cast<const uint2*>(sorted)[j].x;
-    else return reinterpret_cast<const unsigned long long*>(sorted)[j];
-  };
-  auto lower_bound = [&](unsigned long long k) -> uint32_t {
-    uint32_t lo = 0, hi = M;
-    while (lo < hi) {
-      const uint32_t mid = (lo + hi) >> 1;
-      if (key_at(mid) < k) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-  };
-  const uint32_t idx_bits = si.idx_bits;
-  const unsigned long long full_key = key_at(i);
+  const Sorted<KeyT> st = sorted_of<KeyT>(p);
+  const uint32_t idx_bits = p.info->idx_bits;
+  const unsigned long long full_key = st.key(i);
   // clouds are frames of the key; keys of frame >= n_frames are the non-finite points (distance 0: the caller cleared it)
   const unsigned long long frame = idx_bits >= 64 ? 0ull : (full_key >> idx_bits);
   if (frame >= p.n_frames || ((s.too_few >> frame) & 1u)) return;
   const unsigned long long fbits = idx_bits >= 64 ? 0ull : (frame << idx_bits);
   const GridDev g = p.grid[frame];
   if (g.zero_keys) return;  // the host refuses such a call before this kernel is enqueued
+  // query_cell's decode, in signed arithmetic for the cube bounds (on query_cell one instantiation takes two more
+  // registers, DESIGN section 4)
   const long long d0 = g.div_b[0], d1 = g.div_b[1], d2 = g.div_b[2];
   const unsigned long long key = full_key - fbits;
   const long long c0 = (long long)(key % (unsigned long long)d0), t = (long long)(key / (unsigned long long)d0);
@@ -142,8 +123,8 @@ __global__ void __launch_bounds__(SOR_THREADS, 2) k_sor_knn(const VoxelParams p,
             lo = __ldg(s.cell_start + rowk + a);
             hi = __ldg(s.cell_start + rowk + b + 1);
           } else {
-            lo = lower_bound(rowk + a);
-            hi = lower_bound(rowk + b + 1);
+            lo = lower_bound(st, M, rowk + a);
+            hi = lower_bound(st, M, rowk + b + 1);
           }
           cnt = hi - lo;
         }
@@ -161,9 +142,7 @@ __global__ void __launch_bounds__(SOR_THREADS, 2) k_sor_knn(const VoxelParams p,
         const bool valid = j < total;
         float d = 0.f;
         if (valid) {
-          const float4 c = s.sorted_pts[seg_lo + (j - seg_ex)];
-          const float ex = __fsub_rn(q.x, c.x), ey = __fsub_rn(q.y, c.y), ez = __fsub_rn(q.z, c.z);
-          d = __fadd_rn(__fadd_rn(__fmul_rn(ex, ex), __fmul_rn(ey, ey)), __fmul_rn(ez, ez));
+          d = flann_d2(q, s.sorted_pts[seg_lo + (j - seg_ex)]);
         }
         const bool filling = filled < kp1;
         const bool take = valid && (filling || d < thr);
@@ -232,10 +211,7 @@ __global__ void __launch_bounds__(SOR_THREADS, 2) k_sor_knn(const VoxelParams p,
   if (lane == 0) {
     double sum = 0.0;
     for (uint32_t k = 1; k < kp1; ++k) sum = __dadd_rn(sum, root[k]);  // k = 0 is the point itself
-    uint32_t me;
-    if constexpr (REC) me = reinterpret_cast<const uint2*>(sorted)[i].y;
-    else me = vals[i];
-    s.dist[me] = __double2float_rn(__ddiv_rn(sum, (double)s.mean_k));
+    s.dist[st.val(i)] = __double2float_rn(__ddiv_rn(sum, (double)s.mean_k));
   }
 }
 
@@ -350,8 +326,7 @@ __global__ void __launch_bounds__(256) k_sor_select(const SorSumParams s, uint32
 cudaError_t launch_sorted_gather(const VoxelParams& p, float4* sorted_pts, cudaStream_t stream) {
   if (p.max_points == 0) return cudaSuccess;
   const uint32_t gb = (p.max_points + 255) / 256;
-  if (p.key_bytes == 4) k_sor_gather<uint32_t><<<gb, 256, 0, stream>>>(p, sorted_pts);
-  else k_sor_gather<unsigned long long><<<gb, 256, 0, stream>>>(p, sorted_pts);
+  with_key_type(p, [&](auto key) { k_sor_gather<decltype(key)><<<gb, 256, 0, stream>>>(p, sorted_pts); });
   return cudaGetLastError();
 }
 
@@ -361,16 +336,13 @@ cudaError_t launch_sor_knn(const VoxelParams& p, const SorParams& s, float4* sor
   if (ge != cudaSuccess) return ge;
   const uint32_t blocks = (p.max_points + SOR_WARPS - 1) / SOR_WARPS;
   const int ns = s.mean_k + 1 <= 32 ? 1 : s.mean_k + 1 <= 64 ? 2 : 4;
-#define CM_SOR_LAUNCH(KT, TB, NS) k_sor_knn<KT, TB, NS><<<blocks, SOR_THREADS, 0, stream>>>(p, s)
-#define CM_SOR_NS(KT, TB) \
-  do { if (ns == 1) CM_SOR_LAUNCH(KT, TB, 1); else if (ns == 2) CM_SOR_LAUNCH(KT, TB, 2); else CM_SOR_LAUNCH(KT, TB, 4); } while (0)
-  if (p.key_bytes == 4) {
-    if (s.cell_start) CM_SOR_NS(uint32_t, true); else CM_SOR_NS(uint32_t, false);
-  } else {
-    if (s.cell_start) CM_SOR_NS(unsigned long long, true); else CM_SOR_NS(unsigned long long, false);
-  }
-#undef CM_SOR_NS
-#undef CM_SOR_LAUNCH
+  with_cells(p, s.cell_start, [&](auto key, auto table) {
+    using KeyT = decltype(key);
+    constexpr bool TABLE = decltype(table)::value;
+    if (ns == 1) k_sor_knn<KeyT, TABLE, 1><<<blocks, SOR_THREADS, 0, stream>>>(p, s);
+    else if (ns == 2) k_sor_knn<KeyT, TABLE, 2><<<blocks, SOR_THREADS, 0, stream>>>(p, s);
+    else k_sor_knn<KeyT, TABLE, 4><<<blocks, SOR_THREADS, 0, stream>>>(p, s);
+  });
   return cudaGetLastError();
 }
 

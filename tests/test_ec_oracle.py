@@ -91,11 +91,11 @@ def test_equal_size_clusters_through_both_statements():
     assert len(a) == 1504 and _same(a, ec_np.clusters_of(c, 0.5))
 
 
-def test_host_order_is_libstdcxx_sort_through_reverse_iterators():
+def test_host_order_is_libstdcxx_sort_on_the_shared_cell_front_end():
     src = host_function("euclidean_clusters_run")
-    assert 'enqueue_cell_table(h, vp, "CM_EC_NO_TABLE", rp, st)' in src
+    assert 'radius_cell_keys(h, vp, tf, "CM_EC_NO_TABLE", table, st)' in src
     assert "ep.r2 = (float)((double)tf * (double)tf);" in src
-    assert "const float cell = tf * 1.00390625f;" in src
+    assert "const float cell = radius_f * 1.00390625f;" in host_function("radius_cell_keys")
     with open(os.path.join(os.path.dirname(HERE), "cloud_merger_b200", "csrc", "cm_api.cu")) as f:
         api = f.read()
     a = api.index("void ec_order(")

@@ -362,27 +362,30 @@ def _src(name):
         return f.read()
 
 
-def test_ror_constants_match_the_source():
+def test_ror_constants_match_the_cell_search():
     """The N-family restatement mirrors the kernels' constants; a retune must fail here rather than miss the edges."""
-    ror, vox = _src("cm_outlier.cu"), _src("cm_voxel.cu")
-    run, front, keys, table = (host_function(f) for f in ("radius_outlier_run", "cell_keys_begin", "cell_keys_sort",
-                                                          "enqueue_cell_table"))
-    assert "(float)radius * 1.00390625f" in run and E.ROR_MARGIN == 1.00390625
-    assert "worst >= (1 << 14)" in ror and E.ROR_BOUND == 1 << 14
+    ror, cells, vox = _src("cm_outlier.cu"), _src("cm_cells.cuh"), _src("cm_voxel.cu")
+    run, front, keys, table, cell_keys = (host_function(f) for f in ("radius_outlier_run", "cell_keys_begin", "cell_keys_sort",
+                                                                     "enqueue_cell_table", "radius_cell_keys"))
+    assert 'radius_cell_keys(h, vp, (float)radius, "CM_ROR_NO_TABLE", table, st)' in run
+    assert "const float cell = radius_f * 1.00390625f;" in cell_keys and E.ROR_MARGIN == 1.00390625
+    assert "rc = cell_keys_sort(h, vp, 1.0f / cell, st);" in cell_keys
+    assert "return enqueue_cell_table(h, vp, no_table_env, table, st);" in cell_keys
+    assert "worst >= (1 << 14)" in cells and "if (i == 0) check_cell_margin(p);" in ror and E.ROR_BOUND == 1 << 14
     assert "w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25)" in table and E.ROR_TABLE_LOG2 == 25
-    assert 'enqueue_cell_table(h, vp, "CM_ROR_NO_TABLE", rp, st)' in run
     # the launches cm_launch_count reports for the call (ror_launches): a bounding box per cloud and the table in the shared
     # front end, the count in the run
     assert front.count("++w.launches;") == 1 and table.count("++w.launches;") == 1 and run.count("++w.launches;") == 1
-    assert "w.launches" not in keys and "rc = run_voxel(h, w, vp, st, false, false);" in keys
-    assert "rc = cell_keys_sort(h, vp, 1.0f / cell, st);" in run
+    assert "w.launches" not in keys and "w.launches" not in cell_keys and "rc = run_voxel(h, w, vp, st, false, false);" in keys
     assert "constexpr int ROR_THREADS = 256;" in ror and E.ROR_THREADS == 256
     assert "constexpr unsigned long long LONG_GAP = 2048;" in ror and "to - from >= LONG_GAP" in ror and E.ROR_LONG_GAP == 2048
     assert "constexpr int LIST = 32;" in ror and E.ROR_LIST == 32
-    assert "0x28215u" in ror and "0x22161u" in ror and (E.ROR_ROW_DZ, E.ROR_ROW_DY) == (0x28215, 0x22161)
+    assert "0x28215u" in cells and "0x22161u" in cells and (E.ROR_ROW_DZ, E.ROR_ROW_DY) == (0x28215, 0x22161)
+    assert "row_segment<KeyT, TABLE>(s, r.cell_start, M, qc, rr, lo, hi, k_hi)" in ror
     assert E.ror_rows() == [(0, 0), (0, -1), (0, 1), (-1, 0), (1, 0), (-1, -1), (-1, 1), (1, -1), (1, 1)]
     assert "dv > (1ll << 21)" in vox and "1073741824.f" in vox
-    assert "if (g.zero_keys) return;" in ror and "w.plan_error == CM_DEV_E_KEY_RANGE" in keys
+    assert "if (g.zero_keys) { skip = true; return true; }" in cells and "w.plan_error == CM_DEV_E_KEY_RANGE" in keys
+    assert "if (!query_cell<KeyT>(p, s, i, qc, skip) || skip) return;" in ror
 
 
 def _two_apart(x, pairs, cell):

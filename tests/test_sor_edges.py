@@ -34,7 +34,7 @@ def _valid(c, mean_k):
     return int(np.isfinite(np.asarray(c, F32)[:, :3]).all(axis=1).sum()) > mean_k
 
 
-def test_sor_constants_match_the_shared_front_end():
+def test_sor_constants_match_the_cell_search():
     """The S-family restatement mirrors the kernels' constants; a retune must fail here rather than miss the edges."""
     sor, api, vox = _src("cm_statistical.cu"), _src("cm_api.cu"), _src("cm_voxel.cu")
     body, front, keys, table = (host_function(f) for f in ("statistical_outlier_run", "cell_keys_begin", "cell_keys_sort",
@@ -55,7 +55,7 @@ def test_sor_constants_match_the_shared_front_end():
     assert "const float inv = (float)(1.0 / sor_cell_edge(" in body and "rc = cell_keys_sort(h, vp, inv, st);" in body
     assert ("w.plan_idx_bits <= 25 && ((uint64_t)n_clouds << w.plan_idx_bits) <= (1ull << 25) &&\n      "
             "!getenv(no_table_env)") in table and S.TABLE_LOG2 == 25
-    assert 'enqueue_cell_table(h, vp, "CM_SOR_NO_TABLE", rp, st)' in body
+    assert 'enqueue_cell_table(h, vp, "CM_SOR_NO_TABLE", table, st)' in body and "sp.cell_start = table.cell_start;" in body
     assert "dv > (1ll << 21)" in vox and "1073741824.f" in vox
     # the launches cm_launch_count reports for the call (sor_plan's "launches"): a bounding box per cloud and the table in
     # the shared front end, the search, sums and select in the run
